@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- alignments/sec through filter + bam2gtf + update-gtf (BASELINE.json's metric) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--reads R] [--genes G] [--shape iso|ont]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--reads R] [--genes G] [--shape iso|ont] [--dump-outputs DIR]
 
 Workload (the same ONE data set for every N: strong scaling): BASELINE.json configs[3] -- R synthetic spliced alignments
 (default 50 M primaries, Iso-Seq-like as configs[1], + secondaries / rRNA / low-identity / low-coverage rejects) against a
@@ -22,6 +22,9 @@ the gathered table, counters summed) -- the gather and the merge are INSIDE the 
   cpu_baseline, files_e2e (N = 1): the UNMODIFIED reference binary (oracle/_ref/lr2rmats), one thread, on a bounded sample of the
             same stream, and the drop-in CLI on the same files (wall clock files in -> files out, outputs compared byte for byte).
   other_configs (N = 1): configs[1] (1 M Iso-Seq-like) and configs[2] (10 M ONT-like, indel-dense CIGARs) device-resident.
+
+--dump-outputs DIR: after the device-resident steps, what the last one computed is written as DIR/<name>.npy (see dump_outputs), so
+that two builds run with the same arguments (hence the same seeded data set) can be compared output for output.
 
 --impl reference: the reference's own CPU implementation (its CLI, unmodified binary) on the host cores: one process per
 locus-aligned shard of a bounded sample of the same stream, all cores.
@@ -261,6 +264,25 @@ def pinned_copy(arr):
     return t, t.numpy()
 
 
+DUMP_CAP = 1 << 18          # elements per dumped array: the 21 arrays stay below 64 MiB of float64
+
+
+def dump_outputs(out_dir, res, keep_idx):
+    """The arrays a caller of the timed step receives -- the updated_T table (table_*), the BED rows (bed_*), the summary counters and
+    filter's kept-record list -- as float64 .npy files (every value is an integer below 2^53, so it is stored exactly).  An array longer
+    than DUMP_CAP is replaced by its elements at DUMP_CAP sorted positions drawn with its length as the seed: two runs whose arrays have
+    the same length dump the same positions."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"summary": res["summary"], "keep_idx": keep_idx}
+    arrays.update({f"table_{k}": v for k, v in res["table"].items()})
+    arrays.update({f"bed_{k}": v for k, v in res["bed"].items()})
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if len(a) > DUMP_CAP:
+            a = a[np.sort(np.random.default_rng(len(a)).choice(len(a), DUMP_CAP, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float64))
+
+
 def gather_sj(dist, torch, sj, world):
     """Every rank made the SJ rows of its own chromosomes: all-gather them (plumbing) so that rank 0 holds the whole table."""
     if dist is None:
@@ -402,6 +424,9 @@ def bench_ours(args, rank, world, local_rank):
     merged = ctx.gather_fetch() if world > 1 else tb
     summary = merged["summary"].copy() if rank == 0 else local_summary
     n_upd_total = len(merged["table"]["cov"]) if rank == 0 else 0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, merged, ctx.filter_fetch_keep())
+        log(f"[rank {rank}] outputs of the last timed step written to {args.dump_outputs}")
     del tb, merged
 
     # ---- end to end from HOST buffers: upload of the shard from pinned memory, the stages, gather + merge, and the merged
@@ -588,7 +613,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
     ap.add_argument("--e2e-contexts", type=int, default=3, help="lrb contexts (streams + host threads) kept in flight by the e2e leg at N = 1")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (rank 0's results)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":

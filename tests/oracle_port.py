@@ -3,6 +3,9 @@ reference binary (oracle/_ref/lr2rmats).  Never imported by the product."""
 from __future__ import annotations
 
 import ctypes as C
+import gzip
+import hashlib
+import json
 import os
 import subprocess
 
@@ -14,6 +17,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ORACLE_DIR = os.path.join(ROOT, "oracle")
 REF_BIN = os.path.join(ORACLE_DIR, "_ref", "lr2rmats")
 PORT_BIN = os.path.join(ORACLE_DIR, "_ref", "lr2rmats_port")
+REF_SORT_SCRIPT = os.path.join(ORACLE_DIR, "_ref", "sort_gtf.sh")          # the reference's src/sort_gtf.sh, copied by `make ref`
 PORT_SO = os.path.join(ORACLE_DIR, "liboracle_port.so")
 
 
@@ -105,6 +109,49 @@ def bam2sj(batch_soa: dict, is_uniq, params: cabi.SjParams) -> dict:
     out = {k: v.copy() for k, v in cabi.sj_to_np(res).items()}
     lib().orc_free_sj(C.byref(res))
     return out
+
+
+REF_DIGESTS = os.path.join(ROOT, "tests", "golden", "ref_digests.json")
+
+
+def digest(path) -> str:
+    """sha256 of a file's bytes; of the decompressed stream for a .bam (its deflate bytes depend on zlib)."""
+    with (gzip.open(path) if str(path).endswith(".bam") else open(path, "rb")) as f:
+        return hashlib.sha256(f.read()).hexdigest()
+
+
+def stored_digests(key: str, got: dict | None) -> dict:
+    """Entry `key` of tests/golden/ref_digests.json: digests of the reference's outputs on a test's generated inputs (or of those
+    inputs), so that the comparison with the reference holds where it is not built.  `got` maps names to the digests the test
+    computed from the reference's own run; with LRB_RECORD_REF_DIGESTS=1 they are (re)recorded instead."""
+    table = {}
+    if os.path.exists(REF_DIGESTS):
+        with open(REF_DIGESTS) as f:
+            table = json.load(f)
+    if os.environ.get("LRB_RECORD_REF_DIGESTS") == "1" and got is not None:
+        table[key] = got
+        with open(REF_DIGESTS, "w") as f:
+            json.dump(table, f, indent=1, sort_keys=True)
+            f.write("\n")
+    assert key in table, f"no entry {key} in tests/golden/ref_digests.json"
+    return table[key]
+
+
+def ref_digests(key: str, run_ref, paths: dict, available=None) -> dict:
+    """Digests of what the reference writes to `paths` (name -> file) when `run_ref()` runs it: computed live where it is built
+    (`available`, by default the reference binary) and checked against the stored ones, the stored ones elsewhere."""
+    if not (have_ref_bin() if available is None else available):
+        return stored_digests(key, None)
+    run_ref()
+    got = {name: digest(p) for name, p in paths.items()}
+    assert stored_digests(key, got) == got, f"{key}: the reference's outputs differ from entry {key} of tests/golden/ref_digests.json"
+    return got
+
+
+def check_inputs(key: str, paths: dict) -> None:
+    """The generated inputs must be the ones the stored reference digests were taken on."""
+    got = {name: digest(p) for name, p in paths.items()}
+    assert stored_digests(key, got) == got, f"{key}: the generated inputs changed; re-record tests/golden/ref_digests.json with the reference binary"
 
 
 def run_bin(binary: str, args: list, stdout_path: str | None = None, check=True):

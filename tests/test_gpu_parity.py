@@ -423,11 +423,10 @@ def test_rows_sort_replaces_samtools_sort(ctx, data, which, one_chrom):
 
 
 def test_cli_sort_input(data, tmp_path):
-    """LRB_SORT_INPUT=1: `lr2rmats-b200 update-gtf` on filter's unsorted BAM == the reference binary on the sorted records."""
-    import filecmp, os, subprocess
+    """LRB_SORT_INPUT=1: `lr2rmats-b200 update-gtf` on filter's unsorted BAM == the reference binary on the sorted records (run where it
+    is built, known by the digests of entry cli_sort_input of tests/golden/ref_digests.json elsewhere)."""
+    import os, subprocess
     from lr2rmats_b200 import api
-    if not op.have_ref_bin():
-        pytest.skip("reference binary not built")
     anno, rr = data["anno"], data["rr"]
     sh = _shuffle_runs(data["iso"], 12)
     synth.write_gtf(tmp_path / "anno.gtf", anno); synth.write_rm_gtf(tmp_path / "rm.gtf", rr, anno.chrom_names)
@@ -435,21 +434,24 @@ def test_cli_sort_input(data, tmp_path):
     of = op.filter(sh.soa(), rr, cabi.FilterParams.default())
     kept = sh.take(of["keep_idx"])
     synth.write_sam(tmp_path / "sorted.sam", kept.take(_samtools_order(kept)), with_seq=True)     # stands in for `samtools sort`
+    op.check_inputs("cli_sort_input_inputs", {fn: tmp_path / fn for fn in ("anno.gtf", "rm.gtf", "in.sam", "sorted.sam")})
     outs = ["-y", "@sum.txt", "-E", "@bed", "-A", "@detail.txt", "-k", "@known.gtf", "-o", "@updated.gtf"]
-    op.run_bin(op.REF_BIN, ["update-gtf", "-l", "3", str(tmp_path / "sorted.sam"), str(tmp_path / "anno.gtf")] + [x.replace("@", str(tmp_path) + "/ref.") for x in outs])
+    want = op.ref_digests("cli_sort_input", lambda: op.run_bin(op.REF_BIN, ["update-gtf", "-l", "3", str(tmp_path / "sorted.sam"), str(tmp_path / "anno.gtf")]
+                                                                         + [x.replace("@", str(tmp_path) + "/ref.") for x in outs]),
+                          {fn: tmp_path / f"ref.{fn}" for fn in ("sum.txt", "bed", "detail.txt", "known.gtf", "updated.gtf")})
     with open(tmp_path / "f.bam", "wb") as f:
         subprocess.run([api.CLI_PATH, "filter", "-r", str(tmp_path / "rm.gtf"), str(tmp_path / "in.sam")], stdout=f, stderr=subprocess.DEVNULL, check=True)
     env = dict(os.environ, LRB_SORT_INPUT="1")
     subprocess.run([api.CLI_PATH, "update-gtf", "-l", "3", str(tmp_path / "f.bam"), str(tmp_path / "anno.gtf")] + [x.replace("@", str(tmp_path) + "/our.") for x in outs],
                    stderr=subprocess.DEVNULL, check=True, env=env)
     for fn in ("sum.txt", "bed", "detail.txt", "known.gtf", "updated.gtf"):
-        assert filecmp.cmp(tmp_path / f"ref.{fn}", tmp_path / f"our.{fn}", shallow=False), fn
+        assert op.digest(tmp_path / f"our.{fn}") == want[fn], fn
     # the table-only fetch path (-o / -y / -E alone)
     few = ["-y", "@sum.txt", "-E", "@bed", "-o", "@updated.gtf"]
     subprocess.run([api.CLI_PATH, "update-gtf", "-l", "3", str(tmp_path / "f.bam"), str(tmp_path / "anno.gtf")] + [x.replace("@", str(tmp_path) + "/few.") for x in few],
                    stderr=subprocess.DEVNULL, check=True, env=env)
     for fn in ("sum.txt", "bed", "updated.gtf"):
-        assert filecmp.cmp(tmp_path / f"ref.{fn}", tmp_path / f"few.{fn}", shallow=False), fn
+        assert op.digest(tmp_path / f"few.{fn}") == want[fn], fn
     p = subprocess.run([api.CLI_PATH, "update-gtf", "-l", "3", str(tmp_path / "f.bam"), str(tmp_path / "anno.gtf")], stdout=subprocess.DEVNULL, stderr=subprocess.PIPE)
     assert p.returncode != 0                                       # without the knob the unsorted BAM is refused, as documented
 

@@ -1,8 +1,7 @@
 """Pins the CPU restatement (oracle/port) -- and the product's host readers/emitters it shares -- against the compiled
 reference binary on seeded synthetic inputs of a few thousand reads (every output file, both passes, split pieces).
-Runs only where oracle/_ref/lr2rmats exists (the build container; it also travels to the GPU box)."""
-import filecmp
-import gzip
+Where oracle/_ref/lr2rmats is built the reference runs alongside; elsewhere its outputs are known by their digests
+(the pin_* entries of tests/golden/ref_digests.json)."""
 import os
 
 import numpy as np
@@ -10,8 +9,6 @@ import pytest
 
 from lr2rmats_b200 import cabi, synth
 from tests import oracle_port as op
-
-pytestmark = pytest.mark.skipif(not op.have_ref_bin(), reason="reference binary not built (oracle/_ref/lr2rmats)")
 
 
 @pytest.fixture(scope="module")
@@ -26,25 +23,29 @@ def workdir(tmp_path_factory):
         ex = op.bam2gtf(r.soa(), cabi.ExonParams.default())
         sj = synth.make_sj((ex["tid"], ex["exon_off"], ex["exon_start"], ex["exon_end"]), 0.7, seed=5)
         synth.write_sj(d / f"{name}.sj.tab", sj, anno.chrom_names)
+    op.check_inputs("pin_inputs", {fn: d / fn for fn in sorted(os.listdir(d))})
     return d
 
 
+def run_one(workdir, tag, who, binary, args, stdout_name):
+    o = workdir / f"{tag}_{who}"
+    o.mkdir(exist_ok=True)
+    a = [x.replace("@", str(o) + "/") for x in args]
+    op.run_bin(binary, a, str(o / stdout_name) if stdout_name else None)
+    return {fn: op.digest(o / fn) for fn in sorted(os.listdir(o))}
+
+
 def run_both(workdir, tag, args, stdout_name=None):
-    outs = {}
-    for who, binary in (("ref", op.REF_BIN), ("port", op.PORT_BIN)):
-        o = workdir / f"{tag}_{who}"
-        o.mkdir(exist_ok=True)
-        a = [x.replace("@", str(o) + "/") for x in args]
-        op.run_bin(binary, a, str(o / stdout_name) if stdout_name else None)
-        outs[who] = o
-    names = sorted(os.listdir(outs["ref"]))
-    assert names == sorted(os.listdir(outs["port"]))
-    for fn in names:
-        if fn.endswith(".bam"):
-            assert gzip.open(outs["ref"] / fn).read() == gzip.open(outs["port"] / fn).read(), fn
-        else:
-            assert filecmp.cmp(outs["ref"] / fn, outs["port"] / fn, shallow=False), f"{tag}: {fn} differs"
-    return names
+    """Every output file of the port equals the reference's (a .bam after decompression: the deflate bytes depend on zlib)."""
+    got = run_one(workdir, tag, "port", op.PORT_BIN, args, stdout_name)
+    ref = run_one(workdir, tag, "ref", op.REF_BIN, args, stdout_name) if op.have_ref_bin() else None
+    want = op.stored_digests(f"pin_{tag}", ref)
+    if ref is not None:
+        assert ref == want, f"{tag}: the reference's outputs differ from the stored digests"
+    assert sorted(got) == sorted(want)
+    for fn in want:
+        assert got[fn] == want[fn], f"{tag}: {fn} differs"
+    return sorted(want)
 
 
 ALL = ["-A", "@detail.txt", "-y", "@summary.txt", "-E", "@bed", "-a", "@bam.gtf", "-k", "@known.gtf", "-v", "@novel.gtf", "-u", "@unrecog.gtf", "-o", "@updated.gtf"]
@@ -74,10 +75,10 @@ def test_update_pass2(workdir, which, extra):
 def test_gtf_input_mode(workdir):
     """-m g: the novel GTF of pass 1 fed back as input (Snakefile:189-192 uses unique-gtf -m g)."""
     sam = str(workdir / "iso.sam")
-    o = workdir / "gin"; o.mkdir(exist_ok=True)
-    op.run_bin(op.REF_BIN, ["update-gtf", "-l", "3", sam, str(workdir / "anno.gtf")], str(o / "novel.gtf"))
-    run_both(workdir, "gin_uniq", ["unique-gtf", "-m", "g", "-b", sam, str(o / "novel.gtf")], "out.gtf")
-    run_both(workdir, "gin_upd", ["update-gtf", "-m", "g", "-b", sam, "-l", "5", str(o / "novel.gtf"), str(workdir / "anno.gtf")] + ALL)
+    run_both(workdir, "gin", ["update-gtf", "-l", "3", sam, str(workdir / "anno.gtf")], "novel.gtf")
+    novel = str(workdir / "gin_port" / "novel.gtf")                  # byte-equal to the reference's
+    run_both(workdir, "gin_uniq", ["unique-gtf", "-m", "g", "-b", sam, novel], "out.gtf")
+    run_both(workdir, "gin_upd", ["update-gtf", "-m", "g", "-b", sam, "-l", "5", novel, str(workdir / "anno.gtf")] + ALL)
 
 
 @pytest.mark.parametrize("which", ["iso", "ont"])
@@ -91,17 +92,14 @@ def test_bam2sj(workdir, which, tmp_path):
     nh = rng.choice([0, 1, 1, 1, 2, 5], r.n)
     sam = tmp_path / "paired.sam"
     synth.write_sam(sam, r, with_seq=False, nh=nh)
+    op.check_inputs(f"pin_{which}_sj_inputs", {"paired.sam": sam})
     names = run_both(workdir, f"{which}_sj", ["bam2sj", str(sam)], "out.sj")
     run_both(workdir, f"{which}_sj_i", ["bam2sj", "-i", "300", str(sam)], "out.sj")
-    assert sum(1 for _ in open(workdir / f"{which}_sj_ref" / "out.sj")) > 50
+    assert sum(1 for _ in open(workdir / f"{which}_sj_port" / "out.sj")) > 50          # the outputs equal the reference's
     run_both(workdir, f"{which}_sj_se", ["bam2sj", str(workdir / f"{which}.sam")], "out.sj")
-    assert sum(1 for _ in open(workdir / f"{which}_sj_se_ref" / "out.sj")) == 4
+    assert sum(1 for _ in open(workdir / f"{which}_sj_se_port" / "out.sj")) == 4
 
 
-SORT_SCRIPT = "/root/reference/src/sort_gtf.sh"
-
-
-@pytest.mark.skipif(not os.path.exists(SORT_SCRIPT), reason="the reference's sort_gtf.sh is only present in the build container")
 @pytest.mark.parametrize("seed", [1, 2, 3, 4])
 def test_sort_gtf_fuzz(seed, tmp_path):
     """`sort-gtf` (host tagging + stable three-key sort; the port CLI sorts with std::stable_sort where the product uses the device) against
@@ -130,6 +128,9 @@ def test_sort_gtf_fuzz(seed, tmp_path):
     head = ["chr5\tsrc\texon\t10\t20\t.\t+\t.\tgene_id \"pre\";"] if seed % 2 else []
     text = "\n".join(head + [ln for b in blocks for ln in b]) + "\n"
     (tmp_path / "in.gtf").write_text(text)
-    subprocess.run(["bash", SORT_SCRIPT, str(tmp_path / "in.gtf"), str(tmp_path / "ref.gtf")], check=True, env=dict(os.environ, LC_ALL="C"))
+    op.check_inputs(f"pin_sort_gtf_{seed}_inputs", {"in.gtf": tmp_path / "in.gtf"})
+    want = op.ref_digests(f"pin_sort_gtf_{seed}", lambda: subprocess.run(["bash", op.REF_SORT_SCRIPT, str(tmp_path / "in.gtf"), str(tmp_path / "ref.gtf")],
+                                                                          check=True, env=dict(os.environ, LC_ALL="C")), {"sorted.gtf": tmp_path / "ref.gtf"},
+                          available=os.path.isfile(op.REF_SORT_SCRIPT))
     op.run_bin(op.PORT_BIN, ["sort-gtf", str(tmp_path / "in.gtf"), str(tmp_path / "port.gtf")])
-    assert (tmp_path / "port.gtf").read_bytes() == (tmp_path / "ref.gtf").read_bytes()
+    assert op.digest(tmp_path / "port.gtf") == want["sorted.gtf"]
