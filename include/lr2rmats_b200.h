@@ -12,7 +12,14 @@
  * Threading: one host thread per lrb_ctx.  A ctx owns one CUDA device, one
  * stream, all device memory and the pinned host result buffers it hands out.
  * Result pointers stay valid until the next *_run/_fetch call of the same kind
- * on that ctx or lrb_ctx_destroy().
+ * on that ctx or lrb_ctx_destroy().  Each kind has pinned buffers of its own:
+ *   filter  lrb_filter_fetch, lrb_filter, lrb_filter_fetch_keep
+ *   exons   lrb_exon_fetch, lrb_bam2gtf
+ *   update  lrb_update_fetch, lrb_update_gtf, lrb_update_fetch_table
+ *   unique  lrb_unique_fetch, lrb_unique_gtf
+ *   bam2sj  lrb_bam2sj
+ *   sort3   lrb_sort3
+ *   gather  lrb_gather_fetch
  */
 #ifndef LR2RMATS_B200_H
 #define LR2RMATS_B200_H

@@ -14,12 +14,17 @@ using namespace lrbk;
 
 namespace {
 
-int setup_rows(lrb_ctx *c, DRows &r, Buf &read, Buf &tid, Buf &rs, Buf &re, Buf &rev, Buf &beg, Buf &cnt, int64_t cap)
+// r backed by `cols`, sized for cap rows (r.n stays the caller's)
+int setup_rows(lrb_ctx *c, DRows &r, RowsCols<Buf> &cols, int64_t cap)
 {
-    size_t n = (size_t)std::max<int64_t>(cap, 1);
-    NEED(read, n * 4); NEED(tid, n * 4); NEED(rs, n * 4); NEED(re, n * 4); NEED(rev, n); NEED(beg, n * 4); NEED(cnt, n * 4);
-    r.cap = cap; r.read_idx = read.as<uint32_t>(); r.tid = tid.as<int32_t>(); r.start = rs.as<int32_t>(); r.end = re.as<int32_t>();
-    r.is_rev = rev.as<uint8_t>(); r.ex_beg = beg.as<uint32_t>(); r.ex_n = cnt.as<uint32_t>();
+    if (int rc = ensure(c, cols, Extent{std::max<int64_t>(cap, 1)})) return rc;
+    r = view(cols, r); r.cap = cap;
+    return LRB_OK;
+}
+int setup_list(lrb_ctx *c, DTransList &l, ListCols<Buf> &cols, int64_t n)
+{
+    if (int rc = ensure(c, cols, Extent{std::max<int64_t>(n, 1)})) return rc;
+    l = view(cols, DTransList{n, n});
     return LRB_OK;
 }
 int setup_exons(lrb_ctx *c, int64_t cap)
@@ -39,7 +44,7 @@ int run_scan(lrb_ctx *c, int mode, const lrb_filter_params *fp, const lrb_exon_p
     const int64_t n = c->b.n;
     int rc;
     if ((rc = ensure_tiles(c, n)) != LRB_OK) return rc;
-    if ((rc = setup_rows(c, c->rows, c->r_read, c->r_tid, c->r_rs, c->r_re, c->r_rev, c->r_beg, c->r_n, n)) != LRB_OK) return rc;
+    if ((rc = setup_rows(c, c->rows, c->rows_cols, n)) != LRB_OK) return rc;
     if (mode != 1) { NEED(c->f_pass, (size_t)n + 1); NEED(c->f_score, (size_t)n * 4 + 4); NEED(c->f_intron, (size_t)n * 4 + 4); }
     if (n == 0) { c->rows.n = 0; c->ex.n = 0; if (mode != 0 && (rc = setup_exons(c, 16)) != LRB_OK) return rc; return LRB_OK; }
     const double avg = (double)c->b.n_cigar / (double)n;
@@ -62,15 +67,15 @@ int run_scan(lrb_ctx *c, int mode, const lrb_filter_params *fp, const lrb_exon_p
         CK(cudaMemsetAsync(c->tile_state.p, 0, (size_t)n_tiles * 8, c->st));
         CK(cudaMemsetAsync(c->scalars.p, 0, 8 * 8, c->st)); CK(cudaMemsetAsync(d_ticket(c), 0, 4, c->st));
         size_t smem = (size_t)stage_words * 4;
-        tick(c, 8);
+        tick(c, EV_SCAN0);
         launch_cigar_scan(a, n_tiles, stream_mode, smem, c->st);
-        tick(c, 9);
+        tick(c, EV_SCAN1);
         CK(cudaGetLastError());
         if (by_record) return LRB_OK;
         uint64_t t[2];
         if ((rc = read_totals(c, t, 2)) != LRB_OK) return rc;
         c->rows.n = (int64_t)t[0]; c->ex.n = (int64_t)t[1];
-        if (c->timing) cudaEventElapsedTime(&c->ms[LRB_T_K_SCAN], c->ev[8], c->ev[9]);
+        if (c->timing) cudaEventElapsedTime(&c->ms[LRB_T_K_SCAN], c->ev[EV_SCAN0], c->ev[EV_SCAN1]);
         if (mode == 0 || c->ex.n <= c->ex.cap) break;
         if (attempt == 1) return fail(c, LRB_E_NOMEM, "exon pool still too small after regrow");
         if ((rc = setup_exons(c, c->ex.n + 16)) != LRB_OK) return rc;          // exact size known now: walk again
@@ -100,18 +105,10 @@ int setup_merge(lrb_ctx *c, MergeBufs &m, int64_t n_cand)
     size_t n = (size_t)std::max<int64_t>(n_cand, 1);
     NEED(m.keys, n * 8); NEED(m.head, n); NEED(m.locus_start, (n + 1) * 4); NEED(m.locus_cnt, n * 4); NEED(m.dropped, n);
     NEED(m.rep, n * 4); NEED(m.lstart, n * 4); NEED(m.evmask, n * 8); NEED(m.samemask, n * 8); NEED(m.hard, n); NEED(m.desc, n * 2); NEED(m.relsym, n * 8); NEED(m.ckey, (2 * n + 64) * 8); NEED(m.cmin, (2 * n + 64) * 4); NEED(m.cord, n); NEED(m.clist, n * 4); NEED(m.crow, n * 16); NEED(m.fb_list, n * 8); NEED(m.fb_cnt, 64);
-    Buf *w[] = {&m.w_cand, &m.w_cov, &m.w_tid, &m.w_start, &m.w_end, &m.w_fs, &m.w_le, &m.o_cand, &m.o_cov, &m.o_tid, &m.o_start, &m.o_end, &m.o_fs, &m.o_le};
-    for (Buf *b : w) NEED(*b, n * 4);
-    Buf *cb[] = {&m.c_tid, &m.c_start, &m.c_end, &m.c_rev, &m.c_n, &m.c_fs, &m.c_le, &m.c_gbeg};
-    for (Buf *b : cb) NEED(*b, n * 4);
-    NEED(m.c_hash, n * 8); NEED(m.c_j0, n * 8); NEED(m.c_sig, n * 8);
+    const Extent e{(int64_t)n};
+    int rc;
+    if ((rc = ensure(c, m.w, e)) || (rc = ensure(c, m.o, e)) || (rc = ensure(c, m.cd, e))) return rc;
     return LRB_OK;
-}
-DMerged merged_view(Buf &cand, Buf &cov, Buf &tid, Buf &st, Buf &en, Buf &fs, Buf &le, int64_t n)
-{
-    DMerged d; d.n = n; d.cap = n; d.cand = cand.as<uint32_t>(); d.cov = cov.as<int32_t>(); d.tid = tid.as<int32_t>(); d.start = st.as<int32_t>();
-    d.end = en.as<int32_t>(); d.fs = fs.as<int32_t>(); d.le = le.as<int32_t>();
-    return d;
 }
 
 // merge fold over `list`, asynchronous.  n_cand is the number of candidates, or (n_cand_dev != nullptr) the host's upper
@@ -135,11 +132,7 @@ int run_merge_async(lrb_ctx *c, MergeBufs &m, const DTransList &list, int64_t n_
     a.keys = m.keys.as<uint64_t>(); a.head = m.head.as<uint8_t>(); a.locus_start = m.locus_start.as<uint32_t>(); a.locus_cnt = m.locus_cnt.as<uint32_t>();
     a.dropped = m.dropped.as<uint8_t>();
     a.rep = m.rep.as<uint32_t>(); a.lstart = m.lstart.as<uint32_t>(); a.evmask = m.evmask.as<uint64_t>(); a.samemask = m.samemask.as<uint64_t>(); a.hard = m.hard.as<uint8_t>(); a.desc = m.desc.as<uint16_t>(); a.relsym = m.relsym.as<uint64_t>(); a.ckey = m.ckey.as<uint64_t>(); a.cmin = m.cmin.as<uint32_t>(); a.cord = m.cord.as<uint8_t>(); a.clist = m.clist.as<uint32_t>(); a.crow = m.crow.as<uint64_t>(); a.fb_list = m.fb_list.as<uint32_t>(); a.fb_cnt = m.fb_cnt.as<uint32_t>();
-    a.work = merged_view(m.w_cand, m.w_cov, m.w_tid, m.w_start, m.w_end, m.w_fs, m.w_le, n_cand);
-    a.out = merged_view(m.o_cand, m.o_cov, m.o_tid, m.o_start, m.o_end, m.o_fs, m.o_le, n_cand);
-    a.cd.tid = m.c_tid.as<int32_t>(); a.cd.start = m.c_start.as<int32_t>(); a.cd.end = m.c_end.as<int32_t>(); a.cd.rev = m.c_rev.as<int32_t>();
-    a.cd.n = m.c_n.as<int32_t>(); a.cd.fs = m.c_fs.as<int32_t>(); a.cd.le = m.c_le.as<int32_t>(); a.cd.gbeg = m.c_gbeg.as<uint32_t>();
-    a.cd.hash = m.c_hash.as<uint64_t>(); a.cd.j0 = m.c_j0.as<uint64_t>(); a.cd.sig = m.c_sig.as<uint64_t>();
+    a.work = view(m.w, DMerged{n_cand, n_cand}); a.out = view(m.o, DMerged{n_cand, n_cand}); a.cd = view(m.cd, CandSoA{});
     a.tile_state = side ? c->tile_state2.as<uint64_t>() : c->tile_state.as<uint64_t>(); a.ticket = side ? d_ticket2(c) : d_ticket(c); a.totals = totals;
     a.kls = kls; a.class_alive = class_alive; a.single_locus = single_locus ? 1 : 0;
     if (xl) {
@@ -153,9 +146,9 @@ int run_merge_async(lrb_ctx *c, MergeBufs &m, const DTransList &list, int64_t n_
     }
     m.args = a;
     launch_merge_prepare(a, st);
-    if (time_fold) tick(c, 10);
+    if (time_fold) tick(c, EV_FOLD0);
     launch_merge_fold(a, st);                        // locus count is consumed on the device: no host round trip
-    if (time_fold) tick(c, 11);
+    if (time_fold) tick(c, EV_FOLD1);
     if (xl) launch_xlocus_detect(a, c->xl, st);
     if (kls) launch_merge_class_counts(a, st);
     else launch_merge_finish(a, st);
@@ -170,15 +163,7 @@ int run_merge(lrb_ctx *c, MergeBufs &m, const DTransList &list, int64_t n_cand, 
     uint64_t t[2];
     if ((rc = read_totals(c, t, 2)) != LRB_OK) return rc;
     m.n_loci = (int64_t)t[0]; m.n_out = (int64_t)t[1];
-    if (c->timing && n_cand) cudaEventElapsedTime(&c->ms[LRB_T_K_FOLD], c->ev[10], c->ev[11]);
-    return LRB_OK;
-}
-
-int setup_list(lrb_ctx *c, DTransList &l, Buf &row, Buf &lo, Buf &cnt, Buf &piece, int64_t n)
-{
-    size_t k = (size_t)std::max<int64_t>(n, 1);
-    NEED(row, k * 4); NEED(lo, k * 4); NEED(cnt, k * 4); NEED(piece, k * 4);
-    l.n = n; l.cap = n; l.row = row.as<uint32_t>(); l.lo = lo.as<uint32_t>(); l.cnt = cnt.as<uint32_t>(); l.piece = piece.as<int32_t>();
+    if (c->timing && n_cand) cudaEventElapsedTime(&c->ms[LRB_T_K_FOLD], c->ev[EV_FOLD0], c->ev[EV_FOLD1]);
     return LRB_OK;
 }
 
@@ -210,7 +195,7 @@ int lrb_ctx_create(int device, lrb_ctx **out)
     { const char *e = getenv("LRB_FORCE_SINGLE_FOLD"); if (e) c->force_single_fold = atoi(e) != 0; }    // test hook: updated_T always folded by the one-locus replay
     if (!c->scalars.ensure(512) || !c->h_scalars.ensure(512)) { delete c; return LRB_E_NOMEM; }
     cudaMemsetAsync(c->scalars.p, 0, 512, c->st);
-    for (int i = 0; i < 12; ++i) cudaEventCreate(&c->ev[i]);
+    for (cudaEvent_t &e : c->ev) cudaEventCreate(&e);
     for (int i = 0; i < 8; ++i) cudaEventCreate(&c->marks[i]);
     memset(c->ms, 0, sizeof c->ms); memset(c->summary, 0, sizeof c->summary);
     c->launches0 = total_launches();
@@ -223,33 +208,13 @@ void lrb_ctx_destroy(lrb_ctx *c)
     if (!c) return;
     cudaSetDevice(c->device);
     cudaStreamSynchronize(c->st); cudaStreamSynchronize(c->st2); cudaStreamSynchronize(c->st3);
-    Buf *bufs[] = {&c->a_tid, &c->a_start, &c->a_end, &c->a_gene, &c->a_rev, &c->a_off, &c->a_es, &c->a_ee, &c->a_pmax, &c->a_mono, &c->s_tid, &c->s_don, &c->s_acc,
-                   &c->s_u, &c->s_m, &c->s_pmax, &c->s_dkey, &c->r_gtid, &c->r_goff, &c->r_start, &c->r_pmax, &c->b_tid, &c->b_pos, &c->b_lq, &c->b_nm,
-                   &c->b_flag, &c->b_xs, &c->b_qh, &c->b_coff, &c->b_cig, &c->f_pass, &c->f_score, &c->f_intron, &c->f_keep_row_mask, &c->f_keep_rec_mask,
-                   &c->f_keep_idx, &c->f_keep_rows, &c->r_read, &c->r_tid, &c->r_rs, &c->r_re, &c->r_rev, &c->r_beg, &c->r_n, &c->r_nonmono, &c->q_read, &c->q_tid,
-                   &c->q_rs, &c->q_re, &c->q_rev, &c->q_beg, &c->q_n, &c->e_s, &c->e_e, &c->e_f, &c->u_cls, &c->u_ref, &c->u_nnovel, &c->u_noff, &c->u_mk,
-                   &c->u_mu, &c->u_ck, &c->u_cr, &c->u_cu, &c->u_cn, &c->u_known, &c->u_unrecog, &c->u_sub, &c->n_row, &c->n_lo, &c->n_cnt, &c->n_piece,
-                   &c->t_row, &c->t_lo, &c->t_cnt, &c->t_piece, &c->h_khi, &c->h_klo, &c->h_min, &c->h_score, &c->y_barcnt, &c->y_barseg, &c->y_genebar,
-                   &c->y_bedcnt, &c->y_bedoff, &c->y_counts, &c->y_nelem, &c->bd_tid, &c->bd_s, &c->bd_e, &c->bd_sc, &c->bd_ty, &c->bd_rv, &c->q_shared, &c->tb_name, &c->tb_piece, &c->tb_ttid, &c->tb_tstart, &c->tb_tend, &c->tb_trev, &c->tb_etid, &c->tb_erev, &c->tb_cov, &c->tb_ref, &c->tb_cnt, &c->tb_off, &c->tb_es, &c->tb_ee, &c->tb_flag,
-                   &c->s_read, &c->s_rtid, &c->s_rs, &c->s_re, &c->s_rev, &c->s_beg, &c->s_n, &c->s_key0, &c->s_key1, &c->s_idx0, &c->s_idx1, &c->s_hist,
-                   &c->tile_state, &c->tile_state2, &c->scalars, &c->kg_pairs, &c->xl_key, &c->xl_min, &c->xl_max, &c->xl_cnt, &c->xl_forced,
-                   &c->j_cnt, &c->j_off, &c->j_uq, &c->j_tid, &c->j_don, &c->j_acc, &c->j_u, &c->j_head, &c->j_hpos, &c->jo_tid, &c->jo_don, &c->jo_acc, &c->jo_u, &c->jo_m};
-    for (Buf *b : bufs) b->release();
-    for (MergeBufs *m : {&c->mg, &c->mg2}) {
-        Buf *w[] = {&m->keys, &m->head, &m->locus_start, &m->locus_cnt, &m->dropped, &m->rep, &m->lstart, &m->evmask, &m->samemask, &m->hard, &m->desc, &m->relsym, &m->ckey, &m->cmin, &m->cord, &m->clist, &m->crow, &m->fb_list, &m->fb_cnt, &m->w_cand, &m->w_cov, &m->w_tid, &m->w_start, &m->w_end, &m->w_fs,
-                    &m->w_le, &m->o_cand, &m->o_cov, &m->o_tid, &m->o_start, &m->o_end, &m->o_fs, &m->o_le,
-                    &m->c_tid, &m->c_start, &m->c_end, &m->c_rev, &m->c_n, &m->c_fs, &m->c_le, &m->c_gbeg, &m->c_hash, &m->c_j0, &m->c_sig};
-        for (Buf *b : w) b->release();
-    }
     lrbk::multi_release(c);
-    for (PBuf &p : c->p) p.release();
-    c->h_scalars.release();
-    for (int i = 0; i < 12; ++i) cudaEventDestroy(c->ev[i]);
+    for (cudaEvent_t e : c->ev) cudaEventDestroy(e);
     for (int i = 0; i < 8; ++i) cudaEventDestroy(c->marks[i]);
     cudaEventDestroy(c->ev_fork); cudaEventDestroy(c->ev_join);
     cudaEventDestroy(c->ev_fork3); cudaEventDestroy(c->ev_join3); cudaStreamDestroy(c->st3);
     cudaStreamDestroy(c->st2); cudaStreamDestroy(c->st);
-    delete c;
+    delete c;                                       // frees the device and pinned buffers
 }
 
 const char *lrb_last_error(const lrb_ctx *c) { return c ? c->err.c_str() : "null context"; }
@@ -275,22 +240,12 @@ int lrb_anno_upload(lrb_ctx *c, const lrb_anno *a)
             if (a->exon_start[k] <= a->exon_start[k - 1] || a->exon_end[k] <= a->exon_end[k - 1]) { m = 0; break; }
         mono[(size_t)i] = m;
     }
-    int rc;
-    if ((rc = h2d(c, c->a_mono, mono.data(), (size_t)n))) return rc;
-    if ((rc = h2d(c, c->a_tid, a->tid, (size_t)n))) return rc;
-    if ((rc = h2d(c, c->a_start, a->start, (size_t)n))) return rc;
-    if ((rc = h2d(c, c->a_end, a->end, (size_t)n))) return rc;
-    if ((rc = h2d(c, c->a_gene, a->gene, (size_t)n))) return rc;
-    if ((rc = h2d(c, c->a_rev, a->is_rev, (size_t)n))) return rc;
-    if ((rc = h2d(c, c->a_off, a->exon_off, (size_t)n + 1))) return rc;
-    if ((rc = h2d(c, c->a_es, a->exon_start, (size_t)a->n_exon))) return rc;
-    if ((rc = h2d(c, c->a_ee, a->exon_end, (size_t)a->n_exon))) return rc;
-    if ((rc = h2d(c, c->a_pmax, pm.data(), (size_t)n))) return rc;
+    AnnoCols<const void *> src;
+    src.tid = a->tid; src.start = a->start; src.end = a->end; src.gene = a->gene; src.is_rev = a->is_rev; src.exon_off = a->exon_off;
+    src.es = a->exon_start; src.ee = a->exon_end; src.pmax_key = pm.data(); src.mono = mono.data();
+    if (int rc = copy(c, c->anno_cols, src, Extent{n, a->n_exon}, cudaMemcpyHostToDevice)) return rc;
     CK(cudaStreamSynchronize(c->st));               // pm is a local
-    c->anno.n = n; c->anno.n_exon = a->n_exon; c->anno.tid = c->a_tid.as<int32_t>(); c->anno.start = c->a_start.as<int32_t>();
-    c->anno.end = c->a_end.as<int32_t>(); c->anno.gene = c->a_gene.as<int32_t>(); c->anno.is_rev = c->a_rev.as<uint8_t>();
-    c->anno.exon_off = c->a_off.as<uint32_t>(); c->anno.es = c->a_es.as<int32_t>(); c->anno.ee = c->a_ee.as<int32_t>();
-    c->anno.pmax_key = c->a_pmax.as<uint64_t>(); c->anno.mono = c->a_mono.as<uint8_t>();
+    c->anno = view(c->anno_cols, DAnno{n, a->n_exon});
     return LRB_OK;
 }
 
@@ -320,14 +275,11 @@ int lrb_rm_upload(lrb_ctx *c, const lrb_anno *rmt)
         for (auto &iv : g.second) { m = std::max(m, iv.second); st.push_back(iv.first); pe.push_back(m); }
         gt.push_back(g.first); go.push_back((int32_t)st.size());
     }
-    int rc;
-    if ((rc = h2d(c, c->r_gtid, gt.data(), gt.size()))) return rc;
-    if ((rc = h2d(c, c->r_goff, go.data(), go.size()))) return rc;
-    if ((rc = h2d(c, c->r_start, st.data(), st.size()))) return rc;
-    if ((rc = h2d(c, c->r_pmax, pe.data(), pe.size()))) return rc;
+    RmCols<const void *> src;
+    src.g_tid = gt.data(); src.g_off = go.data(); src.start = st.data(); src.pmax_end = pe.data();
+    if (int rc = copy(c, c->rm_cols, src, Extent{(int64_t)gt.size(), (int64_t)st.size()}, cudaMemcpyHostToDevice)) return rc;
     CK(cudaStreamSynchronize(c->st));
-    c->rm.n_groups = (int32_t)gt.size(); c->rm.n = (int32_t)st.size(); c->rm.g_tid = c->r_gtid.as<int32_t>(); c->rm.g_off = c->r_goff.as<int32_t>();
-    c->rm.start = c->r_start.as<int32_t>(); c->rm.pmax_end = c->r_pmax.as<int32_t>();
+    c->rm = view(c->rm_cols, DRmIndex{(int32_t)gt.size(), (int32_t)st.size()});
     return LRB_OK;
 }
 
@@ -346,17 +298,11 @@ int lrb_sj_upload(lrb_ctx *c, const lrb_sj *s)
         dk[(size_t)i] = ((uint64_t)(uint32_t)(s->tid[i] + 1) << 32) | (uint32_t)s->don[i];
         if (i && dk[(size_t)i] < dk[(size_t)i - 1]) return fail(c, LRB_E_ARG, "SJ table is not sorted by (tid,don,acc)");
     }
-    int rc;
-    if ((rc = h2d(c, c->s_tid, s->tid, (size_t)n))) return rc;
-    if ((rc = h2d(c, c->s_don, s->don, (size_t)n))) return rc;
-    if ((rc = h2d(c, c->s_acc, s->acc, (size_t)n))) return rc;
-    if ((rc = h2d(c, c->s_u, s->uniq_c, (size_t)n))) return rc;
-    if ((rc = h2d(c, c->s_m, s->multi_c, (size_t)n))) return rc;
-    if ((rc = h2d(c, c->s_pmax, pm.data(), (size_t)n))) return rc;
-    if ((rc = h2d(c, c->s_dkey, dk.data(), (size_t)n))) return rc;
+    SjCols<const void *> src;
+    src.tid = s->tid; src.don = s->don; src.acc = s->acc; src.cnt_u = s->uniq_c; src.cnt_m = s->multi_c; src.pmax_key = pm.data(); src.don_key = dk.data();
+    if (int rc = copy(c, c->sj_cols, src, Extent{n}, cudaMemcpyHostToDevice)) return rc;
     CK(cudaStreamSynchronize(c->st));
-    c->sj.n = n; c->sj.tid = c->s_tid.as<int32_t>(); c->sj.don = c->s_don.as<int32_t>(); c->sj.acc = c->s_acc.as<int32_t>();
-    c->sj.cnt_u = c->s_u.as<int32_t>(); c->sj.cnt_m = c->s_m.as<int32_t>(); c->sj.pmax_key = c->s_pmax.as<uint64_t>(); c->sj.don_key = c->s_dkey.as<uint64_t>();
+    c->sj = view(c->sj_cols, DSj{n});
     return LRB_OK;
 }
 
@@ -370,21 +316,12 @@ int lrb_batch_upload(lrb_ctx *c, const lrb_batch *b)
     if (b->n >= (1ll << 31) - 1) return fail(c, LRB_E_ARG, "batch too large: at most 2^31-2 records per batch");
     if (n && b->cigar_off[0] != 0) return fail(c, LRB_E_ARG, "cigar_off[0] must be 0");
     if (nc >= (1ull << 40)) return fail(c, LRB_E_ARG, "batch too large: at most 2^40 CIGAR ops per batch");
-    int rc;
-    if ((rc = h2d(c, c->b_tid, b->tid, n))) return rc;
-    if ((rc = h2d(c, c->b_pos, b->pos, n))) return rc;
-    if ((rc = h2d(c, c->b_flag, b->flag, n))) return rc;
-    if ((rc = h2d(c, c->b_lq, b->l_qseq, n))) return rc;
-    if ((rc = h2d(c, c->b_nm, b->nm, n))) return rc;
-    if ((rc = h2d(c, c->b_xs, b->xs, n))) return rc;
-    if ((rc = h2d(c, c->b_qh, b->qname_hash, n))) return rc;
-    if (n) { if ((rc = h2d(c, c->b_coff, b->cigar_off, n + 1))) return rc; }
-    else { NEED(c->b_coff, 8); CK(cudaMemsetAsync(c->b_coff.p, 0, 8, c->st)); }
-    if ((rc = h2d(c, c->b_cig, b->cigar, nc))) return rc;
-    c->b.n = b->n; c->b.n_cigar = (int64_t)nc;
-    c->b.tid = c->b_tid.as<int32_t>(); c->b.pos = c->b_pos.as<int32_t>(); c->b.flag = c->b_flag.as<uint16_t>(); c->b.l_qseq = c->b_lq.as<int32_t>();
-    c->b.nm = c->b_nm.as<int32_t>(); c->b.xs = c->b_xs.as<int8_t>(); c->b.qhash = c->b_qh.as<uint64_t>(); c->b.cigar_off = c->b_coff.as<uint64_t>();
-    c->b.cigar = c->b_cig.as<uint32_t>();
+    static const uint64_t no_cigar = 0;             // cigar_off of an empty batch
+    BatchCols<const void *> src;
+    src.tid = b->tid; src.pos = b->pos; src.l_qseq = b->l_qseq; src.nm = b->nm; src.flag = b->flag; src.xs = b->xs; src.qhash = b->qname_hash;
+    src.cigar_off = n ? b->cigar_off : &no_cigar; src.cigar = b->cigar;
+    if (int rc = copy(c, c->batch_cols, src, Extent{(int64_t)n, (int64_t)nc}, cudaMemcpyHostToDevice)) return rc;
+    c->b = view(c->batch_cols, DBatch{b->n, (int64_t)nc});
     c->have_batch = true; c->have_filter = c->have_exons = c->have_update = c->have_unique = false;
     return LRB_OK;
 }
@@ -409,10 +346,10 @@ int lrb_chains_upload(lrb_ctx *c, const lrb_chains *ch)
     CK(cudaSetDevice(c->device));
     const int64_t n = ch->n; const int64_t ne = n ? ch->exon_off[n] : 0;
     int rc;
-    if ((rc = setup_rows(c, c->rows, c->r_read, c->r_tid, c->r_rs, c->r_re, c->r_rev, c->r_beg, c->r_n, n))) return rc;
+    if ((rc = setup_rows(c, c->rows, c->rows_cols, n))) return rc;
     if ((rc = setup_exons(c, ne + 16))) return rc;
-    if ((rc = h2d(c, c->r_tid, ch->tid, (size_t)n))) return rc;
-    if ((rc = h2d(c, c->r_rev, ch->is_rev, (size_t)n))) return rc;
+    if ((rc = h2d(c, c->rows_cols.tid, ch->tid, (size_t)n))) return rc;
+    if ((rc = h2d(c, c->rows_cols.is_rev, ch->is_rev, (size_t)n))) return rc;
     if ((rc = h2d(c, c->e_s, ch->exon_start, (size_t)ne))) return rc;
     if ((rc = h2d(c, c->e_e, ch->exon_end, (size_t)ne))) return rc;
     if ((rc = h2d(c, c->u_noff, ch->exon_off, (size_t)n + 1))) return rc;          // scratch for the offsets
@@ -429,12 +366,12 @@ int lrb_filter_run(lrb_ctx *c, const lrb_filter_params *p)
     if (!c || !p) return LRB_E_ARG;
     if (!c->have_batch) return fail(c, LRB_E_ARG, "lrb_filter_run: no batch uploaded");
     CK(cudaSetDevice(c->device));
-    int64_t l0 = total_launches(); tick(c, 0);
+    int64_t l0 = total_launches(); tick(c, EV_BEGIN);
     int rc = run_scan(c, 0, p, nullptr, nullptr); if (rc) return rc;
     if ((rc = run_select(c, p))) return rc;
-    tick(c, 1);
+    tick(c, EV_END);
     c->have_filter = true; c->have_exons = false; c->launches_last = total_launches() - l0;
-    if (c->timing) { CK(cudaStreamSynchronize(c->st)); cudaEventElapsedTime(&c->ms[LRB_T_FILTER], c->ev[0], c->ev[1]); }
+    if (c->timing) { CK(cudaStreamSynchronize(c->st)); cudaEventElapsedTime(&c->ms[LRB_T_FILTER], c->ev[EV_BEGIN], c->ev[EV_END]); }
     return LRB_OK;
 }
 
@@ -444,12 +381,12 @@ int lrb_exon_run(lrb_ctx *c, const lrb_exon_params *p, int use_keep_list)
     if (!c->have_batch) return fail(c, LRB_E_ARG, "lrb_exon_run: no batch uploaded");
     if (use_keep_list && !c->have_filter) return fail(c, LRB_E_ARG, "lrb_exon_run: keep list requested but lrb_filter_run has not run");
     CK(cudaSetDevice(c->device));
-    int64_t l0 = total_launches(); tick(c, 0);
+    int64_t l0 = total_launches(); tick(c, EV_BEGIN);
     int rc = run_scan(c, 1, nullptr, p, use_keep_list ? c->f_keep_rec_mask.as<uint8_t>() : nullptr); if (rc) return rc;
-    tick(c, 1);
+    tick(c, EV_END);
     c->cur = &c->rows; c->rows_compact = true; c->have_exons = true; c->have_update = c->have_unique = false;
     c->launches_last = total_launches() - l0;
-    if (c->timing) { CK(cudaStreamSynchronize(c->st)); cudaEventElapsedTime(&c->ms[LRB_T_EXON], c->ev[0], c->ev[1]); }
+    if (c->timing) { CK(cudaStreamSynchronize(c->st)); cudaEventElapsedTime(&c->ms[LRB_T_EXON], c->ev[EV_BEGIN], c->ev[EV_END]); }
     return LRB_OK;
 }
 
@@ -458,11 +395,11 @@ int lrb_pipeline_run(lrb_ctx *c, const lrb_filter_params *fp, const lrb_exon_par
     if (!c || !fp || !ep) return LRB_E_ARG;
     if (!c->have_batch) return fail(c, LRB_E_ARG, "lrb_pipeline_run: no batch uploaded");
     CK(cudaSetDevice(c->device));
-    int64_t l0 = total_launches(); tick(c, 0);
+    int64_t l0 = total_launches(); tick(c, EV_BEGIN);
     const int64_t n = c->b.n;
     int rc;
     NEED(c->f_keep_rec_mask, (size_t)std::max<int64_t>(n, 1)); NEED(c->f_keep_idx, (size_t)std::max<int64_t>(n, 1) * 4);
-    if ((rc = setup_rows(c, c->rows2, c->q_read, c->q_tid, c->q_rs, c->q_re, c->q_rev, c->q_beg, c->q_n, n))) return rc;
+    if ((rc = setup_rows(c, c->rows2, c->rows2_cols, n))) return rc;
     c->rows.n = 0; c->ex.n = 0; c->n_pass = c->n_keep = 0;
     for (int attempt = 0; n > 0; ++attempt) {
         // scan (rows at their record index) -> run selection on the record stream -> compaction + row gather: one
@@ -476,7 +413,7 @@ int lrb_pipeline_run(lrb_ctx *c, const lrb_filter_params *fp, const lrb_exon_par
         uint64_t t[3];
         if ((rc = read_totals(c, t, 3))) return rc;
         c->n_pass = (int64_t)t[0]; c->ex.n = (int64_t)t[1]; c->n_keep = (int64_t)t[2];
-        if (c->timing) cudaEventElapsedTime(&c->ms[LRB_T_K_SCAN], c->ev[8], c->ev[9]);
+        if (c->timing) cudaEventElapsedTime(&c->ms[LRB_T_K_SCAN], c->ev[EV_SCAN0], c->ev[EV_SCAN1]);
         if (c->ex.n <= c->ex.cap) break;
         if (attempt == 1) return fail(c, LRB_E_NOMEM, "exon pool still too small after regrow");
         if ((rc = setup_exons(c, c->ex.n + 16))) return rc;     // exact size known now: walk again
@@ -484,10 +421,10 @@ int lrb_pipeline_run(lrb_ctx *c, const lrb_filter_params *fp, const lrb_exon_par
     if (n == 0 && (rc = setup_exons(c, 16))) return rc;
     c->rows.n = n;                                               // record-indexed: only the passing records' rows are valid
     c->rows2.n = c->n_keep;
-    tick(c, 1);
+    tick(c, EV_END);
     c->cur = &c->rows2; c->rows_compact = false; c->have_filter = true; c->have_exons = true; c->have_update = c->have_unique = false;
     c->launches_last = total_launches() - l0;
-    if (c->timing) { CK(cudaStreamSynchronize(c->st)); cudaEventElapsedTime(&c->ms[LRB_T_FILTER], c->ev[0], c->ev[1]); c->ms[LRB_T_EXON] = 0; }
+    if (c->timing) { CK(cudaStreamSynchronize(c->st)); cudaEventElapsedTime(&c->ms[LRB_T_FILTER], c->ev[EV_BEGIN], c->ev[EV_END]); c->ms[LRB_T_EXON] = 0; }
     return LRB_OK;
 }
 
@@ -535,7 +472,7 @@ int lrb_update_run(lrb_ctx *c, const lrb_update_params *up)
     NEED(c->y_counts, 64); NEED(c->y_nelem, 64);       // y_nelem: element count, then (at +16) the six tickets of sum_scans_kernel
     if ((rc = ensure_tiles(c, std::max<int64_t>(n, c->ex.n)))) return rc;
     CK(cudaMemsetAsync(d_err(c), 0, 4, c->st));
-    tick(c, 0);
+    tick(c, EV_BEGIN);
     // ---- classification (+ SJ support)
     ClassArgs ca{};
     ca.rows = rows; ca.ex = c->ex; ca.anno = c->anno; ca.sj = c->sj; ca.up = *up;
@@ -543,7 +480,7 @@ int lrb_update_run(lrb_ctx *c, const lrb_update_params *up)
     ca.cls = c->u_cls.as<uint32_t>(); ca.ref = c->u_ref.as<int32_t>(); ca.n_novel = c->u_nnovel.as<uint32_t>(); ca.err_flags = d_err(c);
     launch_classify(ca, c->u_mk.as<uint8_t>(), c->st);     // u_mk: scratch for the slow-row mask
     CK(cudaGetLastError());
-    tick(c, 1);
+    tick(c, EV_CLASSIFIED);
 
     // ---- lists, the updated_T fold, the class folds and the element count of the summary sets: one stream of launches,
     // every count stays on the device; ONE copy brings them all back.  novel_T is sized optimistically (pieces are rare);
@@ -568,8 +505,7 @@ int lrb_update_run(lrb_ctx *c, const lrb_update_params *up)
     int64_t n_novel = 0, nu = 0; uint64_t n_elem = 0, n_exon_elem = 0;
     uint32_t cnt16[16];
     for (int attempt = 0; n > 0; ++attempt) {
-        if ((rc = setup_list(c, c->novel, c->n_row, c->n_lo, c->n_cnt, c->n_piece, cap))) return rc;
-        c->novel.cap = cap;
+        if ((rc = setup_list(c, c->novel, c->novel_cols, cap))) return rc;
         CK(cudaMemsetAsync(c->y_counts.p, 0, 64, c->st)); CK(cudaMemsetAsync(c->y_nelem.p, 0, 16, c->st));
         ListArgs la{};
         la.rows = rows; la.ex = c->ex; la.up = *up; la.cls = ca.cls; la.n_novel = ca.n_novel; la.novel = c->novel;
@@ -578,14 +514,14 @@ int lrb_update_run(lrb_ctx *c, const lrb_update_params *up)
         la.tile_state = c->tile_state.as<uint64_t>(); la.ticket = d_ticket(c); la.totals = T + T_NOVEL;
         launch_build_lists(la, c->st);
         CK(cudaGetLastError());
-        if (attempt == 0 && fold_pass == 0) tick(c, 2);
+        if (attempt == 0 && fold_pass == 0) tick(c, EV_LISTED);
         if (up->want_summary) {
             // class counts + uniq_* folds over bam_T (update_gtf.c:501-528): the four classes partition the rows; they are
             // folded in ONE pass over all rows, each candidate seeing only the entries of its own class.  Independent of the
             // updated_T fold and of the sets: forked onto the side stream, joined in front of the round trip below.
             const bool side = c->side_stream;
             cudaStream_t s2 = side ? c->st2 : c->st;
-            if ((rc = setup_list(c, c->tmp_list, c->t_row, c->t_lo, c->t_cnt, c->t_piece, n))) return rc;
+            if ((rc = setup_list(c, c->tmp_list, c->tmp_cols, n))) return rc;
             if (side) { CK(cudaEventRecord(c->ev_fork, c->st)); CK(cudaStreamWaitEvent(c->st2, c->ev_fork, 0)); }
             launch_rows_as_list(rows, nullptr, n, c->tmp_list, s2);
             if ((rc = run_merge_async(c, c->mg2, c->tmp_list, n, nullptr, *up, T + T_LOCI2, c->u_ck.as<uint8_t>(), c->y_counts.as<uint32_t>() + 8, false, side))) return rc;
@@ -594,14 +530,14 @@ int lrb_update_run(lrb_ctx *c, const lrb_update_params *up)
         // updated_T = merge fold over novel_T (update_gtf.c:949,956)
         if (xl_exact) { NEED(c->xl_forced, (size_t)std::max<int64_t>(cap, 1)); CK(cudaMemsetAsync(c->xl_forced.p, 0, (size_t)std::max<int64_t>(cap, 1), c->st)); }
         if ((rc = run_merge_async(c, c->mg, c->novel, cap, T + T_NOVEL, *up, T + T_LOCI, nullptr, nullptr, true, false, single, xl_exact))) return rc;
-        if (attempt == 0 && fold_pass == 0) tick(c, 3);
+        if (attempt == 0 && fold_pass == 0) tick(c, EV_FOLDED);
         if (run_sets) {
             // sets over updated_T: element count (sizes the hash table)
             const size_t capn = (size_t)std::max<int64_t>(cap, 1);
             NEED(c->y_barcnt, capn * 16); NEED(c->y_barseg, capn * 16); NEED(c->y_genebar, capn * 8); NEED(c->y_bedcnt, capn * 4); NEED(c->y_bedoff, capn * 4);
             sa = SummaryArgs{}; sa.sets = up->want_summary ? SUM_ALL : 0; sa.probe = detect ? 1 : 0;
             sa.rows = rows; sa.ex = c->ex; sa.list = c->novel; sa.n_upd = cap; sa.n_upd_dev = T + T_UPD;
-            sa.upd = merged_view(c->mg.o_cand, c->mg.o_cov, c->mg.o_tid, c->mg.o_start, c->mg.o_end, c->mg.o_fs, c->mg.o_le, cap);
+            sa.upd = view(c->mg.o, DMerged{cap, cap});
             sa.ref = c->u_ref.as<int32_t>(); sa.anno_gene = c->anno.gene;
             sa.bar_cnt = c->y_barcnt.as<uint32_t>(); sa.bar_seg = c->y_barseg.as<uint32_t>(); sa.gene_bar = c->y_genebar.as<uint64_t>();
             sa.bed_cnt = c->y_bedcnt.as<uint32_t>(); sa.bed_off = c->y_bedoff.as<uint32_t>(); sa.counts = c->y_counts.as<uint32_t>();
@@ -610,20 +546,20 @@ int lrb_update_run(lrb_ctx *c, const lrb_update_params *up)
         }
         // ---- the one round trip: totals, error flags, class sizes, element count.  The class folds keep running on the
         // side stream underneath the summary sets; they are joined in front of the last copy of this stage.
-        uint8_t *hp = (uint8_t *)c->h_scalars.p;
-        CK(cudaMemcpyAsync(hp, c->scalars.p, T_SLOTS * 8 + 8, cudaMemcpyDeviceToHost, c->st));
-        CK(cudaMemcpyAsync(hp + 320, c->y_counts.p, 64, cudaMemcpyDeviceToHost, c->st));
-        CK(cudaMemcpyAsync(hp + 384, c->y_nelem.p, 16, cudaMemcpyDeviceToHost, c->st));
-        if (xl_exact) CK(cudaMemcpyAsync(hp + 400, c->xl_cnt.p, XL_NCNT * 4, cudaMemcpyDeviceToHost, c->st));
+        UpdateScalars *hs = c->h_scalars.as<UpdateScalars>();
+        CK(cudaMemcpyAsync(hs, c->scalars.p, T_SLOTS * 8 + 8, cudaMemcpyDeviceToHost, c->st));
+        CK(cudaMemcpyAsync(hs->counts, c->y_counts.p, 64, cudaMemcpyDeviceToHost, c->st));
+        CK(cudaMemcpyAsync(&hs->n_elem, c->y_nelem.p, 16, cudaMemcpyDeviceToHost, c->st));
+        if (xl_exact) CK(cudaMemcpyAsync(hs->xl, c->xl_cnt.p, XL_NCNT * 4, cudaMemcpyDeviceToHost, c->st));
         CK(cudaStreamSynchronize(c->st));
-        uint64_t t[T_SLOTS]; uint32_t e[2], xc[XL_NCNT] = {0};
-        memcpy(t, hp, sizeof t); memcpy(e, hp + T_SLOTS * 8, 8); memcpy(cnt16, hp + 320, 64); memcpy(&n_elem, hp + 384, 8); memcpy(&n_exon_elem, hp + 392, 8);
-        if (xl_exact) memcpy(xc, hp + 400, sizeof xc);
-        if (e[1] & 3u) {
+        uint64_t t[T_SLOTS]; uint32_t xc[XL_NCNT] = {0};
+        memcpy(t, hs->t, sizeof t); memcpy(cnt16, hs->counts, 64); n_elem = hs->n_elem; n_exon_elem = hs->n_exon_elem;
+        if (xl_exact) memcpy(xc, hs->xl, sizeof xc);
+        if (hs->err & 3u) {
             // the class folds may still be running on the side stream: they must be over before the caller can start another
             // stage on this context (they share its buffers and counters)
             if (up->want_summary && c->side_stream) cudaStreamSynchronize(c->st2);
-            if (e[1] & 2u) return fail(c, LRB_E_UNMAPPED, "unmapped record / empty exon chain in update/unique input (the reference aborts here, bam2gtf.c:95-100)");
+            if (hs->err & 2u) return fail(c, LRB_E_UNMAPPED, "unmapped record / empty exon chain in update/unique input (the reference aborts here, bam2gtf.c:95-100)");
             return fail(c, LRB_E_UNSORTED, "reads are not sorted by (tid,start) (update_gtf.c:41)");
         }
         n_novel = (int64_t)t[T_NOVEL]; c->n_known = (int64_t)t[T_KNOWN]; c->n_unrecog = (int64_t)t[T_UNREC];
@@ -643,9 +579,9 @@ int lrb_update_run(lrb_ctx *c, const lrb_update_params *up)
                 launch_xlocus_reset(c->mg.args, c->xl, c->st);
                 launch_merge_fold(c->mg.args, c->st);
                 launch_xlocus_detect(c->mg.args, c->xl, c->st);
-                CK(cudaMemcpyAsync(hp + 400, c->xl_cnt.p, XL_NCNT * 4, cudaMemcpyDeviceToHost, c->st));
+                CK(cudaMemcpyAsync(hs->xl, c->xl_cnt.p, XL_NCNT * 4, cudaMemcpyDeviceToHost, c->st));
                 CK(cudaStreamSynchronize(c->st));
-                memcpy(xc, hp + 400, sizeof xc);
+                memcpy(xc, hs->xl, sizeof xc);
             }
             if (xc[XL_OVERFLOW] || xc[XL_CHANGED]) {                 // more hits than the lists hold, or no fixed point in 32 rounds: the exact replay
                 if (up->want_summary && c->side_stream) CK(cudaStreamWaitEvent(c->st, c->ev_join, 0));
@@ -657,18 +593,18 @@ int lrb_update_run(lrb_ctx *c, const lrb_update_params *up)
             launch_merge_finish(c->mg.args, c->st);
             if (run_sets) { CK(cudaMemsetAsync(c->y_nelem.p, 0, 16, c->st)); launch_summary_count(sa, c->y_nelem.as<unsigned long long>(), c->st); }
             CK(cudaGetLastError());
-            CK(cudaMemcpyAsync(hp, c->scalars.p, T_SLOTS * 8 + 8, cudaMemcpyDeviceToHost, c->st));
-            CK(cudaMemcpyAsync(hp + 384, c->y_nelem.p, 16, cudaMemcpyDeviceToHost, c->st));
+            CK(cudaMemcpyAsync(hs, c->scalars.p, T_SLOTS * 8 + 8, cudaMemcpyDeviceToHost, c->st));
+            CK(cudaMemcpyAsync(&hs->n_elem, c->y_nelem.p, 16, cudaMemcpyDeviceToHost, c->st));
             CK(cudaStreamSynchronize(c->st));
-            memcpy(t, hp, sizeof t); memcpy(&n_elem, hp + 384, 8); memcpy(&n_exon_elem, hp + 392, 8);
+            memcpy(t, hs->t, sizeof t); n_elem = hs->n_elem; n_exon_elem = hs->n_exon_elem;
             c->mg.n_out = nu = (int64_t)t[T_UPD];
         }
         break;
     }
     if (n_novel < 0) continue;                                        // the marks did not settle: once more as ONE locus
-    if (n == 0) { if ((rc = setup_list(c, c->novel, c->n_row, c->n_lo, c->n_cnt, c->n_piece, 0))) return rc; c->mg.n_out = c->mg.n_loci = 0; tick(c, 2); tick(c, 3); }
+    if (n == 0) { if ((rc = setup_list(c, c->novel, c->novel_cols, 0))) return rc; c->mg.n_out = c->mg.n_loci = 0; tick(c, EV_LISTED); tick(c, EV_FOLDED); }
     c->novel.n = n_novel; c->novel.cap = std::max<int64_t>(cap, 0);
-    if (c->timing && n && fold_pass == 0) { CK(cudaStreamSynchronize(c->st)); cudaEventElapsedTime(&c->ms[LRB_T_K_FOLD], c->ev[10], c->ev[11]); }
+    if (c->timing && n && fold_pass == 0) { CK(cudaStreamSynchronize(c->st)); cudaEventElapsedTime(&c->ms[LRB_T_K_FOLD], c->ev[EV_FOLD0], c->ev[EV_FOLD1]); }
 
     // ---- summary sets (print_trans_summary, update_gtf.c:421-587) and / or the probe for pieces that meet another chromosome
     if (!(run_sets && n > 0)) break;
@@ -687,21 +623,21 @@ int lrb_update_run(lrb_ctx *c, const lrb_update_params *up)
     sa.tab.cap = capn; sa.tab.slots = c->h_khi.as<HashSlot>();
     // BED rows are the first occurrences of the exon set: at most one per counted element
     const size_t nb = (size_t)std::max<uint64_t>(n_elem, 1);
-    NEED(c->bd_tid, nb * 4); NEED(c->bd_s, nb * 4); NEED(c->bd_e, nb * 4); NEED(c->bd_sc, nb * 4); NEED(c->bd_ty, nb); NEED(c->bd_rv, nb);
-    sa.bed_tid = c->bd_tid.as<int32_t>(); sa.bed_start = c->bd_s.as<int32_t>(); sa.bed_end = c->bd_e.as<int32_t>(); sa.bed_score = c->bd_sc.as<int32_t>();
-    sa.bed_type = c->bd_ty.as<uint8_t>(); sa.bed_rev = c->bd_rv.as<uint8_t>();
+    if ((rc = ensure(c, c->bed, Extent{(int64_t)nb}))) return rc;
+    sa.bed_tid = c->bed.tid.as<int32_t>(); sa.bed_start = c->bed.start.as<int32_t>(); sa.bed_end = c->bed.end.as<int32_t>(); sa.bed_score = c->bed.score.as<int32_t>();
+    sa.bed_type = c->bed.type.as<uint8_t>(); sa.bed_rev = c->bed.is_rev.as<uint8_t>();
     if (c->want_kg_pairs && up->want_summary) { NEED(c->kg_pairs, (size_t)std::max<int64_t>(n_known_reads, 1) * 8); sa.kg_pairs = c->kg_pairs.as<int2>(); }
     CK(cudaMemsetAsync(c->y_counts.p, 0, 32, c->st));
     launch_summary_sets(sa, ca.cls, n, c->tile_state.as<uint64_t>(), (uint32_t *)(c->y_nelem.as<uint8_t>() + 16), T + T_BED, c->st,
                         c->sum_split ? c->st3 : c->st, c->ev_fork3, c->ev_join3);
     CK(cudaGetLastError());
     if (up->want_summary && c->side_stream) CK(cudaStreamWaitEvent(c->st, c->ev_join, 0));
-    uint8_t *hp = (uint8_t *)c->h_scalars.p;
-    CK(cudaMemcpyAsync(hp, T + T_BED, 8, cudaMemcpyDeviceToHost, c->st));
-    CK(cudaMemcpyAsync(hp + 64, c->y_counts.p, 48, cudaMemcpyDeviceToHost, c->st));
+    UpdateScalars *hs = c->h_scalars.as<UpdateScalars>();
+    CK(cudaMemcpyAsync(&hs->t[T_BED], T + T_BED, 8, cudaMemcpyDeviceToHost, c->st));
+    CK(cudaMemcpyAsync(hs->counts, c->y_counts.p, 48, cudaMemcpyDeviceToHost, c->st));
     CK(cudaStreamSynchronize(c->st));
-    uint64_t nbed; uint32_t cnt[12];
-    memcpy(&nbed, hp, 8); memcpy(cnt, hp + 64, 48);
+    const uint64_t nbed = hs->t[T_BED]; uint32_t cnt[12];
+    memcpy(cnt, hs->counts, 48);
     c->xlocus_seen = detect && (cnt[CNT_XLOCUS] != 0 || (up->ss_dis > 0 && cnt[CNT_PARTIAL] != 0));
     if (c->xlocus_seen && !single) { single = true; c->n_xlocus_replays++; continue; }       // replay the fold as one locus
     if (up->want_summary) {
@@ -716,14 +652,14 @@ int lrb_update_run(lrb_ctx *c, const lrb_update_params *up)
     }
     break;
     }   // fold_pass
-    tick(c, 4);
+    tick(c, EV_UPDATED);
     c->have_update = true; c->launches_last = total_launches() - l0;
     if (c->timing) {
         CK(cudaStreamSynchronize(c->st));
-        cudaEventElapsedTime(&c->ms[LRB_T_CLASSIFY], c->ev[0], c->ev[1]);
-        float lists = 0; cudaEventElapsedTime(&lists, c->ev[1], c->ev[2]);
-        cudaEventElapsedTime(&c->ms[LRB_T_MERGE], c->ev[2], c->ev[3]); c->ms[LRB_T_MERGE] += lists;
-        cudaEventElapsedTime(&c->ms[LRB_T_SUMMARY], c->ev[3], c->ev[4]);
+        cudaEventElapsedTime(&c->ms[LRB_T_CLASSIFY], c->ev[EV_BEGIN], c->ev[EV_CLASSIFIED]);
+        float lists = 0; cudaEventElapsedTime(&lists, c->ev[EV_CLASSIFIED], c->ev[EV_LISTED]);
+        cudaEventElapsedTime(&c->ms[LRB_T_MERGE], c->ev[EV_LISTED], c->ev[EV_FOLDED]); c->ms[LRB_T_MERGE] += lists;
+        cudaEventElapsedTime(&c->ms[LRB_T_SUMMARY], c->ev[EV_FOLDED], c->ev[EV_UPDATED]);
     }
     return LRB_OK;
 }
@@ -737,11 +673,11 @@ int lrb_unique_run(lrb_ctx *c, const lrb_update_params *up)
     DRows &rows = *c->cur; const int64_t n = rows.n;
     int rc;
     CK(cudaMemsetAsync(d_err(c), 0, 4, c->st));
-    tick(c, 0);
+    tick(c, EV_BEGIN);
     if (n) { rows_check_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->st>>>(rows, d_err(c), 1); CK(cudaGetLastError()); }
     uint32_t flags = 0;
     if ((rc = check_err_flags(c, &flags))) return rc;
-    if ((rc = setup_list(c, c->tmp_list, c->t_row, c->t_lo, c->t_cnt, c->t_piece, n))) return rc;
+    if ((rc = setup_list(c, c->tmp_list, c->tmp_cols, n))) return rc;
     launch_rows_as_list(rows, nullptr, n, c->tmp_list, c->st);
     // unique-gtf's input may be a concatenation of sorted samples (Snakefile:189-192).  The locus cuts (App. B.3) are only
     // proven for (tid,start)-sorted streams, so an unsorted list is folded as ONE locus: the back-scan of merge_trans is
@@ -757,9 +693,9 @@ int lrb_unique_run(lrb_ctx *c, const lrb_update_params *up)
         uint64_t t; if ((rc = read_totals(c, &t, 1))) return rc;
         c->n_shared = (int64_t)t;
     }
-    tick(c, 1);
+    tick(c, EV_END);
     c->have_unique = true; c->launches_last = total_launches() - l0;
-    if (c->timing) { CK(cudaStreamSynchronize(c->st)); cudaEventElapsedTime(&c->ms[LRB_T_MERGE], c->ev[0], c->ev[1]); }
+    if (c->timing) { CK(cudaStreamSynchronize(c->st)); cudaEventElapsedTime(&c->ms[LRB_T_MERGE], c->ev[EV_BEGIN], c->ev[EV_END]); }
     return LRB_OK;
 }
 
@@ -778,7 +714,7 @@ int lrb_rows_sort(lrb_ctx *c)
     const size_t nn = (size_t)n;
     NEED(c->s_key0, nn * 8); NEED(c->s_key1, nn * 8); NEED(c->s_idx0, nn * 4); NEED(c->s_idx1, nn * 4);
     NEED(c->s_hist, (size_t)256 * (size_t)lrbk::sort_tiles(n) * 4);
-    if ((rc = setup_rows(c, c->rows3, c->s_read, c->s_rtid, c->s_rs, c->s_re, c->s_rev, c->s_beg, c->s_n, n))) return rc;
+    if ((rc = setup_rows(c, c->rows3, c->rows3_cols, n))) return rc;
     unsigned long long *d_max = (unsigned long long *)(d_totals(c) + 3);
     CK(cudaMemsetAsync(d_max, 0, 8, c->st));
     launch_sort_keys(rows, c->have_batch ? c->b.flag : nullptr, c->s_key0.as<uint64_t>(), c->s_idx0.as<uint32_t>(), d_max, c->st);
@@ -815,13 +751,14 @@ int lrb_filter_fetch(lrb_ctx *c, lrb_filter_result *out)
     if (!c->have_filter) return fail(c, LRB_E_ARG, "lrb_filter_fetch: filter stage has not run");
     CK(cudaSetDevice(c->device));
     const size_t n = (size_t)c->b.n; int rc;
-    if ((rc = d2h(c, c->p[0], c->f_pass.as<uint8_t>(), n))) return rc;
-    if ((rc = d2h(c, c->p[1], c->f_score.as<int32_t>(), n))) return rc;
-    if ((rc = d2h(c, c->p[2], c->f_intron.as<int32_t>(), n))) return rc;
-    if ((rc = d2h(c, c->p[3], c->f_keep_idx.as<uint32_t>(), (size_t)c->n_keep))) return rc;
+    FilterOut &o = c->out_filter;
+    if ((rc = d2h(c, o.pass, c->f_pass.as<uint8_t>(), n))) return rc;
+    if ((rc = d2h(c, o.score, c->f_score.as<int32_t>(), n))) return rc;
+    if ((rc = d2h(c, o.intron, c->f_intron.as<int32_t>(), n))) return rc;
+    if ((rc = d2h(c, o.keep_idx, c->f_keep_idx.as<uint32_t>(), (size_t)c->n_keep))) return rc;
     CK(cudaStreamSynchronize(c->st));
-    out->n = c->b.n; out->pass = c->p[0].as<uint8_t>(); out->score = c->p[1].as<int32_t>(); out->intron_n = c->p[2].as<int32_t>();
-    out->n_keep = c->n_keep; out->keep_idx = c->p[3].as<uint32_t>();
+    out->n = c->b.n; out->pass = o.pass.as<uint8_t>(); out->score = o.score.as<int32_t>(); out->intron_n = o.intron.as<int32_t>();
+    out->n_keep = c->n_keep; out->keep_idx = o.keep_idx.as<uint32_t>();
     return LRB_OK;
 }
 
@@ -831,9 +768,9 @@ int lrb_filter_fetch_keep(lrb_ctx *c, int64_t *n_keep, const uint32_t **keep_idx
     if (!c->have_filter) return fail(c, LRB_E_ARG, "lrb_filter_fetch_keep: filter stage has not run");
     CK(cudaSetDevice(c->device));
     int rc;
-    if ((rc = d2h(c, c->p[3], c->f_keep_idx.as<uint32_t>(), (size_t)c->n_keep))) return rc;
+    if ((rc = d2h(c, c->out_filter.keep_idx, c->f_keep_idx.as<uint32_t>(), (size_t)c->n_keep))) return rc;
     CK(cudaStreamSynchronize(c->st));
-    *n_keep = c->n_keep; *keep_idx = c->p[3].as<uint32_t>();
+    *n_keep = c->n_keep; *keep_idx = c->out_filter.keep_idx.as<uint32_t>();
     return LRB_OK;
 }
 
@@ -846,23 +783,16 @@ __global__ void exon_gather_kernel(DRows rows, DExons ex, const uint32_t *__rest
     for (uint32_t j = 0; j < n; ++j) { es[o + j] = ex.es[b + j]; ee[o + j] = ex.ee[b + j]; if (with_flags) fl[o + j] = ex.flag[b + j]; }
 }
 
-static int fetch_exons(lrb_ctx *c, lrb_exon_result *out, bool with_flags, const uint8_t **flags_out, int pbase)
+static int fetch_exons(lrb_ctx *c, ExonsOut &o, lrb_exon_result *out, bool with_flags, const uint8_t **flags_out)
 {
     DRows &rows = *c->cur; const int64_t n = rows.n; int rc;
-    if ((rc = d2h(c, c->p[pbase + 0], rows.read_idx, (size_t)n))) return rc;
-    if ((rc = d2h(c, c->p[pbase + 1], rows.tid, (size_t)n))) return rc;
-    if ((rc = d2h(c, c->p[pbase + 2], rows.is_rev, (size_t)n))) return rc;
-    int64_t ne = 0;
-    NEEDP(c->p[pbase + 3], ((size_t)n + 1) * 4);
-    if (c->rows_compact) {
-        ne = c->ex.n;
-        if (n) CK(cudaMemcpyAsync(c->p[pbase + 3].p, rows.ex_beg, (size_t)n * 4, cudaMemcpyDeviceToHost, c->st));
-        if ((rc = d2h(c, c->p[pbase + 4], c->ex.es, (size_t)ne))) return rc;
-        if ((rc = d2h(c, c->p[pbase + 5], c->ex.ee, (size_t)ne))) return rc;
-        if (with_flags && (rc = d2h(c, c->p[pbase + 6], c->ex.flag, (size_t)ne))) return rc;
-        CK(cudaStreamSynchronize(c->st));
-        c->p[pbase + 3].as<uint32_t>()[n] = (uint32_t)ne;
-    } else {
+    if ((rc = d2h(c, o.read_idx, rows.read_idx, (size_t)n))) return rc;
+    if ((rc = d2h(c, o.tid, rows.tid, (size_t)n))) return rc;
+    if ((rc = d2h(c, o.is_rev, rows.is_rev, (size_t)n))) return rc;
+    int64_t ne = c->ex.n;
+    int32_t *es = c->ex.es, *ee = c->ex.ee; uint8_t *fl = c->ex.flag; uint32_t *off = rows.ex_beg;
+    NEEDP(o.off, ((size_t)n + 1) * 4);
+    if (!c->rows_compact) {
         // exclusive scan of ex_n -> offsets, then gather into scratch (the summary hash buffers are free at fetch time)
         if ((rc = ensure_tiles(c, n))) return rc;
         NEED(c->u_sub, ((size_t)n + 1) * 4);
@@ -871,22 +801,22 @@ static int fetch_exons(lrb_ctx *c, lrb_exon_result *out, bool with_flags, const 
         ne = n ? (int64_t)t : 0;
         const size_t k = (size_t)std::max<int64_t>(ne, 1);
         NEED(c->y_barcnt, k * 4); NEED(c->y_barseg, k * 4); NEED(c->y_bedcnt, k);
+        es = c->y_barcnt.as<int32_t>(); ee = c->y_barseg.as<int32_t>(); fl = c->y_bedcnt.as<uint8_t>(); off = c->u_sub.as<uint32_t>();
         if (n) {
-            exon_gather_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->st>>>(rows, c->ex, c->u_sub.as<uint32_t>(), c->y_barcnt.as<int32_t>(),
-                                                                                 c->y_barseg.as<int32_t>(), c->y_bedcnt.as<uint8_t>(), with_flags ? 1 : 0);
+            exon_gather_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->st>>>(rows, c->ex, off, es, ee, fl, with_flags ? 1 : 0);
             CK(cudaGetLastError());
-            CK(cudaMemcpyAsync(c->p[pbase + 3].p, c->u_sub.p, (size_t)n * 4, cudaMemcpyDeviceToHost, c->st));
         }
-        if ((rc = d2h(c, c->p[pbase + 4], c->y_barcnt.as<int32_t>(), (size_t)ne))) return rc;
-        if ((rc = d2h(c, c->p[pbase + 5], c->y_barseg.as<int32_t>(), (size_t)ne))) return rc;
-        if (with_flags && (rc = d2h(c, c->p[pbase + 6], c->y_bedcnt.as<uint8_t>(), (size_t)ne))) return rc;
-        CK(cudaStreamSynchronize(c->st));
-        c->p[pbase + 3].as<uint32_t>()[n] = (uint32_t)ne;
     }
-    out->n_reads = n; out->read_idx = c->have_batch ? c->p[pbase + 0].as<uint32_t>() : nullptr; out->tid = c->p[pbase + 1].as<int32_t>();
-    out->is_rev = c->p[pbase + 2].as<uint8_t>(); out->exon_off = c->p[pbase + 3].as<uint32_t>();
-    out->exon_start = c->p[pbase + 4].as<int32_t>(); out->exon_end = c->p[pbase + 5].as<int32_t>();
-    if (flags_out) *flags_out = with_flags ? c->p[pbase + 6].as<uint8_t>() : nullptr;
+    if (n) CK(cudaMemcpyAsync(o.off.p, off, (size_t)n * 4, cudaMemcpyDeviceToHost, c->st));
+    if ((rc = d2h(c, o.es, es, (size_t)ne))) return rc;
+    if ((rc = d2h(c, o.ee, ee, (size_t)ne))) return rc;
+    if (with_flags && (rc = d2h(c, o.flag, fl, (size_t)ne))) return rc;
+    CK(cudaStreamSynchronize(c->st));
+    o.off.as<uint32_t>()[n] = (uint32_t)ne;
+    out->n_reads = n; out->read_idx = c->have_batch ? o.read_idx.as<uint32_t>() : nullptr; out->tid = o.tid.as<int32_t>();
+    out->is_rev = o.is_rev.as<uint8_t>(); out->exon_off = o.off.as<uint32_t>();
+    out->exon_start = o.es.as<int32_t>(); out->exon_end = o.ee.as<int32_t>();
+    if (flags_out) *flags_out = with_flags ? o.flag.as<uint8_t>() : nullptr;
     return LRB_OK;
 }
 
@@ -895,18 +825,14 @@ int lrb_exon_fetch(lrb_ctx *c, lrb_exon_result *out)
     if (!c || !out) return LRB_E_ARG;
     if (!c->have_exons) return fail(c, LRB_E_ARG, "lrb_exon_fetch: exon stage has not run");
     CK(cudaSetDevice(c->device));
-    return fetch_exons(c, out, false, nullptr, 4);
+    return fetch_exons(c, c->out_exons, out, false, nullptr);
 }
 
-static int fetch_merged(lrb_ctx *c, MergeBufs &m, lrb_merged_list *o, int pbase)
+static lrb_merged_list merged_result(const MergedCols<PBuf> &h, int64_t n)
 {
-    const size_t n = (size_t)m.n_out; int rc;
-    Buf *src[] = {&m.o_cand, &m.o_cov, &m.o_tid, &m.o_start, &m.o_end, &m.o_fs, &m.o_le};
-    for (int i = 0; i < 7; ++i) if ((rc = d2h(c, c->p[pbase + i], src[i]->as<uint32_t>(), n))) return rc;
-    o->n = m.n_out; o->cand = c->p[pbase].as<uint32_t>(); o->cov = c->p[pbase + 1].as<int32_t>(); o->t_tid = c->p[pbase + 2].as<int32_t>();
-    o->t_start = c->p[pbase + 3].as<int32_t>(); o->t_end = c->p[pbase + 4].as<int32_t>(); o->first_start = c->p[pbase + 5].as<int32_t>();
-    o->last_end = c->p[pbase + 6].as<int32_t>();
-    return LRB_OK;
+    lrb_merged_list o; o.n = n; o.cand = h.cand.as<uint32_t>(); o.cov = h.cov.as<int32_t>(); o.t_tid = h.tid.as<int32_t>(); o.t_start = h.start.as<int32_t>();
+    o.t_end = h.end.as<int32_t>(); o.first_start = h.fs.as<int32_t>(); o.last_end = h.le.as<int32_t>();
+    return o;
 }
 
 int lrb_update_fetch(lrb_ctx *c, lrb_update_result *out)
@@ -916,30 +842,22 @@ int lrb_update_fetch(lrb_ctx *c, lrb_update_result *out)
     CK(cudaSetDevice(c->device));
     memset(out, 0, sizeof *out);
     int rc; const int64_t n = c->cur->n;
-    if ((rc = fetch_exons(c, &out->ex, true, &out->exon_flag, 4))) return rc;
-    if ((rc = d2h(c, c->p[11], c->u_cls.as<uint32_t>(), (size_t)n))) return rc;
-    if ((rc = d2h(c, c->p[12], c->u_ref.as<int32_t>(), (size_t)n))) return rc;
-    if ((rc = d2h(c, c->p[13], c->u_known.as<uint32_t>(), (size_t)c->n_known))) return rc;
-    if ((rc = d2h(c, c->p[14], c->u_unrecog.as<uint32_t>(), (size_t)c->n_unrecog))) return rc;
-    if ((rc = d2h(c, c->p[15], c->novel.row, (size_t)c->novel.n))) return rc;
-    if ((rc = d2h(c, c->p[16], c->novel.lo, (size_t)c->novel.n))) return rc;
-    if ((rc = d2h(c, c->p[17], c->novel.cnt, (size_t)c->novel.n))) return rc;
-    if ((rc = d2h(c, c->p[18], c->novel.piece, (size_t)c->novel.n))) return rc;
-    if ((rc = fetch_merged(c, c->mg, &out->updated, 19))) return rc;
-    if ((rc = d2h(c, c->p[26], c->bd_tid.as<int32_t>(), (size_t)c->n_bed))) return rc;
-    if ((rc = d2h(c, c->p[27], c->bd_s.as<int32_t>(), (size_t)c->n_bed))) return rc;
-    if ((rc = d2h(c, c->p[28], c->bd_e.as<int32_t>(), (size_t)c->n_bed))) return rc;
-    if ((rc = d2h(c, c->p[29], c->bd_sc.as<int32_t>(), (size_t)c->n_bed))) return rc;
-    if ((rc = d2h(c, c->p[30], c->bd_ty.as<uint8_t>(), (size_t)c->n_bed))) return rc;
-    if ((rc = d2h(c, c->p[31], c->bd_rv.as<uint8_t>(), (size_t)c->n_bed))) return rc;
+    UpdateOut &o = c->out_update;
+    if ((rc = fetch_exons(c, o.ex, &out->ex, true, &out->exon_flag))) return rc;
+    if ((rc = d2h(c, o.cls, c->u_cls.as<uint32_t>(), (size_t)n))) return rc;
+    if ((rc = d2h(c, o.ref, c->u_ref.as<int32_t>(), (size_t)n))) return rc;
+    if ((rc = d2h(c, o.known, c->u_known.as<uint32_t>(), (size_t)c->n_known))) return rc;
+    if ((rc = d2h(c, o.unrecog, c->u_unrecog.as<uint32_t>(), (size_t)c->n_unrecog))) return rc;
+    if ((rc = copy(c, o.novel, c->novel_cols, Extent{c->novel.n}, cudaMemcpyDeviceToHost))) return rc;
+    if ((rc = copy(c, o.updated, c->mg.o, Extent{c->mg.n_out}, cudaMemcpyDeviceToHost))) return rc;
+    if ((rc = copy(c, o.bed, c->bed, Extent{c->n_bed}, cudaMemcpyDeviceToHost))) return rc;
     CK(cudaStreamSynchronize(c->st));
-    out->cls = c->p[11].as<uint32_t>(); out->ref_anno = c->p[12].as<int32_t>();
-    out->n_known = c->n_known; out->known_idx = c->p[13].as<uint32_t>(); out->n_unrecog = c->n_unrecog; out->unrecog_idx = c->p[14].as<uint32_t>();
-    out->novel.n = c->novel.n; out->novel.read = c->p[15].as<uint32_t>(); out->novel.exon_lo = c->p[16].as<uint32_t>();
-    out->novel.exon_n = c->p[17].as<uint32_t>(); out->novel.piece = c->p[18].as<int32_t>();
+    out->cls = o.cls.as<uint32_t>(); out->ref_anno = o.ref.as<int32_t>();
+    out->n_known = c->n_known; out->known_idx = o.known.as<uint32_t>(); out->n_unrecog = c->n_unrecog; out->unrecog_idx = o.unrecog.as<uint32_t>();
+    out->novel.n = c->novel.n; out->novel.read = o.novel.row.as<uint32_t>(); out->novel.exon_lo = o.novel.lo.as<uint32_t>();
+    out->novel.exon_n = o.novel.cnt.as<uint32_t>(); out->novel.piece = o.novel.piece.as<int32_t>();
+    out->updated = merged_result(o.updated, c->mg.n_out); out->bed = view(o.bed, lrb_bed_list{c->n_bed});
     memcpy(out->summary, c->summary, sizeof c->summary);
-    out->bed.n = c->n_bed; out->bed.tid = c->p[26].as<int32_t>(); out->bed.start = c->p[27].as<int32_t>(); out->bed.end = c->p[28].as<int32_t>();
-    out->bed.score = c->p[29].as<int32_t>(); out->bed.type = c->p[30].as<uint8_t>(); out->bed.is_rev = c->p[31].as<uint8_t>();
     return LRB_OK;
 }
 
@@ -977,32 +895,32 @@ __global__ void tab_exons_kernel(TabArgs a)
 
 }  // extern "C" (reopened below)
 
-// updated_T as a self-contained table in device memory (c->tb_*): rows + exon offsets + exon pools (+ the exon flag bytes for the
+// updated_T as a self-contained table in device memory (c->tab): rows + exon offsets + exon pools (+ the exon flag bytes for the
 // gather root of a multi-GPU run).  One host round trip (the exon total).
 int lrbk::build_update_table(lrb_ctx *c, int64_t *n_exon_out, bool with_flags)
 {
     int rc;
-    const int64_t nu = c->mg.n_out; const size_t k = (size_t)std::max<int64_t>(nu, 1);
-    Buf *b4[] = {&c->tb_name, &c->tb_piece, &c->tb_ttid, &c->tb_tstart, &c->tb_tend, &c->tb_etid, &c->tb_cov, &c->tb_ref, &c->tb_cnt};
-    for (Buf *b : b4) NEED(*b, k * 4);
-    NEED(c->tb_trev, k); NEED(c->tb_erev, k); NEED(c->tb_off, (k + 1) * 4);
+    const int64_t nu = c->mg.n_out, k = std::max<int64_t>(nu, 1);
+    TableCols<Buf> &tb = c->tab;
+    if ((rc = ensure(c, tb, Extent{k, -1}))) return rc;                // the exon columns once their total is known
+    NEED(c->tb_cnt, (size_t)k * 4);
     TabArgs a{};
     a.rows = *c->cur; a.ex = c->ex; a.list = c->novel; a.ref = c->u_ref.as<int32_t>(); a.rows_have_read_idx = c->have_batch ? 1 : 0;
-    a.upd = merged_view(c->mg.o_cand, c->mg.o_cov, c->mg.o_tid, c->mg.o_start, c->mg.o_end, c->mg.o_fs, c->mg.o_le, nu);
-    a.name_idx = c->tb_name.as<uint32_t>(); a.piece = c->tb_piece.as<int32_t>(); a.t_tid = c->tb_ttid.as<int32_t>(); a.t_start = c->tb_tstart.as<int32_t>();
-    a.t_end = c->tb_tend.as<int32_t>(); a.e_tid = c->tb_etid.as<int32_t>(); a.cov = c->tb_cov.as<int32_t>(); a.ref_out = c->tb_ref.as<int32_t>();
-    a.t_rev = c->tb_trev.as<uint8_t>(); a.e_rev = c->tb_erev.as<uint8_t>(); a.cnt = c->tb_cnt.as<uint32_t>(); a.off = c->tb_off.as<uint32_t>();
+    a.upd = view(c->mg.o, DMerged{nu, nu});
+    a.name_idx = tb.name_idx.as<uint32_t>(); a.piece = tb.piece.as<int32_t>(); a.t_tid = tb.t_tid.as<int32_t>(); a.t_start = tb.t_start.as<int32_t>();
+    a.t_end = tb.t_end.as<int32_t>(); a.e_tid = tb.e_tid.as<int32_t>(); a.cov = tb.cov.as<int32_t>(); a.ref_out = tb.ref_anno.as<int32_t>();
+    a.t_rev = tb.t_rev.as<uint8_t>(); a.e_rev = tb.e_rev.as<uint8_t>(); a.cnt = c->tb_cnt.as<uint32_t>(); a.off = tb.exon_off.as<uint32_t>();
     int64_t ne = 0;
     if (nu) {
         if ((rc = ensure_tiles(c, nu))) return rc;
         tab_rows_kernel<<<(unsigned)((nu + 255) / 256), 256, 0, c->st>>>(a);
-        launch_scan_sum_u32(a.cnt, c->tb_off.as<uint32_t>(), nu, c->tile_state.as<uint64_t>(), d_ticket(c), d_totals(c), c->st);
+        launch_scan_sum_u32(a.cnt, tb.exon_off.as<uint32_t>(), nu, c->tile_state.as<uint64_t>(), d_ticket(c), d_totals(c), c->st);
         CK(cudaGetLastError());
         uint64_t t; if ((rc = read_totals(c, &t, 1))) return rc;
         ne = (int64_t)t;
-        NEED(c->tb_es, (size_t)std::max<int64_t>(ne, 1) * 4); NEED(c->tb_ee, (size_t)std::max<int64_t>(ne, 1) * 4);
+        if ((rc = ensure(c, tb, Extent{k, ne}))) return rc;
         if (with_flags) NEED(c->tb_flag, (size_t)std::max<int64_t>(ne, 1));
-        a.es = c->tb_es.as<int32_t>(); a.ee = c->tb_ee.as<int32_t>(); a.fl = with_flags ? c->tb_flag.as<uint8_t>() : nullptr;
+        a.es = tb.exon_start.as<int32_t>(); a.ee = tb.exon_end.as<int32_t>(); a.fl = with_flags ? c->tb_flag.as<uint8_t>() : nullptr;
         tab_exons_kernel<<<(unsigned)((nu + 255) / 256), 256, 0, c->st>>>(a);
         CK(cudaGetLastError());
     }
@@ -1019,41 +937,20 @@ int lrb_update_fetch_table(lrb_ctx *c, lrb_trans_table *tab, lrb_bed_list *bed, 
     CK(cudaSetDevice(c->device));
     int rc;
     if (summary) memcpy(summary, c->summary, sizeof c->summary);
+    UpdateOut &o = c->out_update;
     if (bed) {
         if (!c->last_up.want_summary) return fail(c, LRB_E_ARG, "lrb_update_fetch_table: BED rows need want_summary");
-        if ((rc = d2h(c, c->p[26], c->bd_tid.as<int32_t>(), (size_t)c->n_bed))) return rc;
-        if ((rc = d2h(c, c->p[27], c->bd_s.as<int32_t>(), (size_t)c->n_bed))) return rc;
-        if ((rc = d2h(c, c->p[28], c->bd_e.as<int32_t>(), (size_t)c->n_bed))) return rc;
-        if ((rc = d2h(c, c->p[29], c->bd_sc.as<int32_t>(), (size_t)c->n_bed))) return rc;
-        if ((rc = d2h(c, c->p[30], c->bd_ty.as<uint8_t>(), (size_t)c->n_bed))) return rc;
-        if ((rc = d2h(c, c->p[31], c->bd_rv.as<uint8_t>(), (size_t)c->n_bed))) return rc;
-        bed->n = c->n_bed; bed->tid = c->p[26].as<int32_t>(); bed->start = c->p[27].as<int32_t>(); bed->end = c->p[28].as<int32_t>();
-        bed->score = c->p[29].as<int32_t>(); bed->type = c->p[30].as<uint8_t>(); bed->is_rev = c->p[31].as<uint8_t>();
+        if ((rc = copy(c, o.bed, c->bed, Extent{c->n_bed}, cudaMemcpyDeviceToHost))) return rc;
+        *bed = view(o.bed, lrb_bed_list{c->n_bed});
     }
     if (tab) {
         int64_t ne = 0;
         if ((rc = lrbk::build_update_table(c, &ne, false))) return rc;
-        const int64_t nu = c->mg.n_out; const size_t n = (size_t)nu;
-        if ((rc = d2h(c, c->p[32], c->tb_name.as<uint32_t>(), n))) return rc;
-        if ((rc = d2h(c, c->p[33], c->tb_piece.as<int32_t>(), n))) return rc;
-        if ((rc = d2h(c, c->p[34], c->tb_ttid.as<int32_t>(), n))) return rc;
-        if ((rc = d2h(c, c->p[35], c->tb_tstart.as<int32_t>(), n))) return rc;
-        if ((rc = d2h(c, c->p[36], c->tb_tend.as<int32_t>(), n))) return rc;
-        if ((rc = d2h(c, c->p[37], c->tb_trev.as<uint8_t>(), n))) return rc;
-        if ((rc = d2h(c, c->p[38], c->tb_etid.as<int32_t>(), n))) return rc;
-        if ((rc = d2h(c, c->p[39], c->tb_erev.as<uint8_t>(), n))) return rc;
-        if ((rc = d2h(c, c->p[40], c->tb_cov.as<int32_t>(), n))) return rc;
-        if ((rc = d2h(c, c->p[41], c->tb_ref.as<int32_t>(), n))) return rc;
-        NEEDP(c->p[42], (n + 1) * 4);
-        if (n) CK(cudaMemcpyAsync(c->p[42].p, c->tb_off.p, n * 4, cudaMemcpyDeviceToHost, c->st));
-        if ((rc = d2h(c, c->p[43], c->tb_es.as<int32_t>(), (size_t)ne))) return rc;
-        if ((rc = d2h(c, c->p[44], c->tb_ee.as<int32_t>(), (size_t)ne))) return rc;
+        const int64_t nu = c->mg.n_out;
+        if ((rc = copy(c, o.tab, c->tab, Extent{nu, ne}, cudaMemcpyDeviceToHost))) return rc;
         CK(cudaStreamSynchronize(c->st));
-        c->p[42].as<uint32_t>()[n] = (uint32_t)ne;
-        tab->n = nu; tab->name_idx = c->p[32].as<uint32_t>(); tab->piece = c->p[33].as<int32_t>(); tab->t_tid = c->p[34].as<int32_t>();
-        tab->t_start = c->p[35].as<int32_t>(); tab->t_end = c->p[36].as<int32_t>(); tab->t_rev = c->p[37].as<uint8_t>(); tab->e_tid = c->p[38].as<int32_t>();
-        tab->e_rev = c->p[39].as<uint8_t>(); tab->cov = c->p[40].as<int32_t>(); tab->ref_anno = c->p[41].as<int32_t>(); tab->exon_off = c->p[42].as<uint32_t>();
-        tab->exon_start = c->p[43].as<int32_t>(); tab->exon_end = c->p[44].as<int32_t>();
+        o.tab.exon_off.as<uint32_t>()[nu] = (uint32_t)ne;
+        *tab = view(o.tab, lrb_trans_table{nu});
     } else CK(cudaStreamSynchronize(c->st));
     return LRB_OK;
 }
@@ -1065,11 +962,13 @@ int lrb_unique_fetch(lrb_ctx *c, lrb_unique_result *out)
     CK(cudaSetDevice(c->device));
     memset(out, 0, sizeof *out);
     int rc;
-    if ((rc = fetch_exons(c, &out->ex, false, nullptr, 4))) return rc;
-    if ((rc = fetch_merged(c, c->mg, &out->uniq, 19))) return rc;
-    if ((rc = d2h(c, c->p[26], c->q_shared.as<uint32_t>(), (size_t)c->n_shared))) return rc;
+    UniqueOut &o = c->out_unique;
+    if ((rc = fetch_exons(c, o.ex, &out->ex, false, nullptr))) return rc;
+    if ((rc = copy(c, o.uniq, c->mg.o, Extent{c->mg.n_out}, cudaMemcpyDeviceToHost))) return rc;
+    if ((rc = d2h(c, o.shared, c->q_shared.as<uint32_t>(), (size_t)c->n_shared))) return rc;
     CK(cudaStreamSynchronize(c->st));
-    out->n_shared = c->n_shared; out->shared_idx = c->p[26].as<uint32_t>();
+    out->uniq = merged_result(o.uniq, c->mg.n_out);
+    out->n_shared = c->n_shared; out->shared_idx = o.shared.as<uint32_t>();
     return LRB_OK;
 }
 

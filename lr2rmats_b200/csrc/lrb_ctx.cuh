@@ -5,6 +5,7 @@
 #include <cstdint>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include "lrb_common.cuh"
 #include "lrb_kernels.cuh"
 #include "lrb_summary.cuh"
@@ -13,40 +14,144 @@ namespace lrbk {
 
 extern int64_t g_launches_update, g_launches_summary, g_launches_sort;
 
-struct Buf {                                        // device buffer, grow-only, contents not preserved on growth
+// grow-only buffer, contents not preserved on growth: device memory (Buf) or pinned host memory (PBuf), freed with its owner
+template <cudaError_t (*Alloc)(void **, size_t), cudaError_t (*Free)(void *)> struct Mem {
     void *p = nullptr; size_t cap = 0;
+    Mem() = default;
+    Mem(const Mem &) = delete; Mem &operator=(const Mem &) = delete;
+    ~Mem() { release(); }
     bool ensure(size_t bytes)
     {
         if (bytes <= cap) return true;
-        if (p) cudaFree(p);
+        if (p) Free(p);
         size_t nc = bytes + bytes / 4 + 256;
-        if (cudaMalloc(&p, nc) != cudaSuccess) { p = nullptr; cap = 0; cudaGetLastError(); return false; }
+        if (Alloc(&p, nc) != cudaSuccess) { p = nullptr; cap = 0; cudaGetLastError(); return false; }
         cap = nc; return true;
     }
-    void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+    void release() { if (p) Free(p); p = nullptr; cap = 0; }
     template <class T> T *as() const { return (T *)p; }
 };
-struct PBuf {                                       // pinned host buffer
-    void *p = nullptr; size_t cap = 0;
-    bool ensure(size_t bytes)
+using Buf = Mem<cudaMalloc, cudaFree>;
+using PBuf = Mem<cudaMallocHost, cudaFreeHost>;
+
+// ---- tables: one struct per table states its columns once.  XCols<Buf> holds the table in HBM, XCols<PBuf> its pinned copy,
+// XCols<const void *> the host arrays of an upload.  cols(f, g...) calls f(per, element size, the column of each g) per column.
+// The columns are named like the pointers of the table's kernel view or result struct, which view() points at them.
+enum Per {
+    ROW,                                            // one entry per row
+    ROW1,                                           // n + 1 entries (offsets given by the host)
+    OFFS,                                           // n + 1 exon offsets of which n are built on the device: the one past the end,
+                                                    // the exon total, is written by whoever receives the table
+    EXON                                            // one entry per exon (per entry of the table's second count)
+};
+struct Extent {
+    int64_t n = 0, ne = 0;                          // rows, exons; ne < 0: exon columns are left alone (not known yet)
+    int64_t held(Per p) const { return p == ROW ? n : p == EXON ? ne : n + 1; }
+    int64_t moved(Per p) const { return p == ROW1 ? n + 1 : p == EXON ? ne : n; }
+};
+
+template <class B> struct BatchCols {               // DBatch; the CIGAR ops are its "exons"
+    B tid, pos, l_qseq, nm, flag, xs, qhash, cigar_off, cigar;
+    template <class F, class... G> static void cols(F &&f, G &...g)
     {
-        if (bytes <= cap) return true;
-        if (p) cudaFreeHost(p);
-        size_t nc = bytes + bytes / 4 + 256;
-        if (cudaMallocHost(&p, nc) != cudaSuccess) { p = nullptr; cap = 0; cudaGetLastError(); return false; }
-        cap = nc; return true;
+        f(ROW, 4, g.tid...); f(ROW, 4, g.pos...); f(ROW, 4, g.l_qseq...); f(ROW, 4, g.nm...); f(ROW, 2, g.flag...); f(ROW, 1, g.xs...);
+        f(ROW, 8, g.qhash...); f(ROW1, 8, g.cigar_off...); f(EXON, 4, g.cigar...);
     }
-    void release() { if (p) cudaFreeHost(p); p = nullptr; cap = 0; }
-    template <class T> T *as() const { return (T *)p; }
 };
+template <class B> struct AnnoCols {                // DAnno
+    B tid, start, end, gene, is_rev, exon_off, es, ee, pmax_key, mono;
+    template <class F, class... G> static void cols(F &&f, G &...g)
+    {
+        f(ROW, 4, g.tid...); f(ROW, 4, g.start...); f(ROW, 4, g.end...); f(ROW, 4, g.gene...); f(ROW, 1, g.is_rev...); f(ROW1, 4, g.exon_off...);
+        f(EXON, 4, g.es...); f(EXON, 4, g.ee...); f(ROW, 8, g.pmax_key...); f(ROW, 1, g.mono...);
+    }
+};
+template <class B> struct SjCols {                  // DSj
+    B tid, don, acc, cnt_u, cnt_m, pmax_key, don_key;
+    template <class F, class... G> static void cols(F &&f, G &...g)
+    {
+        f(ROW, 4, g.tid...); f(ROW, 4, g.don...); f(ROW, 4, g.acc...); f(ROW, 4, g.cnt_u...); f(ROW, 4, g.cnt_m...); f(ROW, 8, g.pmax_key...); f(ROW, 8, g.don_key...);
+    }
+};
+template <class B> struct RmCols {                  // DRmIndex; rows: the per-tid groups, exons: their entries
+    B g_tid, g_off, start, pmax_end;
+    template <class F, class... G> static void cols(F &&f, G &...g) { f(ROW, 4, g.g_tid...); f(ROW1, 4, g.g_off...); f(EXON, 4, g.start...); f(EXON, 4, g.pmax_end...); }
+};
+template <class B> struct RowsCols {                // DRows
+    B read_idx, tid, start, end, is_rev, ex_beg, ex_n;
+    template <class F, class... G> static void cols(F &&f, G &...g)
+    {
+        f(ROW, 4, g.read_idx...); f(ROW, 4, g.tid...); f(ROW, 4, g.start...); f(ROW, 4, g.end...); f(ROW, 1, g.is_rev...); f(ROW, 4, g.ex_beg...); f(ROW, 4, g.ex_n...);
+    }
+};
+template <class B> struct ListCols {                // DTransList
+    B row, lo, cnt, piece;
+    template <class F, class... G> static void cols(F &&f, G &...g) { f(ROW, 4, g.row...); f(ROW, 4, g.lo...); f(ROW, 4, g.cnt...); f(ROW, 4, g.piece...); }
+};
+template <class B> struct MergedCols {              // DMerged
+    B cand, cov, tid, start, end, fs, le;
+    template <class F, class... G> static void cols(F &&f, G &...g)
+    {
+        f(ROW, 4, g.cand...); f(ROW, 4, g.cov...); f(ROW, 4, g.tid...); f(ROW, 4, g.start...); f(ROW, 4, g.end...); f(ROW, 4, g.fs...); f(ROW, 4, g.le...);
+    }
+};
+template <class B> struct CandCols {                // CandSoA
+    B tid, start, end, rev, n, fs, le, gbeg, hash, j0, sig;
+    template <class F, class... G> static void cols(F &&f, G &...g)
+    {
+        f(ROW, 4, g.tid...); f(ROW, 4, g.start...); f(ROW, 4, g.end...); f(ROW, 4, g.rev...); f(ROW, 4, g.n...); f(ROW, 4, g.fs...); f(ROW, 4, g.le...);
+        f(ROW, 4, g.gbeg...); f(ROW, 8, g.hash...); f(ROW, 8, g.j0...); f(ROW, 8, g.sig...);
+    }
+};
+template <class B> struct TableCols {               // lrb_trans_table: updated_T as a self-contained table
+    B name_idx, piece, t_tid, t_start, t_end, t_rev, e_tid, e_rev, cov, ref_anno, exon_off, exon_start, exon_end;
+    template <class F, class... G> static void cols(F &&f, G &...g)
+    {
+        f(ROW, 4, g.name_idx...); f(ROW, 4, g.piece...); f(ROW, 4, g.t_tid...); f(ROW, 4, g.t_start...); f(ROW, 4, g.t_end...); f(ROW, 1, g.t_rev...);
+        f(ROW, 4, g.e_tid...); f(ROW, 1, g.e_rev...); f(ROW, 4, g.cov...); f(ROW, 4, g.ref_anno...); f(OFFS, 4, g.exon_off...);
+        f(EXON, 4, g.exon_start...); f(EXON, 4, g.exon_end...);
+    }
+};
+template <class B> struct BedCols {                 // lrb_bed_list
+    B tid, start, end, score, type, is_rev;
+    template <class F, class... G> static void cols(F &&f, G &...g)
+    {
+        f(ROW, 4, g.tid...); f(ROW, 4, g.start...); f(ROW, 4, g.end...); f(ROW, 4, g.score...); f(ROW, 1, g.type...); f(ROW, 1, g.is_rev...);
+    }
+};
+template <class B> struct JuncCols {                // lrb_sj: the bam2sj output
+    B tid, don, acc, uniq_c, multi_c;
+    template <class F, class... G> static void cols(F &&f, G &...g) { f(ROW, 4, g.tid...); f(ROW, 4, g.don...); f(ROW, 4, g.acc...); f(ROW, 4, g.uniq_c...); f(ROW, 4, g.multi_c...); }
+};
+
+// v (a kernel view or a result struct) with its pointers at the columns of g; its counts are the caller's
+template <class G, class V> V view(const G &g, V v)
+{
+    G::cols([](Per, size_t, auto &ptr, const auto &col) { ptr = (std::remove_reference_t<decltype(ptr)>)col.p; }, v, g);
+    return v;
+}
+
+// ---- pinned results: one set per result kind, so that a fetch of one kind leaves the results of the others intact
+struct ExonsOut { PBuf read_idx, tid, is_rev, off, es, ee, flag; };    // lrb_exon_result (+ the exon flags of an update result)
+struct FilterOut { PBuf pass, score, intron, keep_idx; };
+struct UpdateOut {                                  // lrb_update_fetch, lrb_update_fetch_table
+    ExonsOut ex; PBuf cls, ref, known, unrecog; ListCols<PBuf> novel; MergedCols<PBuf> updated; BedCols<PBuf> bed; TableCols<PBuf> tab;
+};
+struct UniqueOut { ExonsOut ex; MergedCols<PBuf> uniq; PBuf shared; };
 
 struct MergeBufs {                                  // scratch + output of one merge fold
     Buf keys, head, locus_start, locus_cnt, dropped, rep, lstart, evmask, samemask, hard, desc, relsym, ckey, cmin, cord, clist, crow, fb_list, fb_cnt;
-    Buf w_cand, w_cov, w_tid, w_start, w_end, w_fs, w_le;
-    Buf o_cand, o_cov, o_tid, o_start, o_end, o_fs, o_le;
-    Buf c_tid, c_start, c_end, c_rev, c_n, c_fs, c_le, c_gbeg, c_hash, c_j0, c_sig;
+    MergedCols<Buf> w, o;                           // work list, survivors
+    CandCols<Buf> cd;
     int64_t n_out = 0, n_loci = 0;
     MergeArgs args;                                 // of the last fold (refolds of the split-piece rounds reuse them)
+};
+
+// timing events (ev[]): the marks of the stage that runs, then the two kernels timed on their own
+enum {
+    EV_BEGIN = 0, EV_END = 1,                                           // filter, exon, pipeline, unique
+    EV_CLASSIFIED = 1, EV_LISTED = 2, EV_FOLDED = 3, EV_UPDATED = 4,    // update
+    EV_SCAN0 = 8, EV_SCAN1, EV_FOLD0, EV_FOLD1, EV_COUNT
 };
 
 struct MultiState;                                  // lrb_multi.cu
@@ -65,45 +170,43 @@ struct lrb_ctx {
     cudaStream_t st3 = nullptr; cudaEvent_t ev_fork3 = nullptr, ev_join3 = nullptr; bool sum_split = true;   // exon chain of the summary sets
     // tables
     DAnno anno; DSj sj; DRmIndex rm;
-    Buf a_tid, a_start, a_end, a_gene, a_rev, a_off, a_es, a_ee, a_pmax, a_mono;
-    Buf s_tid, s_don, s_acc, s_u, s_m, s_pmax, s_dkey;
-    Buf r_gtid, r_goff, r_start, r_pmax;
+    lrbk::AnnoCols<Buf> anno_cols; lrbk::SjCols<Buf> sj_cols; lrbk::RmCols<Buf> rm_cols;
     // batch
-    DBatch b; Buf b_tid, b_pos, b_lq, b_nm, b_flag, b_xs, b_qh, b_coff, b_cig;
+    DBatch b; lrbk::BatchCols<Buf> batch_cols;
     bool have_batch = false;
     // filter
     Buf f_pass, f_score, f_intron, f_keep_row_mask, f_keep_rec_mask, f_keep_idx, f_keep_rows;
     int64_t n_pass = 0, n_keep = 0; bool have_filter = false;
     // rows + exons
     DRows rows, rows2, rows3; DRows *cur = nullptr; DExons ex;      // rows3: the coordinate-sorted copy made by lrb_rows_sort
-    Buf r_read, r_tid, r_rs, r_re, r_rev, r_beg, r_n, r_nonmono;
-    Buf q_read, q_tid, q_rs, q_re, q_rev, q_beg, q_n;
-    Buf s_read, s_rtid, s_rs, s_re, s_rev, s_beg, s_n, s_key0, s_key1, s_idx0, s_idx1, s_hist;   // lrb_rows_sort
+    lrbk::RowsCols<Buf> rows_cols, rows2_cols, rows3_cols; Buf r_nonmono;
+    Buf s_key0, s_key1, s_idx0, s_idx1, s_hist;                      // lrb_rows_sort
     Buf e_s, e_e, e_f;
     bool have_exons = false, rows_compact = false;
     // update
-    Buf u_cls, u_ref, u_nnovel, u_noff, u_mk, u_mu, u_ck, u_cr, u_cu, u_cn, u_known, u_unrecog, u_sub;
-    DTransList novel; Buf n_row, n_lo, n_cnt, n_piece;
-    DTransList tmp_list; Buf t_row, t_lo, t_cnt, t_piece;
+    Buf u_cls, u_ref, u_nnovel, u_noff, u_mk, u_ck, u_known, u_unrecog, u_sub;
+    DTransList novel; lrbk::ListCols<Buf> novel_cols;
+    DTransList tmp_list; lrbk::ListCols<Buf> tmp_cols;
     MergeBufs mg, mg2;
     int64_t n_known = 0, n_unrecog = 0, novel_cap_hint = 0; bool have_update = false, have_unique = false;
     int32_t summary[LRB_S_COUNT];
     bool force_single_fold = false, test_small_novel_cap = false, xlocus_seen = false, want_kg_pairs = false; int64_t n_xlocus_replays = 0, n_xlocus_pieces = 0, n_kg_pairs = 0; Buf kg_pairs;
     Buf xl_key, xl_min, xl_max, xl_cnt, xl_forced; lrbk::XlArgs xl;      // split pieces that meet another chromosome (xl_* kernels)
     // summary
-    Buf h_khi, h_klo, h_min, h_score, y_barcnt, y_barseg, y_genebar, y_bedcnt, y_bedoff, y_counts, y_nelem;
-    Buf bd_tid, bd_s, bd_e, bd_sc, bd_ty, bd_rv; int64_t n_bed = 0;
+    Buf h_khi, y_barcnt, y_barseg, y_genebar, y_bedcnt, y_bedoff, y_counts, y_nelem;
+    lrbk::BedCols<Buf> bed; int64_t n_bed = 0;
+    // updated_T as a table (build_update_table); the exon flags only for the gather root, tb_cnt is scratch
+    lrbk::TableCols<Buf> tab; Buf tb_flag, tb_cnt;
     // bam2sj
-    Buf j_cnt, j_off, j_uq, j_tid, j_don, j_acc, j_u, j_head, j_hpos, jo_tid, jo_don, jo_acc, jo_u, jo_m;
+    Buf j_cnt, j_off, j_uq, j_tid, j_don, j_acc, j_u, j_head, j_hpos; lrbk::JuncCols<Buf> junc;
     // unique
     Buf q_shared; int64_t n_shared = 0;
     // look-back state, small device scalars and their pinned mirror
     Buf tile_state, tile_state2, scalars; PBuf h_scalars;
-    // pinned result buffers
-    PBuf p[48];
-    Buf tb_name, tb_piece, tb_ttid, tb_tstart, tb_tend, tb_trev, tb_etid, tb_erev, tb_cov, tb_ref, tb_cnt, tb_off, tb_es, tb_ee, tb_flag;
+    // pinned results, one set per kind
+    lrbk::FilterOut out_filter; lrbk::ExonsOut out_exons; lrbk::UpdateOut out_update; lrbk::UniqueOut out_unique; lrbk::JuncCols<PBuf> out_junc; PBuf out_perm;
     // timing
-    bool timing = false; cudaEvent_t ev[12]; cudaEvent_t marks[8]; float ms[LRB_T_COUNT]; int64_t launches0 = 0, launches_last = 0;
+    bool timing = false; cudaEvent_t ev[lrbk::EV_COUNT]; cudaEvent_t marks[8]; float ms[LRB_T_COUNT]; int64_t launches0 = 0, launches_last = 0;
     lrb_update_params last_up;
 };
 
@@ -127,6 +230,15 @@ inline uint64_t *d_totals(lrb_ctx *c) { return c->scalars.as<uint64_t>(); }
 inline uint32_t *d_ticket(lrb_ctx *c) { return (uint32_t *)(c->scalars.as<uint64_t>() + T_SLOTS); }
 inline uint32_t *d_err(lrb_ctx *c) { return d_ticket(c) + 1; }
 inline uint32_t *d_ticket2(lrb_ctx *c) { return d_ticket(c) + 2; }          // ticket of the side stream
+
+// the update stage's pinned round trip (h_scalars, 512 bytes): the device scalars, then the counters it brings back with them
+struct UpdateScalars {
+    uint64_t t[T_SLOTS]; uint32_t ticket, err;      // d_totals, d_ticket, d_err
+    uint32_t counts[16];                            // y_counts
+    uint64_t n_elem, n_exon_elem;                   // y_nelem
+    uint32_t xl[XL_NCNT];                           // xl_cnt
+};
+static_assert(sizeof(UpdateScalars) <= 512, "h_scalars holds 512 bytes");
 
 inline int read_totals(lrb_ctx *c, uint64_t *out, int n)
 {
@@ -156,6 +268,35 @@ template <class T> int d2h(lrb_ctx *c, PBuf &dst, const T *src, size_t n)
     NEEDP(dst, std::max<size_t>(n, 1) * sizeof(T));
     if (n) CK(cudaMemcpyAsync(dst.p, src, n * sizeof(T), cudaMemcpyDeviceToHost, c->st));
     return LRB_OK;
+}
+
+// f(per, element size, columns...) over the columns of g, gs... until one returns an error
+template <class G, class F, class... Gs> int each_col(F &&f, G &g, Gs &...gs)
+{
+    int rc = LRB_OK;
+    G::cols([&](Per p, size_t esz, auto &...col) { if (rc == LRB_OK) rc = f(p, esz, col...); }, g, gs...);
+    return rc;
+}
+// every column of g (device or pinned) sized for e, at least one entry each
+template <class G> int ensure(lrb_ctx *c, G &g, Extent e)
+{
+    return each_col([&](Per p, size_t esz, auto &b) {
+        const int64_t k = e.held(p);
+        if (k >= 0 && !b.ensure(std::max<int64_t>(k, 1) * esz)) return fail(c, LRB_E_NOMEM, "allocation failed for a table of " + std::to_string(e.n) + " rows");
+        return LRB_OK;
+    }, g);
+}
+// the columns of src -> those of dst, sized for e first: host arrays -> HBM (an upload) or HBM -> pinned (a fetch, which leaves
+// an OFFS column's last entry to the caller)
+inline const void *addr(const void *p) { return p; }
+inline const void *addr(const Buf &b) { return b.p; }
+template <class D, class S> int copy(lrb_ctx *c, D &dst, S &src, Extent e, cudaMemcpyKind kind)
+{
+    if (int rc = ensure(c, dst, e)) return rc;
+    return each_col([&](Per p, size_t esz, auto &d, const auto &s) {
+        if (e.moved(p)) CK(cudaMemcpyAsync(d.p, addr(s), (size_t)e.moved(p) * esz, kind, c->st));
+        return LRB_OK;
+    }, dst, src);
 }
 
 }  // namespace lrbk

@@ -64,12 +64,11 @@ struct MultiState {
     NcclApi *api = nullptr; ncclComm_t comm = nullptr; int rank = 0, n_ranks = 1;
     Buf meta_dev, shard_end_dev, flags_dev; PBuf meta_host;
     // gathered on the root
-    Buf g_name, g_piece, g_ttid, g_tstart, g_tend, g_trev, g_etid, g_erev, g_cov, g_ref, g_off, g_es, g_ee, g_flag;
-    Buf g_bd_tid, g_bd_s, g_bd_e, g_bd_sc, g_bd_ty, g_bd_rv, g_kg;
+    TableCols<Buf> g; Buf g_flag; BedCols<Buf> g_bed; Buf g_kg;
     Buf v_ident, v_zeros, v_cnt, v_fs, v_le;          // the gathered table in the shape the set kernels read
     Buf tab, y_barcnt, y_barseg, y_genebar, y_bedcnt, y_bedoff, y_counts, y_nelem, tiles, xs_pl, xs_hx, xs_cnt;
     int64_t n = 0, n_exon = 0, n_bed = 0; int32_t summary[LRB_S_COUNT]; bool have = false, daj_recomputed = false;
-    PBuf p[24];
+    TableCols<PBuf> out_tab; BedCols<PBuf> out_bed;  // lrb_gather_fetch
     float ms_gather = 0, ms_merge = 0; cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
 };
 
@@ -78,15 +77,8 @@ void multi_release(lrb_ctx *c)
     MultiState *m = c->multi;
     if (!m) return;
     if (m->comm && m->api) m->api->CommDestroy(m->comm);
-    Buf *bufs[] = {&m->meta_dev, &m->shard_end_dev, &m->flags_dev, &m->g_name, &m->g_piece, &m->g_ttid, &m->g_tstart, &m->g_tend, &m->g_trev, &m->g_etid, &m->g_erev,
-                   &m->g_cov, &m->g_ref, &m->g_off, &m->g_es, &m->g_ee, &m->g_flag, &m->g_bd_tid, &m->g_bd_s, &m->g_bd_e, &m->g_bd_sc, &m->g_bd_ty, &m->g_bd_rv, &m->g_kg,
-                   &m->v_ident, &m->v_zeros, &m->v_cnt, &m->v_fs, &m->v_le, &m->tab, &m->y_barcnt, &m->y_barseg, &m->y_genebar, &m->y_bedcnt, &m->y_bedoff, &m->y_counts,
-                   &m->y_nelem, &m->tiles, &m->xs_pl, &m->xs_hx, &m->xs_cnt};
-    for (Buf *b : bufs) b->release();
-    m->meta_host.release();
-    for (PBuf &p : m->p) p.release();
     for (cudaEvent_t &e : m->ev) if (e) cudaEventDestroy(e);
-    delete m; c->multi = nullptr;
+    delete m; c->multi = nullptr;                   // frees its buffers
 }
 
 #define NK(call)                                                                                                           \
@@ -178,35 +170,24 @@ int lrb_tables_broadcast(lrb_ctx *c, int root, const lrb_anno *anno, const lrb_a
     CK(cudaMemcpyAsync(hd, m->meta_dev.p, 5 * 8, cudaMemcpyDeviceToHost, c->st));
     CK(cudaStreamSynchronize(c->st));
     const int64_t na = hd[0], nae = hd[1], ns = hd[2], ng = hd[3], nr = hd[4];
-    struct Item { Buf *b; size_t bytes; };
-    std::vector<Item> items;
-    if (na) {
-        items = {{&c->a_tid, (size_t)na * 4}, {&c->a_start, (size_t)na * 4}, {&c->a_end, (size_t)na * 4}, {&c->a_gene, (size_t)na * 4}, {&c->a_rev, (size_t)na},
-                 {&c->a_off, ((size_t)na + 1) * 4}, {&c->a_es, (size_t)nae * 4}, {&c->a_ee, (size_t)nae * 4}, {&c->a_pmax, (size_t)na * 8}, {&c->a_mono, (size_t)na}};
-    }
-    if (ns) for (Item it : {Item{&c->s_tid, (size_t)ns * 4}, Item{&c->s_don, (size_t)ns * 4}, Item{&c->s_acc, (size_t)ns * 4}, Item{&c->s_u, (size_t)ns * 4},
-                            Item{&c->s_m, (size_t)ns * 4}, Item{&c->s_pmax, (size_t)ns * 8}, Item{&c->s_dkey, (size_t)ns * 8}}) items.push_back(it);
-    if (nr) for (Item it : {Item{&c->r_gtid, (size_t)ng * 4}, Item{&c->r_goff, ((size_t)ng + 1) * 4}, Item{&c->r_start, (size_t)nr * 4}, Item{&c->r_pmax, (size_t)nr * 4}}) items.push_back(it);
-    if (!is_root) for (Item &it : items) NEED(*it.b, std::max<size_t>(it.bytes, 1));
+    const Extent e_anno{na, nae}, e_sj{ns}, e_rm{ng, nr};
+    if (!is_root && ((na && (rc = ensure(c, c->anno_cols, e_anno))) || (ns && (rc = ensure(c, c->sj_cols, e_sj))) || (nr && (rc = ensure(c, c->rm_cols, e_rm)))))
+        return rc;
+    auto bcast = [&](Extent e) {
+        return [&, e](Per p, size_t esz, Buf &b) {
+            const size_t bytes = (size_t)e.moved(p) * esz;
+            if (bytes) NK(m->api->Broadcast(b.p, b.p, bytes, ncclChar, root, m->comm, c->st));
+            return LRB_OK;
+        };
+    };
     NK(m->api->GroupStart());
-    for (Item &it : items) if (it.bytes) NK(m->api->Broadcast(it.b->p, it.b->p, it.bytes, ncclChar, root, m->comm, c->st));
+    if ((na && (rc = each_col(bcast(e_anno), c->anno_cols))) || (ns && (rc = each_col(bcast(e_sj), c->sj_cols))) || (nr && (rc = each_col(bcast(e_rm), c->rm_cols))))
+        return rc;
     NK(m->api->GroupEnd());
     if (!is_root) {
-        c->anno = DAnno{}; c->sj = DSj{}; c->rm = DRmIndex{};
-        if (na) {
-            c->anno.n = (int32_t)na; c->anno.n_exon = nae; c->anno.tid = c->a_tid.as<int32_t>(); c->anno.start = c->a_start.as<int32_t>();
-            c->anno.end = c->a_end.as<int32_t>(); c->anno.gene = c->a_gene.as<int32_t>(); c->anno.is_rev = c->a_rev.as<uint8_t>();
-            c->anno.exon_off = c->a_off.as<uint32_t>(); c->anno.es = c->a_es.as<int32_t>(); c->anno.ee = c->a_ee.as<int32_t>();
-            c->anno.pmax_key = c->a_pmax.as<uint64_t>(); c->anno.mono = c->a_mono.as<uint8_t>();
-        }
-        if (ns) {
-            c->sj.n = ns; c->sj.tid = c->s_tid.as<int32_t>(); c->sj.don = c->s_don.as<int32_t>(); c->sj.acc = c->s_acc.as<int32_t>();
-            c->sj.cnt_u = c->s_u.as<int32_t>(); c->sj.cnt_m = c->s_m.as<int32_t>(); c->sj.pmax_key = c->s_pmax.as<uint64_t>(); c->sj.don_key = c->s_dkey.as<uint64_t>();
-        }
-        if (nr) {
-            c->rm.n_groups = (int32_t)ng; c->rm.n = (int32_t)nr; c->rm.g_tid = c->r_gtid.as<int32_t>(); c->rm.g_off = c->r_goff.as<int32_t>();
-            c->rm.start = c->r_start.as<int32_t>(); c->rm.pmax_end = c->r_pmax.as<int32_t>();
-        }
+        c->anno = na ? view(c->anno_cols, DAnno{(int32_t)na, nae}) : DAnno{};
+        c->sj = ns ? view(c->sj_cols, DSj{ns}) : DSj{};
+        c->rm = nr ? view(c->rm_cols, DRmIndex{(int32_t)ng, (int32_t)nr}) : DRmIndex{};
     }
     CK(cudaStreamSynchronize(c->st));
     return LRB_OK;
@@ -248,35 +229,35 @@ int lrb_update_gather(lrb_ctx *c, int64_t name_base)
     }
     const int64_t N = o_n[R], NE = o_e[R], NB = o_b[R], NK_ = o_k[R];
     if (NE >= ((int64_t)1 << 32) || N >= ((int64_t)1 << 31)) return fail(c, LRB_E_ARG, "lrb_update_gather: gathered table exceeds 2^32 exons / 2^31 transcripts");
-    // ---- gatherv: every rank sends its arrays, the root receives each at the shard's offset
-    struct Arr { Buf *src; Buf *dst; int esz; const std::vector<int64_t> *off; int64_t extra; };
+    // ---- gatherv: every rank sends its part of each column, the root receives each part at the shard's offset and then copies its own
     if (root) {
-        const size_t n1 = (size_t)std::max<int64_t>(N, 1), e1 = (size_t)std::max<int64_t>(NE, 1), b1 = (size_t)std::max<int64_t>(NB, 1), k1 = (size_t)std::max<int64_t>(NK_, 1);
-        for (Buf *b : {&m->g_name, &m->g_piece, &m->g_ttid, &m->g_tstart, &m->g_tend, &m->g_etid, &m->g_cov, &m->g_ref}) NEED(*b, n1 * 4);
-        NEED(m->g_off, (n1 + 1) * 4); NEED(m->g_trev, n1); NEED(m->g_erev, n1);
-        NEED(m->g_es, e1 * 4); NEED(m->g_ee, e1 * 4); NEED(m->g_flag, e1);
-        for (Buf *b : {&m->g_bd_tid, &m->g_bd_s, &m->g_bd_e, &m->g_bd_sc}) NEED(*b, b1 * 4);
-        NEED(m->g_bd_ty, b1); NEED(m->g_bd_rv, b1); NEED(m->g_kg, k1 * 8);
+        const int64_t n1 = std::max<int64_t>(N, 1), e1 = std::max<int64_t>(NE, 1);
+        if ((rc = ensure(c, m->g, Extent{n1, e1})) || (rc = ensure(c, m->g_bed, Extent{std::max<int64_t>(NB, 1)}))) return rc;
+        NEED(m->g_flag, (size_t)e1); NEED(m->g_kg, (size_t)std::max<int64_t>(NK_, 1) * 8);
     }
-    const Arr arrs[] = {
-        {&c->tb_name, &m->g_name, 4, &o_n}, {&c->tb_piece, &m->g_piece, 4, &o_n}, {&c->tb_ttid, &m->g_ttid, 4, &o_n}, {&c->tb_tstart, &m->g_tstart, 4, &o_n},
-        {&c->tb_tend, &m->g_tend, 4, &o_n}, {&c->tb_trev, &m->g_trev, 1, &o_n}, {&c->tb_etid, &m->g_etid, 4, &o_n}, {&c->tb_erev, &m->g_erev, 1, &o_n},
-        {&c->tb_cov, &m->g_cov, 4, &o_n}, {&c->tb_ref, &m->g_ref, 4, &o_n}, {&c->tb_off, &m->g_off, 4, &o_n},
-        {&c->tb_es, &m->g_es, 4, &o_e}, {&c->tb_ee, &m->g_ee, 4, &o_e}, {&c->tb_flag, &m->g_flag, 1, &o_e},
-        {&c->bd_tid, &m->g_bd_tid, 4, &o_b}, {&c->bd_s, &m->g_bd_s, 4, &o_b}, {&c->bd_e, &m->g_bd_e, 4, &o_b}, {&c->bd_sc, &m->g_bd_sc, 4, &o_b},
-        {&c->bd_ty, &m->g_bd_ty, 1, &o_b}, {&c->bd_rv, &m->g_bd_rv, 1, &o_b}, {&c->kg_pairs, &m->g_kg, 8, &o_k},
+    auto parts = [&](bool own, const std::vector<int64_t> &row_off) {
+        return [&, own, rows = &row_off](Per p, size_t esz, Buf &src, Buf &dst) {
+            const std::vector<int64_t> &off = p == EXON ? o_e : *rows;            // an OFFS column moves n entries: the root rebases them
+            if (own) { if (off[1]) CK(cudaMemcpyAsync(dst.p, src.p, (size_t)off[1] * esz, cudaMemcpyDeviceToDevice, c->st)); }
+            else if (!root) { const int64_t cnt = off[me + 1] - off[me]; if (cnt) NK(m->api->Send(src.p, (size_t)cnt * esz, ncclChar, 0, m->comm, c->st)); }
+            else for (int r = 1; r < R; ++r) {
+                const int64_t cnt = off[r + 1] - off[r];
+                if (cnt) NK(m->api->Recv((char *)dst.p + (size_t)off[r] * esz, (size_t)cnt * esz, ncclChar, r, m->comm, c->st));
+            }
+            return LRB_OK;
+        };
+    };
+    auto gather = [&](bool own) {
+        int rc2;
+        if ((rc2 = each_col(parts(own, o_n), c->tab, m->g)) || (rc2 = parts(own, o_n)(EXON, 1, c->tb_flag, m->g_flag)) ||
+            (rc2 = each_col(parts(own, o_b), c->bed, m->g_bed)))
+            return rc2;
+        return parts(own, o_k)(ROW, 8, c->kg_pairs, m->g_kg);
     };
     NK(m->api->GroupStart());
-    for (const Arr &a : arrs) {
-        const std::vector<int64_t> &off = *a.off;
-        if (!root) { const int64_t cnt = off[me + 1] - off[me]; if (cnt) NK(m->api->Send(a.src->p, (size_t)cnt * a.esz, ncclChar, 0, m->comm, c->st)); }
-        else for (int r = 1; r < R; ++r) {
-            const int64_t cnt = off[r + 1] - off[r];
-            if (cnt) NK(m->api->Recv((char *)a.dst->p + (size_t)off[r] * a.esz, (size_t)cnt * a.esz, ncclChar, r, m->comm, c->st));
-        }
-    }
+    if ((rc = gather(false))) return rc;
     NK(m->api->GroupEnd());
-    if (root) for (const Arr &a : arrs) { const int64_t cnt = (*a.off)[1]; if (cnt) CK(cudaMemcpyAsync(a.dst->p, a.src->p, (size_t)cnt * a.esz, cudaMemcpyDeviceToDevice, c->st)); }
+    if (root && (rc = gather(true))) return rc;
     CK(cudaEventRecord(m->ev[1], c->st));
     if (!root) {
         CK(cudaStreamSynchronize(c->st));
@@ -287,7 +268,7 @@ int lrb_update_gather(lrb_ctx *c, int64_t name_base)
     // ---- canonical merge on the root
     RebaseArgs ra{}; ra.n = R;
     for (int r = 0; r < R; ++r) { ra.row_end[r] = o_n[r + 1]; ra.exon_base[r] = o_e[r]; ra.name_base[r] = mh[(size_t)r * META_WORDS + M_NAME_BASE]; }
-    rebase_kernel<<<(unsigned)(N / 256 + 1), 256, 0, c->st>>>(ra, m->g_off.as<uint32_t>(), m->g_name.as<uint32_t>(), N, NE);
+    rebase_kernel<<<(unsigned)(N / 256 + 1), 256, 0, c->st>>>(ra, m->g.exon_off.as<uint32_t>(), m->g.name_idx.as<uint32_t>(), N, NE);
     CK(cudaGetLastError());
     m->n = N; m->n_exon = NE; m->n_bed = want_summary ? NB : 0; m->daj_recomputed = false;
     memset(m->summary, 0, sizeof m->summary);
@@ -303,18 +284,19 @@ int lrb_update_gather(lrb_ctx *c, int64_t name_base)
         for (Buf *b : {&m->v_ident, &m->v_zeros, &m->v_cnt, &m->v_fs, &m->v_le}) NEED(*b, n1 * 4);
         NEED(m->y_barcnt, n1 * 16); NEED(m->y_barseg, n1 * 16); NEED(m->y_genebar, n1 * 8); NEED(m->y_bedcnt, n1 * 4); NEED(m->y_bedoff, n1 * 4);
         NEED(m->y_counts, 64); NEED(m->y_nelem, 64); NEED(m->tiles, (size_t)(N / 256 + 1024) * 8 * 6);
-        GatheredTable gt; gt.n = N; gt.n_exon = NE; gt.exon_off = m->g_off.as<uint32_t>(); gt.es = m->g_es.as<int32_t>(); gt.ee = m->g_ee.as<int32_t>();
+        const TableCols<Buf> &g = m->g;
+        GatheredTable gt; gt.n = N; gt.n_exon = NE; gt.exon_off = g.exon_off.as<uint32_t>(); gt.es = g.exon_start.as<int32_t>(); gt.ee = g.exon_end.as<int32_t>();
         launch_table_view(gt, m->v_ident.as<uint32_t>(), m->v_zeros.as<uint32_t>(), m->v_cnt.as<uint32_t>(), m->v_fs.as<int32_t>(), m->v_le.as<int32_t>(), c->st);
         std::vector<int64_t> ends(o_n.begin() + 1, o_n.end());
         memcpy(mh + (size_t)MAX_RANKS * META_WORDS - MAX_RANKS, ends.data(), (size_t)R * 8);            // pinned staging behind the metas
         CK(cudaMemcpyAsync(m->shard_end_dev.p, mh + (size_t)MAX_RANKS * META_WORDS - MAX_RANKS, (size_t)R * 8, cudaMemcpyHostToDevice, c->st));
         SummaryArgs sa{};
-        sa.rows.n = N; sa.rows.tid = m->g_etid.as<int32_t>(); sa.rows.is_rev = m->g_erev.as<uint8_t>(); sa.rows.ex_beg = m->g_off.as<uint32_t>(); sa.rows.ex_n = m->v_cnt.as<uint32_t>();
-        sa.ex.n = NE; sa.ex.es = m->g_es.as<int32_t>(); sa.ex.ee = m->g_ee.as<int32_t>(); sa.ex.flag = m->g_flag.as<uint8_t>();
-        sa.list.n = N; sa.list.row = m->v_ident.as<uint32_t>(); sa.list.lo = m->v_zeros.as<uint32_t>(); sa.list.cnt = m->v_cnt.as<uint32_t>(); sa.list.piece = m->g_piece.as<int32_t>();
-        sa.upd.n = N; sa.upd.cand = m->v_ident.as<uint32_t>(); sa.upd.cov = m->g_cov.as<int32_t>(); sa.upd.tid = m->g_ttid.as<int32_t>(); sa.upd.start = m->g_tstart.as<int32_t>();
-        sa.upd.end = m->g_tend.as<int32_t>(); sa.upd.fs = m->v_fs.as<int32_t>(); sa.upd.le = m->v_le.as<int32_t>();
-        sa.ref = m->g_ref.as<int32_t>(); sa.anno_gene = c->anno.gene; sa.n_upd = N;
+        sa.rows.n = N; sa.rows.tid = g.e_tid.as<int32_t>(); sa.rows.is_rev = g.e_rev.as<uint8_t>(); sa.rows.ex_beg = g.exon_off.as<uint32_t>(); sa.rows.ex_n = m->v_cnt.as<uint32_t>();
+        sa.ex.n = NE; sa.ex.es = g.exon_start.as<int32_t>(); sa.ex.ee = g.exon_end.as<int32_t>(); sa.ex.flag = m->g_flag.as<uint8_t>();
+        sa.list.n = N; sa.list.row = m->v_ident.as<uint32_t>(); sa.list.lo = m->v_zeros.as<uint32_t>(); sa.list.cnt = m->v_cnt.as<uint32_t>(); sa.list.piece = g.piece.as<int32_t>();
+        sa.upd.n = N; sa.upd.cand = m->v_ident.as<uint32_t>(); sa.upd.cov = g.cov.as<int32_t>(); sa.upd.tid = g.t_tid.as<int32_t>(); sa.upd.start = g.t_start.as<int32_t>();
+        sa.upd.end = g.t_end.as<int32_t>(); sa.upd.fs = m->v_fs.as<int32_t>(); sa.upd.le = m->v_le.as<int32_t>();
+        sa.ref = g.ref_anno.as<int32_t>(); sa.anno_gene = c->anno.gene; sa.n_upd = N;
         sa.bar_cnt = m->y_barcnt.as<uint32_t>(); sa.bar_seg = m->y_barseg.as<uint32_t>(); sa.gene_bar = m->y_genebar.as<uint64_t>();
         sa.bed_cnt = m->y_bedcnt.as<uint32_t>(); sa.bed_off = m->y_bedoff.as<uint32_t>(); sa.counts = m->y_counts.as<uint32_t>();
         sa.shard_end = m->shard_end_dev.as<int64_t>(); sa.n_shards = R; sa.probe = detect ? 1 : 0;
@@ -379,38 +361,12 @@ int lrb_gather_fetch(lrb_ctx *c, lrb_trans_table *tab, lrb_bed_list *bed, int32_
     }
     if (!m->have) return fail(c, LRB_E_ARG, "lrb_gather_fetch: lrb_update_gather has not run");
     if (summary) memcpy(summary, m->summary, sizeof m->summary);
-    const size_t n = (size_t)m->n, ne = (size_t)m->n_exon, nb = (size_t)m->n_bed;
-    auto dl = [&](PBuf &dst, const Buf &src, size_t bytes) -> int {
-        NEEDP(dst, std::max<size_t>(bytes, 1));
-        if (bytes) CK(cudaMemcpyAsync(dst.p, src.p, bytes, cudaMemcpyDeviceToHost, c->st));
-        return LRB_OK;
-    };
     int rc;
-    if (tab) {
-        const Buf *src[] = {&m->g_name, &m->g_piece, &m->g_ttid, &m->g_tstart, &m->g_tend, &m->g_trev, &m->g_etid, &m->g_erev, &m->g_cov, &m->g_ref};
-        const int esz[] = {4, 4, 4, 4, 4, 1, 4, 1, 4, 4};
-        for (int i = 0; i < 10; ++i) if ((rc = dl(m->p[i], *src[i], n * esz[i]))) return rc;
-        if ((rc = dl(m->p[10], m->g_off, (n + 1) * 4))) return rc;
-        if ((rc = dl(m->p[11], m->g_es, ne * 4))) return rc;
-        if ((rc = dl(m->p[12], m->g_ee, ne * 4))) return rc;
-    }
-    if (bed) {
-        const Buf *src[] = {&m->g_bd_tid, &m->g_bd_s, &m->g_bd_e, &m->g_bd_sc, &m->g_bd_ty, &m->g_bd_rv};
-        const int esz[] = {4, 4, 4, 4, 1, 1};
-        for (int i = 0; i < 6; ++i) if ((rc = dl(m->p[13 + i], *src[i], nb * esz[i]))) return rc;
-    }
+    if (tab && (rc = copy(c, m->out_tab, m->g, Extent{m->n, m->n_exon}, cudaMemcpyDeviceToHost))) return rc;
+    if (bed && (rc = copy(c, m->out_bed, m->g_bed, Extent{m->n_bed}, cudaMemcpyDeviceToHost))) return rc;
     CK(cudaStreamSynchronize(c->st));
-    if (tab) {
-        if (n == 0) m->p[10].as<uint32_t>()[0] = 0;
-        tab->n = m->n; tab->name_idx = m->p[0].as<uint32_t>(); tab->piece = m->p[1].as<int32_t>(); tab->t_tid = m->p[2].as<int32_t>(); tab->t_start = m->p[3].as<int32_t>();
-        tab->t_end = m->p[4].as<int32_t>(); tab->t_rev = m->p[5].as<uint8_t>(); tab->e_tid = m->p[6].as<int32_t>(); tab->e_rev = m->p[7].as<uint8_t>();
-        tab->cov = m->p[8].as<int32_t>(); tab->ref_anno = m->p[9].as<int32_t>(); tab->exon_off = m->p[10].as<uint32_t>();
-        tab->exon_start = m->p[11].as<int32_t>(); tab->exon_end = m->p[12].as<int32_t>();
-    }
-    if (bed) {
-        bed->n = m->n_bed; bed->tid = m->p[13].as<int32_t>(); bed->start = m->p[14].as<int32_t>(); bed->end = m->p[15].as<int32_t>(); bed->score = m->p[16].as<int32_t>();
-        bed->type = m->p[17].as<uint8_t>(); bed->is_rev = m->p[18].as<uint8_t>();
-    }
+    if (tab) { m->out_tab.exon_off.as<uint32_t>()[m->n] = (uint32_t)m->n_exon; *tab = view(m->out_tab, lrb_trans_table{m->n}); }
+    if (bed) *bed = view(m->out_bed, lrb_bed_list{m->n_bed});
     return LRB_OK;
 }
 

@@ -130,16 +130,15 @@ extern "C" int lrb_bam2sj(lrb_ctx *c, const lrb_batch *b, const uint8_t *is_uniq
         CK(cudaGetLastError());
         uint64_t t; if ((rc = read_totals(c, &t, 1))) return rc;
         nd = (int64_t)t;
-        const size_t d = (size_t)nd;
-        Buf *o[] = {&c->jo_tid, &c->jo_don, &c->jo_acc, &c->jo_u, &c->jo_m};
-        for (Buf *x : o) NEED(*x, d * 4);
+        JuncCols<Buf> &o = c->junc;
+        if ((rc = ensure(c, o, Extent{nd}))) return rc;
         sj_reduce_kernel<<<(unsigned)((nd + 255) / 256), 256, 0, c->st>>>(a.j_tid, a.j_don, a.j_acc, a.j_uniq, v[cur], c->j_hpos.as<uint32_t>(), nd, nj,
-                                                                             c->jo_tid.as<int32_t>(), c->jo_don.as<int32_t>(), c->jo_acc.as<int32_t>(), c->jo_u.as<int32_t>(), c->jo_m.as<int32_t>());
+                                                                             o.tid.as<int32_t>(), o.don.as<int32_t>(), o.acc.as<int32_t>(), o.uniq_c.as<int32_t>(), o.multi_c.as<int32_t>());
         CK(cudaGetLastError());
-        for (int i = 0; i < 5; ++i) if ((rc = d2h(c, c->p[i], o[i]->as<int32_t>(), d))) return rc;
+        if ((rc = copy(c, c->out_junc, o, Extent{nd}, cudaMemcpyDeviceToHost))) return rc;
         CK(cudaStreamSynchronize(c->st));
     }
-    out->n = nd; out->tid = c->p[0].as<int32_t>(); out->don = c->p[1].as<int32_t>(); out->acc = c->p[2].as<int32_t>(); out->uniq_c = c->p[3].as<int32_t>(); out->multi_c = c->p[4].as<int32_t>();
+    *out = view(c->out_junc, lrb_sj{nd});
     c->launches_last = total_launches() - l0;
     return LRB_OK;
 }
@@ -153,7 +152,7 @@ extern "C" int lrb_sort3(lrb_ctx *c, const uint32_t *k0, const uint32_t *k1, con
     CK(cudaSetDevice(c->device));
     const int64_t l0 = total_launches();
     *perm = nullptr;
-    if (n == 0) { NEEDP(c->p[0], 4); *perm = c->p[0].as<uint32_t>(); return LRB_OK; }
+    if (n == 0) { NEEDP(c->out_perm, 4); *perm = c->out_perm.as<uint32_t>(); return LRB_OK; }
     const size_t m = (size_t)n; int rc;
     // the three key columns ride in the junction buffers (tid = k0, don = k1, acc = k2)
     if ((rc = h2d(c, c->j_tid, (const int32_t *)k0, m)) || (rc = h2d(c, c->j_don, (const int32_t *)k1, m)) || (rc = h2d(c, c->j_acc, (const int32_t *)k2, m))) return rc;
@@ -166,9 +165,9 @@ extern "C" int lrb_sort3(lrb_ctx *c, const uint32_t *k0, const uint32_t *k1, con
     sj_key_kernel<<<bl, 256, 0, c->st>>>(c->j_tid.as<int32_t>(), c->j_don.as<int32_t>(), c->j_acc.as<int32_t>(), v[cur], k[cur], nullptr, n, 1);
     for (int shift = 0; shift < 64; shift += 8) { launch_sort_pass(k[cur], v[cur], k[cur ^ 1], v[cur ^ 1], n, shift, c->s_hist.as<uint32_t>(), c->st); cur ^= 1; }
     CK(cudaGetLastError());
-    if ((rc = d2h(c, c->p[0], v[cur], m))) return rc;
+    if ((rc = d2h(c, c->out_perm, v[cur], m))) return rc;
     CK(cudaStreamSynchronize(c->st));
-    *perm = c->p[0].as<uint32_t>();
+    *perm = c->out_perm.as<uint32_t>();
     c->launches_last = total_launches() - l0;
     return LRB_OK;
 }
