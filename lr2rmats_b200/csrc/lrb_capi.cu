@@ -36,10 +36,10 @@ int setup_exons(lrb_ctx *c, int64_t cap)
     return LRB_OK;
 }
 
-// the scan stage in one of its three modes; on return rows.n / ex.n are known on the host
-// by_record (fused pipeline): rows are written at their record index and the totals stay on the device (slots 0/1) -- the
-// caller reads them together with its own counts and repeats the pass if the exon pool was too small
-int run_scan(lrb_ctx *c, int mode, const lrb_filter_params *fp, const lrb_exon_params *ep, const uint8_t *sel_mask, bool by_record = false)
+// the scan stage in one of its three modes; on return the counts are known on the host.  Mode 2 (fused pipeline) writes the rows at
+// their record index and runs the selection, the keep list and the kept rows (rows2) behind the walk: its counts are n_pass, ex.n and
+// n_keep, read back in the same round trip.  If the exon pool was too small the walk is repeated once with its exact size.
+int run_scan(lrb_ctx *c, int mode, const lrb_filter_params *fp, const lrb_exon_params *ep, const uint8_t *sel_mask)
 {
     const int64_t n = c->b.n;
     int rc;
@@ -58,12 +58,12 @@ int run_scan(lrb_ctx *c, int mode, const lrb_filter_params *fp, const lrb_exon_p
         int64_t bound = c->b.n_cigar + n + 16, est = c->b.n_cigar / 2 + n + 4096;
         if ((rc = setup_exons(c, std::min(bound, std::max(est, c->ex.cap)))) != LRB_OK) return rc;
     }
-    for (int attempt = 0; attempt < 2; ++attempt) {
+    for (int attempt = 0;; ++attempt) {
         ScanArgs a{};
         a.b = c->b; if (fp) a.fp = *fp; if (ep) a.ep = *ep; a.rm = c->rm; a.mode = mode; a.sel_mask = sel_mask;
         a.pass = c->f_pass.as<uint8_t>(); a.score = c->f_score.as<int32_t>(); a.intron_n = c->f_intron.as<int32_t>();
         a.rows = c->rows; a.ex = c->ex; a.tile_state = c->tile_state.as<uint64_t>(); a.ticket = d_ticket(c); a.totals = d_totals(c);
-        a.reads_per_tile = R; a.stage_words = stage_words; a.rows_by_record = by_record ? 1 : 0;
+        a.reads_per_tile = R; a.stage_words = stage_words; a.rows_by_record = mode == 2 ? 1 : 0;
         CK(cudaMemsetAsync(c->tile_state.p, 0, (size_t)n_tiles * 8, c->st));
         CK(cudaMemsetAsync(c->scalars.p, 0, 8 * 8, c->st)); CK(cudaMemsetAsync(d_ticket(c), 0, 4, c->st));
         size_t smem = (size_t)stage_words * 4;
@@ -71,16 +71,23 @@ int run_scan(lrb_ctx *c, int mode, const lrb_filter_params *fp, const lrb_exon_p
         launch_cigar_scan(a, n_tiles, stream_mode, smem, c->st);
         tick(c, EV_SCAN1);
         CK(cudaGetLastError());
-        if (by_record) return LRB_OK;
-        uint64_t t[2];
-        if ((rc = read_totals(c, t, 2)) != LRB_OK) return rc;
-        c->rows.n = (int64_t)t[0]; c->ex.n = (int64_t)t[1];
+        if (mode == 2) {                             // run selection on the record stream -> compaction + row gather
+            CK(cudaMemsetAsync(c->f_keep_rec_mask.p, 0, (size_t)n, c->st));
+            launch_select_records(c->b, c->f_pass.as<uint8_t>(), c->f_score.as<int32_t>(), c->f_intron.as<int32_t>(), *fp, c->f_keep_rec_mask.as<uint8_t>(), c->st);
+            launch_compact_gather(c->f_keep_rec_mask.as<uint8_t>(), n, c->rows, c->rows2, c->f_keep_idx.as<uint32_t>(), c->tile_state.as<uint64_t>(),
+                                  d_ticket(c), d_totals(c) + 2, c->st);
+            CK(cudaGetLastError());
+        }
+        uint64_t t[3];
+        if ((rc = read_totals(c, t, mode == 2 ? 3 : 2)) != LRB_OK) return rc;
+        if (mode == 2) { c->n_pass = (int64_t)t[0]; c->n_keep = (int64_t)t[2]; }
+        else c->rows.n = (int64_t)t[0];
+        c->ex.n = (int64_t)t[1];
         if (c->timing) cudaEventElapsedTime(&c->ms[LRB_T_K_SCAN], c->ev[EV_SCAN0], c->ev[EV_SCAN1]);
-        if (mode == 0 || c->ex.n <= c->ex.cap) break;
+        if (mode == 0 || c->ex.n <= c->ex.cap) return LRB_OK;
         if (attempt == 1) return fail(c, LRB_E_NOMEM, "exon pool still too small after regrow");
         if ((rc = setup_exons(c, c->ex.n + 16)) != LRB_OK) return rc;          // exact size known now: walk again
     }
-    return LRB_OK;
 }
 
 int run_select(lrb_ctx *c, const lrb_filter_params *fp)
@@ -111,18 +118,26 @@ int setup_merge(lrb_ctx *c, MergeBufs &m, int64_t n_cand)
     return LRB_OK;
 }
 
+// what a merge fold does beyond folding its list
+struct FoldOpts {
+    const uint8_t *kls = nullptr;                   // set: the list carries four independent sub-streams (class id per candidate) folded
+    uint32_t *class_alive = nullptr;                // in one pass, and only the survivors per sub-stream are counted (class_alive)
+    bool time_fold = false;                         // EV_FOLD0 / EV_FOLD1 around the fold kernels
+    bool side = false;                              // on the side stream, with its own look-back state
+    bool single_locus = false;                      // the whole list is ONE locus: the back-scan replayed entry by entry
+    bool xl = false;                                // split pieces that meet another chromosome are marked by the xl_* kernels
+};
+
 // merge fold over `list`, asynchronous.  n_cand is the number of candidates, or (n_cand_dev != nullptr) the host's upper
-// bound of a count that lives on the device.  kls != nullptr: the list carries four independent sub-streams (class id per
-// candidate) folded in one pass and only the survivors per sub-stream are counted (class_alive); else the survivors are
-// compacted into m.o_*.  totals[0] <- number of loci, totals[1] <- number of survivors (device).
+// bound of a count that lives on the device.  Without o.kls the survivors are compacted into m.o_*.
+// totals[0] <- number of loci, totals[1] <- number of survivors (device).
 int run_merge_async(lrb_ctx *c, MergeBufs &m, const DTransList &list, int64_t n_cand, const uint64_t *n_cand_dev, const lrb_update_params &up,
-                    uint64_t *totals, const uint8_t *kls = nullptr, uint32_t *class_alive = nullptr, bool time_fold = false, bool side = false,
-                    bool single_locus = false, bool xl = false)
+                    uint64_t *totals, const FoldOpts &o)
 {
     int rc;
-    cudaStream_t st = side ? c->st2 : c->st;
+    cudaStream_t st = o.side ? c->st2 : c->st;
     if ((rc = setup_merge(c, m, n_cand)) != LRB_OK) return rc;
-    if (side) { NEED(c->tile_state2, (size_t)(n_cand / 8 + 1024) * 8); }
+    if (o.side) { NEED(c->tile_state2, (size_t)(n_cand / 8 + 1024) * 8); }
     else if ((rc = ensure_tiles(c, n_cand)) != LRB_OK) return rc;
     m.n_out = 0; m.n_loci = 0;
     CK(cudaMemsetAsync(totals, 0, 16, st));
@@ -133,9 +148,9 @@ int run_merge_async(lrb_ctx *c, MergeBufs &m, const DTransList &list, int64_t n_
     a.dropped = m.dropped.as<uint8_t>();
     a.rep = m.rep.as<uint32_t>(); a.lstart = m.lstart.as<uint32_t>(); a.evmask = m.evmask.as<uint64_t>(); a.samemask = m.samemask.as<uint64_t>(); a.hard = m.hard.as<uint8_t>(); a.desc = m.desc.as<uint16_t>(); a.relsym = m.relsym.as<uint64_t>(); a.ckey = m.ckey.as<uint64_t>(); a.cmin = m.cmin.as<uint32_t>(); a.cord = m.cord.as<uint8_t>(); a.clist = m.clist.as<uint32_t>(); a.crow = m.crow.as<uint64_t>(); a.fb_list = m.fb_list.as<uint32_t>(); a.fb_cnt = m.fb_cnt.as<uint32_t>();
     a.work = view(m.w, DMerged{n_cand, n_cand}); a.out = view(m.o, DMerged{n_cand, n_cand}); a.cd = view(m.cd, CandSoA{});
-    a.tile_state = side ? c->tile_state2.as<uint64_t>() : c->tile_state.as<uint64_t>(); a.ticket = side ? d_ticket2(c) : d_ticket(c); a.totals = totals;
-    a.kls = kls; a.class_alive = class_alive; a.single_locus = single_locus ? 1 : 0;
-    if (xl) {
+    a.tile_state = o.side ? c->tile_state2.as<uint64_t>() : c->tile_state.as<uint64_t>(); a.ticket = o.side ? d_ticket2(c) : d_ticket(c); a.totals = totals;
+    a.kls = o.kls; a.class_alive = o.class_alive; a.single_locus = o.single_locus ? 1 : 0;
+    if (o.xl) {
         // split pieces that meet another chromosome (xl_* kernels): marks per candidate, a key set sized for the pieces' junctions
         // (pieces are a small share of the candidates), lists in buffers the fold is done with by then
         const uint64_t tcap = std::max<uint64_t>(1u << 16, (uint64_t)n_cand / 2);
@@ -146,20 +161,21 @@ int run_merge_async(lrb_ctx *c, MergeBufs &m, const DTransList &list, int64_t n_
     }
     m.args = a;
     launch_merge_prepare(a, st);
-    if (time_fold) tick(c, EV_FOLD0);
+    if (o.time_fold) tick(c, EV_FOLD0);
     launch_merge_fold(a, st);                        // locus count is consumed on the device: no host round trip
-    if (time_fold) tick(c, EV_FOLD1);
-    if (xl) launch_xlocus_detect(a, c->xl, st);
-    if (kls) launch_merge_class_counts(a, st);
+    if (o.time_fold) tick(c, EV_FOLD1);
+    if (o.xl) launch_xlocus_detect(a, c->xl, st);
+    if (o.kls) launch_merge_class_counts(a, st);
     else launch_merge_finish(a, st);
     CK(cudaGetLastError());
     return LRB_OK;
 }
 
-int run_merge(lrb_ctx *c, MergeBufs &m, const DTransList &list, int64_t n_cand, const lrb_update_params &up, bool single_locus = false)
+int run_merge(lrb_ctx *c, MergeBufs &m, const DTransList &list, int64_t n_cand, const lrb_update_params &up, bool single_locus)
 {
     int rc;
-    if ((rc = run_merge_async(c, m, list, n_cand, nullptr, up, d_totals(c), nullptr, nullptr, true, false, single_locus)) != LRB_OK) return rc;
+    FoldOpts o; o.time_fold = true; o.single_locus = single_locus;
+    if ((rc = run_merge_async(c, m, list, n_cand, nullptr, up, d_totals(c), o)) != LRB_OK) return rc;
     uint64_t t[2];
     if ((rc = read_totals(c, t, 2)) != LRB_OK) return rc;
     m.n_loci = (int64_t)t[0]; m.n_out = (int64_t)t[1];
@@ -189,8 +205,6 @@ int lrb_ctx_create(int device, lrb_ctx **out)
     cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming); cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming);
     if (cudaStreamCreateWithFlags(&c->st3, cudaStreamNonBlocking) != cudaSuccess) { cudaStreamDestroy(c->st2); cudaStreamDestroy(c->st); delete c; return LRB_E_CUDA; }
     cudaEventCreateWithFlags(&c->ev_fork3, cudaEventDisableTiming); cudaEventCreateWithFlags(&c->ev_join3, cudaEventDisableTiming);
-    { const char *e = getenv("LRB_SUM_SPLIT"); if (e) c->sum_split = atoi(e) != 0; }
-    { const char *e = getenv("LRB_SIDE_STREAM"); if (e) c->side_stream = atoi(e) != 0; }
     { const char *e = getenv("LRB_TEST_SMALL_NOVEL_CAP"); if (e) c->test_small_novel_cap = atoi(e) != 0; }      // test hook: novel_T sized too small on the first attempt
     { const char *e = getenv("LRB_FORCE_SINGLE_FOLD"); if (e) c->force_single_fold = atoi(e) != 0; }    // test hook: updated_T always folded by the one-locus replay
     if (!c->scalars.ensure(512) || !c->h_scalars.ensure(512)) { delete c; return LRB_E_NOMEM; }
@@ -401,25 +415,8 @@ int lrb_pipeline_run(lrb_ctx *c, const lrb_filter_params *fp, const lrb_exon_par
     NEED(c->f_keep_rec_mask, (size_t)std::max<int64_t>(n, 1)); NEED(c->f_keep_idx, (size_t)std::max<int64_t>(n, 1) * 4);
     if ((rc = setup_rows(c, c->rows2, c->rows2_cols, n))) return rc;
     c->rows.n = 0; c->ex.n = 0; c->n_pass = c->n_keep = 0;
-    for (int attempt = 0; n > 0; ++attempt) {
-        // scan (rows at their record index) -> run selection on the record stream -> compaction + row gather: one
-        // round trip for (passing, exons, kept)
-        if ((rc = run_scan(c, 2, fp, ep, nullptr, true))) return rc;
-        CK(cudaMemsetAsync(c->f_keep_rec_mask.p, 0, (size_t)n, c->st));
-        launch_select_records(c->b, c->f_pass.as<uint8_t>(), c->f_score.as<int32_t>(), c->f_intron.as<int32_t>(), *fp, c->f_keep_rec_mask.as<uint8_t>(), c->st);
-        launch_compact_gather(c->f_keep_rec_mask.as<uint8_t>(), n, c->rows, c->rows2, c->f_keep_idx.as<uint32_t>(), c->tile_state.as<uint64_t>(),
-                              d_ticket(c), d_totals(c) + 2, c->st);
-        CK(cudaGetLastError());
-        uint64_t t[3];
-        if ((rc = read_totals(c, t, 3))) return rc;
-        c->n_pass = (int64_t)t[0]; c->ex.n = (int64_t)t[1]; c->n_keep = (int64_t)t[2];
-        if (c->timing) cudaEventElapsedTime(&c->ms[LRB_T_K_SCAN], c->ev[EV_SCAN0], c->ev[EV_SCAN1]);
-        if (c->ex.n <= c->ex.cap) break;
-        if (attempt == 1) return fail(c, LRB_E_NOMEM, "exon pool still too small after regrow");
-        if ((rc = setup_exons(c, c->ex.n + 16))) return rc;     // exact size known now: walk again
-    }
-    if (n == 0 && (rc = setup_exons(c, 16))) return rc;
-    c->rows.n = n;                                               // record-indexed: only the passing records' rows are valid
+    if ((rc = n ? run_scan(c, 2, fp, ep, nullptr) : setup_exons(c, 16))) return rc;
+    c->rows.n = n;                                              // record-indexed: only the passing records' rows are valid
     c->rows2.n = c->n_keep;
     tick(c, EV_END);
     c->cur = &c->rows2; c->rows_compact = false; c->have_filter = true; c->have_exons = true; c->have_update = c->have_unique = false;
@@ -428,16 +425,20 @@ int lrb_pipeline_run(lrb_ctx *c, const lrb_filter_params *fp, const lrb_exon_par
     return LRB_OK;
 }
 
-static int check_err_flags(lrb_ctx *c, uint32_t *flags = nullptr)
+// the error flags of the update / unique input checks (d_err) as a status
+static int err_status(lrb_ctx *c, uint32_t e)
 {
-    uint32_t e = 0;
-    CK(cudaMemcpyAsync(c->h_scalars.p, d_err(c), 4, cudaMemcpyDeviceToHost, c->st));
-    CK(cudaStreamSynchronize(c->st));
-    memcpy(&e, c->h_scalars.p, 4);
-    if (flags) *flags = e;
     if (e & 2u) return fail(c, LRB_E_UNMAPPED, "unmapped record / empty exon chain in update/unique input (the reference aborts here, bam2gtf.c:95-100)");
     if (e & 1u) return fail(c, LRB_E_UNSORTED, "reads are not sorted by (tid,start) (update_gtf.c:41)");
     return LRB_OK;
+}
+
+static int check_err_flags(lrb_ctx *c, uint32_t *flags)
+{
+    CK(cudaMemcpyAsync(c->h_scalars.p, d_err(c), 4, cudaMemcpyDeviceToHost, c->st));
+    CK(cudaStreamSynchronize(c->st));
+    memcpy(flags, c->h_scalars.p, 4);
+    return err_status(c, *flags);
 }
 
 __global__ void invert_mask_kernel(const uint8_t *a, uint8_t *o, int64_t n)
@@ -458,22 +459,48 @@ __global__ void rows_check_kernel(DRows rows, uint32_t *err, int check_sorted)
     }
 }
 
-int lrb_update_run(lrb_ctx *c, const lrb_update_params *up)
+// ---- the update stage in steps; what one step hands to the next
+struct UpdateRun {
+    const lrb_update_params *up;
+    bool xl_exact, detect, run_sets, single;        // see lrb_update_run
+    int64_t cap, n_novel;                           // novel_T: capacity, entries
+    SummaryArgs sa;                                 // the summary sets over updated_T (run_sets)
+};
+
+// the stage's round trips through h_scalars (UpdateScalars): the copies `parts` names, in this order, then one synchronization.
+// RB_SCALARS: totals, ticket, error flags.  RB_SET_COUNTS: y_counts without the class sizes, which keep the value of an earlier read.
+enum { RB_SCALARS = 1, RB_BED = 2, RB_COUNTS = 4, RB_SET_COUNTS = 8, RB_NELEM = 16, RB_XL = 32 };
+static int read_back(lrb_ctx *c, unsigned parts)
 {
-    if (!c || !up) return LRB_E_ARG;
-    if (!c->have_exons) return fail(c, LRB_E_ARG, "lrb_update_run: exon chains missing (run lrb_exon_run / lrb_pipeline_run / lrb_chains_upload)");
-    CK(cudaSetDevice(c->device));
-    int64_t l0 = total_launches();
+    UpdateScalars *hs = c->h_scalars.as<UpdateScalars>();
+    if (parts & RB_SCALARS) CK(cudaMemcpyAsync(hs, c->scalars.p, T_SLOTS * 8 + 8, cudaMemcpyDeviceToHost, c->st));
+    if (parts & RB_BED) CK(cudaMemcpyAsync(&hs->t[T_BED], d_totals(c) + T_BED, 8, cudaMemcpyDeviceToHost, c->st));
+    if (parts & (RB_COUNTS | RB_SET_COUNTS)) CK(cudaMemcpyAsync(hs->counts, c->y_counts.p, (parts & RB_COUNTS) ? 64 : 48, cudaMemcpyDeviceToHost, c->st));
+    if (parts & RB_NELEM) CK(cudaMemcpyAsync(&hs->n_elem, c->y_nelem.p, 16, cudaMemcpyDeviceToHost, c->st));
+    if (parts & RB_XL) CK(cudaMemcpyAsync(hs->xl, c->xl_cnt.p, XL_NCNT * 4, cudaMemcpyDeviceToHost, c->st));
+    CK(cudaStreamSynchronize(c->st));
+    return LRB_OK;
+}
+
+// The class folds run on the side stream.  The main stream waits for them before their counters are read or reset, and before the
+// stage returns early: they share the context's buffers and counters with whatever runs next.
+static int join_class_folds(lrb_ctx *c, const lrb_update_params *up)
+{
+    if (up->want_summary) CK(cudaStreamWaitEvent(c->st, c->ev_join, 0));
+    return LRB_OK;
+}
+
+// classification (+ SJ support)
+static int update_classify(lrb_ctx *c, const lrb_update_params *up)
+{
     DRows &rows = *c->cur; const int64_t n = rows.n; const size_t nn = (size_t)std::max<int64_t>(n, 1);
     int rc;
-    memset(c->summary, 0, sizeof c->summary); c->n_bed = 0; c->last_up = *up; c->n_known = c->n_unrecog = 0;
     NEED(c->u_cls, nn * 4); NEED(c->u_ref, nn * 4); NEED(c->u_nnovel, nn * 4);
     NEED(c->u_mk, nn); NEED(c->u_known, nn * 4); NEED(c->u_unrecog, nn * 4); NEED(c->u_ck, nn);
     NEED(c->y_counts, 64); NEED(c->y_nelem, 64);       // y_nelem: element count, then (at +16) the six tickets of sum_scans_kernel
     if ((rc = ensure_tiles(c, std::max<int64_t>(n, c->ex.n)))) return rc;
     CK(cudaMemsetAsync(d_err(c), 0, 4, c->st));
     tick(c, EV_BEGIN);
-    // ---- classification (+ SJ support)
     ClassArgs ca{};
     ca.rows = rows; ca.ex = c->ex; ca.anno = c->anno; ca.sj = c->sj; ca.up = *up;
     ca.row_nonmono = c->have_batch ? nullptr : c->r_nonmono.as<uint8_t>();
@@ -481,177 +508,200 @@ int lrb_update_run(lrb_ctx *c, const lrb_update_params *up)
     launch_classify(ca, c->u_mk.as<uint8_t>(), c->st);     // u_mk: scratch for the slow-row mask
     CK(cudaGetLastError());
     tick(c, EV_CLASSIFIED);
+    return LRB_OK;
+}
 
-    // ---- lists, the updated_T fold, the class folds and the element count of the summary sets: one stream of launches,
-    // every count stays on the device; ONE copy brings them all back.  novel_T is sized optimistically (pieces are rare);
-    // if it turns out too small the pass is repeated once with the exact size.
+// Lists, the updated_T fold, the class folds and the element count of the summary sets: one stream of launches, every count stays on
+// the device; ONE copy brings them all back.  novel_T is sized optimistically (pieces are rare); if it turns out too small the step is
+// repeated once with the exact size.  The class folds are left running on the side stream underneath the steps that follow.
+static int update_lists_and_folds(lrb_ctx *c, UpdateRun &u, int pass)
+{
+    const lrb_update_params *up = u.up;
+    DRows &rows = *c->cur; const int64_t n = rows.n;
     uint64_t *T = d_totals(c);
-    int64_t cap = up->split_trans ? n + n / 8 + 1024 : n;
-    cap = std::max<int64_t>(cap, std::min<int64_t>(c->novel_cap_hint, n + c->ex.n / 2 + 1));
-    if (c->test_small_novel_cap) cap = std::max<int64_t>(1, n / 4);   // test hook: forces the undersized-list retry
-    // A split piece scans the WHOLE of updated_T in the reference (its tid/start/end are 0: update_gtf.c:148 never stops it), so it
-    // can be absorbed by a chain on another chromosome.  The locus-parallel fold cannot see that; the set kernels probe for the
-    // necessary condition (a junction of a piece that also exists on another chromosome, CNT_XLOCUS) and the fold is then replayed
-    // once more as ONE locus (merge_fold_kernel: the exact back-scan, entry by entry).  With -d > 0 junctions match approximately and
-    // the exact-key probe proves nothing: any surviving piece sends the fold to the replay.
-    // With the default exact matching (-d 0, no -D) that is settled in rounds on the device (xl_* kernels in lrb_update.cu): exact and
-    // cheap.  The one-locus replay remains for -d > 0 / -D, where check_iden depends on the entries' moving ends.
-    const bool xl_exact = up->split_trans != 0 && up->ss_dis == 0 && up->end_dis == 0x7fffffff && !c->force_single_fold;
-    const bool detect = up->split_trans != 0 && !xl_exact, run_sets = up->want_summary || detect;
-    bool single = c->force_single_fold;
-    c->n_xlocus_pieces = 0;
-    for (int fold_pass = 0; fold_pass < 2; ++fold_pass) {
-    SummaryArgs sa{};
-    int64_t n_novel = 0, nu = 0; uint64_t n_elem = 0, n_exon_elem = 0;
-    uint32_t cnt16[16];
-    for (int attempt = 0; n > 0; ++attempt) {
-        if ((rc = setup_list(c, c->novel, c->novel_cols, cap))) return rc;
+    const UpdateScalars &hs = *c->h_scalars.as<UpdateScalars>();
+    int rc;
+    if (n == 0) {
+        if ((rc = setup_list(c, c->novel, c->novel_cols, 0))) return rc;
+        c->mg.n_out = c->mg.n_loci = 0; tick(c, EV_LISTED); tick(c, EV_FOLDED);
+        u.n_novel = 0;
+        return LRB_OK;
+    }
+    for (int attempt = 0;; ++attempt) {
+        if ((rc = setup_list(c, c->novel, c->novel_cols, u.cap))) return rc;
         CK(cudaMemsetAsync(c->y_counts.p, 0, 64, c->st)); CK(cudaMemsetAsync(c->y_nelem.p, 0, 16, c->st));
         ListArgs la{};
-        la.rows = rows; la.ex = c->ex; la.up = *up; la.cls = ca.cls; la.n_novel = ca.n_novel; la.novel = c->novel;
+        la.rows = rows; la.ex = c->ex; la.up = *up; la.cls = c->u_cls.as<uint32_t>(); la.n_novel = c->u_nnovel.as<uint32_t>(); la.novel = c->novel;
         la.known = c->u_known.as<uint32_t>(); la.unrecog = c->u_unrecog.as<uint32_t>();
         la.kls = up->want_summary ? c->u_ck.as<uint8_t>() : nullptr; la.class_n = c->y_counts.as<uint32_t>() + 12;
         la.tile_state = c->tile_state.as<uint64_t>(); la.ticket = d_ticket(c); la.totals = T + T_NOVEL;
         launch_build_lists(la, c->st);
         CK(cudaGetLastError());
-        if (attempt == 0 && fold_pass == 0) tick(c, EV_LISTED);
+        if (attempt == 0 && pass == 0) tick(c, EV_LISTED);
         if (up->want_summary) {
             // class counts + uniq_* folds over bam_T (update_gtf.c:501-528): the four classes partition the rows; they are
             // folded in ONE pass over all rows, each candidate seeing only the entries of its own class.  Independent of the
-            // updated_T fold and of the sets: forked onto the side stream, joined in front of the round trip below.
-            const bool side = c->side_stream;
-            cudaStream_t s2 = side ? c->st2 : c->st;
+            // updated_T fold and of the sets: forked onto the side stream.
             if ((rc = setup_list(c, c->tmp_list, c->tmp_cols, n))) return rc;
-            if (side) { CK(cudaEventRecord(c->ev_fork, c->st)); CK(cudaStreamWaitEvent(c->st2, c->ev_fork, 0)); }
-            launch_rows_as_list(rows, nullptr, n, c->tmp_list, s2);
-            if ((rc = run_merge_async(c, c->mg2, c->tmp_list, n, nullptr, *up, T + T_LOCI2, c->u_ck.as<uint8_t>(), c->y_counts.as<uint32_t>() + 8, false, side))) return rc;
-            if (side) CK(cudaEventRecord(c->ev_join, c->st2));
+            CK(cudaEventRecord(c->ev_fork, c->st)); CK(cudaStreamWaitEvent(c->st2, c->ev_fork, 0));
+            launch_rows_as_list(rows, nullptr, n, c->tmp_list, c->st2);
+            FoldOpts o; o.kls = c->u_ck.as<uint8_t>(); o.class_alive = c->y_counts.as<uint32_t>() + 8; o.side = true;
+            if ((rc = run_merge_async(c, c->mg2, c->tmp_list, n, nullptr, *up, T + T_LOCI2, o))) return rc;
+            CK(cudaEventRecord(c->ev_join, c->st2));
         }
         // updated_T = merge fold over novel_T (update_gtf.c:949,956)
-        if (xl_exact) { NEED(c->xl_forced, (size_t)std::max<int64_t>(cap, 1)); CK(cudaMemsetAsync(c->xl_forced.p, 0, (size_t)std::max<int64_t>(cap, 1), c->st)); }
-        if ((rc = run_merge_async(c, c->mg, c->novel, cap, T + T_NOVEL, *up, T + T_LOCI, nullptr, nullptr, true, false, single, xl_exact))) return rc;
-        if (attempt == 0 && fold_pass == 0) tick(c, EV_FOLDED);
-        if (run_sets) {
+        if (u.xl_exact) { NEED(c->xl_forced, (size_t)std::max<int64_t>(u.cap, 1)); CK(cudaMemsetAsync(c->xl_forced.p, 0, (size_t)std::max<int64_t>(u.cap, 1), c->st)); }
+        FoldOpts o; o.time_fold = true; o.single_locus = u.single; o.xl = u.xl_exact;
+        if ((rc = run_merge_async(c, c->mg, c->novel, u.cap, T + T_NOVEL, *up, T + T_LOCI, o))) return rc;
+        if (attempt == 0 && pass == 0) tick(c, EV_FOLDED);
+        if (u.run_sets) {
             // sets over updated_T: element count (sizes the hash table)
-            const size_t capn = (size_t)std::max<int64_t>(cap, 1);
+            const size_t capn = (size_t)std::max<int64_t>(u.cap, 1);
             NEED(c->y_barcnt, capn * 16); NEED(c->y_barseg, capn * 16); NEED(c->y_genebar, capn * 8); NEED(c->y_bedcnt, capn * 4); NEED(c->y_bedoff, capn * 4);
-            sa = SummaryArgs{}; sa.sets = up->want_summary ? SUM_ALL : 0; sa.probe = detect ? 1 : 0;
-            sa.rows = rows; sa.ex = c->ex; sa.list = c->novel; sa.n_upd = cap; sa.n_upd_dev = T + T_UPD;
-            sa.upd = view(c->mg.o, DMerged{cap, cap});
+            SummaryArgs &sa = u.sa;
+            sa = SummaryArgs{}; sa.sets = up->want_summary ? SUM_ALL : 0; sa.probe = u.detect ? 1 : 0;
+            sa.rows = rows; sa.ex = c->ex; sa.list = c->novel; sa.n_upd = u.cap; sa.n_upd_dev = T + T_UPD;
+            sa.upd = view(c->mg.o, DMerged{u.cap, u.cap});
             sa.ref = c->u_ref.as<int32_t>(); sa.anno_gene = c->anno.gene;
             sa.bar_cnt = c->y_barcnt.as<uint32_t>(); sa.bar_seg = c->y_barseg.as<uint32_t>(); sa.gene_bar = c->y_genebar.as<uint64_t>();
             sa.bed_cnt = c->y_bedcnt.as<uint32_t>(); sa.bed_off = c->y_bedoff.as<uint32_t>(); sa.counts = c->y_counts.as<uint32_t>();
             launch_summary_count(sa, c->y_nelem.as<unsigned long long>(), c->st);
             CK(cudaGetLastError());
         }
-        // ---- the one round trip: totals, error flags, class sizes, element count.  The class folds keep running on the
-        // side stream underneath the summary sets; they are joined in front of the last copy of this stage.
-        UpdateScalars *hs = c->h_scalars.as<UpdateScalars>();
-        CK(cudaMemcpyAsync(hs, c->scalars.p, T_SLOTS * 8 + 8, cudaMemcpyDeviceToHost, c->st));
-        CK(cudaMemcpyAsync(hs->counts, c->y_counts.p, 64, cudaMemcpyDeviceToHost, c->st));
-        CK(cudaMemcpyAsync(&hs->n_elem, c->y_nelem.p, 16, cudaMemcpyDeviceToHost, c->st));
-        if (xl_exact) CK(cudaMemcpyAsync(hs->xl, c->xl_cnt.p, XL_NCNT * 4, cudaMemcpyDeviceToHost, c->st));
-        CK(cudaStreamSynchronize(c->st));
-        uint64_t t[T_SLOTS]; uint32_t xc[XL_NCNT] = {0};
-        memcpy(t, hs->t, sizeof t); memcpy(cnt16, hs->counts, 64); n_elem = hs->n_elem; n_exon_elem = hs->n_exon_elem;
-        if (xl_exact) memcpy(xc, hs->xl, sizeof xc);
-        if (hs->err & 3u) {
-            // the class folds may still be running on the side stream: they must be over before the caller can start another
-            // stage on this context (they share its buffers and counters)
-            if (up->want_summary && c->side_stream) cudaStreamSynchronize(c->st2);
-            if (hs->err & 2u) return fail(c, LRB_E_UNMAPPED, "unmapped record / empty exon chain in update/unique input (the reference aborts here, bam2gtf.c:95-100)");
-            return fail(c, LRB_E_UNSORTED, "reads are not sorted by (tid,start) (update_gtf.c:41)");
-        }
-        n_novel = (int64_t)t[T_NOVEL]; c->n_known = (int64_t)t[T_KNOWN]; c->n_unrecog = (int64_t)t[T_UNREC];
-        if (n_novel > cap) {                          // novel_T did not fit: once more with the exact size
-            if (attempt >= 1) return fail(c, LRB_E_CUDA, "novel_T size changed between passes");
-            cap = n_novel; c->novel_cap_hint = n_novel + n_novel / 16;
-            if (up->want_summary && c->side_stream) CK(cudaStreamWaitEvent(c->st, c->ev_join, 0));   // the counters are reset below
-            continue;
-        }
-        c->mg.n_loci = (int64_t)t[T_LOCI]; c->mg.n_out = nu = (int64_t)t[T_UPD];
-        if (xl_exact && (xc[XL_OVERFLOW] || xc[XL_CHANGED])) {
-            // some piece is absorbed by an entry on another chromosome: fold again with the marks until they are stable (round k fixes
-            // the k-th affected piece at the latest), then let the absorbing entries take cov / ends, compact and count again
-            int rounds = 0;
-            while (!xc[XL_OVERFLOW] && xc[XL_CHANGED] && rounds < 32) {
-                ++rounds;
-                launch_xlocus_reset(c->mg.args, c->xl, c->st);
-                launch_merge_fold(c->mg.args, c->st);
-                launch_xlocus_detect(c->mg.args, c->xl, c->st);
-                CK(cudaMemcpyAsync(hs->xl, c->xl_cnt.p, XL_NCNT * 4, cudaMemcpyDeviceToHost, c->st));
-                CK(cudaStreamSynchronize(c->st));
-                memcpy(xc, hs->xl, sizeof xc);
-            }
-            if (xc[XL_OVERFLOW] || xc[XL_CHANGED]) {                 // more hits than the lists hold, or no fixed point in 32 rounds: the exact replay
-                if (up->want_summary && c->side_stream) CK(cudaStreamWaitEvent(c->st, c->ev_join, 0));
-                single = true; c->n_xlocus_replays++; n_novel = -1; break;
-            }
-            c->n_xlocus_pieces = xc[XL_NFORCED];
-            launch_xlocus_apply(c->mg.args, c->xl, c->st);
-            CK(cudaMemsetAsync(T + T_UPD, 0, 8, c->st));
-            launch_merge_finish(c->mg.args, c->st);
-            if (run_sets) { CK(cudaMemsetAsync(c->y_nelem.p, 0, 16, c->st)); launch_summary_count(sa, c->y_nelem.as<unsigned long long>(), c->st); }
-            CK(cudaGetLastError());
-            CK(cudaMemcpyAsync(hs, c->scalars.p, T_SLOTS * 8 + 8, cudaMemcpyDeviceToHost, c->st));
-            CK(cudaMemcpyAsync(&hs->n_elem, c->y_nelem.p, 16, cudaMemcpyDeviceToHost, c->st));
-            CK(cudaStreamSynchronize(c->st));
-            memcpy(t, hs->t, sizeof t); n_elem = hs->n_elem; n_exon_elem = hs->n_exon_elem;
-            c->mg.n_out = nu = (int64_t)t[T_UPD];
-        }
-        break;
+        // the one round trip: totals, error flags, class sizes, element count
+        if ((rc = read_back(c, RB_SCALARS | RB_COUNTS | RB_NELEM | (u.xl_exact ? RB_XL : 0)))) return rc;
+        if (hs.err & 3u) { join_class_folds(c, up); return err_status(c, hs.err); }
+        u.n_novel = (int64_t)hs.t[T_NOVEL]; c->n_known = (int64_t)hs.t[T_KNOWN]; c->n_unrecog = (int64_t)hs.t[T_UNREC];
+        if (u.n_novel <= u.cap) break;
+        if ((rc = join_class_folds(c, up))) return rc;          // novel_T did not fit: the counters are reset for one more attempt
+        if (attempt >= 1) return fail(c, LRB_E_CUDA, "novel_T size changed between passes");
+        u.cap = u.n_novel; c->novel_cap_hint = u.n_novel + u.n_novel / 16;
     }
-    if (n_novel < 0) continue;                                        // the marks did not settle: once more as ONE locus
-    if (n == 0) { if ((rc = setup_list(c, c->novel, c->novel_cols, 0))) return rc; c->mg.n_out = c->mg.n_loci = 0; tick(c, EV_LISTED); tick(c, EV_FOLDED); }
-    c->novel.n = n_novel; c->novel.cap = std::max<int64_t>(cap, 0);
-    if (c->timing && n && fold_pass == 0) { CK(cudaStreamSynchronize(c->st)); cudaEventElapsedTime(&c->ms[LRB_T_K_FOLD], c->ev[EV_FOLD0], c->ev[EV_FOLD1]); }
+    c->mg.n_loci = (int64_t)hs.t[T_LOCI]; c->mg.n_out = (int64_t)hs.t[T_UPD];
+    return LRB_OK;
+}
 
-    // ---- summary sets (print_trans_summary, update_gtf.c:421-587) and / or the probe for pieces that meet another chromosome
-    if (!(run_sets && n > 0)) break;
-    int32_t *s = c->summary;
-    const int cnt_idx[4] = {LRB_S_KNOWN_TRANS, LRB_S_NOVEL_RELIABLE, LRB_S_NOVEL_UNRELIABLE, LRB_S_UNRECOG};
-    const int uniq_idx[4] = {LRB_S_UNIQ_KNOWN, LRB_S_UNIQ_RELIABLE, LRB_S_UNIQ_UNRELIABLE, LRB_S_UNIQ_UNRECOG};
-    const int64_t n_known_reads = up->want_summary ? (int64_t)cnt16[12] : 0;
+// Split pieces absorbed by an entry on another chromosome (xl_exact): fold again with the marks until they are stable (round k fixes the
+// k-th affected piece at the latest), then let the absorbing entries take cov / ends, compact and count again.  *settled = false: more
+// hits than the lists hold, or no fixed point in 32 rounds.
+static int update_settle_pieces(lrb_ctx *c, UpdateRun &u, bool *settled)
+{
+    const UpdateScalars &hs = *c->h_scalars.as<UpdateScalars>();
+    int rc;
+    *settled = true;
+    if (!u.xl_exact || c->cur->n == 0 || !(hs.xl[XL_OVERFLOW] || hs.xl[XL_CHANGED])) return LRB_OK;
+    for (int round = 0; !hs.xl[XL_OVERFLOW] && hs.xl[XL_CHANGED] && round < 32; ++round) {
+        launch_xlocus_reset(c->mg.args, c->xl, c->st);
+        launch_merge_fold(c->mg.args, c->st);
+        launch_xlocus_detect(c->mg.args, c->xl, c->st);
+        if ((rc = read_back(c, RB_XL))) return rc;
+    }
+    if (hs.xl[XL_OVERFLOW] || hs.xl[XL_CHANGED]) { *settled = false; return LRB_OK; }
+    c->n_xlocus_pieces = hs.xl[XL_NFORCED];
+    launch_xlocus_apply(c->mg.args, c->xl, c->st);
+    CK(cudaMemsetAsync(d_totals(c) + T_UPD, 0, 8, c->st));
+    launch_merge_finish(c->mg.args, c->st);
+    if (u.run_sets) { CK(cudaMemsetAsync(c->y_nelem.p, 0, 16, c->st)); launch_summary_count(u.sa, c->y_nelem.as<unsigned long long>(), c->st); }
+    CK(cudaGetLastError());
+    if ((rc = read_back(c, RB_SCALARS | RB_NELEM))) return rc;
+    c->mg.n_out = (int64_t)hs.t[T_UPD];
+    return LRB_OK;
+}
+
+// Summary sets (print_trans_summary, update_gtf.c:421-587) and / or the probe for pieces that meet another chromosome, then the second
+// round trip.  The class folds are joined in front of it, so they overlap the sets.
+static int update_sets(lrb_ctx *c, UpdateRun &u)
+{
+    const lrb_update_params *up = u.up;
+    const int64_t n = c->cur->n, nu = c->mg.n_out;
+    const UpdateScalars &hs = *c->h_scalars.as<UpdateScalars>();
+    SummaryArgs &sa = u.sa;
+    int rc;
+    const int64_t n_known_reads = up->want_summary ? (int64_t)hs.counts[12] : 0;
     sa.n_upd = nu; sa.n_upd_dev = nullptr; sa.upd.n = nu;
     // distinct table keys: one per exon element, up to two per gene / site / junction element (the tid-0 phase and the
     // segment phase key them differently), one per known read; the table stays below that bound's next power of two
     // (load <= 0.8 in the worst case, ~0.4 on the bench shape; the slot index is a multiply-high, so no power of two is needed)
-    const uint64_t worst = 2 * n_elem - std::min(n_exon_elem, n_elem) + (uint64_t)n_known_reads;
+    const uint64_t worst = 2 * hs.n_elem - std::min(hs.n_exon_elem, hs.n_elem) + (uint64_t)n_known_reads;
     const uint64_t capn = worst + worst / 4 + 1024;
     NEED(c->h_khi, capn * sizeof(HashSlot));
     CK(cudaMemsetAsync(c->h_khi.p, 0xFF, capn * sizeof(HashSlot), c->st));
     sa.tab.cap = capn; sa.tab.slots = c->h_khi.as<HashSlot>();
     // BED rows are the first occurrences of the exon set: at most one per counted element
-    const size_t nb = (size_t)std::max<uint64_t>(n_elem, 1);
+    const size_t nb = (size_t)std::max<uint64_t>(hs.n_elem, 1);
     if ((rc = ensure(c, c->bed, Extent{(int64_t)nb}))) return rc;
     sa.bed_tid = c->bed.tid.as<int32_t>(); sa.bed_start = c->bed.start.as<int32_t>(); sa.bed_end = c->bed.end.as<int32_t>(); sa.bed_score = c->bed.score.as<int32_t>();
     sa.bed_type = c->bed.type.as<uint8_t>(); sa.bed_rev = c->bed.is_rev.as<uint8_t>();
     if (c->want_kg_pairs && up->want_summary) { NEED(c->kg_pairs, (size_t)std::max<int64_t>(n_known_reads, 1) * 8); sa.kg_pairs = c->kg_pairs.as<int2>(); }
     CK(cudaMemsetAsync(c->y_counts.p, 0, 32, c->st));
-    launch_summary_sets(sa, ca.cls, n, c->tile_state.as<uint64_t>(), (uint32_t *)(c->y_nelem.as<uint8_t>() + 16), T + T_BED, c->st,
-                        c->sum_split ? c->st3 : c->st, c->ev_fork3, c->ev_join3);
+    launch_summary_sets(sa, c->u_cls.as<uint32_t>(), n, c->tile_state.as<uint64_t>(), (uint32_t *)(c->y_nelem.as<uint8_t>() + 16), d_totals(c) + T_BED, c->st,
+                        c->st3, c->ev_fork3, c->ev_join3);
     CK(cudaGetLastError());
-    if (up->want_summary && c->side_stream) CK(cudaStreamWaitEvent(c->st, c->ev_join, 0));
-    UpdateScalars *hs = c->h_scalars.as<UpdateScalars>();
-    CK(cudaMemcpyAsync(&hs->t[T_BED], T + T_BED, 8, cudaMemcpyDeviceToHost, c->st));
-    CK(cudaMemcpyAsync(hs->counts, c->y_counts.p, 48, cudaMemcpyDeviceToHost, c->st));
-    CK(cudaStreamSynchronize(c->st));
-    const uint64_t nbed = hs->t[T_BED]; uint32_t cnt[12];
-    memcpy(cnt, hs->counts, 48);
-    c->xlocus_seen = detect && (cnt[CNT_XLOCUS] != 0 || (up->ss_dis > 0 && cnt[CNT_PARTIAL] != 0));
-    if (c->xlocus_seen && !single) { single = true; c->n_xlocus_replays++; continue; }       // replay the fold as one locus
-    if (up->want_summary) {
-        for (int k = 0; k < 4; ++k) s[cnt_idx[k]] = (int32_t)cnt16[12 + k];
-        s[LRB_S_NOVEL_BAM] = s[LRB_S_NOVEL_RELIABLE] + s[LRB_S_NOVEL_UNRELIABLE];
-        for (int k = 0; k < 4; ++k) s[uniq_idx[k]] = (int32_t)cnt[8 + k];
-        c->n_bed = nu ? (int64_t)nbed : 0;
-        s[LRB_S_UPD_GENES] = (int32_t)cnt[CNT_G]; s[LRB_S_NOVEL_TRANS] = (int32_t)nu; s[LRB_S_NOVEL_PARTIAL] = (int32_t)cnt[CNT_PARTIAL];
-        s[LRB_S_NOVEL_FULL] = (int32_t)nu - (int32_t)cnt[CNT_PARTIAL]; s[LRB_S_NOVEL_EXONS] = (int32_t)cnt[CNT_E]; s[LRB_S_NOVEL_SITES] = (int32_t)(cnt[CNT_D] + cnt[CNT_A]);
-        s[LRB_S_NOVEL_JUNC] = (int32_t)cnt[CNT_J]; s[LRB_S_KNOWN_GENES] = (int32_t)cnt[CNT_KG];
-        c->n_kg_pairs = (int64_t)cnt[CNT_KG];
+    if ((rc = join_class_folds(c, up))) return rc;
+    return read_back(c, RB_BED | RB_SET_COUNTS);
+}
+
+// c->summary from the counters of both round trips (the class sizes are the first one's)
+static void update_fill_summary(lrb_ctx *c)
+{
+    const UpdateScalars &hs = *c->h_scalars.as<UpdateScalars>();
+    const uint32_t *cnt = hs.counts; const int64_t nu = c->mg.n_out;
+    int32_t *s = c->summary;
+    const int cnt_idx[4] = {LRB_S_KNOWN_TRANS, LRB_S_NOVEL_RELIABLE, LRB_S_NOVEL_UNRELIABLE, LRB_S_UNRECOG};
+    const int uniq_idx[4] = {LRB_S_UNIQ_KNOWN, LRB_S_UNIQ_RELIABLE, LRB_S_UNIQ_UNRELIABLE, LRB_S_UNIQ_UNRECOG};
+    for (int k = 0; k < 4; ++k) s[cnt_idx[k]] = (int32_t)cnt[12 + k];
+    s[LRB_S_NOVEL_BAM] = s[LRB_S_NOVEL_RELIABLE] + s[LRB_S_NOVEL_UNRELIABLE];
+    for (int k = 0; k < 4; ++k) s[uniq_idx[k]] = (int32_t)cnt[8 + k];
+    c->n_bed = nu ? (int64_t)hs.t[T_BED] : 0;
+    s[LRB_S_UPD_GENES] = (int32_t)cnt[CNT_G]; s[LRB_S_NOVEL_TRANS] = (int32_t)nu; s[LRB_S_NOVEL_PARTIAL] = (int32_t)cnt[CNT_PARTIAL];
+    s[LRB_S_NOVEL_FULL] = (int32_t)nu - (int32_t)cnt[CNT_PARTIAL]; s[LRB_S_NOVEL_EXONS] = (int32_t)cnt[CNT_E]; s[LRB_S_NOVEL_SITES] = (int32_t)(cnt[CNT_D] + cnt[CNT_A]);
+    s[LRB_S_NOVEL_JUNC] = (int32_t)cnt[CNT_J]; s[LRB_S_KNOWN_GENES] = (int32_t)cnt[CNT_KG];
+    c->n_kg_pairs = (int64_t)cnt[CNT_KG];
+}
+
+int lrb_update_run(lrb_ctx *c, const lrb_update_params *up)
+{
+    if (!c || !up) return LRB_E_ARG;
+    if (!c->have_exons) return fail(c, LRB_E_ARG, "lrb_update_run: exon chains missing (run lrb_exon_run / lrb_pipeline_run / lrb_chains_upload)");
+    CK(cudaSetDevice(c->device));
+    const int64_t l0 = total_launches(), n = c->cur->n;
+    int rc;
+    memset(c->summary, 0, sizeof c->summary); c->n_bed = 0; c->last_up = *up; c->n_known = c->n_unrecog = 0; c->n_xlocus_pieces = 0;
+    if ((rc = update_classify(c, up))) return rc;
+    // A split piece scans the WHOLE of updated_T in the reference (its tid/start/end are 0, update_gtf.c:148 never stops it), so it
+    // can be absorbed by a chain on another chromosome.  The locus-parallel fold cannot see that.  With the default exact matching
+    // (-d 0, no -D) that is settled in rounds on the device (xl_* kernels in lrb_update.cu): exact and cheap.  Otherwise the set
+    // kernels probe for the necessary condition (a junction of a piece that also exists on another chromosome, CNT_XLOCUS) and the
+    // fold is then replayed once more as ONE locus (merge_fold_kernel: the exact back-scan, entry by entry).  With -d > 0 junctions
+    // match approximately and the exact-key probe proves nothing: any surviving piece sends the fold to the replay.
+    UpdateRun u{};
+    u.up = up;
+    u.xl_exact = up->split_trans != 0 && up->ss_dis == 0 && up->end_dis == 0x7fffffff && !c->force_single_fold;
+    u.detect = up->split_trans != 0 && !u.xl_exact; u.run_sets = up->want_summary || u.detect; u.single = c->force_single_fold;
+    u.cap = up->split_trans ? n + n / 8 + 1024 : n;
+    u.cap = std::max<int64_t>(u.cap, std::min<int64_t>(c->novel_cap_hint, n + c->ex.n / 2 + 1));
+    if (c->test_small_novel_cap) u.cap = std::max<int64_t>(1, n / 4);   // test hook: forces the undersized-list retry
+    for (int pass = 0; pass < 2; ++pass) {                              // the second pass is the one-locus replay
+        if ((rc = update_lists_and_folds(c, u, pass))) return rc;
+        bool settled;
+        if ((rc = update_settle_pieces(c, u, &settled))) return rc;
+        if (!settled) {                                                 // way 1 into the replay: the xl marks do not settle
+            if ((rc = join_class_folds(c, up))) return rc;
+            u.single = true; c->n_xlocus_replays++;
+            continue;
+        }
+        c->novel.n = u.n_novel; c->novel.cap = std::max<int64_t>(u.cap, 0);
+        if (c->timing && n && pass == 0) { CK(cudaStreamSynchronize(c->st)); cudaEventElapsedTime(&c->ms[LRB_T_K_FOLD], c->ev[EV_FOLD0], c->ev[EV_FOLD1]); }
+        if (!u.run_sets || n == 0) break;
+        if ((rc = update_sets(c, u))) return rc;
+        const uint32_t *cnt = c->h_scalars.as<UpdateScalars>()->counts;
+        if (u.detect && !u.single && (cnt[CNT_XLOCUS] != 0 || (up->ss_dis > 0 && cnt[CNT_PARTIAL] != 0))) {
+            u.single = true; c->n_xlocus_replays++;                     // way 2 into the replay: the probe
+            continue;
+        }
+        if (up->want_summary) update_fill_summary(c);
+        break;
     }
-    break;
-    }   // fold_pass
     tick(c, EV_UPDATED);
     c->have_update = true; c->launches_last = total_launches() - l0;
     if (c->timing) {

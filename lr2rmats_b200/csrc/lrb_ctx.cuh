@@ -166,8 +166,8 @@ struct lrb_ctx {
     int device = 0; cudaStream_t st = nullptr; std::string err;
     // side stream: work of a stage that is independent of its main chain (the class folds of the summary) runs here,
     // forked / joined with events, on its own look-back state
-    cudaStream_t st2 = nullptr; cudaEvent_t ev_fork = nullptr, ev_join = nullptr; bool side_stream = true;
-    cudaStream_t st3 = nullptr; cudaEvent_t ev_fork3 = nullptr, ev_join3 = nullptr; bool sum_split = true;   // exon chain of the summary sets
+    cudaStream_t st2 = nullptr; cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
+    cudaStream_t st3 = nullptr; cudaEvent_t ev_fork3 = nullptr, ev_join3 = nullptr;       // exon chain of the summary sets
     // tables
     DAnno anno; DSj sj; DRmIndex rm;
     lrbk::AnnoCols<Buf> anno_cols; lrbk::SjCols<Buf> sj_cols; lrbk::RmCols<Buf> rm_cols;
@@ -190,7 +190,7 @@ struct lrb_ctx {
     MergeBufs mg, mg2;
     int64_t n_known = 0, n_unrecog = 0, novel_cap_hint = 0; bool have_update = false, have_unique = false;
     int32_t summary[LRB_S_COUNT];
-    bool force_single_fold = false, test_small_novel_cap = false, xlocus_seen = false, want_kg_pairs = false; int64_t n_xlocus_replays = 0, n_xlocus_pieces = 0, n_kg_pairs = 0; Buf kg_pairs;
+    bool force_single_fold = false, test_small_novel_cap = false, want_kg_pairs = false; int64_t n_xlocus_replays = 0, n_xlocus_pieces = 0, n_kg_pairs = 0; Buf kg_pairs;
     Buf xl_key, xl_min, xl_max, xl_cnt, xl_forced; lrbk::XlArgs xl;      // split pieces that meet another chromosome (xl_* kernels)
     // summary
     Buf h_khi, y_barcnt, y_barseg, y_genebar, y_bedcnt, y_bedoff, y_counts, y_nelem;
@@ -225,7 +225,7 @@ inline int fail(lrb_ctx *c, int code, const std::string &msg) { c->err = msg; re
 
 // device scalars: [0..31] uint64 totals, then uint32 ticket, err flags.  Slots 0..7 are scratch of the stage that is
 // running; the update stage parks its results in fixed slots so that ONE copy brings them all to the host:
-enum { T_NOVEL = 8, T_KNOWN = 9, T_UNREC = 10, T_LOCI = 11, T_UPD = 12, T_LOCI2 = 13, T_UPD2 = 14, T_NELEM = 15, T_BED = 16, T_SLOTS = 32 };
+enum { T_NOVEL = 8, T_KNOWN = 9, T_UNREC = 10, T_LOCI = 11, T_UPD = 12, T_LOCI2 = 13, T_BED = 16, T_SLOTS = 32 };
 inline uint64_t *d_totals(lrb_ctx *c) { return c->scalars.as<uint64_t>(); }
 inline uint32_t *d_ticket(lrb_ctx *c) { return (uint32_t *)(c->scalars.as<uint64_t>() + T_SLOTS); }
 inline uint32_t *d_err(lrb_ctx *c) { return d_ticket(c) + 1; }

@@ -80,7 +80,6 @@ void launch_select_records(const DBatch &b, const uint8_t *pass, const int32_t *
                            uint8_t *keep_rec_mask, cudaStream_t st);
 void launch_compact_gather(const uint8_t *mask, int64_t n, const DRows &src_by_record, DRows &dst, uint32_t *keep_idx,
                            uint64_t *tile_state, uint32_t *ticket, uint64_t *total, cudaStream_t st);
-void launch_gather_rows(const DRows &src, const uint32_t *sel, int64_t n_sel, DRows &dst, cudaStream_t st);
 
 // ---- classification
 struct ClassArgs {
@@ -141,7 +140,7 @@ struct MergeArgs {
     uint8_t *hard;                                  // per locus head: 1 = not for the flat kernels, >= 2 = not for fold_big_kernel either (merge_fold_kernel)
     uint8_t *cord; uint32_t *clist; uint64_t *crow;  // big loci: class ordinal per candidate; per locus (at its offset) the class representatives and their 128-bit relation rows
     uint32_t *fb_list, *fb_cnt;                     // big loci: [0, n_cand) list of their locus ordinals, [n_cand, 2 n_cand) those that outgrew tier 0; counters
-    uint64_t *ckey; uint32_t *cmin;                 // class table of the big loci: 2 * n_cand + 64 slots (NULL: big loci go to merge_fold_kernel)
+    uint64_t *ckey; uint32_t *cmin;                 // class table of the big loci: 2 * n_cand + 64 slots
     DMerged out;                                    // compacted result
     uint8_t *forced;                                // optional (split pieces, see XlArgs): 1 = this piece is absorbed by an entry of an earlier locus when its own locus has nothing for it (3: that happened in the last fold)
     uint64_t *tile_state; uint32_t *ticket; uint64_t *totals;  // [0] n_loci, [1] n_out
@@ -169,7 +168,6 @@ void launch_sort_pass(const uint64_t *kin, const uint32_t *vin, uint64_t *kout, 
 void launch_rows_permute(const DRows &in, const DRows &out, const uint32_t *perm, cudaStream_t st);
 
 // generic device scans used by the stages above
-void launch_scan_max_u64(uint64_t *data, int64_t n, uint64_t *tile_state, uint32_t *ticket, cudaStream_t st);   // inclusive prefix max, in place
 void launch_scan_sum_u32(const uint32_t *in, uint32_t *out_excl, int64_t n, uint64_t *tile_state, uint32_t *ticket, uint64_t *total, cudaStream_t st);
 
 int64_t count_launches();   // kernels launched by this library since load (every launch_* bumps it)

@@ -58,7 +58,7 @@ static NcclApi *nccl_api(std::string *err)
 }
 
 static constexpr int META_WORDS = 40, MAX_RANKS = 64;
-enum { M_NU = 0, M_NE, M_NBED, M_NKG, M_NAME_BASE, M_XLOCUS, M_PARTIAL, M_WANT_SUMMARY, M_SUMMARY0 /* .. + LRB_S_COUNT */ };
+enum { M_NU = 0, M_NE, M_NBED, M_NKG, M_NAME_BASE, M_PARTIAL, M_WANT_SUMMARY, M_SUMMARY0 /* .. + LRB_S_COUNT */ };
 
 struct MultiState {
     NcclApi *api = nullptr; ncclComm_t comm = nullptr; int rank = 0, n_ranks = 1;
@@ -212,7 +212,7 @@ int lrb_update_gather(lrb_ctx *c, int64_t name_base)
     // ---- counts of every rank
     int64_t *mh = m->meta_host.as<int64_t>(), *mine = mh + (size_t)me * META_WORDS;
     memset(mine, 0, META_WORDS * 8);
-    mine[M_NU] = nu; mine[M_NE] = ne; mine[M_NBED] = nbed; mine[M_NKG] = nkg; mine[M_NAME_BASE] = name_base; mine[M_XLOCUS] = c->xlocus_seen ? 1 : 0;
+    mine[M_NU] = nu; mine[M_NE] = ne; mine[M_NBED] = nbed; mine[M_NKG] = nkg; mine[M_NAME_BASE] = name_base;
     mine[M_PARTIAL] = c->summary[LRB_S_NOVEL_PARTIAL]; mine[M_WANT_SUMMARY] = c->last_up.want_summary;
     for (int k = 0; k < LRB_S_COUNT; ++k) mine[M_SUMMARY0 + k] = c->summary[k];
     int64_t *md = m->meta_dev.as<int64_t>();
@@ -272,11 +272,11 @@ int lrb_update_gather(lrb_ctx *c, int64_t name_base)
     CK(cudaGetLastError());
     m->n = N; m->n_exon = NE; m->n_bed = want_summary ? NB : 0; m->daj_recomputed = false;
     memset(m->summary, 0, sizeof m->summary);
-    int64_t partial = 0; bool any_xlocus = false;
+    int64_t partial = 0;
     for (int r = 0; r < R; ++r) {
         const int64_t *x = mh + (size_t)r * META_WORDS;
         for (int k = 0; k < LRB_S_COUNT; ++k) m->summary[k] += (int32_t)x[M_SUMMARY0 + k];
-        partial += x[M_PARTIAL]; any_xlocus = any_xlocus || x[M_XLOCUS] != 0;
+        partial += x[M_PARTIAL];
     }
     const bool detect = c->last_up.split_trans != 0;
     if (N > 0 && (want_summary || detect)) {
@@ -338,7 +338,6 @@ int lrb_update_gather(lrb_ctx *c, int64_t name_base)
             if (pass == 0 && hp[16] == 0) break;
         }
     }
-    (void)any_xlocus;
     CK(cudaEventRecord(m->ev[2], c->st));
     CK(cudaStreamSynchronize(c->st));
     CK(cudaEventElapsedTime(&m->ms_gather, m->ev[0], m->ev[1])); CK(cudaEventElapsedTime(&m->ms_merge, m->ev[1], m->ev[2]));

@@ -696,61 +696,8 @@ void launch_compact_mask(const uint8_t *mask, int64_t n, const uint32_t *map, ui
     LRB_COUNT_LAUNCH();
 }
 
-// ------------------------------------------------------------------------------------------------ row gather
-__global__ void gather_rows_kernel(DRows src, const uint32_t *__restrict__ sel, int64_t n_sel, DRows dst)
-{
-    int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= n_sel) return;
-    uint32_t s = sel[k];
-    dst.read_idx[k] = src.read_idx[s]; dst.tid[k] = src.tid[s]; dst.start[k] = src.start[s]; dst.end[k] = src.end[s];
-    dst.is_rev[k] = src.is_rev[s]; dst.ex_beg[k] = src.ex_beg[s]; dst.ex_n[k] = src.ex_n[s];
-}
-void launch_gather_rows(const DRows &src, const uint32_t *sel, int64_t n_sel, DRows &dst, cudaStream_t st)
-{
-    if (n_sel <= 0) return;
-    int th = 256; int64_t bl = (n_sel + th - 1) / th;
-    gather_rows_kernel<<<(unsigned)bl, th, 0, st>>>(src, sel, n_sel, dst);
-    LRB_COUNT_LAUNCH();
-}
-
 // ----------------------------------------------------------------------------------------------- generic scans
 static constexpr int GS_THREADS = 256, GS_ITEMS = 8;
-__global__ void __launch_bounds__(GS_THREADS) scan_max_u64_kernel(uint64_t *data, int64_t n, uint64_t *tile_state, uint32_t *ticket)
-{
-    __shared__ uint64_t s_w[GS_THREADS / 32]; __shared__ uint32_t s_tile; __shared__ uint64_t s_excl;
-    if (threadIdx.x == 0) s_tile = atomicAdd(ticket, 1u);
-    __syncthreads();
-    const int tile = (int)s_tile, lane = lane_id(), w = warp_id();
-    const int64_t base = ((int64_t)tile * GS_THREADS + threadIdx.x) * GS_ITEMS;
-    uint64_t v[GS_ITEMS], run = 0;
-#pragma unroll
-    for (int i = 0; i < GS_ITEMS; ++i) { v[i] = (base + i < n) ? data[base + i] : 0; run = v[i] > run ? v[i] : run; v[i] = run; }
-    uint64_t inc = run;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { uint64_t t = __shfl_up_sync(FULL, inc, o); if (lane >= o && t > inc) inc = t; }
-    if (lane == 31) s_w[w] = inc;
-    __syncthreads();
-    uint64_t pre = 0;                                            // max over warps before mine
-    for (int k = 0; k < w; ++k) pre = s_w[k] > pre ? s_w[k] : pre;
-    uint64_t tot = 0;
-    for (int k = 0; k < GS_THREADS / 32; ++k) tot = s_w[k] > tot ? s_w[k] : tot;
-    uint64_t left = __shfl_up_sync(FULL, inc, 1); if (lane == 0) left = 0;
-    uint64_t tpre = left > pre ? left : pre;                     // exclusive prefix max of this thread inside the tile
-    if (w == 0) { uint64_t e = lookback_exclusive(tile_state, tile, tot, OpMax()); if (lane == 0) s_excl = e; }
-    __syncthreads();
-    uint64_t ex = s_excl > tpre ? s_excl : tpre;
-#pragma unroll
-    for (int i = 0; i < GS_ITEMS; ++i) if (base + i < n) data[base + i] = v[i] > ex ? v[i] : ex;
-}
-void launch_scan_max_u64(uint64_t *data, int64_t n, uint64_t *tile_state, uint32_t *ticket, cudaStream_t st)
-{
-    if (n <= 0) return;
-    int64_t per = (int64_t)GS_THREADS * GS_ITEMS, bl = (n + per - 1) / per;
-    cudaMemsetAsync(tile_state, 0, (size_t)bl * 8, st); cudaMemsetAsync(ticket, 0, 4, st);
-    scan_max_u64_kernel<<<(unsigned)bl, GS_THREADS, 0, st>>>(data, n, tile_state, ticket);
-    LRB_COUNT_LAUNCH();
-}
-
 __global__ void __launch_bounds__(GS_THREADS) scan_sum_u32_kernel(const uint32_t *__restrict__ in, uint32_t *out, int64_t n,
                                                                   uint64_t *tile_state, uint32_t *ticket, uint64_t *total)
 {

@@ -81,6 +81,23 @@ __global__ void __launch_bounds__(256) sj_reduce_kernel(const int32_t *__restric
     o_tid[k] = tid[s]; o_don[k] = don[s]; o_acc[k] = acc[s]; o_u[k] = u; o_m[k] = (int)(hi - lo) - u;
 }
 
+// Stable sort of n records by three keys (k0, k1, k2; most significant first, compared as unsigned): 4 radix passes over k2, then 8 over
+// k0 << 32 | k1.  *perm <- the sorted order (in s_idx0 / s_idx1).
+static int sort3_device(lrb_ctx *c, const int32_t *k0, const int32_t *k1, const int32_t *k2, int64_t n, const uint32_t **perm)
+{
+    const size_t m = (size_t)n;
+    NEED(c->s_key0, m * 8); NEED(c->s_key1, m * 8); NEED(c->s_idx0, m * 4); NEED(c->s_idx1, m * 4); NEED(c->s_hist, (size_t)256 * (size_t)sort_tiles(n) * 4);
+    uint64_t *k[2] = {c->s_key0.as<uint64_t>(), c->s_key1.as<uint64_t>()}; uint32_t *v[2] = {c->s_idx0.as<uint32_t>(), c->s_idx1.as<uint32_t>()};
+    const unsigned bl = (unsigned)((n + 255) / 256);
+    int cur = 0;
+    sj_key_kernel<<<bl, 256, 0, c->st>>>(k0, k1, k2, nullptr, k[0], v[0], n, 0);
+    for (int shift = 0; shift < 32; shift += 8) { launch_sort_pass(k[cur], v[cur], k[cur ^ 1], v[cur ^ 1], n, shift, c->s_hist.as<uint32_t>(), c->st); cur ^= 1; }
+    sj_key_kernel<<<bl, 256, 0, c->st>>>(k0, k1, k2, v[cur], k[cur], nullptr, n, 1);
+    for (int shift = 0; shift < 64; shift += 8) { launch_sort_pass(k[cur], v[cur], k[cur ^ 1], v[cur ^ 1], n, shift, c->s_hist.as<uint32_t>(), c->st); cur ^= 1; }
+    *perm = v[cur];
+    return LRB_OK;
+}
+
 }  // namespace lrbk
 using namespace lrbk;
 
@@ -114,25 +131,19 @@ extern "C" int lrb_bam2sj(lrb_ctx *c, const lrb_batch *b, const uint8_t *is_uniq
     if (nj) {
         const size_t m = (size_t)nj;
         NEED(c->j_tid, m * 4); NEED(c->j_don, m * 4); NEED(c->j_acc, m * 4); NEED(c->j_u, m); NEED(c->j_head, m); NEED(c->j_hpos, m * 4);
-        NEED(c->s_key0, m * 8); NEED(c->s_key1, m * 8); NEED(c->s_idx0, m * 4); NEED(c->s_idx1, m * 4); NEED(c->s_hist, (size_t)256 * (size_t)sort_tiles(nj) * 4);
         if ((rc = ensure_tiles(c, nj))) return rc;
         a.j_tid = c->j_tid.as<int32_t>(); a.j_don = c->j_don.as<int32_t>(); a.j_acc = c->j_acc.as<int32_t>(); a.j_uniq = c->j_u.as<uint8_t>();
         sj_emit_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->st>>>(a);
-        uint64_t *k[2] = {c->s_key0.as<uint64_t>(), c->s_key1.as<uint64_t>()}; uint32_t *v[2] = {c->s_idx0.as<uint32_t>(), c->s_idx1.as<uint32_t>()};
-        const unsigned bl = (unsigned)((nj + 255) / 256);
-        int cur = 0;
-        sj_key_kernel<<<bl, 256, 0, c->st>>>(a.j_tid, a.j_don, a.j_acc, nullptr, k[0], v[0], nj, 0);
-        for (int shift = 0; shift < 32; shift += 8) { launch_sort_pass(k[cur], v[cur], k[cur ^ 1], v[cur ^ 1], nj, shift, c->s_hist.as<uint32_t>(), c->st); cur ^= 1; }
-        sj_key_kernel<<<bl, 256, 0, c->st>>>(a.j_tid, a.j_don, a.j_acc, v[cur], k[cur], nullptr, nj, 1);
-        for (int shift = 0; shift < 64; shift += 8) { launch_sort_pass(k[cur], v[cur], k[cur ^ 1], v[cur ^ 1], nj, shift, c->s_hist.as<uint32_t>(), c->st); cur ^= 1; }
-        sj_heads_kernel<<<bl, 256, 0, c->st>>>(a.j_tid, a.j_don, a.j_acc, v[cur], c->j_head.as<uint8_t>(), nj);
+        const uint32_t *perm;
+        if ((rc = sort3_device(c, a.j_tid, a.j_don, a.j_acc, nj, &perm))) return rc;
+        sj_heads_kernel<<<(unsigned)((nj + 255) / 256), 256, 0, c->st>>>(a.j_tid, a.j_don, a.j_acc, perm, c->j_head.as<uint8_t>(), nj);
         launch_compact_mask(c->j_head.as<uint8_t>(), nj, nullptr, c->j_hpos.as<uint32_t>(), nullptr, c->tile_state.as<uint64_t>(), d_ticket(c), d_totals(c), c->st);
         CK(cudaGetLastError());
         uint64_t t; if ((rc = read_totals(c, &t, 1))) return rc;
         nd = (int64_t)t;
         JuncCols<Buf> &o = c->junc;
         if ((rc = ensure(c, o, Extent{nd}))) return rc;
-        sj_reduce_kernel<<<(unsigned)((nd + 255) / 256), 256, 0, c->st>>>(a.j_tid, a.j_don, a.j_acc, a.j_uniq, v[cur], c->j_hpos.as<uint32_t>(), nd, nj,
+        sj_reduce_kernel<<<(unsigned)((nd + 255) / 256), 256, 0, c->st>>>(a.j_tid, a.j_don, a.j_acc, a.j_uniq, perm, c->j_hpos.as<uint32_t>(), nd, nj,
                                                                              o.tid.as<int32_t>(), o.don.as<int32_t>(), o.acc.as<int32_t>(), o.uniq_c.as<int32_t>(), o.multi_c.as<int32_t>());
         CK(cudaGetLastError());
         if ((rc = copy(c, c->out_junc, o, Extent{nd}, cudaMemcpyDeviceToHost))) return rc;
@@ -156,16 +167,10 @@ extern "C" int lrb_sort3(lrb_ctx *c, const uint32_t *k0, const uint32_t *k1, con
     const size_t m = (size_t)n; int rc;
     // the three key columns ride in the junction buffers (tid = k0, don = k1, acc = k2)
     if ((rc = h2d(c, c->j_tid, (const int32_t *)k0, m)) || (rc = h2d(c, c->j_don, (const int32_t *)k1, m)) || (rc = h2d(c, c->j_acc, (const int32_t *)k2, m))) return rc;
-    NEED(c->s_key0, m * 8); NEED(c->s_key1, m * 8); NEED(c->s_idx0, m * 4); NEED(c->s_idx1, m * 4); NEED(c->s_hist, (size_t)256 * (size_t)sort_tiles(n) * 4);
-    uint64_t *k[2] = {c->s_key0.as<uint64_t>(), c->s_key1.as<uint64_t>()}; uint32_t *v[2] = {c->s_idx0.as<uint32_t>(), c->s_idx1.as<uint32_t>()};
-    const unsigned bl = (unsigned)((n + 255) / 256);
-    int cur = 0;
-    sj_key_kernel<<<bl, 256, 0, c->st>>>(c->j_tid.as<int32_t>(), c->j_don.as<int32_t>(), c->j_acc.as<int32_t>(), nullptr, k[0], v[0], n, 0);
-    for (int shift = 0; shift < 32; shift += 8) { launch_sort_pass(k[cur], v[cur], k[cur ^ 1], v[cur ^ 1], n, shift, c->s_hist.as<uint32_t>(), c->st); cur ^= 1; }
-    sj_key_kernel<<<bl, 256, 0, c->st>>>(c->j_tid.as<int32_t>(), c->j_don.as<int32_t>(), c->j_acc.as<int32_t>(), v[cur], k[cur], nullptr, n, 1);
-    for (int shift = 0; shift < 64; shift += 8) { launch_sort_pass(k[cur], v[cur], k[cur ^ 1], v[cur ^ 1], n, shift, c->s_hist.as<uint32_t>(), c->st); cur ^= 1; }
+    const uint32_t *sorted;
+    if ((rc = sort3_device(c, c->j_tid.as<int32_t>(), c->j_don.as<int32_t>(), c->j_acc.as<int32_t>(), n, &sorted))) return rc;
     CK(cudaGetLastError());
-    if ((rc = d2h(c, c->out_perm, v[cur], m))) return rc;
+    if ((rc = d2h(c, c->out_perm, sorted, m))) return rc;
     CK(cudaStreamSynchronize(c->st));
     *perm = c->out_perm.as<uint32_t>();
     c->launches_last = total_launches() - l0;

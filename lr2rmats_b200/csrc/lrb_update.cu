@@ -1423,29 +1423,26 @@ void launch_merge_fold(const MergeArgs &a, cudaStream_t st)
         // loci beyond the masks and the ones the flat kernels gave up on: classes through one table, then warp per locus with the survivors
         // in shared memory; what outgrows the slots there (hard >= 2) is replayed from global memory
         int64_t bl2 = (a.n_cand / (FF_MAX + 1) + 1 + 3) / 4 + 8; if (bl2 > 148 * 8) bl2 = 148 * 8;
-        if (a.ckey) {
-            using S0 = FbSlots<128, 256>; using S1 = FbSlots<416, 1024>;
-            auto k0 = fold_big_kernel<32, 128, 256, 0>; auto k1 = fold_big_kernel<32, 416, 1024, 1>;
-            const size_t smem0 = sizeof(S0) * (FB_THREADS / 32), smem1 = sizeof(S1) * (FB_THREADS / 32);
-            static bool attr = false;
-            if (!attr) { cudaFuncSetAttribute(k0, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem0); cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1); attr = true; }
-            ClassTab tab{(unsigned long long *)a.ckey, a.cmin, (uint64_t)a.n_cand * 2 + 64};
-            cudaMemsetAsync(a.ckey, 0xFF, tab.cap * 8, st); cudaMemsetAsync(a.cmin, 0xFF, tab.cap * 4, st);
-            cudaMemsetAsync(a.fb_cnt, 0, 32, st);                     // [0] big loci, [1] tier-0 claims, [2] tier-0 overflows, [3] tier-1 claims
-            int64_t blm = (a.n_cand / 8 + 255) / 256 + 1; if (blm > 148 * 8) blm = 148 * 8;
-            fold_big_mark_kernel<<<(unsigned)blm, 256, 0, st>>>(a, a.hard, a.lstart); LRB_COUNT_LAUNCH();
-            fold_class_insert_kernel<<<bl, 256, 0, st>>>(a, tab, a.lstart); LRB_COUNT_LAUNCH();
-            fold_class_verify_kernel<<<bl, 256, 0, st>>>(a, tab, a.rep, a.lstart, a.hard); LRB_COUNT_LAUNCH();
-            fold_class_rows_kernel<<<(unsigned)blm, 256, 0, st>>>(a, a.rep, a.hard, a.fb_cnt + 4); LRB_COUNT_LAUNCH();
-            // one warp per locus, loci claimed from the lists: a whole warp measured fastest (8 / 16 lanes per locus: 17.5 / 15.8 ms per
-            // step against 14.2 ms on the 10 M-read data set -- the lane groups of a warp diverge)
-            int64_t blb = (a.n_cand / (FF_MAX + 1) + 1) / (FB_THREADS / 32) + 1; if (blb > 148 * 6) blb = 148 * 6;
-            k0<<<(unsigned)blb, FB_THREADS, smem0, st>>>(a, a.rep, a.dropped, a.hard, a.fb_cnt + 1); LRB_COUNT_LAUNCH();
-            if (blb > 148 * 2) blb = 148 * 2;
-            k1<<<(unsigned)blb, FB_THREADS, smem1, st>>>(a, a.rep, a.dropped, a.hard, a.fb_cnt + 3); LRB_COUNT_LAUNCH();
-            merge_fold_kernel<32><<<(unsigned)bl2, MF_THREADS, 0, st>>>(a, (uint32_t *)a.keys, a.dropped, a.hard, 0x7fffffff, 0x7fffffff, (1 << 2) | (1 << 3));
-        } else
-            merge_fold_kernel<32><<<(unsigned)bl2, MF_THREADS, 0, st>>>(a, (uint32_t *)a.keys, a.dropped, a.hard, FF_MAX + 1, 0x7fffffff, 0xFE);
+        using S0 = FbSlots<128, 256>; using S1 = FbSlots<416, 1024>;
+        auto k0 = fold_big_kernel<32, 128, 256, 0>; auto k1 = fold_big_kernel<32, 416, 1024, 1>;
+        const size_t smem0 = sizeof(S0) * (FB_THREADS / 32), smem1 = sizeof(S1) * (FB_THREADS / 32);
+        static bool attr = false;
+        if (!attr) { cudaFuncSetAttribute(k0, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem0); cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1); attr = true; }
+        ClassTab tab{(unsigned long long *)a.ckey, a.cmin, (uint64_t)a.n_cand * 2 + 64};
+        cudaMemsetAsync(a.ckey, 0xFF, tab.cap * 8, st); cudaMemsetAsync(a.cmin, 0xFF, tab.cap * 4, st);
+        cudaMemsetAsync(a.fb_cnt, 0, 32, st);                     // [0] big loci, [1] tier-0 claims, [2] tier-0 overflows, [3] tier-1 claims
+        int64_t blm = (a.n_cand / 8 + 255) / 256 + 1; if (blm > 148 * 8) blm = 148 * 8;
+        fold_big_mark_kernel<<<(unsigned)blm, 256, 0, st>>>(a, a.hard, a.lstart); LRB_COUNT_LAUNCH();
+        fold_class_insert_kernel<<<bl, 256, 0, st>>>(a, tab, a.lstart); LRB_COUNT_LAUNCH();
+        fold_class_verify_kernel<<<bl, 256, 0, st>>>(a, tab, a.rep, a.lstart, a.hard); LRB_COUNT_LAUNCH();
+        fold_class_rows_kernel<<<(unsigned)blm, 256, 0, st>>>(a, a.rep, a.hard, a.fb_cnt + 4); LRB_COUNT_LAUNCH();
+        // one warp per locus, loci claimed from the lists: a whole warp measured fastest (8 / 16 lanes per locus: 17.5 / 15.8 ms per
+        // step against 14.2 ms on the 10 M-read data set -- the lane groups of a warp diverge)
+        int64_t blb = (a.n_cand / (FF_MAX + 1) + 1) / (FB_THREADS / 32) + 1; if (blb > 148 * 6) blb = 148 * 6;
+        k0<<<(unsigned)blb, FB_THREADS, smem0, st>>>(a, a.rep, a.dropped, a.hard, a.fb_cnt + 1); LRB_COUNT_LAUNCH();
+        if (blb > 148 * 2) blb = 148 * 2;
+        k1<<<(unsigned)blb, FB_THREADS, smem1, st>>>(a, a.rep, a.dropped, a.hard, a.fb_cnt + 3); LRB_COUNT_LAUNCH();
+        merge_fold_kernel<32><<<(unsigned)bl2, MF_THREADS, 0, st>>>(a, (uint32_t *)a.keys, a.dropped, a.hard, 0x7fffffff, 0x7fffffff, (1 << 2) | (1 << 3));
         LRB_COUNT_LAUNCH();
         return;
     }

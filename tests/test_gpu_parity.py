@@ -499,25 +499,31 @@ def test_single_locus_replay_equals_locus_fold(tmp_path):
 def test_cross_chromosome_piece_replay(ctx, summary):
     """Every read twice, on chromosomes 1-2 and on clones of them at the same coordinates: the split pieces of the clones meet equal
     chains on the originals, which the reference merges across chromosomes (a piece's back-scan never stops, update_gtf.c:148; golden
-    c8_xlocus).  The set kernels must notice and the fold must be replayed as one locus: every table equals the port's."""
+    c8_xlocus).  The fold must notice, and every table equals the port's.  With -d 0 the pieces are settled by rounds on the device;
+    with -d 2 junctions match approximately, the probe of the set kernels proves nothing and the fold is replayed as one locus."""
     anno = synth.make_annotation(1500, n_chrom=2, seed=41)
     reads = synth.make_reads(anno, 12_000, seed=43, reject_frac=0.0)
     sj = synth.make_sj_from_reads(reads, frac=0.7, seed=44)
     a2, both, s2 = synth.clone_chromosome(anno.soa(), reads, sj, 2)
     ep = cabi.ExonParams.default()
-    up = cabi.UpdateParams.default(full_level=3, split_trans=1, min_sj_cnt=1, want_summary=summary)
     oex = op.bam2gtf(both.soa(), ep)
-    rc, ou = op.update(oex, a2, s2, up)
-    assert rc == 0
     ctx.set_anno(a2); ctx.set_sj(s2)
-    gu = ctx.update_gtf(both.soa(), ep, up)
-    ou["ex"]["read_idx"] = gu["ex"]["read_idx"]
-    assert_dict_equal(gu, ou)
-    # the case is live: at least one piece of a clone chromosome was absorbed by an original (cov > 1 on a piece)
-    upd = gu["updated"]; piece = gu["novel"]["piece"][upd["cand"]]
-    assert ((piece >= 0) & (upd["cov"] > 1)).sum() > 0
-    d = ctx.update_diag()
-    assert d["pieces_across_chromosomes"] > 0, d         # settled by the rounds on the device, not by the one-locus replay
+    for ss_dis in (0, 2):
+        up = cabi.UpdateParams.default(full_level=3, split_trans=1, min_sj_cnt=1, want_summary=summary, ss_dis=ss_dis)
+        rc, ou = op.update(oex, a2, s2, up)
+        assert rc == 0
+        replays = ctx.update_diag()["one_locus_replays"]
+        gu = ctx.update_gtf(both.soa(), ep, up)
+        ou["ex"]["read_idx"] = gu["ex"]["read_idx"]
+        assert_dict_equal(gu, ou, f"-d {ss_dis}")
+        # the case is live: at least one piece of a clone chromosome was absorbed by an original (cov > 1 on a piece)
+        upd = gu["updated"]; piece = gu["novel"]["piece"][upd["cand"]]
+        assert ((piece >= 0) & (upd["cov"] > 1)).sum() > 0, ss_dis
+        d = ctx.update_diag()
+        if ss_dis == 0:
+            assert d["pieces_across_chromosomes"] > 0, d     # settled by the rounds on the device, not by the one-locus replay
+        else:
+            assert d["one_locus_replays"] > replays, d       # the detect probe sent the fold to the one-locus replay
 
 
 @pytest.mark.parametrize("which", ["iso", "ont"])
