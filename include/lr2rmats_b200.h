@@ -20,6 +20,7 @@
  *   bam2sj  lrb_bam2sj
  *   sort3   lrb_sort3
  *   gather  lrb_gather_fetch
+ *   gather reads  lrb_gather_fetch_reads
  */
 #ifndef LR2RMATS_B200_H
 #define LR2RMATS_B200_H
@@ -344,6 +345,13 @@ void lrb_host_free(void *p);
  *      recomputed / unioned over the gathered table, the piece-aware tid-0 sets (update_gtf.c:421-534, SURVEY A.8)
  *      recomputed when two shards share a tid-0 key;
  *   6. lrb_gather_fetch on rank 0: the result exactly as one GPU (and the reference) would produce it for the whole stream.
+ *
+ * The per-read outputs (update-gtf -a/-A/-k/-v/-u, the records `lr2rmats filter` writes) need no merge: every row is a function
+ * of its read and the replicated tables, and shards never cut a qname run, so the shards' results concatenate (App. B.3):
+ *   5'. lrb_update_gather_reads: per-shard bam_T chains, class words, known / unrecog / novel lists, updated_T entries and
+ *       the filter's per-record results go to rank 0 (count all-gather + send/recv gatherv), which shifts their row / exon /
+ *       record indices to the whole stream;
+ *   6'. lrb_gather_fetch_reads on rank 0: what lrb_update_fetch / lrb_filter_fetch return on one GPU for the whole stream.
  */
 #define LRB_COMM_ID_BYTES 128
 int lrb_comm_id(void *id_out /* LRB_COMM_ID_BYTES */);
@@ -358,6 +366,15 @@ int lrb_update_gather(lrb_ctx *ctx, int64_t name_base);
 /* rank 0: merged updated_T + BED rows + summary (anno counters [0],[1] left 0); other ranks: empty.  Any argument may be NULL. */
 int lrb_gather_fetch(lrb_ctx *ctx, lrb_trans_table *updated, lrb_bed_list *bed, int32_t summary[LRB_S_COUNT]);
 int lrb_gather_timing(lrb_ctx *ctx, float *ms_gather, float *ms_merge);   /* CUDA-event times of the last lrb_update_gather */
+/* collective, after lrb_update_run on every rank (each on its shard of ONE stream); name_base as for lrb_update_gather.
+ * Does not depend on the outcome of lrb_update_gather: every rank may call it even where the root got LRB_E_XSHARD.
+ * LRB_E_ARG on every rank when the gathered results exceed 2^32 exons or records. */
+int lrb_update_gather_reads(lrb_ctx *ctx, int64_t name_base);
+/* rank 0: what lrb_update_fetch / lrb_filter_fetch return on ONE GPU for the whole stream; other ranks: zeroed, LRB_OK.
+ * Either argument may be NULL.  update: ex.read_idx is NULL when the shards were chains (lrb_chains_upload); its BED rows and
+ * summary come from lrb_update_gather, which must have succeeded after the same lrb_update_run (LRB_E_ARG otherwise).  filter: LRB_E_ARG unless
+ * the filter stage ran on every shard (lrb_pipeline_run / lrb_filter_run). */
+int lrb_gather_fetch_reads(lrb_ctx *ctx, lrb_update_result *update, lrb_filter_result *filter);
 
 /* Read shards are cut at locus gaps (SURVEY App. B.3: where a read starts beyond every earlier end on its chromosome the
  * outputs concatenate exactly); this helper finds n_shards-1 such cuts near the ideal boundaries on the host.

@@ -23,7 +23,8 @@ ENTRY_POINTS = [
     "lrb_update_gtf", "lrb_unique_gtf", "lrb_timing_enable", "lrb_timing_get", "lrb_launch_count", "lrb_shard_cuts",
     "lrb_mark", "lrb_elapsed_ms", "lrb_host_alloc", "lrb_host_free", "lrb_update_fetch_table", "lrb_filter_fetch_keep",
     "lrb_comm_id", "lrb_comm_init", "lrb_comm_destroy", "lrb_comm_rank", "lrb_tables_broadcast", "lrb_update_gather", "lrb_gather_fetch",
-    "lrb_gather_timing", "lrb_shard_cuts_weighted", "lrb_update_diag", "lrb_bam2sj", "lrb_sort3",
+    "lrb_gather_timing", "lrb_shard_cuts_weighted", "lrb_update_diag", "lrb_bam2sj", "lrb_sort3", "lrb_update_gather_reads",
+    "lrb_gather_fetch_reads",
 ]
 
 T_NAMES = ["filter", "exon", "classify", "merge", "summary", "k_scan", "k_fold"]
@@ -91,6 +92,8 @@ def load_library():
     L.lrb_update_gather.argtypes = [vp, C.c_int64]
     L.lrb_gather_fetch.argtypes = [vp, P(cabi.TransTable), P(cabi.BedList), P(C.c_int32 * cabi.S_COUNT)]
     L.lrb_gather_timing.argtypes = [vp, P(C.c_float), P(C.c_float)]
+    L.lrb_update_gather_reads.argtypes = [vp, C.c_int64]
+    L.lrb_gather_fetch_reads.argtypes = [vp, P(cabi.UpdateResult), P(cabi.FilterResult)]
     L.lrb_update_diag.argtypes = [vp, P(C.c_int64), P(C.c_int64)]
     L.lrb_bam2sj.argtypes = [vp, P(cabi.Batch), cabi.u8p, P(cabi.SjParams), P(cabi.Sj)]
     L.lrb_sort3.argtypes = [vp, cabi.u32p, cabi.u32p, cabi.u32p, C.c_int64, P(cabi.u32p)]
@@ -254,6 +257,17 @@ class Context:
         if raw:
             return t, b, s
         return dict(table=cabi.table_to_np(t), bed=cabi.bed_to_np(b) if want_bed else None, summary=np.array(list(s), np.int32))
+
+    def update_gather_reads(self, name_base: int): self._ck(self.L.lrb_update_gather_reads(self.h, int(name_base)))
+
+    def gather_fetch_reads(self, want_filter=True, want_update=True, raw=False):
+        """Rank 0: the per-read results of the whole stream, as update_fetch() / filter_fetch() give them on one GPU; other ranks: empty."""
+        u = cabi.UpdateResult() if want_update else None
+        f = cabi.FilterResult() if want_filter else None
+        self._ck(self.L.lrb_gather_fetch_reads(self.h, C.byref(u) if u is not None else None, C.byref(f) if f is not None else None))
+        if raw:
+            return u, f
+        return dict(update=cabi.update_to_np(u) if u is not None else None, filter=cabi.filter_to_np(f) if f is not None else None)
 
     def gather_timing(self):
         a = C.c_float(); b = C.c_float(); self._ck(self.L.lrb_gather_timing(self.h, C.byref(a), C.byref(b))); return float(a.value), float(b.value)

@@ -667,6 +667,7 @@ int lrb_update_run(lrb_ctx *c, const lrb_update_params *up)
     const int64_t l0 = total_launches(), n = c->cur->n;
     int rc;
     memset(c->summary, 0, sizeof c->summary); c->n_bed = 0; c->last_up = *up; c->n_known = c->n_unrecog = 0; c->n_xlocus_pieces = 0;
+    ++c->update_gen;
     if ((rc = update_classify(c, up))) return rc;
     // A split piece scans the WHOLE of updated_T in the reference (its tid/start/end are 0, update_gtf.c:148 never stops it), so it
     // can be absorbed by a chain on another chromosome.  The locus-parallel fold cannot see that.  With the default exact matching
@@ -833,34 +834,46 @@ __global__ void exon_gather_kernel(DRows rows, DExons ex, const uint32_t *__rest
     for (uint32_t j = 0; j < n; ++j) { es[o + j] = ex.es[b + j]; ee[o + j] = ex.ee[b + j]; if (with_flags) fl[o + j] = ex.flag[b + j]; }
 }
 
+}  // extern "C" (reopened below)
+
+int lrbk::compact_exons(lrb_ctx *c, bool with_flags, CompactExons *out)
+{
+    DRows &rows = *c->cur; const int64_t n = rows.n; int rc;
+    *out = CompactExons{rows.ex_beg, c->ex.es, c->ex.ee, c->ex.flag, c->ex.n};
+    if (c->rows_compact) return LRB_OK;
+    // exclusive scan of ex_n -> offsets, then gather into scratch (the summary hash buffers are free at fetch time)
+    if ((rc = ensure_tiles(c, n))) return rc;
+    NEED(c->u_sub, ((size_t)n + 1) * 4);
+    launch_scan_sum_u32(rows.ex_n, c->u_sub.as<uint32_t>(), n, c->tile_state.as<uint64_t>(), d_ticket(c), d_totals(c), c->st);
+    uint64_t t; if ((rc = read_totals(c, &t, 1))) return rc;
+    const int64_t ne = n ? (int64_t)t : 0;
+    const size_t k = (size_t)std::max<int64_t>(ne, 1);
+    NEED(c->y_barcnt, k * 4); NEED(c->y_barseg, k * 4); NEED(c->y_bedcnt, k);
+    *out = CompactExons{c->u_sub.as<uint32_t>(), c->y_barcnt.as<int32_t>(), c->y_barseg.as<int32_t>(), c->y_bedcnt.as<uint8_t>(), ne};
+    if (n) {
+        exon_gather_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->st>>>(rows, c->ex, out->off, (int32_t *)out->es, (int32_t *)out->ee,
+                                                                              (uint8_t *)out->flag, with_flags ? 1 : 0);
+        CK(cudaGetLastError());
+    }
+    return LRB_OK;
+}
+
+extern "C" {
+
 static int fetch_exons(lrb_ctx *c, ExonsOut &o, lrb_exon_result *out, bool with_flags, const uint8_t **flags_out)
 {
     DRows &rows = *c->cur; const int64_t n = rows.n; int rc;
     if ((rc = d2h(c, o.read_idx, rows.read_idx, (size_t)n))) return rc;
     if ((rc = d2h(c, o.tid, rows.tid, (size_t)n))) return rc;
     if ((rc = d2h(c, o.is_rev, rows.is_rev, (size_t)n))) return rc;
-    int64_t ne = c->ex.n;
-    int32_t *es = c->ex.es, *ee = c->ex.ee; uint8_t *fl = c->ex.flag; uint32_t *off = rows.ex_beg;
     NEEDP(o.off, ((size_t)n + 1) * 4);
-    if (!c->rows_compact) {
-        // exclusive scan of ex_n -> offsets, then gather into scratch (the summary hash buffers are free at fetch time)
-        if ((rc = ensure_tiles(c, n))) return rc;
-        NEED(c->u_sub, ((size_t)n + 1) * 4);
-        launch_scan_sum_u32(rows.ex_n, c->u_sub.as<uint32_t>(), n, c->tile_state.as<uint64_t>(), d_ticket(c), d_totals(c), c->st);
-        uint64_t t; if ((rc = read_totals(c, &t, 1))) return rc;
-        ne = n ? (int64_t)t : 0;
-        const size_t k = (size_t)std::max<int64_t>(ne, 1);
-        NEED(c->y_barcnt, k * 4); NEED(c->y_barseg, k * 4); NEED(c->y_bedcnt, k);
-        es = c->y_barcnt.as<int32_t>(); ee = c->y_barseg.as<int32_t>(); fl = c->y_bedcnt.as<uint8_t>(); off = c->u_sub.as<uint32_t>();
-        if (n) {
-            exon_gather_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->st>>>(rows, c->ex, off, es, ee, fl, with_flags ? 1 : 0);
-            CK(cudaGetLastError());
-        }
-    }
-    if (n) CK(cudaMemcpyAsync(o.off.p, off, (size_t)n * 4, cudaMemcpyDeviceToHost, c->st));
-    if ((rc = d2h(c, o.es, es, (size_t)ne))) return rc;
-    if ((rc = d2h(c, o.ee, ee, (size_t)ne))) return rc;
-    if (with_flags && (rc = d2h(c, o.flag, fl, (size_t)ne))) return rc;
+    CompactExons ce;
+    if ((rc = compact_exons(c, with_flags, &ce))) return rc;
+    const int64_t ne = ce.n_exon;
+    if (n) CK(cudaMemcpyAsync(o.off.p, ce.off, (size_t)n * 4, cudaMemcpyDeviceToHost, c->st));
+    if ((rc = d2h(c, o.es, ce.es, (size_t)ne))) return rc;
+    if ((rc = d2h(c, o.ee, ce.ee, (size_t)ne))) return rc;
+    if (with_flags && (rc = d2h(c, o.flag, ce.flag, (size_t)ne))) return rc;
     CK(cudaStreamSynchronize(c->st));
     o.off.as<uint32_t>()[n] = (uint32_t)ne;
     out->n_reads = n; out->read_idx = c->have_batch ? o.read_idx.as<uint32_t>() : nullptr; out->tid = o.tid.as<int32_t>();
@@ -876,13 +889,6 @@ int lrb_exon_fetch(lrb_ctx *c, lrb_exon_result *out)
     if (!c->have_exons) return fail(c, LRB_E_ARG, "lrb_exon_fetch: exon stage has not run");
     CK(cudaSetDevice(c->device));
     return fetch_exons(c, c->out_exons, out, false, nullptr);
-}
-
-static lrb_merged_list merged_result(const MergedCols<PBuf> &h, int64_t n)
-{
-    lrb_merged_list o; o.n = n; o.cand = h.cand.as<uint32_t>(); o.cov = h.cov.as<int32_t>(); o.t_tid = h.tid.as<int32_t>(); o.t_start = h.start.as<int32_t>();
-    o.t_end = h.end.as<int32_t>(); o.first_start = h.fs.as<int32_t>(); o.last_end = h.le.as<int32_t>();
-    return o;
 }
 
 int lrb_update_fetch(lrb_ctx *c, lrb_update_result *out)

@@ -119,6 +119,18 @@ template <class B> struct BedCols {                 // lrb_bed_list
         f(ROW, 4, g.tid...); f(ROW, 4, g.start...); f(ROW, 4, g.end...); f(ROW, 4, g.score...); f(ROW, 1, g.type...); f(ROW, 1, g.is_rev...);
     }
 };
+template <class B> struct ReadCols {                // lrb_update_result's per-read part: bam_T chains (lrb_exon_result), class words, flags
+    B read_idx, tid, is_rev, cls, ref_anno, exon_off, exon_start, exon_end, exon_flag;
+    template <class F, class... G> static void cols(F &&f, G &...g)
+    {
+        f(ROW, 4, g.read_idx...); f(ROW, 4, g.tid...); f(ROW, 1, g.is_rev...); f(ROW, 4, g.cls...); f(ROW, 4, g.ref_anno...); f(OFFS, 4, g.exon_off...);
+        f(EXON, 4, g.exon_start...); f(EXON, 4, g.exon_end...); f(EXON, 1, g.exon_flag...);
+    }
+};
+template <class B> struct FilterCols {              // lrb_filter_result; rows: the records, exons: the kept records
+    B pass, score, intron_n, keep_idx;
+    template <class F, class... G> static void cols(F &&f, G &...g) { f(ROW, 1, g.pass...); f(ROW, 4, g.score...); f(ROW, 4, g.intron_n...); f(EXON, 4, g.keep_idx...); }
+};
 template <class B> struct JuncCols {                // lrb_sj: the bam2sj output
     B tid, don, acc, uniq_c, multi_c;
     template <class F, class... G> static void cols(F &&f, G &...g) { f(ROW, 4, g.tid...); f(ROW, 4, g.don...); f(ROW, 4, g.acc...); f(ROW, 4, g.uniq_c...); f(ROW, 4, g.multi_c...); }
@@ -129,6 +141,13 @@ template <class G, class V> V view(const G &g, V v)
 {
     G::cols([](Per, size_t, auto &ptr, const auto &col) { ptr = (std::remove_reference_t<decltype(ptr)>)col.p; }, v, g);
     return v;
+}
+
+inline lrb_merged_list merged_result(const MergedCols<PBuf> &h, int64_t n)
+{
+    lrb_merged_list o; o.n = n; o.cand = h.cand.as<uint32_t>(); o.cov = h.cov.as<int32_t>(); o.t_tid = h.tid.as<int32_t>(); o.t_start = h.start.as<int32_t>();
+    o.t_end = h.end.as<int32_t>(); o.first_start = h.fs.as<int32_t>(); o.last_end = h.le.as<int32_t>();
+    return o;
 }
 
 // ---- pinned results: one set per result kind, so that a fetch of one kind leaves the results of the others intact
@@ -208,11 +227,17 @@ struct lrb_ctx {
     // timing
     bool timing = false; cudaEvent_t ev[lrbk::EV_COUNT]; cudaEvent_t marks[8]; float ms[LRB_T_COUNT]; int64_t launches0 = 0, launches_last = 0;
     lrb_update_params last_up;
+    int64_t update_gen = 0;                         // bumped by every lrb_update_run: ties a gathered result to the run it came from
 };
 
 namespace lrbk {
 
 int build_update_table(lrb_ctx *c, int64_t *n_exon_out, bool with_flags);      // lrb_capi.cu
+// the current rows' exon chains (+ flags) in the layout of lrb_exon_result, in HBM: n offsets from 0 (the exon total is the caller's),
+// the chains back to back.  Rows that are not compact are gathered into summary scratch (free once the update stage has run) after
+// one host round trip for the exon total.  The pointers stay valid until the next stage run or compaction.
+struct CompactExons { const uint32_t *off; const int32_t *es, *ee; const uint8_t *flag; int64_t n_exon; };
+int compact_exons(lrb_ctx *c, bool with_flags, CompactExons *out);                // lrb_capi.cu
 void multi_release(lrb_ctx *c);                                                   // lrb_multi.cu
 
 inline int64_t total_launches() { return lrbk::count_launches() + lrbk::g_launches_update + lrbk::g_launches_summary + lrbk::g_launches_sort; }

@@ -13,6 +13,10 @@
 //                              three sets recomputed over the gathered table when two shards share one;
 //                            * a split piece whose junction also exists in ANOTHER shard could have been absorbed there in the
 //                              reference (Q14.2): that is reported as LRB_E_XSHARD, the caller reruns unsharded.
+//   lrb_update_gather_reads  the per-read results (bam_T chains, class words, known / unrecog / novel lists, the filter's
+//                          records and keep list) of every shard go to rank 0 the same way; they need no merge: each row is
+//                          a function of its read and the replicated tables, so the root only concatenates the shards and
+//                          shifts their row / exon / record indices to the whole stream (App. B.3).
 //
 // NCCL is bound at run time (dlopen of libnccl.so.2): the library loads on a box without NCCL, and inside a process that already
 // carries NCCL (torch) it binds to that copy instead of a second one.
@@ -59,6 +63,18 @@ static NcclApi *nccl_api(std::string *err)
 
 static constexpr int META_WORDS = 40, MAX_RANKS = 64;
 enum { M_NU = 0, M_NE, M_NBED, M_NKG, M_NAME_BASE, M_PARTIAL, M_WANT_SUMMARY, M_SUMMARY0 /* .. + LRB_S_COUNT */ };
+// the per-rank block of lrb_update_gather_reads
+enum { R_REC = 0, R_KEEP, R_ROWS, R_EXON, R_KNOWN, R_UNREC, R_NOVEL, R_UPD, R_NAME_BASE, R_FILTER, R_READ_IDX, R_WORDS };
+static_assert(R_WORDS <= META_WORDS, "meta block");
+
+struct GatherReads {                                // lrb_update_gather_reads, gathered on the root
+    ReadCols<Buf> rd; Buf known, unrecog; ListCols<Buf> novel; MergedCols<Buf> upd; FilterCols<Buf> filt;
+    int64_t n_rec = 0, n_keep = 0, n_rows = 0, n_exon = 0, n_known = 0, n_unrecog = 0, n_novel = 0, n_upd = 0;
+    int64_t gen = -1;                               // lrb_ctx::update_gen of the run gathered
+    bool have = false, with_filter = false, with_read_idx = false;
+    // lrb_gather_fetch_reads
+    ReadCols<PBuf> o_rd; PBuf o_known, o_unrecog; ListCols<PBuf> o_novel; MergedCols<PBuf> o_upd; BedCols<PBuf> o_bed; FilterCols<PBuf> o_filt;
+};
 
 struct MultiState {
     NcclApi *api = nullptr; ncclComm_t comm = nullptr; int rank = 0, n_ranks = 1;
@@ -68,7 +84,9 @@ struct MultiState {
     Buf v_ident, v_zeros, v_cnt, v_fs, v_le;          // the gathered table in the shape the set kernels read
     Buf tab, y_barcnt, y_barseg, y_genebar, y_bedcnt, y_bedoff, y_counts, y_nelem, tiles, xs_pl, xs_hx, xs_cnt;
     int64_t n = 0, n_exon = 0, n_bed = 0; int32_t summary[LRB_S_COUNT]; bool have = false, daj_recomputed = false;
+    int64_t gen = -1;                               // lrb_ctx::update_gen of the run merged
     TableCols<PBuf> out_tab; BedCols<PBuf> out_bed;  // lrb_gather_fetch
+    GatherReads reads;
     float ms_gather = 0, ms_merge = 0; cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
 };
 
@@ -84,16 +102,56 @@ void multi_release(lrb_ctx *c)
 #define NK(call)                                                                                                           \
     do { ncclResult_t r_ = (call); if (r_ != ncclSuccess) return fail(c, LRB_E_NCCL, std::string(#call) + ": " + m->api->GetErrorString(r_)); } while (0)
 
-// exon offsets of shard r start at 0: shift them to the shard's place in the gathered pools; name_idx becomes an index into
-// the whole read stream
-struct RebaseArgs { int64_t row_end[MAX_RANKS]; int64_t exon_base[MAX_RANKS]; int64_t name_base[MAX_RANKS]; int n; };
-__global__ void rebase_kernel(RebaseArgs a, uint32_t *exon_off, uint32_t *name_idx, int64_t n, int64_t n_exon)
+// Indices of shard r count from 0 within the shard (exon offsets, rows, novel entries, records): the root shifts them to the
+// shard's place in the gathered whole.  A segmented add over a few uint32 columns in one launch, blockIdx.y = column: element i
+// lies in shard k, the first with i < end[k], and gets add[k].  *term = term_val writes an OFFS column's last entry.
+static constexpr int REBASE_COLS = 7;
+struct RebaseCol { uint32_t *p; int64_t n; uint32_t end[MAX_RANKS], add[MAX_RANKS]; };
+struct RebaseArgs { RebaseCol col[REBASE_COLS]; int n_cols, n_shards; uint32_t *term, term_val; };
+static_assert(sizeof(RebaseArgs) <= 4096, "kernel parameter space");
+__global__ void rebase_kernel(const __grid_constant__ RebaseArgs a)
 {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i == 0) exon_off[n] = (uint32_t)n_exon;
-    if (i >= n) return;
-    int k = 0; while (k < a.n - 1 && i >= a.row_end[k]) ++k;
-    exon_off[i] += (uint32_t)a.exon_base[k]; name_idx[i] += (uint32_t)a.name_base[k];
+    if (a.term && i == 0 && blockIdx.y == 0) *a.term = a.term_val;
+    const RebaseCol &c = a.col[blockIdx.y];
+    if (i >= c.n) return;
+    int k = 0; while (k < a.n_shards - 1 && i >= c.end[k]) ++k;
+    c.p[i] += c.add[k];
+}
+
+// a column of the gathered shards: shard r holds entries [off[r], off[r + 1]) and gets add[r]
+static void rebase_col(RebaseArgs &a, void *p, const std::vector<int64_t> &off, const std::vector<int64_t> &add)
+{
+    RebaseCol &col = a.col[a.n_cols++];
+    col.p = (uint32_t *)p; col.n = off[a.n_shards];
+    for (int r = 0; r < a.n_shards; ++r) { col.end[r] = (uint32_t)off[r + 1]; col.add[r] = (uint32_t)add[r]; }
+}
+
+static int launch_rebase(lrb_ctx *c, const RebaseArgs &a)
+{
+    int64_t n = 0;
+    for (int j = 0; j < a.n_cols; ++j) n = std::max(n, a.col[j].n);
+    rebase_kernel<<<dim3((unsigned)(n / 256 + 1), (unsigned)a.n_cols), 256, 0, c->st>>>(a);
+    CK(cudaGetLastError());
+    return LRB_OK;
+}
+
+// one table's part of a gatherv to the root, as an each_col callback: a rank sends rows [rows[me], rows[me + 1]) and exons
+// [exons[me], exons[me + 1]) of each column, the root receives part r at that offset (both inside one ncclGroup); own: the root
+// copies its own part instead.  An OFFS column moves n entries: the root rebases them.
+static auto gather_parts(lrb_ctx *c, MultiState *m, bool own, const std::vector<int64_t> &rows, const std::vector<int64_t> &exons)
+{
+    return [c, m, own, &rows, &exons](Per p, size_t esz, auto &src, Buf &dst) {
+        const std::vector<int64_t> &off = p == EXON ? exons : rows;
+        const int me = m->rank;
+        if (own) { if (off[1]) CK(cudaMemcpyAsync(dst.p, addr(src), (size_t)off[1] * esz, cudaMemcpyDeviceToDevice, c->st)); }
+        else if (me != 0) { const int64_t cnt = off[me + 1] - off[me]; if (cnt) NK(m->api->Send(addr(src), (size_t)cnt * esz, ncclChar, 0, m->comm, c->st)); }
+        else for (int r = 1; r < m->n_ranks; ++r) {
+            const int64_t cnt = off[r + 1] - off[r];
+            if (cnt) NK(m->api->Recv((char *)dst.p + (size_t)off[r] * esz, (size_t)cnt * esz, ncclChar, r, m->comm, c->st));
+        }
+        return LRB_OK;
+    };
 }
 
 }  // namespace lrbk
@@ -235,18 +293,7 @@ int lrb_update_gather(lrb_ctx *c, int64_t name_base)
         if ((rc = ensure(c, m->g, Extent{n1, e1})) || (rc = ensure(c, m->g_bed, Extent{std::max<int64_t>(NB, 1)}))) return rc;
         NEED(m->g_flag, (size_t)e1); NEED(m->g_kg, (size_t)std::max<int64_t>(NK_, 1) * 8);
     }
-    auto parts = [&](bool own, const std::vector<int64_t> &row_off) {
-        return [&, own, rows = &row_off](Per p, size_t esz, Buf &src, Buf &dst) {
-            const std::vector<int64_t> &off = p == EXON ? o_e : *rows;            // an OFFS column moves n entries: the root rebases them
-            if (own) { if (off[1]) CK(cudaMemcpyAsync(dst.p, src.p, (size_t)off[1] * esz, cudaMemcpyDeviceToDevice, c->st)); }
-            else if (!root) { const int64_t cnt = off[me + 1] - off[me]; if (cnt) NK(m->api->Send(src.p, (size_t)cnt * esz, ncclChar, 0, m->comm, c->st)); }
-            else for (int r = 1; r < R; ++r) {
-                const int64_t cnt = off[r + 1] - off[r];
-                if (cnt) NK(m->api->Recv((char *)dst.p + (size_t)off[r] * esz, (size_t)cnt * esz, ncclChar, r, m->comm, c->st));
-            }
-            return LRB_OK;
-        };
-    };
+    auto parts = [&](bool own, const std::vector<int64_t> &row_off) { return gather_parts(c, m, own, row_off, o_e); };
     auto gather = [&](bool own) {
         int rc2;
         if ((rc2 = each_col(parts(own, o_n), c->tab, m->g)) || (rc2 = parts(own, o_n)(EXON, 1, c->tb_flag, m->g_flag)) ||
@@ -266,10 +313,11 @@ int lrb_update_gather(lrb_ctx *c, int64_t name_base)
         return LRB_OK;
     }
     // ---- canonical merge on the root
-    RebaseArgs ra{}; ra.n = R;
-    for (int r = 0; r < R; ++r) { ra.row_end[r] = o_n[r + 1]; ra.exon_base[r] = o_e[r]; ra.name_base[r] = mh[(size_t)r * META_WORDS + M_NAME_BASE]; }
-    rebase_kernel<<<(unsigned)(N / 256 + 1), 256, 0, c->st>>>(ra, m->g.exon_off.as<uint32_t>(), m->g.name_idx.as<uint32_t>(), N, NE);
-    CK(cudaGetLastError());
+    std::vector<int64_t> names(R);
+    for (int r = 0; r < R; ++r) names[r] = mh[(size_t)r * META_WORDS + M_NAME_BASE];
+    RebaseArgs ra{}; ra.n_shards = R; ra.term = m->g.exon_off.as<uint32_t>() + N; ra.term_val = (uint32_t)NE;
+    rebase_col(ra, m->g.exon_off.p, o_n, o_e); rebase_col(ra, m->g.name_idx.p, o_n, names);
+    if ((rc = launch_rebase(c, ra))) return rc;
     m->n = N; m->n_exon = NE; m->n_bed = want_summary ? NB : 0; m->daj_recomputed = false;
     memset(m->summary, 0, sizeof m->summary);
     int64_t partial = 0;
@@ -341,7 +389,7 @@ int lrb_update_gather(lrb_ctx *c, int64_t name_base)
     CK(cudaEventRecord(m->ev[2], c->st));
     CK(cudaStreamSynchronize(c->st));
     CK(cudaEventElapsedTime(&m->ms_gather, m->ev[0], m->ev[1])); CK(cudaEventElapsedTime(&m->ms_merge, m->ev[1], m->ev[2]));
-    m->have = true;
+    m->have = true; m->gen = c->update_gen;
     c->launches_last = total_launches() - l0;
     return LRB_OK;
 }
@@ -366,6 +414,134 @@ int lrb_gather_fetch(lrb_ctx *c, lrb_trans_table *tab, lrb_bed_list *bed, int32_
     CK(cudaStreamSynchronize(c->st));
     if (tab) { m->out_tab.exon_off.as<uint32_t>()[m->n] = (uint32_t)m->n_exon; *tab = view(m->out_tab, lrb_trans_table{m->n}); }
     if (bed) *bed = view(m->out_bed, lrb_bed_list{m->n_bed});
+    return LRB_OK;
+}
+
+// ------------------------------------------------------------------------------------------- gather of the per-read results
+int lrb_update_gather_reads(lrb_ctx *c, int64_t name_base)
+{
+    if (!c) return LRB_E_ARG;
+    MultiState *m = c->multi;
+    if (!m) return fail(c, LRB_E_ARG, "lrb_update_gather_reads: no communicator (lrb_comm_init)");
+    if (!c->have_update) return fail(c, LRB_E_ARG, "lrb_update_gather_reads: update stage has not run");
+    CK(cudaSetDevice(c->device));
+    int rc; const int R = m->n_ranks, me = m->rank; const bool root = me == 0;
+    const int64_t l0 = total_launches();
+    GatherReads &gr = m->reads;
+    gr.have = false;
+    // ---- this shard's exon chains in the layout lrb_update_fetch hands out
+    CompactExons ce;
+    if ((rc = compact_exons(c, true, &ce))) return rc;
+    const DRows &rows = *c->cur;
+    // ---- counts of every rank
+    int64_t *mh = m->meta_host.as<int64_t>(), *mine = mh + (size_t)me * META_WORDS;
+    memset(mine, 0, META_WORDS * 8);
+    mine[R_REC] = c->have_filter ? c->b.n : 0; mine[R_KEEP] = c->have_filter ? c->n_keep : 0; mine[R_ROWS] = rows.n; mine[R_EXON] = ce.n_exon;
+    mine[R_KNOWN] = c->n_known; mine[R_UNREC] = c->n_unrecog; mine[R_NOVEL] = c->novel.n; mine[R_UPD] = c->mg.n_out;
+    mine[R_NAME_BASE] = name_base; mine[R_FILTER] = c->have_filter; mine[R_READ_IDX] = c->have_batch;
+    int64_t *md = m->meta_dev.as<int64_t>();
+    CK(cudaMemcpyAsync(md + (size_t)me * META_WORDS, mine, META_WORDS * 8, cudaMemcpyHostToDevice, c->st));
+    NK(m->api->AllGather(md + (size_t)me * META_WORDS, md, META_WORDS, ncclInt64, m->comm, c->st));
+    CK(cudaMemcpyAsync(mh, md, (size_t)R * META_WORDS * 8, cudaMemcpyDeviceToHost, c->st));
+    CK(cudaStreamSynchronize(c->st));
+    // o_x[r]: entries of x in the shards before r
+    std::vector<int64_t> o_rec(R + 1, 0), o_keep(R + 1, 0), o_rows(R + 1, 0), o_exon(R + 1, 0), o_known(R + 1, 0), o_unrec(R + 1, 0), o_novel(R + 1, 0),
+        o_upd(R + 1, 0), names(R);
+    bool with_filter = true, with_read_idx = true;
+    for (int r = 0; r < R; ++r) {
+        const int64_t *x = mh + (size_t)r * META_WORDS;
+        o_rec[r + 1] = o_rec[r] + x[R_REC]; o_keep[r + 1] = o_keep[r] + x[R_KEEP]; o_rows[r + 1] = o_rows[r] + x[R_ROWS];
+        o_exon[r + 1] = o_exon[r] + x[R_EXON]; o_known[r + 1] = o_known[r] + x[R_KNOWN]; o_unrec[r + 1] = o_unrec[r] + x[R_UNREC];
+        o_novel[r + 1] = o_novel[r] + x[R_NOVEL]; o_upd[r + 1] = o_upd[r] + x[R_UPD]; names[r] = x[R_NAME_BASE];
+        with_filter = with_filter && x[R_FILTER] != 0; with_read_idx = with_read_idx && x[R_READ_IDX] != 0;
+    }
+    const int64_t lim = (int64_t)1 << 32;
+    if (o_exon[R] >= lim || o_rows[R] >= lim || o_novel[R] >= lim || (with_filter && o_rec[R] >= lim))
+        return fail(c, LRB_E_ARG, "lrb_update_gather_reads: gathered results exceed 2^32 exons / records");
+    // ---- gatherv of every column, as in lrb_update_gather
+    if (root) {
+        if ((rc = ensure(c, gr.rd, Extent{o_rows[R], o_exon[R]})) || (rc = ensure(c, gr.novel, Extent{o_novel[R]})) || (rc = ensure(c, gr.upd, Extent{o_upd[R]})) ||
+            (with_filter && (rc = ensure(c, gr.filt, Extent{o_rec[R], o_keep[R]}))))
+            return rc;
+        NEED(gr.known, (size_t)std::max<int64_t>(o_known[R], 1) * 4); NEED(gr.unrecog, (size_t)std::max<int64_t>(o_unrec[R], 1) * 4);
+    }
+    ReadCols<const void *> my_rd{rows.read_idx, rows.tid, rows.is_rev, c->u_cls.p, c->u_ref.p, ce.off, ce.es, ce.ee, ce.flag};
+    FilterCols<const void *> my_filt{c->f_pass.p, c->f_score.p, c->f_intron.p, c->f_keep_idx.p};
+    auto gather = [&](bool own) {
+        int rc2;
+        if ((rc2 = each_col(gather_parts(c, m, own, o_rows, o_exon), my_rd, gr.rd)) ||
+            (rc2 = gather_parts(c, m, own, o_known, o_exon)(ROW, 4, c->u_known, gr.known)) ||
+            (rc2 = gather_parts(c, m, own, o_unrec, o_exon)(ROW, 4, c->u_unrecog, gr.unrecog)) ||
+            (rc2 = each_col(gather_parts(c, m, own, o_novel, o_exon), c->novel_cols, gr.novel)) ||
+            (rc2 = each_col(gather_parts(c, m, own, o_upd, o_exon), c->mg.o, gr.upd)))
+            return rc2;
+        return with_filter ? each_col(gather_parts(c, m, own, o_rec, o_keep), my_filt, gr.filt) : LRB_OK;
+    };
+    NK(m->api->GroupStart());
+    if ((rc = gather(false))) return rc;
+    NK(m->api->GroupEnd());
+    if (root) {
+        if ((rc = gather(true))) return rc;
+        // ---- shard-local indices -> indices of the whole stream (the exon total of ex.exon_off is written by the fetch)
+        RebaseArgs ra{}; ra.n_shards = R;
+        if (with_read_idx) rebase_col(ra, gr.rd.read_idx.p, o_rows, names);
+        rebase_col(ra, gr.rd.exon_off.p, o_rows, o_exon);
+        rebase_col(ra, gr.known.p, o_known, o_rows); rebase_col(ra, gr.unrecog.p, o_unrec, o_rows); rebase_col(ra, gr.novel.row.p, o_novel, o_rows);
+        rebase_col(ra, gr.upd.cand.p, o_upd, o_novel);
+        if (with_filter) rebase_col(ra, gr.filt.keep_idx.p, o_keep, names);
+        if ((rc = launch_rebase(c, ra))) return rc;
+        gr.n_rec = o_rec[R]; gr.n_keep = o_keep[R]; gr.n_rows = o_rows[R]; gr.n_exon = o_exon[R]; gr.n_known = o_known[R]; gr.n_unrecog = o_unrec[R];
+        gr.n_novel = o_novel[R]; gr.n_upd = o_upd[R]; gr.with_filter = with_filter; gr.with_read_idx = with_read_idx;
+    }
+    CK(cudaStreamSynchronize(c->st));
+    gr.have = root; gr.gen = c->update_gen;
+    c->launches_last = total_launches() - l0;
+    return LRB_OK;
+}
+
+int lrb_gather_fetch_reads(lrb_ctx *c, lrb_update_result *update, lrb_filter_result *filter)
+{
+    if (!c) return LRB_E_ARG;
+    MultiState *m = c->multi;
+    if (!m) return fail(c, LRB_E_ARG, "lrb_gather_fetch_reads: no communicator (lrb_comm_init)");
+    CK(cudaSetDevice(c->device));
+    if (update) memset(update, 0, sizeof *update);
+    if (filter) memset(filter, 0, sizeof *filter);
+    if (m->rank != 0) return LRB_OK;                 // only the root holds the gathered results
+    GatherReads &gr = m->reads;
+    if (!gr.have) return fail(c, LRB_E_ARG, "lrb_gather_fetch_reads: lrb_update_gather_reads has not run");
+    if (update && (!m->have || m->gen != gr.gen))
+        return fail(c, LRB_E_ARG, "lrb_gather_fetch_reads: an update result takes its BED rows and counters from lrb_update_gather, which has not "
+                                  "succeeded for the lrb_update_run these reads come from");
+    if (filter && !gr.with_filter) return fail(c, LRB_E_ARG, "lrb_gather_fetch_reads: the filter stage did not run on every shard");
+    int rc;
+    if (update) {
+        if ((rc = copy(c, gr.o_rd, gr.rd, Extent{gr.n_rows, gr.n_exon}, cudaMemcpyDeviceToHost))) return rc;
+        if ((rc = d2h(c, gr.o_known, gr.known.as<uint32_t>(), (size_t)gr.n_known))) return rc;
+        if ((rc = d2h(c, gr.o_unrecog, gr.unrecog.as<uint32_t>(), (size_t)gr.n_unrecog))) return rc;
+        if ((rc = copy(c, gr.o_novel, gr.novel, Extent{gr.n_novel}, cudaMemcpyDeviceToHost))) return rc;
+        if ((rc = copy(c, gr.o_upd, gr.upd, Extent{gr.n_upd}, cudaMemcpyDeviceToHost))) return rc;
+        if ((rc = copy(c, gr.o_bed, m->g_bed, Extent{m->n_bed}, cudaMemcpyDeviceToHost))) return rc;
+    }
+    if (filter && (rc = copy(c, gr.o_filt, gr.filt, Extent{gr.n_rec, gr.n_keep}, cudaMemcpyDeviceToHost))) return rc;
+    CK(cudaStreamSynchronize(c->st));
+    if (update) {
+        const ReadCols<PBuf> &h = gr.o_rd;
+        h.exon_off.as<uint32_t>()[gr.n_rows] = (uint32_t)gr.n_exon;
+        lrb_exon_result &ex = update->ex;
+        ex.n_reads = gr.n_rows; ex.read_idx = gr.with_read_idx ? h.read_idx.as<uint32_t>() : nullptr; ex.tid = h.tid.as<int32_t>();
+        ex.is_rev = h.is_rev.as<uint8_t>(); ex.exon_off = h.exon_off.as<uint32_t>(); ex.exon_start = h.exon_start.as<int32_t>(); ex.exon_end = h.exon_end.as<int32_t>();
+        update->cls = h.cls.as<uint32_t>(); update->ref_anno = h.ref_anno.as<int32_t>(); update->exon_flag = h.exon_flag.as<uint8_t>();
+        update->n_known = gr.n_known; update->known_idx = gr.o_known.as<uint32_t>(); update->n_unrecog = gr.n_unrecog; update->unrecog_idx = gr.o_unrecog.as<uint32_t>();
+        update->novel.n = gr.n_novel; update->novel.read = gr.o_novel.row.as<uint32_t>(); update->novel.exon_lo = gr.o_novel.lo.as<uint32_t>();
+        update->novel.exon_n = gr.o_novel.cnt.as<uint32_t>(); update->novel.piece = gr.o_novel.piece.as<int32_t>();
+        update->updated = merged_result(gr.o_upd, gr.n_upd); update->bed = view(gr.o_bed, lrb_bed_list{m->n_bed});
+        memcpy(update->summary, m->summary, sizeof m->summary);
+    }
+    if (filter) {
+        *filter = view(gr.o_filt, lrb_filter_result{});
+        filter->n = gr.n_rec; filter->n_keep = gr.n_keep;
+    }
     return LRB_OK;
 }
 

@@ -4,6 +4,7 @@
     ctx.comm_init(id, rank, world)              # id = api.comm_id() on rank 0, shipped by the launcher (torch.distributed, a file, MPI)
     ctx.tables_broadcast(0, anno, rm, sj)       # rank 0 passes the tables, the others None
     res = run_shard(ctx, shard_soa, name_base, fp, ep, up)   # rank 0: the merged result; others: None
+    res = run_shard(..., reads=True)            # + res["reads"]: the per-read results (update-gtf -a/-A/-k/-v/-u, filter's records)
 
 Everything numeric happens in the CUDA library; this file only slices arrays and orders calls.
 """
@@ -64,8 +65,10 @@ def take_rows(batch: dict, idx) -> dict:
     return d
 
 
-def run_shard(ctx: api.Context, shard: dict | None, name_base: int, fp, ep, up, filtered: bool = True, fetch: bool = True):
-    """One rank's part: upload, (filter +) CIGAR walk, update, gather to rank 0.  Returns the merged result on rank 0."""
+def run_shard(ctx: api.Context, shard: dict | None, name_base: int, fp, ep, up, filtered: bool = True, fetch: bool = True,
+              reads: bool = False):
+    """One rank's part: upload, (filter +) CIGAR walk, update, gather to rank 0.  Returns the merged result on rank 0.
+    reads: also gather the per-read results; rank 0's result then has them under "reads" (Context.gather_fetch_reads)."""
     if shard is not None:
         ctx.upload(shard)
     if filtered:
@@ -73,5 +76,14 @@ def run_shard(ctx: api.Context, shard: dict | None, name_base: int, fp, ep, up, 
     else:
         ctx.exon_run(ep)
     ctx.update_run(up)
-    ctx.update_gather(name_base)
-    return ctx.gather_fetch() if fetch else None
+    try:
+        ctx.update_gather(name_base)
+    finally:
+        if reads:                                   # collective: every rank joins it, also where the root's table gather failed
+            ctx.update_gather_reads(name_base)
+    if not fetch:
+        return None
+    res = ctx.gather_fetch()
+    if reads:
+        res["reads"] = ctx.gather_fetch_reads(want_filter=filtered)
+    return res
