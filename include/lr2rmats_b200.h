@@ -326,6 +326,24 @@ int lrb_elapsed_ms(lrb_ctx *ctx, int slot_from, int slot_to, float *ms);   /* sy
 /* Diagnostics of the last lrb_update_run: split pieces that were absorbed by an entry on ANOTHER chromosome (the reference's
  * back-scan of a piece never stops, update_gtf.c:148; settled in rounds on the device) and folds replayed as one locus. */
 int lrb_update_diag(const lrb_ctx *ctx, int64_t *pieces_across_chromosomes, int64_t *one_locus_replays);
+/* Fold census, a test hook: which path of the merge fold (update-gtf's updated_T and class folds, unique-gtf) folded each locus.
+ * Counted only when LRB_TEST_FOLD_CENSUS is set to a non-zero number at lrb_ctx_create; each fold then reads its locus table back
+ * and synchronises its stream.  Cumulative over the context's life; the repeated folds that settle split pieces absorbed on another
+ * chromosome are not counted.  Per locus unless stated, by the final state of the fold:
+ *   -d 0:  FLAT         <= 64 candidates, folded by the flat kernels
+ *          TIER0        > 64 candidates or given up by the flat kernels, folded by the 128-slot warp replay
+ *          TIER1        outgrew tier 0, folded by the 416-slot replay
+ *          MERGE_OVER   outgrew tier 1, or >= 32768 candidates: replayed by merge_fold_kernel
+ *          MERGE_VERIFY a class hash collision: replayed by merge_fold_kernel
+ *          NOROWS       (locus, sub-stream) pairs of the warp replay with more than 127 multi-exon classes (no relation rows)
+ *   -d >0: D_SMALL / D_LARGE  loci of <= 32 / >= 33 candidates
+ *   both:  SINGLE       loci of folds replayed as one locus (also counted above)
+ * Counters [0, LRB_FC_COUNT) are the folds on the main stream (updated_T, unique-gtf), [LRB_FC_COUNT, 2 * LRB_FC_COUNT) those on
+ * the side stream (update-gtf's four class folds of the summary).  Writes min(n, 2 * LRB_FC_COUNT) counters to out and returns
+ * 2 * LRB_FC_COUNT. */
+enum { LRB_FC_FLAT, LRB_FC_TIER0, LRB_FC_TIER1, LRB_FC_MERGE_OVER, LRB_FC_MERGE_VERIFY, LRB_FC_NOROWS, LRB_FC_D_SMALL, LRB_FC_D_LARGE,
+       LRB_FC_SINGLE, LRB_FC_COUNT };
+int lrb_fold_census(const lrb_ctx *ctx, int64_t *out, int n);
 /* pinned host memory for record batches (what the host decoder fills) */
 void *lrb_host_alloc(size_t bytes);
 void lrb_host_free(void *p);

@@ -24,8 +24,11 @@ ENTRY_POINTS = [
     "lrb_mark", "lrb_elapsed_ms", "lrb_host_alloc", "lrb_host_free", "lrb_update_fetch_table", "lrb_filter_fetch_keep",
     "lrb_comm_id", "lrb_comm_init", "lrb_comm_destroy", "lrb_comm_rank", "lrb_tables_broadcast", "lrb_update_gather", "lrb_gather_fetch",
     "lrb_gather_timing", "lrb_shard_cuts_weighted", "lrb_update_diag", "lrb_bam2sj", "lrb_sort3", "lrb_update_gather_reads",
-    "lrb_gather_fetch_reads",
+    "lrb_gather_fetch_reads", "lrb_fold_census",
 ]
+
+# lrb_fold_census counters per stream, in the order of the LRB_FC_* enum
+FOLD_CENSUS_NAMES = ["flat", "tier0", "tier1", "merge_overflow", "merge_verify", "norows", "d_small", "d_large", "single"]
 
 T_NAMES = ["filter", "exon", "classify", "merge", "summary", "k_scan", "k_fold"]
 
@@ -95,6 +98,7 @@ def load_library():
     L.lrb_update_gather_reads.argtypes = [vp, C.c_int64]
     L.lrb_gather_fetch_reads.argtypes = [vp, P(cabi.UpdateResult), P(cabi.FilterResult)]
     L.lrb_update_diag.argtypes = [vp, P(C.c_int64), P(C.c_int64)]
+    L.lrb_fold_census.argtypes = [vp, P(C.c_int64), C.c_int]
     L.lrb_bam2sj.argtypes = [vp, P(cabi.Batch), cabi.u8p, P(cabi.SjParams), P(cabi.Sj)]
     L.lrb_sort3.argtypes = [vp, cabi.u32p, cabi.u32p, cabi.u32p, C.c_int64, P(cabi.u32p)]
     _lib = L
@@ -275,6 +279,16 @@ class Context:
     def update_diag(self):
         a = C.c_int64(); b = C.c_int64(); self._ck(self.L.lrb_update_diag(self.h, C.byref(a), C.byref(b)))
         return dict(pieces_across_chromosomes=int(a.value), one_locus_replays=int(b.value))
+
+    def fold_census(self) -> dict:
+        """Loci per merge-fold path since the context was created, {"main": {name: n}, "side": {name: n}} (names: FOLD_CENSUS_NAMES).
+        Counted only when LRB_TEST_FOLD_CENSUS=1 was in the environment when the context was created; all zero otherwise."""
+        k = len(FOLD_CENSUS_NAMES)
+        out = (C.c_int64 * (2 * k))()
+        n = self.L.lrb_fold_census(self.h, out, 2 * k)
+        if n != 2 * k:
+            raise LrbError(n, f"lrb_fold_census returned {n} counters, the binding knows {2 * k}")
+        return {s: dict(zip(FOLD_CENSUS_NAMES, list(out)[i * k:(i + 1) * k])) for i, s in enumerate(("main", "side"))}
 
     # ---- measurement
     def timing(self, on=True): self._ck(self.L.lrb_timing_enable(self.h, 1 if on else 0))

@@ -164,6 +164,7 @@ int run_merge_async(lrb_ctx *c, MergeBufs &m, const DTransList &list, int64_t n_
     if (o.time_fold) tick(c, EV_FOLD0);
     launch_merge_fold(a, st);                        // locus count is consumed on the device: no host round trip
     if (o.time_fold) tick(c, EV_FOLD1);
+    if (c->fold_census) CK(merge_fold_census(a, st, c->census[o.side ? 1 : 0]));
     if (o.xl) launch_xlocus_detect(a, c->xl, st);
     if (o.kls) launch_merge_class_counts(a, st);
     else launch_merge_finish(a, st);
@@ -207,6 +208,7 @@ int lrb_ctx_create(int device, lrb_ctx **out)
     cudaEventCreateWithFlags(&c->ev_fork3, cudaEventDisableTiming); cudaEventCreateWithFlags(&c->ev_join3, cudaEventDisableTiming);
     { const char *e = getenv("LRB_TEST_SMALL_NOVEL_CAP"); if (e) c->test_small_novel_cap = atoi(e) != 0; }      // test hook: novel_T sized too small on the first attempt
     { const char *e = getenv("LRB_FORCE_SINGLE_FOLD"); if (e) c->force_single_fold = atoi(e) != 0; }    // test hook: updated_T always folded by the one-locus replay
+    { const char *e = getenv("LRB_TEST_FOLD_CENSUS"); if (e) c->fold_census = atoi(e) != 0; }       // test hook: loci tallied by fold path (lrb_fold_census)
     if (!c->scalars.ensure(512) || !c->h_scalars.ensure(512)) { delete c; return LRB_E_NOMEM; }
     cudaMemsetAsync(c->scalars.p, 0, 512, c->st);
     for (cudaEvent_t &e : c->ev) cudaEventCreate(&e);
@@ -1089,6 +1091,12 @@ int lrb_update_diag(const lrb_ctx *c, int64_t *pieces, int64_t *replays)
     if (pieces) *pieces = c->n_xlocus_pieces;
     if (replays) *replays = c->n_xlocus_replays;
     return LRB_OK;
+}
+int lrb_fold_census(const lrb_ctx *c, int64_t *out, int n)
+{
+    if (!c || n < 0 || (n > 0 && !out)) return LRB_E_ARG;
+    if (n > 0) memcpy(out, c->census, sizeof(int64_t) * (size_t)std::min(n, 2 * LRB_FC_COUNT));
+    return 2 * LRB_FC_COUNT;
 }
 void *lrb_host_alloc(size_t bytes) { void *p = nullptr; if (cudaMallocHost(&p, bytes ? bytes : 1) != cudaSuccess) { cudaGetLastError(); return nullptr; } return p; }
 void lrb_host_free(void *p) { if (p) cudaFreeHost(p); }

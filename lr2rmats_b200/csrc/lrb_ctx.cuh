@@ -210,6 +210,7 @@ struct lrb_ctx {
     int64_t n_known = 0, n_unrecog = 0, novel_cap_hint = 0; bool have_update = false, have_unique = false;
     int32_t summary[LRB_S_COUNT];
     bool force_single_fold = false, test_small_novel_cap = false, want_kg_pairs = false; int64_t n_xlocus_replays = 0, n_xlocus_pieces = 0, n_kg_pairs = 0; Buf kg_pairs;
+    bool fold_census = false; int64_t census[2][LRB_FC_COUNT] = {};   // test hook LRB_TEST_FOLD_CENSUS: loci per fold path, main / side stream
     Buf xl_key, xl_min, xl_max, xl_cnt, xl_forced; lrbk::XlArgs xl;      // split pieces that meet another chromosome (xl_* kernels)
     // summary
     Buf h_khi, y_barcnt, y_barseg, y_genebar, y_bedcnt, y_bedoff, y_counts, y_nelem;

@@ -158,6 +158,7 @@ void launch_xlocus_apply(const MergeArgs &a, const XlArgs &x, cudaStream_t st);
 void launch_xlocus_reset(const MergeArgs &a, const XlArgs &x, cudaStream_t st);     // before the fold runs again with new marks
 void launch_merge_prepare(MergeArgs a, cudaStream_t st);            // candidates, locus heads, locus_start; totals[0] = number of loci
 void launch_merge_fold(const MergeArgs &a, cudaStream_t st);        // number of loci is read from a.totals[0] on the device
+cudaError_t merge_fold_census(const MergeArgs &a, cudaStream_t st, int64_t *counts);   // test hook: synchronises st, adds to counts[LRB_FC_*]
 void launch_merge_class_counts(const MergeArgs &a, cudaStream_t st);
 void launch_merge_finish(MergeArgs a, cudaStream_t st);             // survivors compacted into a.out; totals[1] = their number
 

@@ -12,6 +12,7 @@
 // parallel, one warp each, the warp evaluating a whole window of the back-scan per step.
 #include <cstdlib>
 #include <climits>
+#include <vector>
 #include "lrb_common.cuh"
 #include "lrb_kernels.cuh"
 
@@ -1458,6 +1459,39 @@ void launch_merge_fold(const MergeArgs &a, cudaStream_t st)
         merge_fold_kernel<32><<<(unsigned)bl, MF_THREADS, 0, st>>>(a, (uint32_t *)a.keys, a.dropped, nullptr, 33, 0x7fffffff, 0);
         LRB_COUNT_LAUNCH();
     }
+}
+
+// Test hook (lrb_fold_census): after launch_merge_fold on the same stream, read the locus table back and tally each locus by the path
+// that folded it.  Every kernel writes hard[] at the locus head, and only to hand the locus on (0 flat -> 1 tier 0 -> 4 tier 1 -> 2
+// merge_fold_kernel; 2 also at >= FB_MAXREL members, 3 after a failed class verify), so the final value names the path that finished
+// the locus.  A big locus's locus_cnt holds one byte per sub-stream, written by fold_class_rows_kernel unless class verification had
+// already sent the locus to merge_fold_kernel (hard 3): that byte is stale then and not read.
+cudaError_t merge_fold_census(const MergeArgs &a, cudaStream_t st, int64_t *k)
+{
+    uint64_t n_loci = 0, n_dev = (uint64_t)a.n_cand;
+    cudaError_t e;
+    if ((e = cudaMemcpyAsync(&n_loci, a.totals, 8, cudaMemcpyDeviceToHost, st))) return e;
+    if (a.n_cand_dev && (e = cudaMemcpyAsync(&n_dev, a.n_cand_dev, 8, cudaMemcpyDeviceToHost, st))) return e;
+    if ((e = cudaStreamSynchronize(st))) return e;
+    const int64_t n = n_dev > (uint64_t)a.n_cand ? 0 : (int64_t)n_dev;      // as cand_count: an undersized list is folded empty
+    if (a.n_cand <= 0 || n == 0 || n_loci == 0) return cudaSuccess;
+    const bool exact = a.up.ss_dis == 0;
+    std::vector<uint32_t> ls(n_loci), cnt(n_loci); std::vector<uint8_t> hard(n);
+    if ((e = cudaMemcpyAsync(ls.data(), a.locus_start, n_loci * 4, cudaMemcpyDeviceToHost, st))) return e;
+    if (exact && (e = cudaMemcpyAsync(cnt.data(), a.locus_cnt, n_loci * 4, cudaMemcpyDeviceToHost, st))) return e;
+    if (exact && (e = cudaMemcpyAsync(hard.data(), a.hard, (size_t)n, cudaMemcpyDeviceToHost, st))) return e;
+    if ((e = cudaStreamSynchronize(st))) return e;
+    for (uint64_t loc = 0; loc < n_loci; ++loc) {
+        const int64_t m = (loc + 1 < n_loci ? (int64_t)ls[loc + 1] : n) - (int64_t)ls[loc];
+        if (a.single_locus) ++k[LRB_FC_SINGLE];
+        if (!exact) { ++k[m <= 32 ? LRB_FC_D_SMALL : LRB_FC_D_LARGE]; continue; }   // merge_fold_kernel<8> / <32>
+        const int h = hard[ls[loc]];
+        if (h == 0 && m <= FF_MAX) { ++k[LRB_FC_FLAT]; continue; }
+        ++k[h <= 1 ? LRB_FC_TIER0 : h == 4 ? LRB_FC_TIER1 : h == 2 ? LRB_FC_MERGE_OVER : LRB_FC_MERGE_VERIFY];
+        if (h == 3) continue;
+        for (int s = 0; s < (a.kls ? 4 : 1); ++s) k[LRB_FC_NOROWS] += ((const uint8_t *)&cnt[loc])[s] == FB_NOROWS;
+    }
+    return cudaSuccess;
 }
 
 // ------------------------------------------------------------------------------ split pieces that meet ANOTHER chromosome
