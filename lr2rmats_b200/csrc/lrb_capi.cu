@@ -110,7 +110,7 @@ int run_select(lrb_ctx *c, const lrb_filter_params *fp)
 int setup_merge(lrb_ctx *c, MergeBufs &m, int64_t n_cand)
 {
     size_t n = (size_t)std::max<int64_t>(n_cand, 1);
-    NEED(m.keys, n * 8); NEED(m.head, n); NEED(m.locus_start, (n + 1) * 4); NEED(m.locus_cnt, n * 4); NEED(m.dropped, n);
+    NEED(m.tlist, n * 8); NEED(m.head, n); NEED(m.locus_start, (n + 1) * 4); NEED(m.locus_cnt, n * 4); NEED(m.alive, n);
     NEED(m.rep, n * 4); NEED(m.lstart, n * 4); NEED(m.evmask, n * 8); NEED(m.samemask, n * 8); NEED(m.hard, n); NEED(m.desc, n * 2); NEED(m.relsym, n * 8); NEED(m.ckey, (2 * n + 64) * 8); NEED(m.cmin, (2 * n + 64) * 4); NEED(m.cord, n); NEED(m.clist, n * 4); NEED(m.crow, n * 16); NEED(m.fb_list, n * 8); NEED(m.fb_cnt, 64);
     const Extent e{(int64_t)n};
     int rc;
@@ -144,8 +144,8 @@ int run_merge_async(lrb_ctx *c, MergeBufs &m, const DTransList &list, int64_t n_
     if (n_cand == 0) return LRB_OK;
     MergeArgs a{};
     a.rows = *c->cur; a.ex = c->ex; a.up = up; a.list = list; a.n_cand = n_cand; a.n_cand_dev = n_cand_dev;
-    a.keys = m.keys.as<uint64_t>(); a.head = m.head.as<uint8_t>(); a.locus_start = m.locus_start.as<uint32_t>(); a.locus_cnt = m.locus_cnt.as<uint32_t>();
-    a.dropped = m.dropped.as<uint8_t>();
+    a.tlist = m.tlist.as<uint32_t>(); a.head = m.head.as<uint8_t>(); a.locus_start = m.locus_start.as<uint32_t>(); a.locus_cnt = m.locus_cnt.as<uint32_t>();
+    a.alive = m.alive.as<uint8_t>();
     a.rep = m.rep.as<uint32_t>(); a.lstart = m.lstart.as<uint32_t>(); a.evmask = m.evmask.as<uint64_t>(); a.samemask = m.samemask.as<uint64_t>(); a.hard = m.hard.as<uint8_t>(); a.desc = m.desc.as<uint16_t>(); a.relsym = m.relsym.as<uint64_t>(); a.ckey = m.ckey.as<uint64_t>(); a.cmin = m.cmin.as<uint32_t>(); a.cord = m.cord.as<uint8_t>(); a.clist = m.clist.as<uint32_t>(); a.crow = m.crow.as<uint64_t>(); a.fb_list = m.fb_list.as<uint32_t>(); a.fb_cnt = m.fb_cnt.as<uint32_t>();
     a.work = view(m.w, DMerged{n_cand, n_cand}); a.out = view(m.o, DMerged{n_cand, n_cand}); a.cd = view(m.cd, CandSoA{});
     a.tile_state = o.side ? c->tile_state2.as<uint64_t>() : c->tile_state.as<uint64_t>(); a.ticket = o.side ? d_ticket2(c) : d_ticket(c); a.totals = totals;
@@ -209,6 +209,7 @@ int lrb_ctx_create(int device, lrb_ctx **out)
     { const char *e = getenv("LRB_TEST_SMALL_NOVEL_CAP"); if (e) c->test_small_novel_cap = atoi(e) != 0; }      // test hook: novel_T sized too small on the first attempt
     { const char *e = getenv("LRB_FORCE_SINGLE_FOLD"); if (e) c->force_single_fold = atoi(e) != 0; }    // test hook: updated_T always folded by the one-locus replay
     { const char *e = getenv("LRB_TEST_FOLD_CENSUS"); if (e) c->fold_census = atoi(e) != 0; }       // test hook: loci tallied by fold path (lrb_fold_census)
+    { const char *e = getenv("LRB_TEST_CLASSIFY_GENERAL"); if (e) c->classify_general = atoi(e) != 0; }   // test hook: every row through classify_kernel
     if (!c->scalars.ensure(512) || !c->h_scalars.ensure(512)) { delete c; return LRB_E_NOMEM; }
     cudaMemsetAsync(c->scalars.p, 0, 512, c->st);
     for (cudaEvent_t &e : c->ev) cudaEventCreate(&e);
@@ -507,7 +508,7 @@ static int update_classify(lrb_ctx *c, const lrb_update_params *up)
     ca.rows = rows; ca.ex = c->ex; ca.anno = c->anno; ca.sj = c->sj; ca.up = *up;
     ca.row_nonmono = c->have_batch ? nullptr : c->r_nonmono.as<uint8_t>();
     ca.cls = c->u_cls.as<uint32_t>(); ca.ref = c->u_ref.as<int32_t>(); ca.n_novel = c->u_nnovel.as<uint32_t>(); ca.err_flags = d_err(c);
-    launch_classify(ca, c->u_mk.as<uint8_t>(), c->st);     // u_mk: scratch for the slow-row mask
+    launch_classify(ca, c->classify_general ? nullptr : c->u_mk.as<uint8_t>(), c->st);     // u_mk: scratch for the slow-row mask
     CK(cudaGetLastError());
     tick(c, EV_CLASSIFIED);
     return LRB_OK;
@@ -736,11 +737,11 @@ int lrb_unique_run(lrb_ctx *c, const lrb_update_params *up)
     // proven for (tid,start)-sorted streams, so an unsorted list is folded as ONE locus: the back-scan of merge_trans is
     // replayed entry by entry (merge_fold_kernel), early-termination quirks included.
     if ((rc = run_merge(c, c->mg, c->tmp_list, n, *up, (flags & 4u) != 0))) return rc;
-    // shared_T = rows the fold absorbed: complement of the alive mask (kept in mg.dropped); mg.head is free again
+    // shared_T = rows the fold absorbed: complement of the alive mask (kept in mg.alive); mg.head is free again
     NEED(c->q_shared, (size_t)std::max<int64_t>(n, 1) * 4);
     c->n_shared = 0;
     if (n) {
-        invert_mask_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->st>>>(c->mg.dropped.as<uint8_t>(), c->mg.head.as<uint8_t>(), n);
+        invert_mask_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->st>>>(c->mg.alive.as<uint8_t>(), c->mg.head.as<uint8_t>(), n);
         launch_compact_mask(c->mg.head.as<uint8_t>(), n, nullptr, c->q_shared.as<uint32_t>(), nullptr, c->tile_state.as<uint64_t>(), d_ticket(c), d_totals(c), c->st);
         CK(cudaGetLastError());
         uint64_t t; if ((rc = read_totals(c, &t, 1))) return rc;

@@ -105,11 +105,25 @@ template <int G> LRB_DEVINL int group_or(unsigned m, int v)
     return v;
 }
 
+// first index in [lo, hi) with a[idx] > key (a non-decreasing)
+template <class T> LRB_DEVINL int64_t upper_bound_dev(const T *a, int64_t lo, int64_t hi, T key)
+{
+    while (lo < hi) { int64_t mid = (lo + hi) >> 1; if (a[mid] > key) hi = mid; else lo = mid + 1; }
+    return lo;
+}
+// first index in [lo, hi) with a[idx] >= key
+template <class T> LRB_DEVINL int64_t lower_bound_dev(const T *a, int64_t lo, int64_t hi, T key)
+{
+    while (lo < hi) { int64_t mid = (lo + hi) >> 1; if (a[mid] < key) lo = mid + 1; else hi = mid; }
+    return lo;
+}
+
 // cooperative (G+1)-ary searches: the G lanes of a group probe G pivots per step (one load each, in parallel), so a
 // search over n keys costs ~log_{G+1}(n) dependent loads instead of log_2(n).  `a` non-decreasing; all lanes of the
-// group must call with the same arguments and receive the same result.
+// group must call with the same arguments and receive the same result.  A group of one lane runs the plain binary search.
 template <int G, class T> LRB_DEVINL int64_t group_upper_bound(unsigned m, int gl, const T *a, int64_t lo, int64_t hi, T key)
 {
+    if constexpr (G == 1) return upper_bound_dev(a, lo, hi, key);
     const int sh = (lane_id() / G) * G;
     while (hi - lo > G) {
         const int64_t span = hi - lo;
@@ -128,6 +142,7 @@ template <int G, class T> LRB_DEVINL int64_t group_upper_bound(unsigned m, int g
 }
 template <int G, class T> LRB_DEVINL int64_t group_lower_bound(unsigned m, int gl, const T *a, int64_t lo, int64_t hi, T key)
 {
+    if constexpr (G == 1) return lower_bound_dev(a, lo, hi, key);
     const int sh = (lane_id() / G) * G;
     while (hi - lo > G) {
         const int64_t span = hi - lo;
@@ -148,19 +163,6 @@ template <int G, class T> LRB_DEVINL int64_t group_lower_bound(unsigned m, int g
 // --------------------------------------------------------------------------------------------- memory helpers
 LRB_DEVINL uint4 ldg_stream_u4(const uint4 *p) { uint4 r; asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p)); return r; }
 LRB_DEVINL uint32_t ldg_stream_u32(const uint32_t *p) { uint32_t r; asm volatile("ld.global.nc.L1::no_allocate.u32 %0, [%1];" : "=r"(r) : "l"(p)); return r; }
-
-// first index in [lo, hi) with a[idx] > key (a non-decreasing)
-template <class T> LRB_DEVINL int64_t upper_bound_dev(const T *a, int64_t lo, int64_t hi, T key)
-{
-    while (lo < hi) { int64_t mid = (lo + hi) >> 1; if (a[mid] > key) hi = mid; else lo = mid + 1; }
-    return lo;
-}
-// first index in [lo, hi) with a[idx] >= key
-template <class T> LRB_DEVINL int64_t lower_bound_dev(const T *a, int64_t lo, int64_t hi, T key)
-{
-    while (lo < hi) { int64_t mid = (lo + hi) >> 1; if (a[mid] < key) lo = mid + 1; else hi = mid; }
-    return lo;
-}
 
 LRB_DEVINL int iabs_dev(int x) { return x < 0 ? -x : x; }
 

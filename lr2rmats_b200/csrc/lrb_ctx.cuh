@@ -159,7 +159,7 @@ struct UpdateOut {                                  // lrb_update_fetch, lrb_upd
 struct UniqueOut { ExonsOut ex; MergedCols<PBuf> uniq; PBuf shared; };
 
 struct MergeBufs {                                  // scratch + output of one merge fold
-    Buf keys, head, locus_start, locus_cnt, dropped, rep, lstart, evmask, samemask, hard, desc, relsym, ckey, cmin, cord, clist, crow, fb_list, fb_cnt;
+    Buf tlist, head, locus_start, locus_cnt, alive, rep, lstart, evmask, samemask, hard, desc, relsym, ckey, cmin, cord, clist, crow, fb_list, fb_cnt;
     MergedCols<Buf> w, o;                           // work list, survivors
     CandCols<Buf> cd;
     int64_t n_out = 0, n_loci = 0;
@@ -211,6 +211,7 @@ struct lrb_ctx {
     int32_t summary[LRB_S_COUNT];
     bool force_single_fold = false, test_small_novel_cap = false, want_kg_pairs = false; int64_t n_xlocus_replays = 0, n_xlocus_pieces = 0, n_kg_pairs = 0; Buf kg_pairs;
     bool fold_census = false; int64_t census[2][LRB_FC_COUNT] = {};   // test hook LRB_TEST_FOLD_CENSUS: loci per fold path, main / side stream
+    bool classify_general = false;                  // test hook LRB_TEST_CLASSIFY_GENERAL: classify_row_kernel is not launched
     Buf xl_key, xl_min, xl_max, xl_cnt, xl_forced; lrbk::XlArgs xl;      // split pieces that meet another chromosome (xl_* kernels)
     // summary
     Buf h_khi, y_barcnt, y_barseg, y_genebar, y_bedcnt, y_bedoff, y_counts, y_nelem;

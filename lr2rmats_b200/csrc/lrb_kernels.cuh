@@ -111,7 +111,7 @@ struct DMerged {
     int64_t n = 0, cap = 0;
     uint32_t *cand = nullptr; int32_t *cov = nullptr, *tid = nullptr, *start = nullptr, *end = nullptr, *fs = nullptr, *le = nullptr;
 };
-struct CandSoA {                                    // flattened fold candidates (see merge_cand_kernel)
+struct CandSoA {                                    // flattened fold candidates (see fold_prepare_kernel)
     int32_t *tid = nullptr, *start = nullptr, *end = nullptr, *rev = nullptr, *n = nullptr, *fs = nullptr, *le = nullptr;
     uint32_t *gbeg = nullptr; uint64_t *hash = nullptr;
     uint64_t *j0 = nullptr;                         // first junction (exon[0].end << 32 | exon[1].start), 0 for single-exon chains
@@ -129,16 +129,18 @@ struct MergeArgs {
     uint64_t *samemask;                             // flat fold with kls: earlier candidates of the locus in the same sub-stream
     uint32_t *class_alive;                          // [4] surviving entries per sub-stream
     // scratch
-    uint64_t *keys;                                 // per candidate (tid+1)<<32|real_end, then prefix max
+    uint32_t *tlist;                                // merge_fold_kernel: candidate index of each entry of T, at the locus' offset
     uint8_t *head;                                  // locus head flags
     uint32_t *locus_start;                          // compacted heads (+ sentinel)
     DMerged work;                                   // per-candidate slots (T entries live at their locus' range)
-    uint32_t *locus_cnt;                            // big loci: number of multi-exon classes (FB_NOROWS: too many for the relation rows)
-    uint8_t *dropped;                               // per candidate: absorbed/dropped by the fold
+    uint32_t *locus_cnt;                            // big loci: number of multi-exon classes per sub-stream (CLASSES_UNTABULATED: too many for the relation rows)
+    uint8_t *alive;                                 // per candidate: 1 = an entry of T after the fold (0: absorbed / dropped)
     uint32_t *rep, *lstart; uint64_t *evmask;       // flat fold: class representative, locus head, absorber mask per candidate
     uint16_t *desc; uint64_t *relsym;               // flat fold: class descriptor per candidate; per representative the related representatives
-    uint8_t *hard;                                  // per locus head: 1 = not for the flat kernels, >= 2 = not for fold_big_kernel either (merge_fold_kernel)
-    uint8_t *cord; uint32_t *clist; uint64_t *crow;  // big loci: class ordinal per candidate; per locus (at its offset) the class representatives and their 128-bit relation rows
+    uint8_t *hard;                                  // per locus head: the path that folds the locus next (LocusPath, lrb_update.cu)
+    uint8_t *cord; uint64_t *crow;                  // big loci: class ordinal per candidate; per representative its 128-bit relation row
+    uint32_t *clist;                                // not used by the fold: the split-piece rounds' piece list (XlArgs::pl)
+    // lent to XlArgs once the fold is done, as well: lstart as its hit list hx, relsym as best
     uint32_t *fb_list, *fb_cnt;                     // big loci: [0, n_cand) list of their locus ordinals, [n_cand, 2 n_cand) those that outgrew tier 0; counters
     uint64_t *ckey; uint32_t *cmin;                 // class table of the big loci: 2 * n_cand + 64 slots
     DMerged out;                                    // compacted result

@@ -43,6 +43,157 @@ LRB_DEVINL int small_lower_bound(const int *a, int n, int key)
     return lo;
 }
 
+// ------------------------------------------------------------------------- classification rules (both kernels below)
+// A rule that lanes share is templated on the group width G (G lanes per read, G == 1: one thread per read); all lanes of a group
+// call it with the same arguments.
+LRB_DEVINL uint64_t tid_key(int tid) { return (uint64_t)(uint32_t)(tid + 1) << 32; }     // high half of the (tid+1)<<32 | coordinate keys
+
+// Rows are sorted by (tid,start), so the annotation cursor F(b), the SJ cursor S(b) and the first SJ row at or after start - dis are
+// monotone in the row index: six searches bracket them for the rows [r0, r1) of a tile.  Search q: F (q = 0, 1), S (2, 3), the donor
+// row (4, 5), each at the first (even q) and the last (odd q) row.
+template <int G>
+LRB_DEVINL int tile_window(const ClassArgs &a, int q, int64_t r0, int64_t r1, unsigned gm, int gl)
+{
+    const int64_t rr = (q & 1) ? r1 - 1 : r0;
+    const uint64_t tk = tid_key(a.rows.tid[rr]);
+    const int st = a.rows.start[rr];
+    if (q < 2) return (int)group_upper_bound<G, uint64_t>(gm, gl, a.anno.pmax_key, 0, a.anno.n, tk | (uint32_t)st);
+    if (!a.sj.n) return 0;
+    if (q < 4) return (int)group_upper_bound<G, uint64_t>(gm, gl, a.sj.pmax_key, 0, a.sj.n, tk | (uint32_t)st);
+    return (int)group_lower_bound<G, uint64_t>(gm, gl, a.sj.don_key, 0, a.sj.n, tk | (uint32_t)max(st - a.up.ss_dis, 0));
+}
+struct TileWin { int Flo, Fhi, Slo, Shi, Dlo, Dhi; };
+LRB_DEVINL TileWin tile_windows(const int *s) { return {s[0], max(s[0], s[1]), s[2], max(s[2], s[3]), s[4], max(s[4], s[5])}; }
+
+// the closed forms need the rows in (tid,start) order: a row out of order sets err_flags bit 0
+LRB_DEVINL void check_row_order(const ClassArgs &a, int64_t row, int tid_b, int start_b)
+{
+    if (row == 0) return;
+    const int pt = a.rows.tid[row - 1], ps = a.rows.start[row - 1];
+    if (pt > tid_b || (pt == tid_b && ps > start_b)) atomicOr(a.err_flags, 1u);
+}
+
+// comp_trans (the sweep of update_gtf.c:792-835): the transcript lies after the read (< 0: the sweep ends) or before it (> 0: skipped)
+LRB_DEVINL bool anno_after(int tid_b, int end_b, int at, int as) { return tid_b < at || (tid_b == at && end_b <= as); }
+LRB_DEVINL bool anno_before(int tid_b, int start_b, int at, int ae) { return at < tid_b || (at == tid_b && ae <= start_b); }
+
+struct ClassState {
+    int lfull = 0, rfull = 0, lnoth = 1, rnoth = 1;   // check_full
+    int known = 0, known_site = 0, ref = -1;
+};
+
+// check_full, update_gtf.c:629-681: the read's first exon [b0s, b0e] and last exon [bls, ble] against transcript (xs, xe, na)
+template <int G>
+LRB_DEVINL void check_full(ClassState &c, int level, int b0s, int b0e, int bls, int ble, const int *xs, const int *xe, int na, unsigned gm, int gl)
+{
+    if ((c.lfull && c.rfull) || level > 4) return;
+    const int a0s = xs[0], a0e = xe[0], als = xs[na - 1], ale = xe[na - 1];
+    if (level == 1) {
+        if (!c.lfull && b0e == a0e) c.lfull = 1;
+        if (!c.rfull && bls == als) c.rfull = 1;
+    } else if (level == 2) {
+        if (!c.lfull && ex_ovlp(b0s, b0e, a0s, a0e)) c.lfull = 1;
+        if (!c.rfull && ex_ovlp(bls, ble, als, ale)) c.rfull = 1;
+    } else if (level == 3 || level == 4) {
+        bool need_l = false, need_r = false;
+        if (!c.lfull) { if (ex_ovlp(b0s, b0e, a0s, a0e)) c.lfull = 1; else need_l = c.lnoth; }
+        if (level == 3 && !c.rfull) { if (ex_ovlp(bls, ble, als, ale)) c.rfull = 1; else need_r = c.rnoth; }
+        if (need_l | need_r) {
+            int lany = 0, rany = 0;
+            for (int k = gl; k < na; k += G) { const int s2 = xs[k], e2 = xe[k]; lany |= ex_ovlp(b0s, b0e, s2, e2); rany |= ex_ovlp(bls, ble, s2, e2); }
+            if (need_l && group_or<G>(gm, lany)) c.lnoth = 0;
+            if (need_r && group_or<G>(gm, rany)) c.rnoth = 0;
+        }
+    }
+}
+
+// update_gtf.c:806-811: a single-exon read is known through a single-exon transcript it overlaps by at least -f
+LRB_DEVINL bool single_exon_known(const ClassArgs &a, int b0s, int b0e, int a0s, int a0e)
+{
+    return ovlp_frac(b0s, b0e, a0s, a0e) >= a.up.single_exon_ovlp_frac;
+}
+
+// check_splice_site's verdict for transcript i (update_gtf.c:812-821): every splice site of the read inside the overlap matches -> known,
+// and the sweep ends (true); some match -> known_site through this transcript
+LRB_DEVINL bool splice_verdict(ClassState &c, int n, int ovl, int iden, int i)
+{
+    if (2 * (n - 1) == ovl && ovl == iden) { c.known = 1; c.ref = i; return true; }
+    if (iden > 0) { c.known_site = 1; c.ref = i; }
+    return false;
+}
+
+// set_full, update_gtf.c:683-696
+LRB_DEVINL int set_full(const ClassState &c, int level)
+{
+    if (level == 5) return 1;
+    if (level == 4) return c.lfull || c.lnoth;
+    if (level == 3) return (c.lfull || c.lnoth) && (c.rfull || c.rnoth);
+    return c.lfull && c.rfull;
+}
+
+// check_with_short_sj, update_gtf.c:589-627, cursor closed form (App. B.2): false when the SJ cursor S(b) has no junction row left that
+// starts inside the read.  Else R0 = the first row with the read's tid and donor >= start - dis, never below S.
+template <int G>
+LRB_DEVINL bool sj_cursor(const ClassArgs &a, const TileWin &w, uint64_t key_b, int tid_b, int start_b, int end_b, unsigned gm, int gl, int64_t &R0)
+{
+    const int64_t S = group_upper_bound<G, uint64_t>(gm, gl, a.sj.pmax_key, w.Slo, w.Shi, key_b);
+    if (S >= a.sj.n) return false;
+    const int st = a.sj.tid[S];
+    if (st > tid_b || (st == tid_b && a.sj.don[S] >= end_b)) return false;
+    R0 = group_lower_bound<G, uint64_t>(gm, gl, a.sj.don_key, w.Dlo, w.Dhi, tid_key(tid_b) | (uint32_t)max(start_b - a.up.ss_dis, 0));
+    if (R0 < S) R0 = S;
+    return true;
+}
+
+// check_short_sj / check_short_sj1 (:698-709) for the intron [is, ie]: an SJ row with the read's tid, donor in [is-dis, is+dis] and below
+// ie, acceptor within dis of ie and enough reads (-j, -J).  The rows are searched from `from` on (gallop, then bisect); `from` moves to
+// the first row of the donor window, where the search for a later intron of a chain with ascending introns may start.
+LRB_DEVINL bool sj_supported(const ClassArgs &a, int tid_b, int is, int ie, int64_t &from)
+{
+    const int dis = a.up.ss_dis;
+    const uint64_t tk = tid_key(tid_b);
+    int dlo = is - dis; if (dlo < 0) dlo = 0;
+    int64_t dhi = (int64_t)is + dis + 1; if (dhi > ie) dhi = ie; if (dhi < 0) dhi = 0;
+    const uint64_t klo = tk | (uint32_t)dlo, khi = tk | (uint64_t)dhi;
+    int64_t lo = from, step = 1, hi = from;
+    while (hi < a.sj.n && a.sj.don_key[hi] < klo) { lo = hi + 1; hi += step; step <<= 1; }
+    if (hi > a.sj.n) hi = a.sj.n;
+    lo = lower_bound_dev<uint64_t>(a.sj.don_key, lo, hi, klo);
+    from = lo;
+    for (int64_t q = lo; q < a.sj.n; ++q) {
+        if (a.sj.don_key[q] >= khi) break;
+        if (iabs_dev(a.sj.acc[q] - ie) <= dis) {
+            const int c = a.up.use_multi ? a.sj.cnt_u[q] + a.sj.cnt_m[q] : a.sj.cnt_u[q];
+            if (c >= a.up.min_sj_cnt) return true;
+        }
+    }
+    return false;
+}
+
+// split_trans (update_gtf.c:837-913): the chain of n exons is cut after every unreliable junction; a piece of at least two exons with a
+// novel and a known junction is emitted as emit(first exon, last exon).  novel_junc(k) / unreliable(k): flags of junction k (< n - 1).
+template <class NovelJ, class Unrel, class Emit>
+LRB_DEVINL void split_trans(int n, NovelJ novel_junc, Unrel unreliable, Emit emit)
+{
+    int last = 0, has_novel = 0, has_known = 0;
+    for (int k = 0; k <= n - 1; ++k) {
+        const bool at_end = k == n - 1;
+        if (!at_end) { if (novel_junc(k)) has_novel = 1; else has_known = 1; }
+        if (at_end || unreliable(k)) {
+            if (has_novel && has_known && k - last >= 1) emit(last, k);
+            last = k + 1; has_novel = 0; has_known = 0;
+        }
+    }
+}
+
+LRB_DEVINL uint32_t class_word(const ClassState &c, int full, int sj_checked, int unreliable)
+{
+    return (c.known ? LRB_C_KNOWN : 0) | (c.known_site ? LRB_C_KNOWN_SITE : 0) | (unreliable ? LRB_C_UNRELIABLE : 0) | (full ? LRB_C_FULL : 0) |
+           (c.lfull ? LRB_C_LFULL : 0) | (c.rfull ? LRB_C_RFULL : 0) | (c.lnoth ? LRB_C_LNOTH : 0) | (c.rnoth ? LRB_C_RNOTH : 0) |
+           (sj_checked ? LRB_C_SJ_CHECKED : 0);
+}
+
+// ------------------------------------------------------------------------------------- classification, lane group per read
 // G lanes per read (power of two), CL_SLOTS exon slots per read staged in shared memory
 template <int G, int CL_SLOTS>
 __global__ void __launch_bounds__(CL_THREADS) classify_kernel(ClassArgs a, const uint8_t *__restrict__ only)
@@ -52,13 +203,11 @@ __global__ void __launch_bounds__(CL_THREADS) classify_kernel(ClassArgs a, const
     static_assert(((STRIDE / G) & 1) == 1 && STRIDE % G == 0, "bank-conflict-free stride");
     __shared__ int s_es[GPB][STRIDE], s_ee[GPB][STRIDE];
     __shared__ uint8_t s_fl[GPB][STRIDE];
-    __shared__ int s_win[6];                         // search windows of this block's rows: F, S, don_key lower bounds
+    __shared__ int s_win[6];
     const int g = threadIdx.x / G, gl = threadIdx.x % G;
     const unsigned gm = group_mask<G>();
     const int dis = a.up.ss_dis, level = a.up.full_level;
 
-    // Rows are sorted by (tid,start), so the annotation cursor F(b), the SJ cursor S(b) and the first SJ row at or after
-    // the read start are monotone in the row index: six full binary searches per block bracket them for all its rows.
     const int64_t r0 = (int64_t)blockIdx.x * GPB * CL_ITERS;
     const int64_t r1 = min(a.rows.n, r0 + (int64_t)GPB * CL_ITERS);
     if (only) {                                      // nothing left for this block after classify_row_kernel?
@@ -66,32 +215,17 @@ __global__ void __launch_bounds__(CL_THREADS) classify_kernel(ClassArgs a, const
         for (int64_t r = r0 + threadIdx.x; r < r1; r += CL_THREADS) any |= only[r];
         if (!__syncthreads_or(any)) return;
     }
-    if (threadIdx.x < 6) {
-        const int64_t rr = (threadIdx.x & 1) ? r1 - 1 : r0;
-        const int t = a.rows.tid[rr], st = a.rows.start[rr];
-        const uint64_t key = ((uint64_t)(uint32_t)(t + 1) << 32) | (uint32_t)st;
-        int v;
-        if (threadIdx.x < 2) v = (int)upper_bound_dev<uint64_t>(a.anno.pmax_key, 0, a.anno.n, key);
-        else if (threadIdx.x < 4) v = a.sj.n ? (int)upper_bound_dev<uint64_t>(a.sj.pmax_key, 0, a.sj.n, key) : 0;
-        else {
-            int wlo = st - dis; if (wlo < 0) wlo = 0;
-            v = a.sj.n ? (int)lower_bound_dev<uint64_t>(a.sj.don_key, 0, a.sj.n, (((uint64_t)(uint32_t)(t + 1)) << 32) | (uint32_t)wlo) : 0;
-        }
-        s_win[threadIdx.x] = v;
-    }
+    if (threadIdx.x < 6) s_win[threadIdx.x] = tile_window<1>(a, threadIdx.x, r0, r1, FULL, 0);      // one thread per search
     __syncthreads();
-    const int Flo = s_win[0], Fhi = max(s_win[0], s_win[1]), Slo = s_win[2], Shi = max(s_win[2], s_win[3]), Dlo = s_win[4], Dhi = max(s_win[4], s_win[5]);
+    const TileWin w = tile_windows(s_win);
 
     for (int64_t row = r0 + g; row < r1; row += GPB) {
-        if (only && !only[row]) continue;               // classified by classify_fast_kernel
+        if (only && !only[row]) continue;               // classified by classify_row_kernel
         const int n = (int)a.rows.ex_n[row];
         const uint32_t beg = a.rows.ex_beg[row];
         const int tid_b = a.rows.tid[row], start_b = a.rows.start[row], end_b = a.rows.end[row];
         if (n == 0) { if (gl == 0) { atomicOr(a.err_flags, 2u); a.cls[row] = 0; a.ref[row] = -1; a.n_novel[row] = 0; } continue; }
-        if (row > 0 && gl == 0) {
-            int pt = a.rows.tid[row - 1], ps = a.rows.start[row - 1];
-            if (pt > tid_b || (pt == tid_b && ps > start_b)) atomicOr(a.err_flags, 1u);
-        }
+        if (gl == 0) check_row_order(a, row, tid_b, start_b);
         // exon chain + flags: shared memory when it fits, else straight on the HBM arrays
         const bool in_smem = n <= CL_SLOTS;
         int *es = in_smem ? s_es[g] : a.ex.es + beg, *ee = in_smem ? s_ee[g] : a.ex.ee + beg;
@@ -105,45 +239,17 @@ __global__ void __launch_bounds__(CL_THREADS) classify_kernel(ClassArgs a, const
         const int b0s = es[0], b0e = ee[0], bls = es[n - 1], ble = ee[n - 1];
 
         // ---- annotation window: F(b) by a cooperative search on the prefix-max keys, sweep to the first "after"
-        const uint64_t key_b = ((uint64_t)(uint32_t)(tid_b + 1) << 32) | (uint32_t)start_b;
-        int i = (int)group_upper_bound<G, uint64_t>(gm, gl, a.anno.pmax_key, Flo, Fhi, key_b);
-        int lfull = 0, rfull = 0, lnoth = 1, rnoth = 1, known = 0, known_site = 0, ref = -1;
-        for (; i < a.anno.n; ++i) {
+        const uint64_t key_b = tid_key(tid_b) | (uint32_t)start_b;
+        ClassState c;
+        for (int i = (int)group_upper_bound<G, uint64_t>(gm, gl, a.anno.pmax_key, w.Flo, w.Fhi, key_b); i < a.anno.n; ++i) {
             const int at = a.anno.tid[i], as_ = a.anno.start[i], ae_ = a.anno.end[i];
-            if (tid_b < at || (tid_b == at && end_b <= as_)) break;                       // comp_trans < 0
-            if (at < tid_b || (at == tid_b && ae_ <= start_b)) continue;                  // comp_trans > 0
+            if (anno_after(tid_b, end_b, at, as_)) break;
+            if (anno_before(tid_b, start_b, at, ae_)) continue;
             const uint32_t ao = a.anno.exon_off[i]; const int na = (int)(a.anno.exon_off[i + 1] - ao);
             const int *xs = a.anno.es + ao, *xe = a.anno.ee + ao;
-            // check_full, update_gtf.c:629-681
-            if (!(lfull && rfull) && level <= 4) {
-                const int a0s = xs[0], a0e = xe[0], als = xs[na - 1], ale = xe[na - 1];
-                if (level == 1) {
-                    if (!lfull && b0e == a0e) lfull = 1;
-                    if (!rfull && bls == als) rfull = 1;
-                } else if (level == 2) {
-                    if (!lfull && ex_ovlp(b0s, b0e, a0s, a0e)) lfull = 1;
-                    if (!rfull && ex_ovlp(bls, ble, als, ale)) rfull = 1;
-                } else if (level == 3 || level == 4) {
-                    if (!lfull) {
-                        if (ex_ovlp(b0s, b0e, a0s, a0e)) lfull = 1;
-                        else if (lnoth) {
-                            int any = 0;
-                            for (int ii = gl; ii < na; ii += G) any |= ex_ovlp(b0s, b0e, xs[ii], xe[ii]);
-                            if (group_or<G>(gm, any)) lnoth = 0;
-                        }
-                    }
-                    if (level == 3 && !rfull) {
-                        if (ex_ovlp(bls, ble, als, ale)) rfull = 1;
-                        else if (rnoth) {
-                            int any = 0;
-                            for (int ii = gl; ii < na; ii += G) any |= ex_ovlp(bls, ble, xs[ii], xe[ii]);
-                            if (group_or<G>(gm, any)) rnoth = 0;
-                        }
-                    }
-                }
-            }
-            if (n == 1 && na == 1) {                                                       // update_gtf.c:806-811
-                if (ovlp_frac(b0s, b0e, xs[0], xe[0]) >= a.up.single_exon_ovlp_frac) { ref = i; known = 1; break; }
+            check_full<G>(c, level, b0s, b0e, bls, ble, xs, xe, na, gm, gl);
+            if (n == 1 && na == 1) {
+                if (single_exon_known(a, b0s, b0e, xs[0], xe[0])) { c.ref = i; c.known = 1; break; }
             } else if (n > 1 && na > 1) {                                                  // check_splice_site :717-779
                 const int os = max(start_b, as_), oe = min(end_b, ae_);
                 int ovl = 0, iden = 0;
@@ -193,88 +299,43 @@ __global__ void __launch_bounds__(CL_THREADS) classify_kernel(ClassArgs a, const
                         }
                     }
                 }
-                ovl = group_sum<G>(gm, ovl); iden = group_sum<G>(gm, iden);
-                if (2 * (n - 1) == ovl && ovl == iden) { known = 1; ref = i; break; }
-                else if (iden > 0) { known_site = 1; ref = i; }
+                if (splice_verdict(c, n, group_sum<G>(gm, ovl), group_sum<G>(gm, iden), i)) break;
             }
         }
         int is_rev = a.rows.is_rev[row];
-        if (ref != -1) is_rev = a.anno.is_rev[ref];                                       // update_gtf.c:823-833
-        int full;                                                                          // set_full :683-696
-        if (level == 5) full = 1;
-        else if (level == 4) full = (lfull || lnoth);
-        else if (level == 3) full = ((lfull || lnoth) && (rfull || rnoth));
-        else full = (lfull && rfull);
+        if (c.ref != -1) is_rev = a.anno.is_rev[c.ref];                                   // update_gtf.c:823-833
+        const int full = set_full(c, level);
         __syncwarp(gm);
 
-        // ---- short-read SJ support, update_gtf.c:589-627,698-709 (cursor closed form, App. B.2)
+        // ---- short-read SJ support; a chain here need not have ascending introns, so every intron is searched from R0
         int sj_checked = 0, unreliable = 0;
-        if (full && !known && known_site && a.sj.n > 0) {
+        if (full && !c.known && c.known_site && a.sj.n > 0) {
             sj_checked = 1;
-            const int64_t S = group_upper_bound<G, uint64_t>(gm, gl, a.sj.pmax_key, Slo, Shi, key_b);
-            int ok = 1;
-            if (S >= a.sj.n) ok = 0;
-            else {
-                int st = a.sj.tid[S];
-                if (st > tid_b || (st == tid_b && a.sj.don[S] >= end_b)) ok = 0;
-                else {
-                    int bad = 0;
-                    const uint64_t tk = (uint64_t)(uint32_t)(tid_b + 1) << 32;
-                    // first row with tid == tid_b and don >= start_b - dis (never below the cursor S)
-                    int wlo = start_b - dis; if (wlo < 0) wlo = 0;
-                    int64_t R0 = group_lower_bound<G, uint64_t>(gm, gl, a.sj.don_key, Dlo, Dhi, tk | (uint32_t)wlo);
-                    if (R0 < S) R0 = S;
-                    for (int j = gl; j < n - 1; j += G) {
-                        if (!(fl[j] & LRB_F_NOVEL_JUNC)) continue;
-                        const int is = ee[j] + 1, ie = es[j + 1] - 1;                      // intron [is, ie]
-                        // rows with tid==tid_b, don in [is-dis, is+dis], don < ie, index >= S: gallop from R0, then bisect
-                        int dlo = is - dis; if (dlo < 0) dlo = 0;
-                        int64_t dhi = (int64_t)is + dis + 1; if (dhi > ie) dhi = ie; if (dhi < 0) dhi = 0;
-                        const uint64_t klo = tk | (uint32_t)dlo, khi = tk | (uint64_t)dhi;
-                        int64_t lo = R0, step = 1, hi = R0;
-                        while (hi < a.sj.n && a.sj.don_key[hi] < klo) { lo = hi + 1; hi += step; step <<= 1; }
-                        if (hi > a.sj.n) hi = a.sj.n;
-                        lo = lower_bound_dev<uint64_t>(a.sj.don_key, lo, hi, klo);
-                        int found = 0;
-                        for (int64_t q = lo; q < a.sj.n && !found; ++q) {
-                            if (a.sj.don_key[q] >= khi) break;
-                            if (iabs_dev(a.sj.acc[q] - ie) <= dis) {
-                                int c = a.up.use_multi ? a.sj.cnt_u[q] + a.sj.cnt_m[q] : a.sj.cnt_u[q];
-                                if (c >= a.up.min_sj_cnt) found = 1;
-                            }
-                        }
-                        if (!found) { fl[j] |= LRB_F_UNRELIABLE; bad = 1; }
-                    }
-                    if (group_or<G>(gm, bad)) ok = 0;
+            int64_t R0;
+            unreliable = !sj_cursor<G>(a, w, key_b, tid_b, start_b, end_b, gm, gl, R0);
+            if (!unreliable) {
+                int bad = 0;
+                for (int j = gl; j < n - 1; j += G) {
+                    int64_t from = R0;
+                    if ((fl[j] & LRB_F_NOVEL_JUNC) && !sj_supported(a, tid_b, ee[j] + 1, es[j + 1] - 1, from)) { fl[j] |= LRB_F_UNRELIABLE; bad = 1; }
                 }
+                unreliable = group_or<G>(gm, bad);
             }
-            unreliable = !ok;
         }
         __syncwarp(gm);
 
-        // ---- novel_T contribution: the read itself, or its split pieces (split_trans :837-913)
+        // ---- novel_T contribution: the read itself, or its split pieces
         uint32_t nn = 0;
-        if (full && !known && known_site) {
+        if (full && !c.known && c.known_site) {
             if (!sj_checked || !unreliable) nn = 1;
-            else if (a.up.split_trans && gl == 0) {
-                int last = 0, has_novel = 0, has_known = 0;
-                for (int k = 0; k <= n - 1; ++k) {
-                    bool at_end = k == n - 1;
-                    uint8_t f = fl[k];
-                    if (!at_end) { if (f & LRB_F_NOVEL_JUNC) has_novel = 1; else has_known = 1; }
-                    if (at_end || (f & LRB_F_UNRELIABLE)) {
-                        if (has_novel && has_known && k - last >= 1) ++nn;
-                        last = k + 1; has_novel = 0; has_known = 0;
-                    }
-                }
-            }
+            else if (a.up.split_trans && gl == 0)
+                split_trans(n, [&](int k) { return (fl[k] & LRB_F_NOVEL_JUNC) != 0; }, [&](int k) { return (fl[k] & LRB_F_UNRELIABLE) != 0; },
+                            [&](int, int) { ++nn; });
         }
         if (in_smem) for (int j = gl; j < n; j += G) a.ex.flag[beg + j] = fl[j];
         if (gl == 0) {
-            a.cls[row] = (known ? LRB_C_KNOWN : 0) | (known_site ? LRB_C_KNOWN_SITE : 0) | (unreliable ? LRB_C_UNRELIABLE : 0) |
-                         (full ? LRB_C_FULL : 0) | (lfull ? LRB_C_LFULL : 0) | (rfull ? LRB_C_RFULL : 0) | (lnoth ? LRB_C_LNOTH : 0) |
-                         (rnoth ? LRB_C_RNOTH : 0) | (sj_checked ? LRB_C_SJ_CHECKED : 0);
-            a.ref[row] = ref;
+            a.cls[row] = class_word(c, full, sj_checked, unreliable);
+            a.ref[row] = c.ref;
             a.rows.is_rev[row] = (uint8_t)is_rev;
             a.n_novel[row] = nn;
         }
@@ -297,21 +358,9 @@ __global__ void __launch_bounds__(CR_THREADS, CR_MINB) classify_row_kernel(Class
     int t = threadIdx.x;
     const int dis = a.up.ss_dis, level = a.up.full_level;
     const int64_t r0 = (int64_t)blockIdx.x * CR_THREADS, r1 = min(a.rows.n, r0 + (int64_t)CR_THREADS);
-    {   // bracket the three cursors for the rows of this tile (rows are sorted): six cooperative 33-ary searches, warps 0..3
-        const int w = warp_id(), lane = lane_id();
-        for (int q = w; q < 6; q += CR_THREADS / 32) {
-            const int64_t rr = (q & 1) ? r1 - 1 : r0;
-            const int tt = a.rows.tid[rr], st = a.rows.start[rr];
-            const uint64_t key = ((uint64_t)(uint32_t)(tt + 1) << 32) | (uint32_t)st;
-            int v;
-            if (q < 2) v = (int)group_upper_bound<32, uint64_t>(FULL, lane, a.anno.pmax_key, 0, a.anno.n, key);
-            else if (q < 4) v = a.sj.n ? (int)group_upper_bound<32, uint64_t>(FULL, lane, a.sj.pmax_key, 0, a.sj.n, key) : 0;
-            else {
-                int wlo = st - dis; if (wlo < 0) wlo = 0;
-                v = a.sj.n ? (int)group_lower_bound<32, uint64_t>(FULL, lane, a.sj.don_key, 0, a.sj.n, (((uint64_t)(uint32_t)(tt + 1)) << 32) | (uint32_t)wlo) : 0;
-            }
-            if (lane == 0) s_win[q] = v;
-        }
+    for (int q = warp_id(); q < 6; q += CR_THREADS / 32) {          // six cooperative 33-ary searches, warps 0..3
+        const int v = tile_window<32>(a, q, r0, r1, FULL, lane_id());
+        if (lane_id() == 0) s_win[q] = v;
     }
     __syncthreads();
     if (by_exon_count) {
@@ -341,52 +390,30 @@ __global__ void __launch_bounds__(CR_THREADS, CR_MINB) classify_row_kernel(Class
     }
     const int64_t row = r0 + t;
     if (row >= r1) return;
-    const int Flo = s_win[0], Fhi = max(s_win[0], s_win[1]), Slo = s_win[2], Shi = max(s_win[2], s_win[3]), Dlo = s_win[4], Dhi = max(s_win[4], s_win[5]);
+    const TileWin w = tile_windows(s_win);
     const int n = (int)a.rows.ex_n[row];
     const uint32_t beg = a.rows.ex_beg[row];
     const int tid_b = a.rows.tid[row], start_b = a.rows.start[row], end_b = a.rows.end[row];
-    if (row > 0) {
-        const int pt = a.rows.tid[row - 1], ps = a.rows.start[row - 1];
-        if (pt > tid_b || (pt == tid_b && ps > start_b)) atomicOr(a.err_flags, 1u);             // the closed forms need (tid,start) order
-    }
+    check_row_order(a, row, tid_b, start_b);
     if (dis != 0 || n < 1 || n > 32 || (row_nonmono && row_nonmono[row])) { slow[row] = 1; return; }
     const int *__restrict__ es = a.ex.es + beg, *__restrict__ ee = a.ex.ee + beg;
     const int b0s = es[0], b0e = ee[0], bls = es[n - 1], ble = ee[n - 1];
-    const uint64_t key_b = ((uint64_t)(uint32_t)(tid_b + 1) << 32) | (uint32_t)start_b;
+    const uint64_t key_b = tid_key(tid_b) | (uint32_t)start_b;
 
     // ---- annotation window: F(b) on the prefix-max keys, sweep to the first "after" (update_gtf.c:792-835)
-    int lfull = 0, rfull = 0, lnoth = 1, rnoth = 1, known = 0, known_site = 0, ref = -1;
+    ClassState c;
     uint32_t c_don = 0, c_acc = 0, c_junc = 0, c_exon = 0;                                     // cleared novel_* flags, bit j
-    for (int i = (int)upper_bound_dev<uint64_t>(a.anno.pmax_key, Flo, Fhi, key_b); i < a.anno.n; ++i) {
+    for (int i = (int)upper_bound_dev<uint64_t>(a.anno.pmax_key, w.Flo, w.Fhi, key_b); i < a.anno.n; ++i) {
         const int at = a.anno.tid[i], as_ = a.anno.start[i];
-        if (tid_b < at || (tid_b == at && end_b <= as_)) break;                                 // comp_trans < 0
+        if (anno_after(tid_b, end_b, at, as_)) break;
         const int ae_ = a.anno.end[i];
-        if (at < tid_b || (at == tid_b && ae_ <= start_b)) continue;                            // comp_trans > 0
+        if (anno_before(tid_b, start_b, at, ae_)) continue;
         if (!a.anno.mono[i]) { slow[row] = 1; return; }                                         // nothing was written yet
         const uint32_t ao = a.anno.exon_off[i]; const int na = (int)(a.anno.exon_off[i + 1] - ao);
         const int *__restrict__ xs = a.anno.es + ao, *__restrict__ xe = a.anno.ee + ao;
-        if (!(lfull && rfull) && level <= 4) {                                                  // check_full, update_gtf.c:629-681
-            const int a0s = xs[0], a0e = xe[0], als = xs[na - 1], ale = xe[na - 1];
-            if (level == 1) {
-                if (!lfull && b0e == a0e) lfull = 1;
-                if (!rfull && bls == als) rfull = 1;
-            } else if (level == 2) {
-                if (!lfull && ex_ovlp(b0s, b0e, a0s, a0e)) lfull = 1;
-                if (!rfull && ex_ovlp(bls, ble, als, ale)) rfull = 1;
-            } else if (level == 3 || level == 4) {
-                bool need_l = false, need_r = false;
-                if (!lfull) { if (ex_ovlp(b0s, b0e, a0s, a0e)) lfull = 1; else need_l = lnoth; }
-                if (level == 3 && !rfull) { if (ex_ovlp(bls, ble, als, ale)) rfull = 1; else need_r = rnoth; }
-                if (need_l | need_r) {
-                    bool lany = false, rany = false;
-                    for (int k = 0; k < na; ++k) { const int s2 = xs[k], e2 = xe[k]; lany |= ex_ovlp(b0s, b0e, s2, e2); rany |= ex_ovlp(bls, ble, s2, e2); }
-                    if (need_l && lany) lnoth = 0;
-                    if (need_r && rany) rnoth = 0;
-                }
-            }
-        }
-        if (n == 1 && na == 1) {                                                                // update_gtf.c:806-811
-            if (ovlp_frac(b0s, b0e, xs[0], xe[0]) >= a.up.single_exon_ovlp_frac) { ref = i; known = 1; break; }
+        check_full<1>(c, level, b0s, b0e, bls, ble, xs, xe, na, FULL, 0);
+        if (n == 1 && na == 1) {
+            if (single_exon_known(a, b0s, b0e, xs[0], xe[0])) { c.ref = i; c.known = 1; break; }
         } else if (n > 1 && na > 1) {                                                           // check_splice_site :717-779, exact matching
             const int os = max(start_b, as_), oe = min(end_b, ae_);
             int ovl = 0, iden = 0, ps = 0, pe = 0, bs = b0s, be = b0e;
@@ -428,75 +455,34 @@ __global__ void __launch_bounds__(CR_THREADS, CR_MINB) classify_row_kernel(Class
                     bs = sn; be = ee[j + 1];
                 }
             }
-            if (2 * (n - 1) == ovl && ovl == iden) { known = 1; ref = i; break; }
-            else if (iden > 0) { known_site = 1; ref = i; }
+            if (splice_verdict(c, n, ovl, iden, i)) break;
         }
     }
-    int full;                                                                                    // set_full :683-696
-    if (level == 5) full = 1;
-    else if (level == 4) full = (lfull || lnoth);
-    else if (level == 3) full = ((lfull || lnoth) && (rfull || rnoth));
-    else full = (lfull && rfull);
+    const int full = set_full(c, level);
 
-    // ---- short-read SJ support, update_gtf.c:589-627,698-709 (cursor closed form, App. B.2)
+    // ---- short-read SJ support: the introns of a chain here ascend, so each search starts where the last one ended
     int sj_checked = 0, unreliable = 0;
     uint32_t unrel = 0;
-    if (full && !known && known_site && a.sj.n > 0) {
+    if (full && !c.known && c.known_site && a.sj.n > 0) {
         sj_checked = 1;
-        const int64_t S = upper_bound_dev<uint64_t>(a.sj.pmax_key, Slo, Shi, key_b);
-        int ok = 1;
-        if (S >= a.sj.n) ok = 0;
-        else {
-            const int st = a.sj.tid[S];
-            if (st > tid_b || (st == tid_b && a.sj.don[S] >= end_b)) ok = 0;
-            else {
-                const uint64_t tk = (uint64_t)(uint32_t)(tid_b + 1) << 32;
-                int wlo = start_b - dis; if (wlo < 0) wlo = 0;
-                int64_t R0 = lower_bound_dev<uint64_t>(a.sj.don_key, Dlo, Dhi, tk | (uint32_t)wlo);
-                if (R0 < S) R0 = S;
-                uint32_t nj = ~c_junc & (n >= 2 ? (0xffffffffu >> (33 - n)) : 0u);              // novel junctions j < n-1, ascending
-                while (nj) {
-                    const int j = __ffs(nj) - 1; nj &= nj - 1;
-                    const int is = ee[j] + 1, ie = es[j + 1] - 1;                               // intron [is, ie]
-                    int dlo = is - dis; if (dlo < 0) dlo = 0;
-                    int64_t dhi = (int64_t)is + dis + 1; if (dhi > ie) dhi = ie; if (dhi < 0) dhi = 0;
-                    const uint64_t klo = tk | (uint32_t)dlo, khi = tk | (uint64_t)dhi;
-                    int64_t l2 = R0, step = 1, h2 = R0;
-                    while (h2 < a.sj.n && a.sj.don_key[h2] < klo) { l2 = h2 + 1; h2 += step; step <<= 1; }
-                    if (h2 > a.sj.n) h2 = a.sj.n;
-                    l2 = lower_bound_dev<uint64_t>(a.sj.don_key, l2, h2, klo);
-                    R0 = l2;                                                                    // junctions ascend: the next search starts here
-                    int found = 0;
-                    for (int64_t q = l2; q < a.sj.n && !found; ++q) {
-                        if (a.sj.don_key[q] >= khi) break;
-                        if (iabs_dev(a.sj.acc[q] - ie) <= dis) {
-                            const int c = a.up.use_multi ? a.sj.cnt_u[q] + a.sj.cnt_m[q] : a.sj.cnt_u[q];
-                            if (c >= a.up.min_sj_cnt) found = 1;
-                        }
-                    }
-                    if (!found) unrel |= 1u << j;
-                }
-                if (unrel) ok = 0;
+        int64_t R0;
+        unreliable = !sj_cursor<1>(a, w, key_b, tid_b, start_b, end_b, FULL, 0, R0);
+        if (!unreliable) {
+            uint32_t nj = ~c_junc & (n >= 2 ? (0xffffffffu >> (33 - n)) : 0u);              // novel junctions j < n-1, ascending
+            while (nj) {
+                const int j = __ffs(nj) - 1; nj &= nj - 1;
+                if (!sj_supported(a, tid_b, ee[j] + 1, es[j + 1] - 1, R0)) unrel |= 1u << j;
             }
+            unreliable = unrel != 0;
         }
-        unreliable = !ok;
     }
 
-    // ---- novel_T contribution: the read itself, or its split pieces (split_trans :837-913)
+    // ---- novel_T contribution: the read itself, or its split pieces
     uint32_t nn = 0;
-    if (full && !known && known_site) {
+    if (full && !c.known && c.known_site) {
         if (!sj_checked || !unreliable) nn = 1;
-        else if (a.up.split_trans) {
-            int last = 0, has_novel = 0, has_known = 0;
-            for (int k = 0; k <= n - 1; ++k) {
-                const bool at_end = k == n - 1;
-                if (!at_end) { if (!((c_junc >> k) & 1u)) has_novel = 1; else has_known = 1; }
-                if (at_end || ((unrel >> k) & 1u)) {
-                    if (has_novel && has_known && k - last >= 1) ++nn;
-                    last = k + 1; has_novel = 0; has_known = 0;
-                }
-            }
-        }
+        else if (a.up.split_trans)
+            split_trans(n, [&](int k) { return !((c_junc >> k) & 1u); }, [&](int k) { return ((unrel >> k) & 1u) != 0; }, [&](int, int) { ++nn; });
     }
     uint8_t *fl = a.ex.flag + beg;
     for (int j = 0; j < n; ++j) {
@@ -510,11 +496,9 @@ __global__ void __launch_bounds__(CR_THREADS, CR_MINB) classify_row_kernel(Class
         fl[j] = (uint8_t)f;
     }
     slow[row] = 0;
-    a.cls[row] = (known ? LRB_C_KNOWN : 0) | (known_site ? LRB_C_KNOWN_SITE : 0) | (unreliable ? LRB_C_UNRELIABLE : 0) |
-                 (full ? LRB_C_FULL : 0) | (lfull ? LRB_C_LFULL : 0) | (rfull ? LRB_C_RFULL : 0) | (lnoth ? LRB_C_LNOTH : 0) |
-                 (rnoth ? LRB_C_RNOTH : 0) | (sj_checked ? LRB_C_SJ_CHECKED : 0);
-    a.ref[row] = ref;
-    if (ref != -1) a.rows.is_rev[row] = a.anno.is_rev[ref];                                     // update_gtf.c:823-833
+    a.cls[row] = class_word(c, full, sj_checked, unreliable);
+    a.ref[row] = c.ref;
+    if (c.ref != -1) a.rows.is_rev[row] = a.anno.is_rev[c.ref];                                 // update_gtf.c:823-833
     a.n_novel[row] = nn;
 }
 
@@ -602,19 +586,11 @@ __global__ void __launch_bounds__(LS_THREADS) build_lists_kernel(ListArgs a)
             continue;
         }
         const uint8_t *fl = a.ex.flag + a.rows.ex_beg[row];
-        int last = 0, has_novel = 0, has_known = 0, k2 = 0; uint32_t w = o0;
-        for (int j = 0; j <= n - 1; ++j) {
-            const bool at_end = j == n - 1;
-            const uint8_t f = fl[j];
-            if (!at_end) { if (f & LRB_F_NOVEL_JUNC) has_novel = 1; else has_known = 1; }
-            if (at_end || (f & LRB_F_UNRELIABLE)) {
-                if (has_novel && has_known && j - last >= 1) {
-                    a.novel.row[w] = (uint32_t)row; a.novel.lo[w] = (uint32_t)last; a.novel.cnt[w] = (uint32_t)(j - last + 1); a.novel.piece[w] = k2;
-                    ++w; ++k2;
-                }
-                last = j + 1; has_novel = 0; has_known = 0;
-            }
-        }
+        int k2 = 0; uint32_t w = o0;
+        split_trans(n, [&](int k) { return (fl[k] & LRB_F_NOVEL_JUNC) != 0; }, [&](int k) { return (fl[k] & LRB_F_UNRELIABLE) != 0; }, [&](int lo, int hi) {
+            a.novel.row[w] = (uint32_t)row; a.novel.lo[w] = (uint32_t)lo; a.novel.cnt[w] = (uint32_t)(hi - lo + 1); a.novel.piece[w] = k2;
+            ++w; ++k2;
+        });
     }
 }
 void launch_build_lists(ListArgs a, cudaStream_t st)
@@ -654,6 +630,26 @@ LRB_DEVINL bool sig_has(uint64_t sig, uint64_t jk) { const uint64_t m = junc_mas
 // (an undersized list -- more candidates on the device than the host's bound -- folds as EMPTY: its tail was never written, the host
 // sees the true count in the same round trip and repeats the pass with the exact size)
 LRB_DEVINL int64_t cand_count(const MergeArgs &a) { if (!a.n_cand_dev) return a.n_cand; const int64_t n = (int64_t)*a.n_cand_dev; return n > a.n_cand ? 0 : n; }
+// the candidates [ls, le) of locus loc
+LRB_DEVINL void locus_range(const MergeArgs &a, int64_t n_loci, int64_t loc, int64_t &ls, int64_t &le)
+{
+    ls = a.locus_start[loc]; le = (loc + 1 < n_loci) ? a.locus_start[loc + 1] : cand_count(a);
+}
+
+// Hand-off state of a locus, kept at its head in hard[]: the path that folds the locus next.  A kernel writes it only to hand the
+// locus on, so the last value names the path that finished it (merge_fold_census).
+enum LocusPath : uint8_t {
+    LP_FLAT = 0,                // fold_seq_kernel (at most FF_MAX candidates)
+    LP_TIER0 = 1,               // fold_big_kernel tier 0: beyond the flat masks, or given up by the flat kernels
+    LP_MERGE_OVER = 2,          // merge_fold_kernel: tier 1's slots overflowed, or FB_MAXREL candidates or more
+    LP_MERGE_VERIFY = 3,        // merge_fold_kernel: class verification failed
+    LP_TIER1 = 4,               // fold_big_kernel tier 1: tier 0's slots overflowed
+};
+LRB_DEVINL bool for_merge_fold(int h) { return h == LP_MERGE_OVER || h == LP_MERGE_VERIFY; }
+// the other in-band hand-offs of the fold's scratch
+static constexpr uint32_t LSTART_DEEP = 0xffffffffu;    // lstart[c]: the locus is deeper than the flat masks: not for the flat relation kernels
+static constexpr uint16_t DESC_BIG = 0xFFFFu;           // desc[c]: a member of a locus of the big-locus path (the flat kernels are done with desc by then)
+static constexpr uint8_t CLASSES_UNTABULATED = 0xffu;   // locus_cnt byte: too many classes for the relation rows: fold_big_kernel uses its cache
 
 // One pass over the candidates: flatten (CandSoA), running max of (tid,end) across tiles (look-back, max), locus heads
 // (a candidate that starts beyond every earlier end on its chromosome, App. B.3) and their compaction into locus_start
@@ -756,8 +752,36 @@ void launch_merge_prepare(MergeArgs a, cudaStream_t st)
 
 // check_iden (gtf.c:54-92) between candidate t and fold entry E (first start / last end may have been extended)
 struct Entry { int n; uint32_t gbeg; int fs, le; uint64_t hash; int mono; uint64_t j0, sig; };
+// candidate c as an entry of T, with its (possibly extended) first start fs and last end le
+LRB_DEVINL Entry entry_of(const CandSoA &cd, int64_t c, int fs, int le) { return {cd.n[c], cd.gbeg[c], fs, le, cd.hash[c], cd.rev[c] & 2, cd.j0[c], cd.sig[c]}; }
 LRB_DEVINL int x_s(const DExons &ex, const Entry &e, int i) { return i == 0 ? e.fs : ex.es[e.gbeg + i]; }
 LRB_DEVINL int x_e(const DExons &ex, const Entry &e, int i) { return i == e.n - 1 ? e.le : ex.ee[e.gbeg + i]; }
+// the partial match of gtf.c:76-91: does the chain s (fewer exons, at least two; s_j0 its first junction) continue the chain l from the
+// first occurrence of its first junction on, every boundary within ss_dis?  l_mono: the exon ends of l never decrease
+LRB_DEVINL bool chain_continues(const DExons &ex, uint32_t l_gbeg, int l_n, bool l_mono, uint64_t s_j0, uint32_t s_gbeg, int s_n, int ss_dis)
+{
+    const int s_e0 = (int)(uint32_t)(s_j0 >> 32), s_s1 = (int)(uint32_t)s_j0;
+    int i = 0;
+    const bool jump = ss_dis == 0 && l_mono;
+    if (jump) {                                                  // exact matching on non-decreasing ends: jump to the first candidate
+        int lo = 0, hi = l_n - 1;
+        while (lo < hi) { int mid = (lo + hi) >> 1; if (ex.ee[l_gbeg + mid] < s_e0) lo = mid + 1; else hi = mid; }
+        i = lo;
+    }
+    for (; i < l_n - 1; ++i) {
+        const int le_i = ex.ee[l_gbeg + i];
+        if (jump && le_i > s_e0) return false;
+        if (iabs_dev(le_i - s_e0) <= ss_dis && iabs_dev(ex.es[l_gbeg + i + 1] - s_s1) <= ss_dis) {
+            int j = 1;
+            for (i = i + 1; i < l_n - 1 && j < s_n - 1; ++i, ++j) {
+                if (iabs_dev(ex.ee[l_gbeg + i] - ex.ee[s_gbeg + j]) > ss_dis) return false;
+                if (iabs_dev(ex.es[l_gbeg + i + 1] - ex.es[s_gbeg + j + 1]) > ss_dis) return false;
+            }
+            return true;
+        }
+    }
+    return false;
+}
 LRB_DEVINL int chain_iden(const DExons &ex, const Entry &t1, const Entry &t2, int ss_dis, int end_dis)
 {
     const Entry &l = t1.n >= t2.n ? t1 : t2, &s = t1.n >= t2.n ? t2 : t1;
@@ -771,129 +795,123 @@ LRB_DEVINL int chain_iden(const DExons &ex, const Entry &t1, const Entry &t2, in
         if (iabs_dev(l.le - s.le) > end_dis) return -1;
         return 0;
     }
-    int pm = -1;
     if (iabs_dev(l.fs - s.fs) > end_dis) return -1;
     if (ss_dis == 0 && !sig_has(l.sig, s.j0)) return -1;   // the first junction of s is not a junction of l
-    const int s_e0 = (int)(uint32_t)(s.j0 >> 32), s_s1 = (int)(uint32_t)s.j0;   // s has >= 2 exons
-    int i = 0;
-    const bool jump = ss_dis == 0 && l.mono;
-    if (jump) {                                                  // exon ends of this chain never decrease: jump to the first candidate
-        int lo = 0, hi = l.n - 1;
-        while (lo < hi) { int mid = (lo + hi) >> 1; if (ex.ee[l.gbeg + mid] < s_e0) lo = mid + 1; else hi = mid; }
-        i = lo;
-    }
-    for (; i < l.n - 1; ++i) {
-        const int le_i = ex.ee[l.gbeg + i];
-        if (jump && le_i > s_e0) break;
-        if (iabs_dev(le_i - s_e0) <= ss_dis && iabs_dev(ex.es[l.gbeg + i + 1] - s_s1) <= ss_dis) {
-            pm = 2;
-            int j = 1;
-            for (i = i + 1; i < l.n - 1 && j < s.n - 1; ++i, ++j) {
-                if (iabs_dev(ex.ee[l.gbeg + i] - ex.ee[s.gbeg + j]) > ss_dis) return -1;
-                if (iabs_dev(ex.es[l.gbeg + i + 1] - ex.es[s.gbeg + j + 1]) > ss_dis) return -1;
-            }
-            break;
-        }
-    }
+    if (!chain_continues(ex, l.gbeg, l.n, l.mono, s.j0, s.gbeg, s.n, ss_dis)) return -1;
     if (iabs_dev(l.le - s.le) > end_dis) return -1;
-    return pm;
+    return 2;
+}
+
+// ---- one step of merge_trans's back-scan (update_gtf.c:145-160), shared by the replays of merge_fold_kernel and fold_big_kernel
+enum { EV_NONE = 0, EV_STOP = 1, EV_MERGE = 2, EV_DROP = 3 };
+// merge_trans2's single-exon test (update_gtf.c:122-140); its first two tests are check_iden's end tests
+LRB_DEVINL bool ends_match(const MergeArgs &a, int t_fs, int t_le, int e_fs, int e_le)
+{
+    return iabs_dev(t_fs - e_fs) <= a.up.end_dis && iabs_dev(t_le - e_le) <= a.up.end_dis;
+}
+LRB_DEVINL bool single_exon_match(const MergeArgs &a, int t_fs, int t_le, int e_fs, int e_le)
+{
+    return ends_match(a, t_fs, t_le, e_fs, e_le) && ovlp_frac(t_fs, t_le, e_fs, e_le) >= a.up.single_exon_ovlp_frac;
+}
+// The event of entry e for candidate t: visible = e is of t's sub-stream, stop = the stop rule (:148), same_strand (:149, under -c).
+// multi(): the relation of two multi-exon chains whose ends passed the end tests (0 identical, 2 partial, -1 none).
+template <class Multi>
+LRB_DEVINL int fold_event(const MergeArgs &a, bool visible, bool stop, bool same_strand, int t_n, int t_fs, int t_le, int e_n, int e_fs, int e_le, Multi multi)
+{
+    if (!visible) return EV_NONE;
+    if (stop) return EV_STOP;
+    if (a.up.force_strand && !same_strand) return EV_NONE;
+    if (t_n == 1 && e_n == 1) return single_exon_match(a, t_fs, t_le, e_fs, e_le) ? EV_MERGE : EV_NONE;          // merge_trans2
+    if (t_n > 1 && e_n > 1 && ends_match(a, t_fs, t_le, e_fs, e_le)) {                                           // merge_trans1 :98-119
+        const int r = multi();
+        return r == 0 ? EV_MERGE : r == 2 ? EV_DROP : EV_NONE;
+    }
+    return EV_NONE;
+}
+// A lane group tests G entries at once (lane l: the entry base - l).  The lowest lane with an event holds the entry nearest to the end
+// of T and decides: -1 no event in this window, 0 the scan stops (t is appended), 1 t is absorbed (that lane has run absorb()) or dropped.
+template <int G, class Absorb>
+LRB_DEVINL int fold_winner(unsigned gm, int gl, int ev, Absorb absorb)
+{
+    const int sh = (lane_id() / G) * G;
+    const unsigned m = (__ballot_sync(gm, ev != EV_NONE) >> sh) & lane_bits<G>();
+    if (!m) return -1;
+    const int win = __ffs(m) - 1;
+    const int wev = __shfl_sync(gm, ev, sh + win);
+    if (wev == EV_MERGE && gl == win) absorb();
+    return wev == EV_STOP ? 0 : 1;
+}
+// merge_trans1 / merge_trans2 (update_gtf.c:104-111, 130-137): the entry counts t and takes t's first start / last end where they extend it
+LRB_DEVINL void absorb_into(int &cov, int &fs, int &start, int &le, int &end, int t_fs, int t_le)
+{
+    cov += 1;
+    if (t_fs < fs) { fs = t_fs; start = t_fs; }
+    if (t_le > le) { le = t_le; end = t_le; }
+}
+// a candidate nothing of its locus absorbs is not appended when an entry of an earlier locus absorbs it (xl_* below); the writer lane
+// records (forced = 3) that it happened in this fold
+LRB_DEVINL bool absorbed_elsewhere(const MergeArgs &a, int64_t c, bool writer)
+{
+    if (!a.forced || !a.forced[c]) return false;
+    if (writer) a.forced[c] = 3;
+    return true;
+}
+// the internal boundaries of two chains of n exons are equal (on the pools: what a class key or chain hash only suggests)
+LRB_DEVINL bool same_chain(const DExons &ex, uint32_t g1, uint32_t g2, int n)
+{
+    bool same = true;
+    for (int i = 0; i < n - 1; ++i) same = same && ex.ee[g1 + i] == ex.ee[g2 + i] && ex.es[g1 + i + 1] == ex.es[g2 + i + 1];
+    return same;
 }
 
 static constexpr int MF_THREADS = 128;
-// G lanes per locus; tlist[ls + k] = candidate index of the k-th entry of the locus' T; mutable entry data lives at work[cand]
+// G lanes per locus; tlist[ls + k] = candidate index of the k-th entry of the locus' T; mutable entry data lives at work[cand].
+// Loci of [min_m, max_m] candidates, and those whose hand-off state is in hard_mask.  The whole-warp instance is held to 40 registers
+// (12 blocks per SM): left free, the compiler takes more registers to avoid a few spills.
 template <int G>
-__global__ void __launch_bounds__(MF_THREADS) merge_fold_kernel(MergeArgs a, uint32_t *tlist, uint8_t *alive, const uint8_t *locus_hard, int min_m, int max_m, int hard_mask)
+__global__ void __launch_bounds__(MF_THREADS, G == 32 ? 12 : 0) merge_fold_kernel(MergeArgs a, int min_m, int max_m, int hard_mask)
 {
     const int64_t n_loci = (int64_t)a.totals[0];
     constexpr int GPB = MF_THREADS / G;
     const int gl = threadIdx.x % G;
     const unsigned gm = group_mask<G>();
-    const int sh = (lane_id() / G) * G;
     const CandSoA &cd = a.cd;
     for (int64_t loc = (int64_t)blockIdx.x * GPB + threadIdx.x / G; loc < n_loci; loc += (int64_t)gridDim.x * GPB) {
-        const int64_t ls = a.locus_start[loc], le = (loc + 1 < n_loci) ? a.locus_start[loc + 1] : cand_count(a);
-        if ((le - ls < min_m || le - ls > max_m) && !(locus_hard && ((hard_mask >> locus_hard[ls]) & 1))) continue;   // other loci: flat kernels / another group width
+        int64_t ls, le; locus_range(a, n_loci, loc, ls, le);
+        if ((le - ls < min_m || le - ls > max_m) && !(hard_mask && ((hard_mask >> a.hard[ls]) & 1))) continue;   // other loci: flat kernels / another group width
         int cnt = 0;
         for (int64_t c = ls; c < le; ++c) {
-            const int t_tid = cd.tid[c], t_start = cd.start[c], t_rv = cd.rev[c], t_rev = t_rv & 1;
-            const Entry te = {cd.n[c], cd.gbeg[c], cd.fs[c], cd.le[c], cd.hash[c], t_rv & 2, cd.j0[c], cd.sig[c]};
+            const int t_tid = cd.tid[c], t_start = cd.start[c], t_rev = cd.rev[c] & 1;
+            const Entry te = entry_of(cd, c, cd.fs[c], cd.le[c]);
             int result = 0;                                      // 0 append, 1 absorbed / dropped
             for (int base = cnt - 1; base >= 0; base -= G) {
                 const int k = base - gl;
-                int ev = 0;                                      // 1 stop, 2 merge (identical), 3 drop (partial)
+                int ev = EV_NONE;
                 uint32_t ec = 0;
                 if (k >= 0) {
-                    ec = tlist[ls + k];
-                    if (a.kls && a.kls[ec] != a.kls[c]) ev = 0;                                       // another sub-stream: invisible
-                    else if (t_tid > cd.tid[ec] || t_start > a.work.end[ec]) ev = 1;                  // update_gtf.c:148
-                    else if (!(a.up.force_strand && t_rev != (cd.rev[ec] & 1))) {                     // :149
-                        const Entry E = {cd.n[ec], cd.gbeg[ec], a.work.fs[ec], a.work.le[ec], cd.hash[ec], cd.rev[ec] & 2, cd.j0[ec], cd.sig[ec]};
-                        if (te.n == 1 && E.n == 1) {                                                  // merge_trans2 :122-140
-                            if (iabs_dev(te.fs - E.fs) <= a.up.end_dis && iabs_dev(te.le - E.le) <= a.up.end_dis &&
-                                ovlp_frac(te.fs, te.le, E.fs, E.le) >= a.up.single_exon_ovlp_frac) ev = 2;
-                        } else if (te.n > 1 && E.n > 1) {                                             // merge_trans1 :98-119
-                            int r = chain_iden(a.ex, te, E, a.up.ss_dis, a.up.end_dis);
-                            if (r == 0) ev = 2; else if (r == 2) ev = 3;
-                        }
-                    }
+                    ec = a.tlist[ls + k];
+                    const int e_fs = a.work.fs[ec], e_le = a.work.le[ec];
+                    ev = fold_event(a, !a.kls || a.kls[ec] == a.kls[c], t_tid > cd.tid[ec] || t_start > a.work.end[ec], t_rev == (cd.rev[ec] & 1),
+                                    te.n, te.fs, te.le, cd.n[ec], e_fs, e_le, [&] { return chain_iden(a.ex, te, entry_of(cd, ec, e_fs, e_le), a.up.ss_dis, a.up.end_dis); });
                 }
-                const unsigned m = (__ballot_sync(gm, ev != 0) >> sh) & (G == 32 ? 0xffffffffu : ((1u << G) - 1u));
-                if (m) {
-                    const int win = __ffs(m) - 1;                // lowest lane = entry nearest to the end of T
-                    const int wev = __shfl_sync(gm, ev, sh + win);
-                    if (wev == 2 && gl == win) {
-                        a.work.cov[ec] += 1;
-                        if (te.fs < a.work.fs[ec]) { a.work.fs[ec] = te.fs; a.work.start[ec] = te.fs; }
-                        if (te.le > a.work.le[ec]) { a.work.le[ec] = te.le; a.work.end[ec] = te.le; }
-                    }
-                    result = wev == 1 ? 0 : 1;
-                    break;
-                }
+                const int w = fold_winner<G>(gm, gl, ev, [&] { absorb_into(a.work.cov[ec], a.work.fs[ec], a.work.start[ec], a.work.le[ec], a.work.end[ec], te.fs, te.le); });
+                if (w >= 0) { result = w; break; }
             }
             __syncwarp(gm);
-            if (result == 0 && a.forced && a.forced[c]) {             // absorbed by an entry of an earlier locus (xl_* below): not appended
-                if (gl == 0) a.forced[c] = 3;
-                result = 1;
-            }
+            if (result == 0 && absorbed_elsewhere(a, c, gl == 0)) result = 1;
             if (result == 0) {
                 if (gl == 0) {
-                    tlist[ls + cnt] = (uint32_t)c; alive[c] = 1;
+                    a.tlist[ls + cnt] = (uint32_t)c; a.alive[c] = 1;
                     a.work.cov[c] = 1; a.work.start[c] = t_start; a.work.end[c] = cd.end[c]; a.work.fs[c] = te.fs; a.work.le[c] = te.le;
                 }
                 ++cnt;
-            } else if (gl == 0) alive[c] = 0;
+            } else if (gl == 0) a.alive[c] = 0;
             __syncwarp(gm);
         }
     }
 }
 
 static constexpr int FF_MAX = 64;                   // loci up to this many candidates; larger ones -> fold_big_kernel
-static constexpr uint32_t FF_BIG = 0xffffffffu;
-
-// does the chain s (fewer exons) continue the chain l from the first occurrence of its first junction on?  (gtf.c:79-88, dis 0)
-LRB_DEVINL bool partial_static(const DExons &ex, uint32_t l_gbeg, int l_n, bool l_mono, uint64_t s_j0, uint32_t s_gbeg, int s_n)
-{
-    const int s_e0 = (int)(uint32_t)(s_j0 >> 32), s_s1 = (int)(uint32_t)s_j0;
-    int i = 0;
-    if (l_mono) {
-        int lo = 0, hi = l_n - 1;
-        while (lo < hi) { int mid = (lo + hi) >> 1; if (ex.ee[l_gbeg + mid] < s_e0) lo = mid + 1; else hi = mid; }
-        i = lo;
-    }
-    for (; i < l_n - 1; ++i) {
-        const int le_i = ex.ee[l_gbeg + i];
-        if (l_mono && le_i > s_e0) return false;
-        if (le_i == s_e0 && ex.es[l_gbeg + i + 1] == s_s1) {
-            int j = 1;
-            for (i = i + 1; i < l_n - 1 && j < s_n - 1; ++i, ++j) {
-                if (ex.ee[l_gbeg + i] != ex.ee[s_gbeg + j]) return false;
-                if (ex.es[l_gbeg + i + 1] != ex.es[s_gbeg + j + 1]) return false;
-            }
-            return true;
-        }
-    }
-    return false;
-}
 
 // ------------------------------------------------------------------------------- big loci (ss_dis == 0): classes + warp replay
 // Deep data (hundreds of reads per gene) puts most candidates into loci beyond the 64-candidate masks of the flat fold.  Replaying
@@ -907,9 +925,8 @@ LRB_DEVINL bool partial_static(const DExons &ex, uint32_t l_gbeg, int l_n, bool 
 //                            compare of class ids, the partial-match relation between two classes (junction-signature pre-filter, then
 //                            the pools) is decided once and kept in a direct-mapped per-warp cache, the stop rule reads the slots.
 //                            32 survivors per step, 32 candidates loaded per batch, one per lane.
-// A locus whose survivors outgrow the slots (hard = 2) is redone by merge_fold_kernel -- exact either way.
+// A locus whose survivors outgrow the slots of both tiers (LP_MERGE_OVER) is redone by merge_fold_kernel -- exact either way.
 static constexpr int FB_THREADS = 128, FB_MAXREL = 32768;
-static constexpr uint16_t FB_MEMBER = 0xFFFFu;      // desc[] of a member of a big locus (the flat kernels are done with desc by then)
 // G lanes per locus: lane l reads slot base - l (conflict free inside the group); two tiers -- 8 lanes / 64 slots for the common
 // locus (a few dozen survivors: four loci per warp), a whole warp / 416 slots for what outgrows that
 template <int SLOTS, int CACHE>
@@ -922,20 +939,20 @@ struct FbSlots {
 };
 struct ClassTab { unsigned long long *key; uint32_t *minidx; uint64_t cap; };
 
-__global__ void __launch_bounds__(256) fold_big_mark_kernel(MergeArgs a, const uint8_t *__restrict__ locus_hard, uint32_t *__restrict__ lstart)
+__global__ void __launch_bounds__(256) fold_big_mark_kernel(MergeArgs a)
 {
     const int64_t n_loci = (int64_t)a.totals[0];
     const int lane = lane_id();
     for (int64_t loc = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / 32; loc < n_loci; loc += (int64_t)gridDim.x * blockDim.x / 32) {
-        const int64_t ls = a.locus_start[loc], le = (loc + 1 < n_loci) ? a.locus_start[loc + 1] : cand_count(a);
-        if (le - ls <= FF_MAX && !locus_hard[ls]) continue;
+        int64_t ls, le; locus_range(a, n_loci, loc, ls, le);
+        if (le - ls <= FF_MAX && a.hard[ls] == LP_FLAT) continue;
         // the later passes walk this list, not all loci; an entry is (locus, sub-stream): the four class folds of the summary run over the
         // same rows but never see each other's entries, so each gets its own replay (and its own, four times shorter, survivor list)
         if (lane < (a.kls ? 4 : 1)) {
             const uint32_t i = atomicAdd(&a.fb_cnt[0], 1u);
-            if (i < (uint32_t)a.n_cand) a.fb_list[i] = ((uint32_t)loc << 2) | (uint32_t)lane; else a.hard[ls] = 2;    // (cannot happen for loci beyond the masks)
+            if (i < (uint32_t)a.n_cand) a.fb_list[i] = ((uint32_t)loc << 2) | (uint32_t)lane; else a.hard[ls] = LP_MERGE_OVER;    // (cannot happen for loci beyond the masks)
         }
-        for (int64_t c = ls + lane; c < le; c += 32) { a.desc[c] = FB_MEMBER; lstart[c] = (uint32_t)ls; }
+        for (int64_t c = ls + lane; c < le; c += 32) { a.desc[c] = DESC_BIG; a.lstart[c] = (uint32_t)ls; }
     }
 }
 LRB_DEVINL uint64_t class_key(const MergeArgs &a, int64_t c, uint32_t ls)
@@ -946,11 +963,11 @@ LRB_DEVINL uint64_t class_key(const MergeArgs &a, int64_t c, uint32_t ls)
     return k == ~0ull ? 0x1234567ull : k;
 }
 LRB_DEVINL uint64_t class_slot(const ClassTab &t, uint64_t k) { return __umul64hi(k * 0x9E3779B97F4A7C15ull, t.cap); }
-__global__ void __launch_bounds__(256) fold_class_insert_kernel(MergeArgs a, ClassTab t, const uint32_t *__restrict__ lstart)
+__global__ void __launch_bounds__(256) fold_class_insert_kernel(MergeArgs a, ClassTab t)
 {
     const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= cand_count(a) || a.desc[c] != FB_MEMBER || a.cd.n[c] < 2) return;
-    const uint64_t k = class_key(a, c, lstart[c]);
+    if (c >= cand_count(a) || a.desc[c] != DESC_BIG || a.cd.n[c] < 2) return;
+    const uint64_t k = class_key(a, c, a.lstart[c]);
     uint64_t s = class_slot(t, k);
     for (;;) {
         const unsigned long long p = atomicCAS(&t.key[s], ~0ull, (unsigned long long)k);
@@ -958,37 +975,36 @@ __global__ void __launch_bounds__(256) fold_class_insert_kernel(MergeArgs a, Cla
         s = s + 1 == t.cap ? 0 : s + 1;
     }
 }
-__global__ void __launch_bounds__(256) fold_class_verify_kernel(MergeArgs a, ClassTab t, uint32_t *__restrict__ rep, const uint32_t *__restrict__ lstart, uint8_t *locus_hard)
+__global__ void __launch_bounds__(256) fold_class_verify_kernel(MergeArgs a, ClassTab t)
 {
     const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= cand_count(a) || a.desc[c] != FB_MEMBER) return;
+    if (c >= cand_count(a) || a.desc[c] != DESC_BIG) return;
     const CandSoA &cd = a.cd;
     const int nc = cd.n[c];
-    if (nc < 2) { rep[c] = (uint32_t)c; return; }
-    const uint32_t ls = lstart[c];
+    if (nc < 2) { a.rep[c] = (uint32_t)c; return; }
+    const uint32_t ls = a.lstart[c];
     const uint64_t k = class_key(a, c, ls);
     uint64_t s = class_slot(t, k);
     while (t.key[s] != k) s = s + 1 == t.cap ? 0 : s + 1;
     const uint32_t r = t.minidx[s];
-    rep[c] = r;
+    a.rep[c] = r;
     if (r == (uint32_t)c) return;
     bool same = r >= ls && cd.n[r] == nc;           // same key in another locus (only an unsorted concatenation can do that) or a collision
     if (same) {
-        const uint32_t gc = cd.gbeg[c], gr = cd.gbeg[r];
-        for (int i = 0; i < nc - 1; ++i) same = same && a.ex.ee[gc + i] == a.ex.ee[gr + i] && a.ex.es[gc + i + 1] == a.ex.es[gr + i + 1];
+        same = same_chain(a.ex, cd.gbeg[c], cd.gbeg[r], nc);
         if (a.up.force_strand) same = same && ((cd.rev[c] ^ cd.rev[r]) & 1) == 0;
         if (a.kls) same = same && a.kls[c] == a.kls[r];
     }
-    if (!same) locus_hard[ls] = 3;                  // merge_fold_kernel replays this locus on the pools
+    if (!same) a.hard[ls] = LP_MERGE_VERIFY;        // merge_fold_kernel replays this locus on the pools
 }
 
 // Warp per big locus: the multi-exon classes of the locus get dense ordinals in order of first occurrence (single-exon candidates share
 // the pseudo class FB_SINGLE: their relation is dynamic, decided on the slots), and the STATIC relation between every two classes of
 // the locus (identity on the diagonal, partial match elsewhere: gtf.c:76-91 on the chains of the two representatives) becomes a
 // 128-bit row per class.  The replay then needs no exon pool at all: "can this survivor absorb the candidate" is one bit test.
-// Loci with more than FB_MAXCLS classes keep locus_cnt = FB_NOROWS and the replay falls back to its relation cache.
-static constexpr int FB_MAXCLS = 127; static constexpr uint32_t FB_SINGLE = 127u, FB_NOROWS = 0xffu;
-__global__ void __launch_bounds__(256) fold_class_rows_kernel(MergeArgs a, const uint32_t *__restrict__ rep, const uint8_t *__restrict__ locus_hard, uint32_t *next_entry)
+// Loci with more than FB_MAXCLS classes keep locus_cnt = CLASSES_UNTABULATED and the replay falls back to its relation cache.
+static constexpr int FB_MAXCLS = 127; static constexpr uint32_t FB_SINGLE = 127u;
+__global__ void __launch_bounds__(256) fold_class_rows_kernel(MergeArgs a, uint32_t *next_entry)
 {
     // per warp: the classes of the locus (exon count, sub-stream, junction signature, first junction, representative)
     __shared__ uint64_t s_sig[8][128], s_j0[8][128]; __shared__ uint32_t s_rep[8][128]; __shared__ uint32_t s_nk[8][128];
@@ -1001,12 +1017,12 @@ __global__ void __launch_bounds__(256) fold_class_rows_kernel(MergeArgs a, const
         bi = __shfl_sync(FULL, bi, 0);
         if ((int64_t)bi >= n_big) return;
         const int64_t loc = a.fb_list[bi] >> 2; const uint32_t my = a.fb_list[bi] & 3u;
-        const int64_t ls = a.locus_start[loc], le = (loc + 1 < n_loci) ? a.locus_start[loc + 1] : cand_count(a);
-        if (locus_hard[ls] >= 2) continue;
+        int64_t ls, le; locus_range(a, n_loci, loc, ls, le);
+        if (for_merge_fold(a.hard[ls])) continue;
         int K = 0;
         for (int64_t c0 = ls; c0 < le; c0 += 32) {
             const int64_t c = c0 + lane;
-            const bool headc = c < le && cd.n[c] > 1 && rep[c] == (uint32_t)c && (!a.kls || a.kls[c] == my);
+            const bool headc = c < le && cd.n[c] > 1 && a.rep[c] == (uint32_t)c && (!a.kls || a.kls[c] == my);
             const unsigned b = __ballot_sync(FULL, headc);
             if (headc) {
                 const int o = K + __popc(b & ((1u << lane) - 1u));
@@ -1017,13 +1033,13 @@ __global__ void __launch_bounds__(256) fold_class_rows_kernel(MergeArgs a, const
             }
             K += __popc(b);
         }
-        if (lane == 0) ((uint8_t *)&a.locus_cnt[loc])[my] = K <= FB_MAXCLS ? (uint8_t)K : (uint8_t)FB_NOROWS;
+        if (lane == 0) ((uint8_t *)&a.locus_cnt[loc])[my] = K <= FB_MAXCLS ? (uint8_t)K : CLASSES_UNTABULATED;
         if (K > FB_MAXCLS) continue;
         __syncwarp();
         for (int64_t c = ls + lane; c < le; c += 32) {
             if (a.kls && a.kls[c] != my) continue;
             if (cd.n[c] < 2) a.cord[c] = (uint8_t)FB_SINGLE;
-            else if (rep[c] != (uint32_t)c) a.cord[c] = a.cord[rep[c]];
+            else if (a.rep[c] != (uint32_t)c) a.cord[c] = a.cord[a.rep[c]];
         }
         for (int p = lane; p < K * K; p += 32) {
             const int i = p / K, j = p - i * K;
@@ -1034,7 +1050,7 @@ __global__ void __launch_bounds__(256) fold_class_rows_kernel(MergeArgs a, const
             const uint64_t sj0 = s_j0[w][Sh];
             if (!sig_has(s_sig[w][L], sj0)) continue;
             const uint32_t cl = s_rep[w][L], cs = s_rep[w][Sh];
-            if (!partial_static(a.ex, cd.gbeg[cl], cd.n[cl], (cd.rev[cl] & 2) != 0, sj0, cd.gbeg[cs], cd.n[cs])) continue;
+            if (!chain_continues(a.ex, cd.gbeg[cl], cd.n[cl], (cd.rev[cl] & 2) != 0, sj0, cd.gbeg[cs], cd.n[cs], 0)) continue;
             atomicOr((unsigned long long *)&a.crow[2 * (size_t)s_rep[w][i] + (j >> 6)], 1ull << (j & 63));
             atomicOr((unsigned long long *)&a.crow[2 * (size_t)s_rep[w][j] + (i >> 6)], 1ull << (i & 63));
         }
@@ -1042,19 +1058,16 @@ __global__ void __launch_bounds__(256) fold_class_rows_kernel(MergeArgs a, const
     }
 }
 
-// tier 0: loci beyond the masks or left over by the flat kernels (hard == 1); overflow -> hard = 4.  tier 1: hard == 4; overflow -> hard = 2.
+// tier 0: loci beyond the masks or left over by the flat kernels (LP_TIER0); overflow -> LP_TIER1.  tier 1: overflow -> LP_MERGE_OVER.
 template <int G, int SLOTS, int CACHE, int TIER>
-__global__ void __launch_bounds__(FB_THREADS) fold_big_kernel(MergeArgs a, const uint32_t *__restrict__ rep, uint8_t *alive, uint8_t *locus_hard, uint32_t *next_locus)
+__global__ void __launch_bounds__(FB_THREADS) fold_big_kernel(MergeArgs a, uint32_t *next_locus)
 {
     extern __shared__ __align__(16) unsigned char fb_smem[];
     FbSlots<SLOTS, CACHE> &S = reinterpret_cast<FbSlots<SLOTS, CACHE> *>(fb_smem)[threadIdx.x / G];
     const int64_t n_loci = (int64_t)a.totals[0];
     const int lane = threadIdx.x % G;
     const unsigned gm = group_mask<G>();
-    const int sh = (lane_id() / G) * G;
     const CandSoA &cd = a.cd;
-    const bool force = a.up.force_strand != 0;
-    const int end_dis = a.up.end_dis;
     for (;;) {
         // loci are claimed one at a time (their sizes differ by orders of magnitude)
         // tier 0 walks the list of big loci (fold_big_mark_kernel), tier 1 the list of those whose survivors outgrew tier 0's slots
@@ -1065,11 +1078,11 @@ __global__ void __launch_bounds__(FB_THREADS) fold_big_kernel(MergeArgs a, const
         li = __shfl_sync(gm, li, 0, G);
         if (li >= n_list) return;
         const int64_t loc = (int64_t)(list[li] >> 2); const int my = (int)(list[li] & 3u);      // (locus, sub-stream)
-        const int64_t ls = a.locus_start[loc], le = (loc + 1 < n_loci) ? a.locus_start[loc + 1] : cand_count(a);
-        const int hd = locus_hard[ls];
-        if (TIER == 0 ? (hd == 2 || hd == 3) : hd != 4) continue;    // merge_fold_kernel's (class verification failed, list overflow)
-        if (le - ls >= FB_MAXREL) { if (lane == 0) locus_hard[ls] = 2; continue; }
-        const bool use_rows = ((const uint8_t *)&a.locus_cnt[loc])[my] != FB_NOROWS;      // the static relation of the sub-stream's classes is tabulated
+        int64_t ls, le; locus_range(a, n_loci, loc, ls, le);
+        const int hd = a.hard[ls];
+        if (TIER == 0 ? for_merge_fold(hd) : hd != LP_TIER1) continue;
+        if (le - ls >= FB_MAXREL) { if (lane == 0) a.hard[ls] = LP_MERGE_OVER; continue; }
+        const bool use_rows = ((const uint8_t *)&a.locus_cnt[loc])[my] != CLASSES_UNTABULATED;      // the static relation of the sub-stream's classes is tabulated
         if (!use_rows) for (int i = lane; i < CACHE; i += G) S.cache[i] = 0;
         __syncwarp(gm);
         int cnt = 0; bool overflow = false;
@@ -1082,7 +1095,7 @@ __global__ void __launch_bounds__(FB_THREADS) fold_big_kernel(MergeArgs a, const
             const int l_tid = mine ? cd.tid[cl] : 0, l_start = mine ? cd.start[cl] : 0, l_end = mine ? cd.end[cl] : 0, l_rv = mine ? cd.rev[cl] : 0;
             const int l_n = mine ? cd.n[cl] : 0, l_fs = mine ? cd.fs[cl] : 0, l_le = mine ? cd.le[cl] : 0; const uint32_t l_gbeg = mine ? cd.gbeg[cl] : 0;
             const uint64_t l_j0 = mine ? cd.j0[cl] : 0, l_sig = mine ? cd.sig[cl] : 0;
-            const uint32_t l_rep = mine ? rep[cl] : 0;
+            const uint32_t l_rep = mine ? a.rep[cl] : 0;
             const uint32_t l_ord = (mine && use_rows) ? a.cord[cl] : FB_SINGLE;
             const uint64_t l_row0 = l_ord != FB_SINGLE ? a.crow[2 * (size_t)l_rep] : 0, l_row1 = l_ord != FB_SINGLE ? a.crow[2 * (size_t)l_rep + 1] : 0;
             int l_alive = 0;
@@ -1095,67 +1108,46 @@ __global__ void __launch_bounds__(FB_THREADS) fold_big_kernel(MergeArgs a, const
                 const uint64_t t_j0 = __shfl_sync(gm, l_j0, q, G), t_sig = __shfl_sync(gm, l_sig, q, G);
                 const uint64_t t_row0 = __shfl_sync(gm, l_row0, q, G), t_row1 = __shfl_sync(gm, l_row1, q, G);
                 const uint32_t t_ord = __shfl_sync(gm, l_ord, q, G);
-                const int t_rev = t_rv & 1;
                 const uint32_t t_rel = t_rep - (uint32_t)ls;
                 int result = 0;                                      // 0 append, 1 absorbed / dropped
                 for (int base = cnt - 1; base >= 0; base -= G) {
                     const int k = base - lane;
-                    int ev = 0;                                      // 1 stop, 2 merge (identical), 3 drop (partial)
+                    int ev = EV_NONE;
                     if (k >= 0) {
                         const uint32_t mt = S.meta[k];
                         const int e_n = (int)(mt >> 8);
-                        if (a.kls && (int)((mt >> 2) & 3u) != t_kls) ev = 0;                          // another sub-stream: invisible
-                        else if (t_tid > S.tid[k] || t_start > S.end[k]) ev = 1;                      // update_gtf.c:148
-                        else if (!(force && t_rev != (int)(mt & 1u))) {                               // :149
-                            const int e_fs = S.fs[k], e_le = S.le[k];
-                            if (t_n == 1 && e_n == 1) {                                               // merge_trans2 :122-140
-                                if (iabs_dev(t_fs - e_fs) <= end_dis && iabs_dev(t_le - e_le) <= end_dis &&
-                                    ovlp_frac(t_fs, t_le, e_fs, e_le) >= a.up.single_exon_ovlp_frac) ev = 2;
-                            } else if (t_n > 1 && e_n > 1 && iabs_dev(t_fs - e_fs) <= end_dis && iabs_dev(t_le - e_le) <= end_dis) {   // merge_trans1 :98-119, check_iden
-                                if (use_rows) {
-                                    const uint32_t e_ord = S.cand[k] >> 16;
-                                    if ((((e_ord & 64u) ? t_row1 : t_row0) >> (e_ord & 63u)) & 1ull) ev = e_ord == t_ord ? 2 : 3;
-                                } else if (t_n == e_n) { if (S.rep[k] == t_rep) ev = 2; }
-                                else {
-                                    // the shorter chain's first junction must be a junction of the longer (signature), then the static relation
-                                    const bool t_long = t_n > e_n;
-                                    const uint64_t lsig = t_long ? t_sig : S.sig[k], sj0 = t_long ? S.j0[k] : t_j0;
-                                    if (sig_has(lsig, sj0)) {
-                                        const uint32_t e_rel = S.rep[k] - (uint32_t)ls;
-                                        const uint32_t pair = (t_rel << 15) | e_rel;
-                                        const uint32_t ci = ((t_rel * 0x9E37u) ^ (e_rel * 0x85EBu) ^ (e_rel >> 5)) & (CACHE - 1);
-                                        const uint32_t ce = S.cache[ci];
-                                        bool rel;
-                                        if ((ce >> 31) && (ce & 0x3FFFFFFFu) == pair) rel = (ce >> 30) & 1u;
-                                        else {
-                                            rel = t_long ? partial_static(a.ex, t_gbeg, t_n, (t_rv & 2) != 0, sj0, S.gbeg[k], e_n)
-                                                         : partial_static(a.ex, S.gbeg[k], e_n, (mt & 2u) != 0, sj0, t_gbeg, t_n);
-                                            S.cache[ci] = 0x80000000u | (rel ? 0x40000000u : 0u) | pair;
-                                        }
-                                        if (rel) ev = 3;
-                                    }
-                                }
+                        // the static relation of two multi-exon classes: the class rows, else the identity of the representatives or the
+                        // partial match (the shorter chain's first junction must be a junction of the longer, then the cached relation)
+                        ev = fold_event(a, !a.kls || (int)((mt >> 2) & 3u) == t_kls, t_tid > S.tid[k] || t_start > S.end[k], (t_rv & 1) == (int)(mt & 1u),
+                                        t_n, t_fs, t_le, e_n, S.fs[k], S.le[k], [&] {
+                            if (use_rows) {
+                                const uint32_t e_ord = S.cand[k] >> 16;
+                                if (!((((e_ord & 64u) ? t_row1 : t_row0) >> (e_ord & 63u)) & 1ull)) return -1;
+                                return e_ord == t_ord ? 0 : 2;
                             }
-                        }
+                            if (t_n == e_n) return S.rep[k] == t_rep ? 0 : -1;
+                            const bool t_long = t_n > e_n;
+                            const uint64_t lsig = t_long ? t_sig : S.sig[k], sj0 = t_long ? S.j0[k] : t_j0;
+                            if (!sig_has(lsig, sj0)) return -1;
+                            const uint32_t e_rel = S.rep[k] - (uint32_t)ls;
+                            const uint32_t pair = (t_rel << 15) | e_rel;
+                            const uint32_t ci = ((t_rel * 0x9E37u) ^ (e_rel * 0x85EBu) ^ (e_rel >> 5)) & (CACHE - 1);
+                            const uint32_t ce = S.cache[ci];
+                            bool rel;
+                            if ((ce >> 31) && (ce & 0x3FFFFFFFu) == pair) rel = (ce >> 30) & 1u;
+                            else {
+                                rel = t_long ? chain_continues(a.ex, t_gbeg, t_n, (t_rv & 2) != 0, sj0, S.gbeg[k], e_n, 0)
+                                             : chain_continues(a.ex, S.gbeg[k], e_n, (mt & 2u) != 0, sj0, t_gbeg, t_n, 0);
+                                S.cache[ci] = 0x80000000u | (rel ? 0x40000000u : 0u) | pair;
+                            }
+                            return rel ? 2 : -1;
+                        });
                     }
-                    const unsigned m = (__ballot_sync(gm, ev != 0) >> sh) & lane_bits<G>();
-                    if (m) {
-                        const int win = __ffs(m) - 1;                // lowest lane = entry nearest to the end of T
-                        const int wev = __shfl_sync(gm, ev, win, G);
-                        if (wev == 2 && lane == win) {
-                            S.cov[k] += 1;
-                            if (t_fs < S.fs[k]) { S.fs[k] = t_fs; S.start[k] = t_fs; }
-                            if (t_le > S.le[k]) { S.le[k] = t_le; S.end[k] = t_le; }
-                        }
-                        result = wev == 1 ? 0 : 1;
-                        break;
-                    }
+                    const int w = fold_winner<G>(gm, lane, ev, [&] { absorb_into(S.cov[k], S.fs[k], S.start[k], S.le[k], S.end[k], t_fs, t_le); });
+                    if (w >= 0) { result = w; break; }
                 }
                 __syncwarp(gm);
-                if (result == 0 && a.forced && a.forced[c0 + q]) {   // absorbed by an entry of an earlier locus (xl_* below): not appended
-                    if (lane == 0) a.forced[c0 + q] = 3;
-                    result = 1;
-                }
+                if (result == 0 && absorbed_elsewhere(a, c0 + q, lane == 0)) result = 1;
                 if (result == 0) {
                     if (cnt == SLOTS) { overflow = true; break; }
                     if (lane == 0) {
@@ -1168,10 +1160,10 @@ __global__ void __launch_bounds__(FB_THREADS) fold_big_kernel(MergeArgs a, const
                 }
                 __syncwarp(gm);
             }
-            if (!overflow && have && (!a.kls || l_kls == my)) alive[cl] = (uint8_t)l_alive;
+            if (!overflow && have && (!a.kls || l_kls == my)) a.alive[cl] = (uint8_t)l_alive;
         }
         if (overflow) {                                              // the next tier / merge_fold_kernel redoes the locus from scratch
-            if (lane == 0) { locus_hard[ls] = TIER == 0 ? 4 : 2; if (TIER == 0) a.fb_list[a.n_cand + atomicAdd(&a.fb_cnt[2], 1u)] = list[li]; }
+            if (lane == 0) { a.hard[ls] = TIER == 0 ? LP_TIER1 : LP_MERGE_OVER; if (TIER == 0) a.fb_list[a.n_cand + atomicAdd(&a.fb_cnt[2], 1u)] = list[li]; }
             continue;
         }
         for (int k = lane; k < cnt; k += G) {
@@ -1187,8 +1179,8 @@ __global__ void __launch_bounds__(FB_THREADS) fold_big_kernel(MergeArgs a, const
 // mutable first start / last end enter through the end_dis tests alone), identity is transitive, and the partial-match
 // relation is a relation between identity classes.  That moves every exon-pool access out of the ordered part:
 //   fold_rep_kernel   thread per candidate: its identity class = first earlier candidate of the locus with the same
-//                     (exon count, chain hash[, strand]), verified once on the pools (a hash collision marks the locus
-//                     "hard": it is left to merge_fold_kernel);
+//                     (exon count, chain hash[, strand]), verified once on the pools (a hash collision hands the locus
+//                     to the big-locus path, LP_TIER0);
 //   fold_rel_kernel   thread per candidate: bit mask (over the <= 64 earlier candidates of its locus) of the entries that
 //                     could absorb it -- same class, a class in partial-match relation (junction-signature pre-filter,
 //                     verified on the pools, decided once per class representative), other single-exon reads;
@@ -1196,7 +1188,7 @@ __global__ void __launch_bounds__(FB_THREADS) fold_big_kernel(MergeArgs a, const
 //                     the alive entries from the newest, stop on the reference's stop rule (dynamic end), take the first
 //                     confirmed event.  A warp folds 32 loci in lock step.
 
-__global__ void __launch_bounds__(256) fold_rep_kernel(MergeArgs a, uint32_t *__restrict__ rep, uint32_t *__restrict__ lstart, uint8_t *locus_hard)
+__global__ void __launch_bounds__(256) fold_rep_kernel(MergeArgs a)
 {
     const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= cand_count(a)) return;
@@ -1208,18 +1200,12 @@ __global__ void __launch_bounds__(256) fold_rep_kernel(MergeArgs a, uint32_t *__
     int64_t e = c, r = c;
     int steps = 0;
     while (!a.head[e]) {
-        if (++steps >= FF_MAX) { lstart[c] = FF_BIG; rep[c] = (uint32_t)c; a.desc[c] = 0; return; }   // deeper than the masks reach
+        if (++steps >= FF_MAX) { a.lstart[c] = LSTART_DEEP; a.rep[c] = (uint32_t)c; a.desc[c] = 0; return; }   // deeper than the masks reach
         --e;
         if (nc > 1 && cd.n[e] == nc && cd.hash[e] == hc && (!force || (cd.rev[e] & 1) == rvc) && (!a.kls || a.kls[e] == kc)) r = e;
     }
-    if (r != c) {
-        const uint32_t gc = cd.gbeg[c], gr = cd.gbeg[r];
-        bool same = true;
-        for (int i = 0; i < nc - 1; ++i)
-            same = same && a.ex.ee[gc + i] == a.ex.ee[gr + i] && a.ex.es[gc + i + 1] == a.ex.es[gr + i + 1];
-        if (!same) locus_hard[e] = 1;
-    }
-    rep[c] = (uint32_t)r; lstart[c] = (uint32_t)e;
+    if (r != c && !same_chain(a.ex, cd.gbeg[c], cd.gbeg[r], nc)) a.hard[e] = LP_TIER0;     // a hash collision: not for the flat kernels
+    a.rep[c] = (uint32_t)r; a.lstart[c] = (uint32_t)e;
     // class descriptor for the relation passes: [0:5] representative (locus-local), [6] single exon, [7] strand, [8:9] sub-stream
     a.desc[c] = (uint16_t)((uint32_t)(r - e) | (nc == 1 ? 64u : 0u) | ((uint32_t)rvc << 7) | ((uint32_t)kc << 8));
     a.relsym[c] = 0;
@@ -1227,12 +1213,12 @@ __global__ void __launch_bounds__(256) fold_rep_kernel(MergeArgs a, uint32_t *__
 
 // partial-match relation between the class representatives of a locus (threads of non-representatives leave at once):
 // relsym[r] gets a bit for every representative r' (earlier or later) whose class can absorb / be absorbed by r's
-__global__ void __launch_bounds__(256) fold_relrep_kernel(MergeArgs a, const uint32_t *__restrict__ lstart)
+__global__ void __launch_bounds__(256) fold_relrep_kernel(MergeArgs a)
 {
     const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= cand_count(a)) return;
-    const uint32_t ls = lstart[c];
-    if (ls == FF_BIG) return;
+    const uint32_t ls = a.lstart[c];
+    if (ls == LSTART_DEEP) return;
     const uint32_t d = a.desc[c];
     if ((d & 64u) || (d & 63u) != (uint32_t)c - ls) return;          // single exon, or not the representative of its class
     const CandSoA &cd = a.cd;
@@ -1250,9 +1236,9 @@ __global__ void __launch_bounds__(256) fold_relrep_kernel(MergeArgs a, const uin
         bool hit;
         if (nc > ne) {
             const uint64_t j0_e = cd.j0[e];
-            hit = sig_has(sig_c, j0_e) && partial_static(a.ex, gb_c, nc, mono_c, j0_e, cd.gbeg[e], ne);
+            hit = sig_has(sig_c, j0_e) && chain_continues(a.ex, gb_c, nc, mono_c, j0_e, cd.gbeg[e], ne, 0);
         } else
-            hit = sig_has(cd.sig[e], j0_c) && partial_static(a.ex, cd.gbeg[e], ne, (cd.rev[e] & 2) != 0, j0_c, gb_c, nc);
+            hit = sig_has(cd.sig[e], j0_c) && chain_continues(a.ex, cd.gbeg[e], ne, (cd.rev[e] & 2) != 0, j0_c, gb_c, nc, 0);
         if (hit) {
             atomicOr((unsigned long long *)&a.relsym[c], 1ull << (e - ls));
             atomicOr((unsigned long long *)&a.relsym[e], 1ull << ((uint32_t)c - ls));
@@ -1263,12 +1249,12 @@ __global__ void __launch_bounds__(256) fold_relrep_kernel(MergeArgs a, const uin
 // per candidate: the mask (over the <= 63 earlier candidates of its locus) of the entries that could absorb it -- members of its
 // own class (identical chains), members of classes in partial-match relation, other single-exon reads -- and, for class
 // folds, the mask of the earlier candidates of its own sub-stream
-__global__ void __launch_bounds__(256) fold_relasm_kernel(MergeArgs a, const uint32_t *__restrict__ lstart, uint64_t *__restrict__ evmask)
+__global__ void __launch_bounds__(256) fold_relasm_kernel(MergeArgs a)
 {
     const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= cand_count(a)) return;
-    const uint32_t ls = lstart[c];
-    if (ls == FF_BIG) return;
+    const uint32_t ls = a.lstart[c];
+    if (ls == LSTART_DEEP) return;
     const uint32_t d = a.desc[c];
     const bool force = a.up.force_strand != 0;
     uint64_t mask = 0, same = 0;
@@ -1288,21 +1274,20 @@ __global__ void __launch_bounds__(256) fold_relasm_kernel(MergeArgs a, const uin
             if (!(de & 64u) && ((rel >> (de & 63u)) & 1ull)) mask |= bit;
         }
     }
-    evmask[c] = mask;
+    a.evmask[c] = mask;
     if (a.kls) a.samemask[c] = same;
 }
 
 // thread per locus.  The entries of T (the survivors so far) live in shared-memory slots in insertion order -- the back-scan
-// of merge_trans is a walk down the slots; a locus with more than FS_SLOTS survivors is handed to merge_fold_kernel.
+// of merge_trans is a walk down the slots; a locus with more than FS_SLOTS survivors is handed to fold_big_kernel.
 // A slot keeps exon[0].start / exon[last].end; T.start / T.end equal them except for a split piece that was not extended
 // yet (0 / 0, SURVEY Q14) -- two flag bits.
 // T.tid of an entry is not stored: the candidates of a locus carry one non-zero tid (checked; a locus mixing chromosomes -- unsorted
-// input -- goes to merge_fold_kernel), so "t.tid > T.tid" (update_gtf.c:148) can only hold for an entry with tid 0 (a split piece,
+// input -- goes to fold_big_kernel), so "t.tid > T.tid" (update_gtf.c:148) can only hold for an entry with tid 0 (a split piece,
 // flag bit 4) under a candidate with tid > 0.
 static constexpr int FS_THREADS = 64;
 template <int FS_SLOTS>
-__global__ void __launch_bounds__(FS_THREADS) fold_seq_kernel(MergeArgs a, const uint32_t *__restrict__ rep, const uint64_t *__restrict__ evmask,
-                                                              uint8_t *locus_hard, uint8_t *alive_out)
+__global__ void __launch_bounds__(FS_THREADS) fold_seq_kernel(MergeArgs a)
 {
     __shared__ int s_fs[FS_SLOTS][FS_THREADS], s_le[FS_SLOTS][FS_THREADS];
     __shared__ uint8_t s_cov[FS_SLOTS][FS_THREADS], s_rep[FS_SLOTS][FS_THREADS], s_cand[FS_SLOTS][FS_THREADS], s_flag[FS_SLOTS][FS_THREADS];
@@ -1310,27 +1295,26 @@ __global__ void __launch_bounds__(FS_THREADS) fold_seq_kernel(MergeArgs a, const
     const int64_t loc = (int64_t)blockIdx.x * FS_THREADS + t;
     const int64_t n_loci = (int64_t)a.totals[0];
     if (loc >= n_loci) return;
-    const int64_t ls = a.locus_start[loc], le = (loc + 1 < n_loci) ? a.locus_start[loc + 1] : cand_count(a);
-    if (le - ls > FF_MAX || locus_hard[ls]) return;
+    int64_t ls, le; locus_range(a, n_loci, loc, ls, le);
+    if (le - ls > FF_MAX || a.hard[ls] != LP_FLAT) return;
     const int m = (int)(le - ls);
     const CandSoA &cd = a.cd;
-    const int end_dis = a.up.end_dis;
-    const bool end_free = end_dis == 0x7fffffff;                      // the default: check_iden's end tests always pass
+    const bool end_free = a.up.end_dis == 0x7fffffff;                // the default: check_iden's end tests always pass
     uint64_t alive = 0;
     int cnt = 0, ltid = 0;
     // candidate k+1 is loaded while candidate k is folded
     int t_tid = cd.tid[ls], t_start = cd.start[ls], t_end = cd.end[ls], nc = cd.n[ls], fs = cd.fs[ls], lend = cd.le[ls];
-    uint32_t rc = rep[ls]; uint64_t ev = evmask[ls], same = a.kls ? a.samemask[ls] : ~0ull;
+    uint32_t rc = a.rep[ls]; uint64_t ev = a.evmask[ls], same = a.kls ? a.samemask[ls] : ~0ull;
     for (int k = 0; k < m; ++k) {
         const int64_t c = ls + k;
         const int c_tid = t_tid, c_start = t_start, c_end = t_end, c_n = nc, c_fs = fs, c_le = lend;
         const uint32_t c_rep = rc - (uint32_t)ls; const uint64_t c_ev = ev, c_same = same;
         if (k + 1 < m) {
             t_tid = cd.tid[c + 1]; t_start = cd.start[c + 1]; t_end = cd.end[c + 1]; nc = cd.n[c + 1]; fs = cd.fs[c + 1]; lend = cd.le[c + 1];
-            rc = rep[c + 1]; ev = evmask[c + 1]; if (a.kls) same = a.samemask[c + 1];
+            rc = a.rep[c + 1]; ev = a.evmask[c + 1]; if (a.kls) same = a.samemask[c + 1];
         }
         if (c_tid != 0) {                                             // unsorted input can put two chromosomes into one locus: not for the slots
-            if (ltid == 0) ltid = c_tid; else if (c_tid != ltid) { locus_hard[ls] = 1; return; }
+            if (ltid == 0) ltid = c_tid; else if (c_tid != ltid) { a.hard[ls] = LP_TIER0; return; }
         }
         int kind = 0, hit = 0;                                        // kind: 0 append, 1 merge (identical), 2 drop (partial)
         for (int sl = cnt - 1; sl >= 0; --sl) {
@@ -1342,11 +1326,7 @@ __global__ void __launch_bounds__(FS_THREADS) fold_seq_kernel(MergeArgs a, const
             const int e_end = (fl & 2) ? 0 : ele;                     // T.end
             if (((fl & 4) && c_tid > 0) || c_start > e_end) break;    // update_gtf.c:148
             if ((c_ev >> b) & 1ull) {
-                bool ok = true;
-                if (!end_free || c_n == 1) {
-                    ok = iabs_dev(c_fs - efs) <= end_dis && iabs_dev(c_le - ele) <= end_dis; // merge_trans2 :124-125 / check_iden's end tests
-                    if (c_n == 1) ok = ok && ovlp_frac(c_fs, c_le, efs, ele) >= a.up.single_exon_ovlp_frac;
-                }
+                const bool ok = c_n == 1 ? single_exon_match(a, c_fs, c_le, efs, ele) : end_free || ends_match(a, c_fs, c_le, efs, ele);
                 if (ok) { hit = sl; kind = (c_n == 1 || s_rep[sl][t] == (uint8_t)c_rep) ? 1 : 2; break; }
             }
         }
@@ -1354,17 +1334,17 @@ __global__ void __launch_bounds__(FS_THREADS) fold_seq_kernel(MergeArgs a, const
             s_cov[hit][t] += 1;                                       // <= 64 candidates per locus: fits a byte
             if (c_fs < s_fs[hit][t]) { s_fs[hit][t] = c_fs; s_flag[hit][t] &= ~1; }
             if (c_le > s_le[hit][t]) { s_le[hit][t] = c_le; s_flag[hit][t] &= ~2; }
-        } else if (kind == 0 && a.forced && a.forced[c]) {
-            a.forced[c] = 3; kind = 3;                                // absorbed by an entry of an earlier locus (see xl_* below): not appended
+        } else if (kind == 0 && absorbed_elsewhere(a, c, true)) {
+            kind = 3;
         } else if (kind == 0) {
-            if (cnt == FS_SLOTS) { locus_hard[ls] = 1; return; }      // too many survivors for the slots: merge_fold_kernel redoes the locus
+            if (cnt == FS_SLOTS) { a.hard[ls] = LP_TIER0; return; }   // too many survivors for the slots: fold_big_kernel redoes the locus
             alive |= 1ull << k;
             s_fs[cnt][t] = c_fs; s_le[cnt][t] = c_le; s_cov[cnt][t] = 1;
             s_rep[cnt][t] = (uint8_t)c_rep; s_cand[cnt][t] = (uint8_t)k;
             s_flag[cnt][t] = (uint8_t)((c_start != c_fs ? 1 : 0) | (c_end != c_le ? 2 : 0) | (c_tid == 0 ? 4 : 0));   // bits 0,1: only an unextended piece (start = end = 0)
             ++cnt;
         }
-        alive_out[c] = kind == 0 ? 1 : 0;
+        a.alive[c] = kind == 0 ? 1 : 0;
     }
     for (int sl = 0; sl < cnt; ++sl) {
         const int64_t c = ls + s_cand[sl][t];
@@ -1375,7 +1355,7 @@ __global__ void __launch_bounds__(FS_THREADS) fold_seq_kernel(MergeArgs a, const
 
 // survivors of the fold, compacted in candidate order with their mutated fields (one pass, look-back sum)
 static constexpr int FF_ITEMS = 8;
-__global__ void __launch_bounds__(FP_THREADS) fold_finish_kernel(MergeArgs a, const uint8_t *__restrict__ alive)
+__global__ void __launch_bounds__(FP_THREADS) fold_finish_kernel(MergeArgs a)
 {
     __shared__ uint32_t s_scan[33];
     __shared__ uint32_t s_tile; __shared__ uint64_t s_excl;
@@ -1385,7 +1365,7 @@ __global__ void __launch_bounds__(FP_THREADS) fold_finish_kernel(MergeArgs a, co
     const int64_t c0 = ((int64_t)tile * FP_THREADS + threadIdx.x) * FF_ITEMS, n = cand_count(a);
     uint32_t al = 0, cnt = 0;
 #pragma unroll
-    for (int i = 0; i < FF_ITEMS; ++i) if (c0 + i < n && alive[c0 + i]) { al |= 1u << i; ++cnt; }
+    for (int i = 0; i < FF_ITEMS; ++i) if (c0 + i < n && a.alive[c0 + i]) { al |= 1u << i; ++cnt; }
     uint32_t tot; const uint32_t ex = block_excl_sum(cnt, s_scan, &tot);
     if (warp_id() == 0) { const uint64_t e = lookback_exclusive(a.tile_state, tile, (uint64_t)tot, OpAdd()); if (lane_id() == 0) s_excl = e; }
     __syncthreads();
@@ -1405,24 +1385,23 @@ void launch_merge_finish(MergeArgs a, cudaStream_t st)
     if (a.n_cand <= 0) return;
     a.n_tiles = (int)((a.n_cand + FP_THREADS * FF_ITEMS - 1) / (FP_THREADS * FF_ITEMS));
     cudaMemsetAsync(a.tile_state, 0, (size_t)a.n_tiles * 8, st); cudaMemsetAsync(a.ticket, 0, 4, st);
-    fold_finish_kernel<<<(unsigned)a.n_tiles, FP_THREADS, 0, st>>>(a, a.dropped); LRB_COUNT_LAUNCH();
+    fold_finish_kernel<<<(unsigned)a.n_tiles, FP_THREADS, 0, st>>>(a); LRB_COUNT_LAUNCH();
 }
 
 void launch_merge_fold(const MergeArgs &a, cudaStream_t st)
 {
     if (a.n_cand <= 0) return;
-    // tlist reuses the (no longer needed) 64-bit key scratch; alive goes to `dropped`.  Grids are sized for the worst
-    // case (every candidate its own locus); the locus count is read on the device.
+    // Grids are sized for the worst case (every candidate its own locus); the locus count is read on the device.
     if (a.up.ss_dis == 0) {
         cudaMemsetAsync(a.hard, 0, (size_t)a.n_cand, st);
         const unsigned bl = (unsigned)((a.n_cand + 255) / 256);
-        fold_rep_kernel<<<bl, 256, 0, st>>>(a, a.rep, a.lstart, a.hard); LRB_COUNT_LAUNCH();
-        fold_relrep_kernel<<<bl, 256, 0, st>>>(a, a.lstart); LRB_COUNT_LAUNCH();
-        fold_relasm_kernel<<<bl, 256, 0, st>>>(a, a.lstart, a.evmask); LRB_COUNT_LAUNCH();
+        fold_rep_kernel<<<bl, 256, 0, st>>>(a); LRB_COUNT_LAUNCH();
+        fold_relrep_kernel<<<bl, 256, 0, st>>>(a); LRB_COUNT_LAUNCH();
+        fold_relasm_kernel<<<bl, 256, 0, st>>>(a); LRB_COUNT_LAUNCH();
         const unsigned bs = (unsigned)((a.n_cand + FS_THREADS - 1) / FS_THREADS);
-        fold_seq_kernel<32><<<bs, FS_THREADS, 0, st>>>(a, a.rep, a.evmask, a.hard, a.dropped); LRB_COUNT_LAUNCH();
+        fold_seq_kernel<32><<<bs, FS_THREADS, 0, st>>>(a); LRB_COUNT_LAUNCH();
         // loci beyond the masks and the ones the flat kernels gave up on: classes through one table, then warp per locus with the survivors
-        // in shared memory; what outgrows the slots there (hard >= 2) is replayed from global memory
+        // in shared memory; what outgrows the slots there (LP_MERGE_OVER) is replayed from global memory
         int64_t bl2 = (a.n_cand / (FF_MAX + 1) + 1 + 3) / 4 + 8; if (bl2 > 148 * 8) bl2 = 148 * 8;
         using S0 = FbSlots<128, 256>; using S1 = FbSlots<416, 1024>;
         auto k0 = fold_big_kernel<32, 128, 256, 0>; auto k1 = fold_big_kernel<32, 416, 1024, 1>;
@@ -1433,17 +1412,17 @@ void launch_merge_fold(const MergeArgs &a, cudaStream_t st)
         cudaMemsetAsync(a.ckey, 0xFF, tab.cap * 8, st); cudaMemsetAsync(a.cmin, 0xFF, tab.cap * 4, st);
         cudaMemsetAsync(a.fb_cnt, 0, 32, st);                     // [0] big loci, [1] tier-0 claims, [2] tier-0 overflows, [3] tier-1 claims
         int64_t blm = (a.n_cand / 8 + 255) / 256 + 1; if (blm > 148 * 8) blm = 148 * 8;
-        fold_big_mark_kernel<<<(unsigned)blm, 256, 0, st>>>(a, a.hard, a.lstart); LRB_COUNT_LAUNCH();
-        fold_class_insert_kernel<<<bl, 256, 0, st>>>(a, tab, a.lstart); LRB_COUNT_LAUNCH();
-        fold_class_verify_kernel<<<bl, 256, 0, st>>>(a, tab, a.rep, a.lstart, a.hard); LRB_COUNT_LAUNCH();
-        fold_class_rows_kernel<<<(unsigned)blm, 256, 0, st>>>(a, a.rep, a.hard, a.fb_cnt + 4); LRB_COUNT_LAUNCH();
+        fold_big_mark_kernel<<<(unsigned)blm, 256, 0, st>>>(a); LRB_COUNT_LAUNCH();
+        fold_class_insert_kernel<<<bl, 256, 0, st>>>(a, tab); LRB_COUNT_LAUNCH();
+        fold_class_verify_kernel<<<bl, 256, 0, st>>>(a, tab); LRB_COUNT_LAUNCH();
+        fold_class_rows_kernel<<<(unsigned)blm, 256, 0, st>>>(a, a.fb_cnt + 4); LRB_COUNT_LAUNCH();
         // one warp per locus, loci claimed from the lists: a whole warp measured fastest (8 / 16 lanes per locus: 17.5 / 15.8 ms per
         // step against 14.2 ms on the 10 M-read data set -- the lane groups of a warp diverge)
         int64_t blb = (a.n_cand / (FF_MAX + 1) + 1) / (FB_THREADS / 32) + 1; if (blb > 148 * 6) blb = 148 * 6;
-        k0<<<(unsigned)blb, FB_THREADS, smem0, st>>>(a, a.rep, a.dropped, a.hard, a.fb_cnt + 1); LRB_COUNT_LAUNCH();
+        k0<<<(unsigned)blb, FB_THREADS, smem0, st>>>(a, a.fb_cnt + 1); LRB_COUNT_LAUNCH();
         if (blb > 148 * 2) blb = 148 * 2;
-        k1<<<(unsigned)blb, FB_THREADS, smem1, st>>>(a, a.rep, a.dropped, a.hard, a.fb_cnt + 3); LRB_COUNT_LAUNCH();
-        merge_fold_kernel<32><<<(unsigned)bl2, MF_THREADS, 0, st>>>(a, (uint32_t *)a.keys, a.dropped, a.hard, 0x7fffffff, 0x7fffffff, (1 << 2) | (1 << 3));
+        k1<<<(unsigned)blb, FB_THREADS, smem1, st>>>(a, a.fb_cnt + 3); LRB_COUNT_LAUNCH();
+        merge_fold_kernel<32><<<(unsigned)bl2, MF_THREADS, 0, st>>>(a, 0x7fffffff, 0x7fffffff, (1 << LP_MERGE_OVER) | (1 << LP_MERGE_VERIFY));
         LRB_COUNT_LAUNCH();
         return;
     }
@@ -1451,21 +1430,20 @@ void launch_merge_fold(const MergeArgs &a, cudaStream_t st)
     {
         constexpr int GPB = MF_THREADS / 8;
         int64_t bl = (a.n_cand + GPB - 1) / GPB; if (bl > 148 * 12) bl = 148 * 12;
-        merge_fold_kernel<8><<<(unsigned)bl, MF_THREADS, 0, st>>>(a, (uint32_t *)a.keys, a.dropped, nullptr, 1, 32, 0);
+        merge_fold_kernel<8><<<(unsigned)bl, MF_THREADS, 0, st>>>(a, 1, 32, 0);
         LRB_COUNT_LAUNCH();
     }
     {
         int64_t bl = (a.n_cand / 33 + 1 + 3) / 4; if (bl > 148 * 8) bl = 148 * 8;
-        merge_fold_kernel<32><<<(unsigned)bl, MF_THREADS, 0, st>>>(a, (uint32_t *)a.keys, a.dropped, nullptr, 33, 0x7fffffff, 0);
+        merge_fold_kernel<32><<<(unsigned)bl, MF_THREADS, 0, st>>>(a, 33, 0x7fffffff, 0);
         LRB_COUNT_LAUNCH();
     }
 }
 
 // Test hook (lrb_fold_census): after launch_merge_fold on the same stream, read the locus table back and tally each locus by the path
-// that folded it.  Every kernel writes hard[] at the locus head, and only to hand the locus on (0 flat -> 1 tier 0 -> 4 tier 1 -> 2
-// merge_fold_kernel; 2 also at >= FB_MAXREL members, 3 after a failed class verify), so the final value names the path that finished
-// the locus.  A big locus's locus_cnt holds one byte per sub-stream, written by fold_class_rows_kernel unless class verification had
-// already sent the locus to merge_fold_kernel (hard 3): that byte is stale then and not read.
+// that folded it: the final LocusPath at its head.  A big locus's locus_cnt holds one byte per sub-stream, written by
+// fold_class_rows_kernel unless class verification had already sent the locus to merge_fold_kernel (LP_MERGE_VERIFY): that byte is
+// stale then and not read.
 cudaError_t merge_fold_census(const MergeArgs &a, cudaStream_t st, int64_t *k)
 {
     uint64_t n_loci = 0, n_dev = (uint64_t)a.n_cand;
@@ -1486,10 +1464,10 @@ cudaError_t merge_fold_census(const MergeArgs &a, cudaStream_t st, int64_t *k)
         if (a.single_locus) ++k[LRB_FC_SINGLE];
         if (!exact) { ++k[m <= 32 ? LRB_FC_D_SMALL : LRB_FC_D_LARGE]; continue; }   // merge_fold_kernel<8> / <32>
         const int h = hard[ls[loc]];
-        if (h == 0 && m <= FF_MAX) { ++k[LRB_FC_FLAT]; continue; }
-        ++k[h <= 1 ? LRB_FC_TIER0 : h == 4 ? LRB_FC_TIER1 : h == 2 ? LRB_FC_MERGE_OVER : LRB_FC_MERGE_VERIFY];
-        if (h == 3) continue;
-        for (int s = 0; s < (a.kls ? 4 : 1); ++s) k[LRB_FC_NOROWS] += ((const uint8_t *)&cnt[loc])[s] == FB_NOROWS;
+        if (h == LP_FLAT && m <= FF_MAX) { ++k[LRB_FC_FLAT]; continue; }
+        ++k[h <= LP_TIER0 ? LRB_FC_TIER0 : h == LP_TIER1 ? LRB_FC_TIER1 : h == LP_MERGE_OVER ? LRB_FC_MERGE_OVER : LRB_FC_MERGE_VERIFY];
+        if (h == LP_MERGE_VERIFY) continue;
+        for (int s = 0; s < (a.kls ? 4 : 1); ++s) k[LRB_FC_NOROWS] += ((const uint8_t *)&cnt[loc])[s] == CLASSES_UNTABULATED;
     }
     return cudaSuccess;
 }
@@ -1529,12 +1507,12 @@ LRB_DEVINL bool xl_other_chrom(const XlArgs &x, uint64_t k, uint32_t rt)      //
     }
     return true;
 }
-__global__ void __launch_bounds__(256) xl_insert_kernel(MergeArgs a, XlArgs x, const uint8_t *__restrict__ alive)
+__global__ void __launch_bounds__(256) xl_insert_kernel(MergeArgs a, XlArgs x)
 {
     const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= cand_count(a) || a.list.piece[c] < 0) return;
     const int n = a.cd.n[c];
-    if (n < 2 || !(alive[c] || a.forced[c])) return;
+    if (n < 2 || !(a.alive[c] || a.forced[c])) return;
     const uint32_t i = atomicAdd(&x.cnt[XL_NPL], 1u);
     x.pl[i] = (uint32_t)c; x.best[c] = 0;
     const uint32_t g = a.cd.gbeg[c], rt = (uint32_t)a.rows.tid[a.list.row[c]];
@@ -1546,11 +1524,11 @@ __global__ void __launch_bounds__(256) xl_insert_kernel(MergeArgs a, XlArgs x, c
     }
     if (!ok) x.cnt[XL_OVERFLOW] = 1u;
 }
-__global__ void __launch_bounds__(256) xl_probe_kernel(MergeArgs a, XlArgs x, const uint8_t *__restrict__ alive)
+__global__ void __launch_bounds__(256) xl_probe_kernel(MergeArgs a, XlArgs x)
 {
     if (x.cnt[XL_NPL] == 0) return;
     const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= cand_count(a) || !alive[c]) return;
+    if (c >= cand_count(a) || !a.alive[c]) return;
     const int n = a.cd.n[c];
     if (n < 2) return;
     const uint32_t g = a.cd.gbeg[c], rt = (uint32_t)a.rows.tid[a.list.row[c]];
@@ -1568,12 +1546,12 @@ __global__ void __launch_bounds__(256) xl_join_kernel(MergeArgs a, XlArgs x)
     for (uint32_t h = blockIdx.y; h < n_hx; h += gridDim.y) {
         const uint32_t e = x.hx[h];
         const int e_tid = a.rows.tid[a.list.row[e]];
-        const Entry E = {cd.n[e], cd.gbeg[e], a.work.fs[e], a.work.le[e], cd.hash[e], cd.rev[e] & 2, cd.j0[e], cd.sig[e]};
+        const Entry E = entry_of(cd, e, a.work.fs[e], a.work.le[e]);
         for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_pl; i += gridDim.x * blockDim.x) {
             const uint32_t p = x.pl[i];
             if (e >= p || a.rows.tid[a.list.row[p]] == e_tid) continue;          // only EARLIER entries, and its own chromosome is the fold's business
             if (a.up.force_strand && ((cd.rev[e] ^ cd.rev[p]) & 1)) continue;    // pieces carry is_rev 0 in cd.rev (update_gtf.c:149)
-            const Entry P = {cd.n[p], cd.gbeg[p], cd.fs[p], cd.le[p], cd.hash[p], cd.rev[p] & 2, cd.j0[p], cd.sig[p]};
+            const Entry P = entry_of(cd, p, cd.fs[p], cd.le[p]);
             const int r = chain_iden(a.ex, P, E, 0, a.up.end_dis);
             if (r == 0 || r == 2) atomicMax((unsigned long long *)&x.best[p], ((unsigned long long)(e + 1u) << 2) | (r == 0 ? 1ull : 2ull));
         }
@@ -1619,8 +1597,8 @@ void launch_xlocus_detect(const MergeArgs &a, const XlArgs &x, cudaStream_t st)
     cudaMemsetAsync(x.tkey, 0xFF, x.tcap * 8, st); cudaMemsetAsync(x.tmin, 0xFF, x.tcap * 4, st); cudaMemsetAsync(x.tmax, 0, x.tcap * 4, st);
     cudaMemsetAsync(x.cnt, 0, XL_NCNT * 4, st);
     const unsigned bl = (unsigned)((a.n_cand + 255) / 256);
-    xl_insert_kernel<<<bl, 256, 0, st>>>(a, x, a.dropped); LRB_COUNT_LAUNCH();
-    xl_probe_kernel<<<bl, 256, 0, st>>>(a, x, a.dropped); LRB_COUNT_LAUNCH();
+    xl_insert_kernel<<<bl, 256, 0, st>>>(a, x); LRB_COUNT_LAUNCH();
+    xl_probe_kernel<<<bl, 256, 0, st>>>(a, x); LRB_COUNT_LAUNCH();
     xl_join_kernel<<<dim3(64, 64), 256, 0, st>>>(a, x); LRB_COUNT_LAUNCH();
     int64_t blp = (a.n_cand / 16 + 255) / 256 + 1;                   // pieces are a small share of the candidates; the kernel checks the true count
     xl_force_kernel<<<(unsigned)blp, 256, 0, st>>>(a, x); LRB_COUNT_LAUNCH();
@@ -1632,7 +1610,7 @@ void launch_xlocus_apply(const MergeArgs &a, const XlArgs &x, cudaStream_t st)
     for (int pass = 0; pass < 2; ++pass) { xl_apply_kernel<<<(unsigned)blp, 256, 0, st>>>(a, x, pass); LRB_COUNT_LAUNCH(); }
 }
 
-__global__ void __launch_bounds__(256) merge_class_counts_kernel(MergeArgs a, const uint8_t *__restrict__ alive)
+__global__ void __launch_bounds__(256) merge_class_counts_kernel(MergeArgs a)
 {
     __shared__ uint32_t s_class[4];
     if (threadIdx.x < 4) s_class[threadIdx.x] = 0;
@@ -1640,7 +1618,7 @@ __global__ void __launch_bounds__(256) merge_class_counts_kernel(MergeArgs a, co
     const int64_t n = cand_count(a);
     uint32_t ccnt = 0;                                               // four 8-bit counters
     for (int64_t c = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 4, i = 0; i < 4 && c + i < n; ++i)
-        if (alive[c + i]) ccnt += 1u << (8 * a.kls[c + i]);
+        if (a.alive[c + i]) ccnt += 1u << (8 * a.kls[c + i]);
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) ccnt += __shfl_xor_sync(FULL, ccnt, o);         // <= 128 per class and warp
     if (lane_id() == 0) for (int q = 0; q < 4; ++q) { const uint32_t v = (ccnt >> (8 * q)) & 0xffu; if (v) atomicAdd(&s_class[q], v); }
@@ -1650,7 +1628,7 @@ __global__ void __launch_bounds__(256) merge_class_counts_kernel(MergeArgs a, co
 void launch_merge_class_counts(const MergeArgs &a, cudaStream_t st)
 {
     if (a.n_cand <= 0) return;
-    merge_class_counts_kernel<<<(unsigned)((a.n_cand + 1023) / 1024), 256, 0, st>>>(a, a.dropped);
+    merge_class_counts_kernel<<<(unsigned)((a.n_cand + 1023) / 1024), 256, 0, st>>>(a);
     LRB_COUNT_LAUNCH();
 }
 
