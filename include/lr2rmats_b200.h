@@ -338,11 +338,13 @@ int lrb_update_diag(const lrb_ctx *ctx, int64_t *pieces_across_chromosomes, int6
  *          NOROWS       (locus, sub-stream) pairs of the warp replay with more than 127 multi-exon classes (no relation rows)
  *   -d >0: D_SMALL / D_LARGE  loci of <= 32 / >= 33 candidates
  *   both:  SINGLE       loci of folds replayed as one locus (also counted above)
+ *   -d 0:  INDEXED      multi-exon candidates the warp replay decided by its class index (tabulated classes, no end tests)
+ *                       instead of a back-scan; per candidate
  * Counters [0, LRB_FC_COUNT) are the folds on the main stream (updated_T, unique-gtf), [LRB_FC_COUNT, 2 * LRB_FC_COUNT) those on
  * the side stream (update-gtf's four class folds of the summary).  Writes min(n, 2 * LRB_FC_COUNT) counters to out and returns
  * 2 * LRB_FC_COUNT. */
 enum { LRB_FC_FLAT, LRB_FC_TIER0, LRB_FC_TIER1, LRB_FC_MERGE_OVER, LRB_FC_MERGE_VERIFY, LRB_FC_NOROWS, LRB_FC_D_SMALL, LRB_FC_D_LARGE,
-       LRB_FC_SINGLE, LRB_FC_COUNT };
+       LRB_FC_SINGLE, LRB_FC_INDEXED, LRB_FC_COUNT };
 int lrb_fold_census(const lrb_ctx *ctx, int64_t *out, int n);
 /* pinned host memory for record batches (what the host decoder fills) */
 void *lrb_host_alloc(size_t bytes);

@@ -28,7 +28,7 @@ ENTRY_POINTS = [
 ]
 
 # lrb_fold_census counters per stream, in the order of the LRB_FC_* enum
-FOLD_CENSUS_NAMES = ["flat", "tier0", "tier1", "merge_overflow", "merge_verify", "norows", "d_small", "d_large", "single"]
+FOLD_CENSUS_NAMES = ["flat", "tier0", "tier1", "merge_overflow", "merge_verify", "norows", "d_small", "d_large", "single", "indexed"]
 
 T_NAMES = ["filter", "exon", "classify", "merge", "summary", "k_scan", "k_fold"]
 

@@ -147,6 +147,7 @@ int run_merge_async(lrb_ctx *c, MergeBufs &m, const DTransList &list, int64_t n_
     a.tlist = m.tlist.as<uint32_t>(); a.head = m.head.as<uint8_t>(); a.locus_start = m.locus_start.as<uint32_t>(); a.locus_cnt = m.locus_cnt.as<uint32_t>();
     a.alive = m.alive.as<uint8_t>();
     a.rep = m.rep.as<uint32_t>(); a.lstart = m.lstart.as<uint32_t>(); a.evmask = m.evmask.as<uint64_t>(); a.samemask = m.samemask.as<uint64_t>(); a.hard = m.hard.as<uint8_t>(); a.desc = m.desc.as<uint16_t>(); a.relsym = m.relsym.as<uint64_t>(); a.ckey = m.ckey.as<uint64_t>(); a.cmin = m.cmin.as<uint32_t>(); a.cord = m.cord.as<uint8_t>(); a.clist = m.clist.as<uint32_t>(); a.crow = m.crow.as<uint64_t>(); a.fb_list = m.fb_list.as<uint32_t>(); a.fb_cnt = m.fb_cnt.as<uint32_t>();
+    a.n_indexed = c->fold_census ? a.fb_cnt + 5 : nullptr;
     a.work = view(m.w, DMerged{n_cand, n_cand}); a.out = view(m.o, DMerged{n_cand, n_cand}); a.cd = view(m.cd, CandSoA{});
     a.tile_state = o.side ? c->tile_state2.as<uint64_t>() : c->tile_state.as<uint64_t>(); a.ticket = o.side ? d_ticket2(c) : d_ticket(c); a.totals = totals;
     a.kls = o.kls; a.class_alive = o.class_alive; a.single_locus = o.single_locus ? 1 : 0;

@@ -143,6 +143,7 @@ struct MergeArgs {
     // lent to XlArgs once the fold is done, as well: lstart as its hit list hx, relsym as best
     uint32_t *fb_list, *fb_cnt;                     // big loci: [0, n_cand) list of their locus ordinals, [n_cand, 2 n_cand) those that outgrew tier 0; counters
     uint64_t *ckey; uint32_t *cmin;                 // class table of the big loci: 2 * n_cand + 64 slots
+    uint32_t *n_indexed;                            // optional (fold census): multi-exon candidates fold_big_kernel decided by its class index
     DMerged out;                                    // compacted result
     uint8_t *forced;                                // optional (split pieces, see XlArgs): 1 = this piece is absorbed by an entry of an earlier locus when its own locus has nothing for it (3: that happened in the last fold)
     uint64_t *tile_state; uint32_t *ticket; uint64_t *totals;  // [0] n_loci, [1] n_out

@@ -1050,6 +1050,9 @@ __global__ void __launch_bounds__(256) fold_class_rows_kernel(MergeArgs a, uint3
             const uint64_t sj0 = s_j0[w][Sh];
             if (!sig_has(s_sig[w][L], sj0)) continue;
             const uint32_t cl = s_rep[w][L], cs = s_rep[w][Sh];
+            // under -c a survivor of the other strand never absorbs (fold_event): the rows leave such pairs out, so that the class
+            // index of fold_big_kernel sees only same-strand classes (the back-scan tests the strand first and reads no row for them)
+            if (a.up.force_strand && ((cd.rev[cl] ^ cd.rev[cs]) & 1)) continue;
             if (!chain_continues(a.ex, cd.gbeg[cl], cd.n[cl], (cd.rev[cl] & 2) != 0, sj0, cd.gbeg[cs], cd.n[cs], 0)) continue;
             atomicOr((unsigned long long *)&a.crow[2 * (size_t)s_rep[w][i] + (j >> 6)], 1ull << (j & 63));
             atomicOr((unsigned long long *)&a.crow[2 * (size_t)s_rep[w][j] + (i >> 6)], 1ull << (i & 63));
@@ -1058,10 +1061,59 @@ __global__ void __launch_bounds__(256) fold_class_rows_kernel(MergeArgs a, uint3
     }
 }
 
-// tier 0: loci beyond the masks or left over by the flat kernels (LP_TIER0); overflow -> LP_TIER1.  tier 1: overflow -> LP_MERGE_OVER.
-template <int G, int SLOTS, int CACHE, int TIER>
-__global__ void __launch_bounds__(FB_THREADS) fold_big_kernel(MergeArgs a, uint32_t *next_locus)
+// The class index of a replay: with tabulated rows and no end tests (end_dis = INT_MAX: check_iden's end tests always pass) the
+// event of a slot for a multi-exon candidate t does not depend on the slot's position: STOP where t_tid > tid or t_start > end,
+// else MERGE / DROP where the slot's class is in t's row (same class / partial match), else NONE.  The back-scan takes the newest
+// slot with an event, so its winner is max(F, A): F the newest stopping slot, A the newest slot of a class in t's row.  A comes from
+// last[o], the newest slot of class o (lane l keeps l, l + 32, l + 64, l + 96); F needs only be looked for at or above A, and only
+// in 32-slot chunks whose lower bounds of tid and end allow a stop (lane j keeps chunk j's; tid is fixed and end only grows, so a
+// bound stays a lower bound).  A split piece (tid = start = 0) never stops.
+struct FbIndex {
+    int last[4] = {-1, -1, -1, -1};
+    int lo_tid = INT_MAX, lo_end = INT_MAX;
+};
+// -1: no slot stops or absorbs at or above A (t is appended), else 0 (a slot stops the scan: t is appended) or 1 (absorbed / dropped)
+template <int SLOTS, int CACHE>
+LRB_DEVINL int fold_index_decide(FbSlots<SLOTS, CACHE> &S, FbIndex &ix, int cnt, int lane, int t_tid, int t_start, int t_fs, int t_le,
+                                 uint32_t t_ord, uint64_t t_row0, uint64_t t_row1)
 {
+    int A = -1;
+    if ((t_row0 >> lane) & 1ull) A = max(A, ix.last[0]);
+    if ((t_row0 >> (lane + 32)) & 1ull) A = max(A, ix.last[1]);
+    if ((t_row1 >> lane) & 1ull) A = max(A, ix.last[2]);
+    if ((t_row1 >> (lane + 32)) & 1ull) A = max(A, ix.last[3]);
+    A = __reduce_max_sync(FULL, A);
+    unsigned maybe = __ballot_sync(FULL, lane * 32 + 31 >= A && (t_tid > ix.lo_tid || t_start > ix.lo_end));
+    while (maybe) {
+        const int j = 31 - __clz(maybe);                         // newest chunk first
+        maybe &= ~(1u << j);
+        const int k = j * 32 + lane;
+        const bool live = k < cnt;
+        if (__any_sync(FULL, live && k >= A && (t_tid > S.tid[k] || t_start > S.end[k]))) return 0;
+        const int e = __reduce_min_sync(FULL, live ? S.end[k] : INT_MAX);     // no stop there: the bound becomes exact again
+        if (lane == j) ix.lo_end = e;
+    }
+    if (A < 0) return -1;
+    if (lane == 0 && (S.cand[A] >> 16) == t_ord) absorb_into(S.cov[A], S.fs[A], S.start[A], S.le[A], S.end[A], t_fs, t_le);
+    return 1;
+}
+// slot `slot` takes a candidate of class ord (FB_SINGLE: none)
+LRB_DEVINL void fold_index_append(FbIndex &ix, int lane, int slot, uint32_t ord, int tid, int end)
+{
+    if (ord != FB_SINGLE && lane == (int)(ord & 31u)) {
+        const int s = (int)(ord >> 5);
+        ix.last[0] = s == 0 ? slot : ix.last[0]; ix.last[1] = s == 1 ? slot : ix.last[1];
+        ix.last[2] = s == 2 ? slot : ix.last[2]; ix.last[3] = s == 3 ? slot : ix.last[3];
+    }
+    if (lane == (slot >> 5)) { ix.lo_tid = min(ix.lo_tid, tid); ix.lo_end = min(ix.lo_end, end); }
+}
+
+// tier 0: loci beyond the masks or left over by the flat kernels (LP_TIER0); overflow -> LP_TIER1.  tier 1: overflow -> LP_MERGE_OVER.
+// Tier 0 runs 6 blocks per SM (its slots take 222 KB of shared memory): at most 80 registers.
+template <int G, int SLOTS, int CACHE, int TIER>
+__global__ void __launch_bounds__(FB_THREADS, TIER == 0 ? 6 : 1) fold_big_kernel(MergeArgs a, uint32_t *next_locus)
+{
+    static_assert(G == 32 && SLOTS <= 32 * 32, "the class index takes a whole warp, one chunk of 32 slots per lane");
     extern __shared__ __align__(16) unsigned char fb_smem[];
     FbSlots<SLOTS, CACHE> &S = reinterpret_cast<FbSlots<SLOTS, CACHE> *>(fb_smem)[threadIdx.x / G];
     const int64_t n_loci = (int64_t)a.totals[0];
@@ -1084,6 +1136,10 @@ __global__ void __launch_bounds__(FB_THREADS) fold_big_kernel(MergeArgs a, uint3
         if (le - ls >= FB_MAXREL) { if (lane == 0) a.hard[ls] = LP_MERGE_OVER; continue; }
         const bool use_rows = ((const uint8_t *)&a.locus_cnt[loc])[my] != CLASSES_UNTABULATED;      // the static relation of the sub-stream's classes is tabulated
         if (!use_rows) for (int i = lane; i < CACHE; i += G) S.cache[i] = 0;
+        // multi-exon candidates are decided by the class index; single-exon ones (their overlap test reads the moving first start /
+        // last end), untabulated classes and finite end_dis keep the back-scan, the only exact path for them
+        const bool indexed = use_rows && a.up.end_dis == INT_MAX;
+        FbIndex ix; uint32_t n_indexed = 0;
         __syncwarp(gm);
         int cnt = 0; bool overflow = false;
         for (int64_t c0 = ls; c0 < le && !overflow; c0 += G) {
@@ -1110,7 +1166,10 @@ __global__ void __launch_bounds__(FB_THREADS) fold_big_kernel(MergeArgs a, uint3
                 const uint32_t t_ord = __shfl_sync(gm, l_ord, q, G);
                 const uint32_t t_rel = t_rep - (uint32_t)ls;
                 int result = 0;                                      // 0 append, 1 absorbed / dropped
-                for (int base = cnt - 1; base >= 0; base -= G) {
+                if (indexed && t_ord != FB_SINGLE) {
+                    result = fold_index_decide(S, ix, cnt, lane, t_tid, t_start, t_fs, t_le, t_ord, t_row0, t_row1) > 0;
+                    ++n_indexed;
+                } else for (int base = cnt - 1; base >= 0; base -= G) {
                     const int k = base - lane;
                     int ev = EV_NONE;
                     if (k >= 0) {
@@ -1155,6 +1214,7 @@ __global__ void __launch_bounds__(FB_THREADS) fold_big_kernel(MergeArgs a, uint3
                         S.tid[cnt] = t_tid; S.cov[cnt] = 1; S.gbeg[cnt] = t_gbeg; S.cand[cnt] = (uint32_t)(c0 + q - ls) | (t_ord << 16); S.rep[cnt] = t_rep;
                         S.meta[cnt] = ((uint32_t)t_n << 8) | ((uint32_t)t_kls << 2) | (uint32_t)(t_rv & 3);
                     }
+                    fold_index_append(ix, lane, cnt, t_ord, t_tid, t_end);
                     ++cnt;
                     if (lane == q) l_alive = 1;
                 }
@@ -1166,6 +1226,7 @@ __global__ void __launch_bounds__(FB_THREADS) fold_big_kernel(MergeArgs a, uint3
             if (lane == 0) { a.hard[ls] = TIER == 0 ? LP_TIER1 : LP_MERGE_OVER; if (TIER == 0) a.fb_list[a.n_cand + atomicAdd(&a.fb_cnt[2], 1u)] = list[li]; }
             continue;
         }
+        if (a.n_indexed && lane == 0 && n_indexed) atomicAdd(a.n_indexed, n_indexed);
         for (int k = lane; k < cnt; k += G) {
             const int64_t c = ls + (S.cand[k] & 0xFFFFu);
             a.work.cov[c] = S.cov[k]; a.work.start[c] = S.start[k]; a.work.end[c] = S.end[k]; a.work.fs[c] = S.fs[k]; a.work.le[c] = S.le[k];
@@ -1410,7 +1471,7 @@ void launch_merge_fold(const MergeArgs &a, cudaStream_t st)
         if (!attr) { cudaFuncSetAttribute(k0, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem0); cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1); attr = true; }
         ClassTab tab{(unsigned long long *)a.ckey, a.cmin, (uint64_t)a.n_cand * 2 + 64};
         cudaMemsetAsync(a.ckey, 0xFF, tab.cap * 8, st); cudaMemsetAsync(a.cmin, 0xFF, tab.cap * 4, st);
-        cudaMemsetAsync(a.fb_cnt, 0, 32, st);                     // [0] big loci, [1] tier-0 claims, [2] tier-0 overflows, [3] tier-1 claims
+        cudaMemsetAsync(a.fb_cnt, 0, 32, st);                     // [0] big loci, [1] tier-0 claims, [2] tier-0 overflows, [3] tier-1 claims, [4] class-row claims, [5] n_indexed
         int64_t blm = (a.n_cand / 8 + 255) / 256 + 1; if (blm > 148 * 8) blm = 148 * 8;
         fold_big_mark_kernel<<<(unsigned)blm, 256, 0, st>>>(a); LRB_COUNT_LAUNCH();
         fold_class_insert_kernel<<<bl, 256, 0, st>>>(a, tab); LRB_COUNT_LAUNCH();
@@ -1458,7 +1519,10 @@ cudaError_t merge_fold_census(const MergeArgs &a, cudaStream_t st, int64_t *k)
     if ((e = cudaMemcpyAsync(ls.data(), a.locus_start, n_loci * 4, cudaMemcpyDeviceToHost, st))) return e;
     if (exact && (e = cudaMemcpyAsync(cnt.data(), a.locus_cnt, n_loci * 4, cudaMemcpyDeviceToHost, st))) return e;
     if (exact && (e = cudaMemcpyAsync(hard.data(), a.hard, (size_t)n, cudaMemcpyDeviceToHost, st))) return e;
+    uint32_t n_indexed = 0;
+    if (exact && a.n_indexed && (e = cudaMemcpyAsync(&n_indexed, a.n_indexed, 4, cudaMemcpyDeviceToHost, st))) return e;
     if ((e = cudaStreamSynchronize(st))) return e;
+    k[LRB_FC_INDEXED] += n_indexed;
     for (uint64_t loc = 0; loc < n_loci; ++loc) {
         const int64_t m = (loc + 1 < n_loci ? (int64_t)ls[loc + 1] : n) - (int64_t)ls[loc];
         if (a.single_locus) ++k[LRB_FC_SINGLE];
