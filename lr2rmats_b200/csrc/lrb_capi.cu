@@ -111,7 +111,7 @@ int setup_merge(lrb_ctx *c, MergeBufs &m, int64_t n_cand)
 {
     size_t n = (size_t)std::max<int64_t>(n_cand, 1);
     NEED(m.tlist, n * 8); NEED(m.head, n); NEED(m.locus_start, (n + 1) * 4); NEED(m.locus_cnt, n * 4); NEED(m.alive, n);
-    NEED(m.rep, n * 4); NEED(m.lstart, n * 4); NEED(m.evmask, n * 8); NEED(m.samemask, n * 8); NEED(m.hard, n); NEED(m.desc, n * 2); NEED(m.relsym, n * 8); NEED(m.ckey, (2 * n + 64) * 8); NEED(m.cmin, (2 * n + 64) * 4); NEED(m.cord, n); NEED(m.clist, n * 4); NEED(m.crow, n * 16); NEED(m.fb_list, n * 8); NEED(m.fb_cnt, 64);
+    NEED(m.rep, n * 4); NEED(m.lstart, n * 4); NEED(m.evmask, n * 8); NEED(m.samemask, n * 8); NEED(m.hard, n); NEED(m.desc, n * 2); NEED(m.relsym, n * 8); NEED(m.ckey, (2 * n + 64) * 8); NEED(m.cmin, (2 * n + 64) * 4); NEED(m.cord, n); NEED(m.clist, n * 4); NEED(m.crow, n * 16); NEED(m.fb_list, n * 8); NEED(m.fb_cnt, 64); NEED(m.fb_state, fold_resume_bytes((int64_t)n));
     const Extent e{(int64_t)n};
     int rc;
     if ((rc = ensure(c, m.w, e)) || (rc = ensure(c, m.o, e)) || (rc = ensure(c, m.cd, e))) return rc;
@@ -120,8 +120,9 @@ int setup_merge(lrb_ctx *c, MergeBufs &m, int64_t n_cand)
 
 // what a merge fold does beyond folding its list
 struct FoldOpts {
-    const uint8_t *kls = nullptr;                   // set: the list carries four independent sub-streams (class id per candidate) folded
-    uint32_t *class_alive = nullptr;                // in one pass, and only the survivors per sub-stream are counted (class_alive)
+    const uint8_t *kls = nullptr;                   // set: every row is folded, as four independent sub-streams (class id per row) in one
+    uint32_t *class_alive = nullptr;                // pass; the list is built here, in class order (launch_class_order), and only the
+                                                    // survivors per sub-stream are counted (class_alive)
     bool time_fold = false;                         // EV_FOLD0 / EV_FOLD1 around the fold kernels
     bool side = false;                              // on the side stream, with its own look-back state
     bool single_locus = false;                      // the whole list is ONE locus: the back-scan replayed entry by entry
@@ -129,7 +130,8 @@ struct FoldOpts {
 };
 
 // merge fold over `list`, asynchronous.  n_cand is the number of candidates, or (n_cand_dev != nullptr) the host's upper
-// bound of a count that lives on the device.  Without o.kls the survivors are compacted into m.o_*.
+// bound of a count that lives on the device.  With o.kls `list` is only the storage the class-ordered list of every row is built in.
+// Without o.kls the survivors are compacted into m.o_*.
 // totals[0] <- number of loci, totals[1] <- number of survivors (device).
 int run_merge_async(lrb_ctx *c, MergeBufs &m, const DTransList &list, int64_t n_cand, const uint64_t *n_cand_dev, const lrb_update_params &up,
                     uint64_t *totals, const FoldOpts &o)
@@ -146,7 +148,7 @@ int run_merge_async(lrb_ctx *c, MergeBufs &m, const DTransList &list, int64_t n_
     a.rows = *c->cur; a.ex = c->ex; a.up = up; a.list = list; a.n_cand = n_cand; a.n_cand_dev = n_cand_dev;
     a.tlist = m.tlist.as<uint32_t>(); a.head = m.head.as<uint8_t>(); a.locus_start = m.locus_start.as<uint32_t>(); a.locus_cnt = m.locus_cnt.as<uint32_t>();
     a.alive = m.alive.as<uint8_t>();
-    a.rep = m.rep.as<uint32_t>(); a.lstart = m.lstart.as<uint32_t>(); a.evmask = m.evmask.as<uint64_t>(); a.samemask = m.samemask.as<uint64_t>(); a.hard = m.hard.as<uint8_t>(); a.desc = m.desc.as<uint16_t>(); a.relsym = m.relsym.as<uint64_t>(); a.ckey = m.ckey.as<uint64_t>(); a.cmin = m.cmin.as<uint32_t>(); a.cord = m.cord.as<uint8_t>(); a.clist = m.clist.as<uint32_t>(); a.crow = m.crow.as<uint64_t>(); a.fb_list = m.fb_list.as<uint32_t>(); a.fb_cnt = m.fb_cnt.as<uint32_t>();
+    a.rep = m.rep.as<uint32_t>(); a.lstart = m.lstart.as<uint32_t>(); a.evmask = m.evmask.as<uint64_t>(); a.samemask = m.samemask.as<uint64_t>(); a.hard = m.hard.as<uint8_t>(); a.desc = m.desc.as<uint16_t>(); a.relsym = m.relsym.as<uint64_t>(); a.ckey = m.ckey.as<uint64_t>(); a.cmin = m.cmin.as<uint32_t>(); a.cord = m.cord.as<uint8_t>(); a.clist = m.clist.as<uint32_t>(); a.crow = m.crow.as<uint64_t>(); a.fb_list = m.fb_list.as<uint32_t>(); a.fb_cnt = m.fb_cnt.as<uint32_t>(); a.fb_state = m.fb_state.p;
     a.n_indexed = c->fold_census ? a.fb_cnt + 5 : nullptr;
     a.work = view(m.w, DMerged{n_cand, n_cand}); a.out = view(m.o, DMerged{n_cand, n_cand}); a.cd = view(m.cd, CandSoA{});
     a.tile_state = o.side ? c->tile_state2.as<uint64_t>() : c->tile_state.as<uint64_t>(); a.ticket = o.side ? d_ticket2(c) : d_ticket(c); a.totals = totals;
@@ -159,6 +161,13 @@ int run_merge_async(lrb_ctx *c, MergeBufs &m, const DTransList &list, int64_t n_
         a.forced = c->xl_forced.as<uint8_t>();
         c->xl = XlArgs{c->xl_key.as<unsigned long long>(), c->xl_min.as<uint32_t>(), c->xl_max.as<uint32_t>(), tcap, a.clist, a.lstart, (uint32_t)std::min<int64_t>(n_cand, 1 << 20),
                        a.relsym, c->xl_cnt.as<uint32_t>()};
+    }
+    if (o.kls) {
+        NEED(m.cbase, ((size_t)n_cand + 1) * 16); NEED(m.cperm, (size_t)n_cand * 4); NEED(m.ckls, (size_t)n_cand);
+        a.cbase = m.cbase.as<uint4>(); a.kls = m.ckls.as<uint8_t>(); a.presegmented = 1;
+        launch_class_order(a, o.kls, m.cperm.as<uint32_t>(), m.ckls.as<uint8_t>(), st);
+        DTransList rows_list = list;                // a view: its columns are the list's
+        launch_rows_as_list(a.rows, m.cperm.as<uint32_t>(), n_cand, rows_list, st);
     }
     m.args = a;
     launch_merge_prepare(a, st);
@@ -548,7 +557,6 @@ static int update_lists_and_folds(lrb_ctx *c, UpdateRun &u, int pass)
             // updated_T fold and of the sets: forked onto the side stream.
             if ((rc = setup_list(c, c->tmp_list, c->tmp_cols, n))) return rc;
             CK(cudaEventRecord(c->ev_fork, c->st)); CK(cudaStreamWaitEvent(c->st2, c->ev_fork, 0));
-            launch_rows_as_list(rows, nullptr, n, c->tmp_list, c->st2);
             FoldOpts o; o.kls = c->u_ck.as<uint8_t>(); o.class_alive = c->y_counts.as<uint32_t>() + 8; o.side = true;
             if ((rc = run_merge_async(c, c->mg2, c->tmp_list, n, nullptr, *up, T + T_LOCI2, o))) return rc;
             CK(cudaEventRecord(c->ev_join, c->st2));

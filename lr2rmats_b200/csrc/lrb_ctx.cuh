@@ -159,7 +159,8 @@ struct UpdateOut {                                  // lrb_update_fetch, lrb_upd
 struct UniqueOut { ExonsOut ex; MergedCols<PBuf> uniq; PBuf shared; };
 
 struct MergeBufs {                                  // scratch + output of one merge fold
-    Buf tlist, head, locus_start, locus_cnt, alive, rep, lstart, evmask, samemask, hard, desc, relsym, ckey, cmin, cord, clist, crow, fb_list, fb_cnt;
+    Buf tlist, head, locus_start, locus_cnt, alive, rep, lstart, evmask, samemask, hard, desc, relsym, ckey, cmin, cord, clist, crow, fb_list, fb_cnt, fb_state;
+    Buf cbase, cperm, ckls;                         // class folds: class order of the rows (launch_class_order)
     MergedCols<Buf> w, o;                           // work list, survivors
     CandCols<Buf> cd;
     int64_t n_out = 0, n_loci = 0;

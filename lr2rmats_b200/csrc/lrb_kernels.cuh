@@ -125,7 +125,10 @@ struct MergeArgs {
     const uint64_t *n_cand_dev;                     // optional: the true count, produced on the device
     int n_tiles;
     int single_locus;                               // 1: the whole list is ONE locus (unsorted input: no cut is safe, the fold is replayed in order)
+    int presegmented;                               // 1: head, locus_start and totals[0] were written by launch_class_order
     const uint8_t *kls;                             // optional: sub-stream id per candidate (class folds: four independent folds in one pass); NULL: one stream
+    uint4 *cbase;                                   // with kls: per locus the candidates of each sub-stream before its head, [n_loci] the totals
+                                                    // (the list is in class order: inside a locus the sub-streams follow each other, class_range)
     uint64_t *samemask;                             // flat fold with kls: earlier candidates of the locus in the same sub-stream
     uint32_t *class_alive;                          // [4] surviving entries per sub-stream
     // scratch
@@ -142,6 +145,7 @@ struct MergeArgs {
     uint32_t *clist;                                // not used by the fold: the split-piece rounds' piece list (XlArgs::pl)
     // lent to XlArgs once the fold is done, as well: lstart as its hit list hx, relsym as best
     uint32_t *fb_list, *fb_cnt;                     // big loci: [0, n_cand) list of their locus ordinals, [n_cand, 2 n_cand) those that outgrew tier 0; counters
+    void *fb_state;                                 // big loci: tier 0's replay state per entry that outgrew it (fold_resume_bytes)
     uint64_t *ckey; uint32_t *cmin;                 // class table of the big loci: 2 * n_cand + 64 slots
     uint32_t *n_indexed;                            // optional (fold census): multi-exon candidates fold_big_kernel decided by its class index
     DMerged out;                                    // compacted result
@@ -159,8 +163,13 @@ struct XlArgs {
 void launch_xlocus_detect(const MergeArgs &a, const XlArgs &x, cudaStream_t st);    // after launch_merge_fold, before launch_merge_finish
 void launch_xlocus_apply(const MergeArgs &a, const XlArgs &x, cudaStream_t st);
 void launch_xlocus_reset(const MergeArgs &a, const XlArgs &x, cudaStream_t st);     // before the fold runs again with new marks
+// class folds: the rows (a.rows, all of them, a.n_cand) cut into loci in row order, then each locus's rows grouped by their class
+// row_kls (known, reliable, unreliable, unrecognized), each group in row order: perm[c] = row of candidate c, cand_kls[c] = its class;
+// head, locus_start, cbase and totals[0] as launch_merge_prepare would leave them for the rows in row order (a.tlist is scratch)
+void launch_class_order(MergeArgs a, const uint8_t *row_kls, uint32_t *perm, uint8_t *cand_kls, cudaStream_t st);
 void launch_merge_prepare(MergeArgs a, cudaStream_t st);            // candidates, locus heads, locus_start; totals[0] = number of loci
 void launch_merge_fold(const MergeArgs &a, cudaStream_t st);        // number of loci is read from a.totals[0] on the device
+size_t fold_resume_bytes(int64_t n_cand);                           // size of MergeArgs::fb_state
 cudaError_t merge_fold_census(const MergeArgs &a, cudaStream_t st, int64_t *counts);   // test hook: synchronises st, adds to counts[LRB_FC_*]
 void launch_merge_class_counts(const MergeArgs &a, cudaStream_t st);
 void launch_merge_finish(MergeArgs a, cudaStream_t st);             // survivors compacted into a.out; totals[1] = their number

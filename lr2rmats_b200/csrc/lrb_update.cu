@@ -635,6 +635,20 @@ LRB_DEVINL void locus_range(const MergeArgs &a, int64_t n_loci, int64_t loc, int
 {
     ls = a.locus_start[loc]; le = (loc + 1 < n_loci) ? a.locus_start[loc + 1] : cand_count(a);
 }
+// class order (launch_class_order): the candidates [cs, ce) of sub-stream k of the locus loc that starts at ls
+LRB_DEVINL void class_range(const MergeArgs &a, int64_t loc, int64_t ls, int k, int64_t &cs, int64_t &ce)
+{
+    const uint4 b0 = a.cbase[loc], b1 = a.cbase[loc + 1];
+    const uint32_t n0 = b1.x - b0.x, n1 = b1.y - b0.y, n2 = b1.z - b0.z, n3 = b1.w - b0.w;
+    cs = ls + (k > 0 ? n0 : 0u) + (k > 1 ? n1 : 0u) + (k > 2 ? n2 : 0u);
+    ce = cs + (k == 0 ? n0 : k == 1 ? n1 : k == 2 ? n2 : n3);
+}
+// the candidates a replay of (locus, sub-stream my) walks: with sub-streams their own range, else the whole locus
+LRB_DEVINL void replay_range(const MergeArgs &a, int64_t n_loci, int64_t loc, int my, int64_t &ls, int64_t &le, int64_t &cs, int64_t &ce)
+{
+    locus_range(a, n_loci, loc, ls, le);
+    if (a.kls) class_range(a, loc, ls, my, cs, ce); else { cs = ls; ce = le; }
+}
 
 // Hand-off state of a locus, kept at its head in hard[]: the path that folds the locus next.  A kernel writes it only to hand the
 // locus on, so the last value names the path that finished it (merge_fold_census).
@@ -656,29 +670,18 @@ static constexpr uint8_t CLASSES_UNTABULATED = 0xffu;   // locus_cnt byte: too m
 // (second look-back chain, sum).  The number of candidates may live on the device (n_cand_dev): the grid is sized by the
 // host's upper bound and surplus tiles only pass the chain on.
 static constexpr int FP_THREADS = 256, FP_ITEMS = 4;
-__global__ void __launch_bounds__(FP_THREADS) fold_prepare_kernel(MergeArgs a)
+// The locus heads of one tile (FP_THREADS threads, items [c0, c0 + FP_ITEMS) per thread, look-back chain `state` under max): head[c]
+// for every item, bit i of the result for item i.  keys(c, key_start, key_end): (tid + 1) << 32 | first start / last end of item c.
+template <class Keys>
+LRB_DEVINL uint32_t tile_locus_heads(uint64_t *state, int tile, int64_t c0, int64_t n, bool single_locus, uint8_t *head_out, Keys keys)
 {
-    __shared__ uint64_t s_w[FP_THREADS / 32];
-    __shared__ uint32_t s_scan[33];
-    __shared__ uint32_t s_tile; __shared__ uint64_t s_excl[2];
-    if (threadIdx.x == 0) s_tile = atomicAdd(a.ticket, 1u);
-    __syncthreads();
-    const int tile = (int)s_tile, lane = lane_id(), w = warp_id();
-    const int64_t n_cand = cand_count(a);
-    const int64_t c0 = ((int64_t)tile * FP_THREADS + threadIdx.x) * FP_ITEMS;
-    // locus segmentation first (cheap loads, two look-back chains): the per-exon work below then overlaps the chains of later tiles
+    __shared__ uint64_t s_w[FP_THREADS / 32], s_excl;
+    const int lane = lane_id(), w = warp_id();
     uint64_t key_end[FP_ITEMS], key_start[FP_ITEMS], run = 0;
 #pragma unroll
     for (int i = 0; i < FP_ITEMS; ++i) {
         key_end[i] = 0; key_start[i] = 0;
-        if (c0 + i < n_cand) {
-            const int64_t c = c0 + i;
-            const uint32_t rw = a.list.row[c]; const int ni = (int)a.list.cnt[c];
-            const uint32_t g = a.rows.ex_beg[rw] + a.list.lo[c];
-            const uint64_t tk = (uint64_t)(uint32_t)(a.rows.tid[rw] + 1) << 32;
-            key_end[i] = tk | (uint32_t)a.ex.ee[g + ni - 1];                               // real coordinates: locus segmentation
-            key_start[i] = tk | (uint32_t)a.ex.es[g];
-        }
+        if (c0 + i < n) keys(c0 + i, key_start[i], key_end[i]);
         run = key_end[i] > run ? key_end[i] : run;
     }
     // inclusive max over the block (one value per thread: the max of its items)
@@ -691,26 +694,48 @@ __global__ void __launch_bounds__(FP_THREADS) fold_prepare_kernel(MergeArgs a)
     for (int k = 0; k < FP_THREADS / 32; ++k) { const uint64_t v = s_w[k]; if (k < w && v > pre) pre = v; if (v > tot) tot = v; }
     uint64_t left = __shfl_up_sync(FULL, inc, 1); if (lane == 0) left = 0;
     const uint64_t tpre = left > pre ? left : pre;                             // exclusive prefix max of this thread inside the tile
-    if (w == 0) { const uint64_t e = lookback_exclusive(a.tile_state, tile, tot, OpMax()); if (lane == 0) s_excl[0] = e; }
+    if (w == 0) { const uint64_t e = lookback_exclusive(state, tile, tot, OpMax()); if (lane == 0) s_excl = e; }
     __syncthreads();
-    uint64_t before = s_excl[0] > tpre ? s_excl[0] : tpre;
-    uint32_t head = 0, nhead = 0;                                              // bit i: item i starts a locus
+    uint64_t before = s_excl > tpre ? s_excl : tpre;
+    uint32_t head = 0;
 #pragma unroll
     for (int i = 0; i < FP_ITEMS; ++i) {
-        if (c0 + i < n_cand) {
-            const bool h = (c0 + i == 0) || (!a.single_locus && key_start[i] > before);
-            if (h) { head |= 1u << i; ++nhead; }
-            a.head[c0 + i] = h ? 1 : 0;
+        if (c0 + i < n) {
+            const bool h = (c0 + i == 0) || (!single_locus && key_start[i] > before);
+            if (h) head |= 1u << i;
+            head_out[c0 + i] = h ? 1 : 0;
             before = key_end[i] > before ? key_end[i] : before;
         }
     }
-    uint32_t htot; const uint32_t hex = block_excl_sum(nhead, s_scan, &htot);
-    if (w == 0) { const uint64_t e = lookback_exclusive(a.tile_state + a.n_tiles, tile, (uint64_t)htot, OpAdd()); if (lane == 0) s_excl[1] = e; }
+    return head;
+}
+
+__global__ void __launch_bounds__(FP_THREADS) fold_prepare_kernel(MergeArgs a)
+{
+    __shared__ uint32_t s_scan[33];
+    __shared__ uint32_t s_tile; __shared__ uint64_t s_excl;
+    if (threadIdx.x == 0) s_tile = atomicAdd(a.ticket, 1u);
     __syncthreads();
-    uint32_t ho = (uint32_t)s_excl[1] + hex;
+    const int tile = (int)s_tile, lane = lane_id(), w = warp_id();
+    const int64_t n_cand = cand_count(a);
+    const int64_t c0 = ((int64_t)tile * FP_THREADS + threadIdx.x) * FP_ITEMS;
+    // locus segmentation first (cheap loads, two look-back chains): the per-exon work below then overlaps the chains of later tiles
+    if (!a.presegmented) {
+        const uint32_t head = tile_locus_heads(a.tile_state, tile, c0, n_cand, a.single_locus, a.head, [&](int64_t c, uint64_t &ks, uint64_t &ke) {
+            const uint32_t rw = a.list.row[c]; const int ni = (int)a.list.cnt[c];
+            const uint32_t g = a.rows.ex_beg[rw] + a.list.lo[c];
+            const uint64_t tk = (uint64_t)(uint32_t)(a.rows.tid[rw] + 1) << 32;
+            ke = tk | (uint32_t)a.ex.ee[g + ni - 1];                               // real coordinates: locus segmentation
+            ks = tk | (uint32_t)a.ex.es[g];
+        });
+        uint32_t htot; const uint32_t hex = block_excl_sum(__popc(head), s_scan, &htot);
+        if (w == 0) { const uint64_t e = lookback_exclusive(a.tile_state + a.n_tiles, tile, (uint64_t)htot, OpAdd()); if (lane == 0) s_excl = e; }
+        __syncthreads();
+        uint32_t ho = (uint32_t)s_excl + hex;
 #pragma unroll
-    for (int i = 0; i < FP_ITEMS; ++i) if ((head >> i) & 1u) a.locus_start[ho++] = (uint32_t)(c0 + i);
-    if (tile == a.n_tiles - 1 && threadIdx.x == 0) a.totals[0] = s_excl[1] + htot;
+        for (int i = 0; i < FP_ITEMS; ++i) if ((head >> i) & 1u) a.locus_start[ho++] = (uint32_t)(c0 + i);
+        if (tile == a.n_tiles - 1 && threadIdx.x == 0) a.totals[0] = s_excl + htot;
+    }
     // flatten the candidates: trans-level fields, chain hash, junction signature.  Striped over the tile (thread t takes the
     // candidates t, t + 256, ...): the exon ranges of neighbouring threads are adjacent in the pools, so the per-exon loads of a
     // warp fall into a few lines instead of one line per lane
@@ -748,6 +773,81 @@ void launch_merge_prepare(MergeArgs a, cudaStream_t st)
     a.n_tiles = (int)((a.n_cand + FP_THREADS * FP_ITEMS - 1) / (FP_THREADS * FP_ITEMS));
     cudaMemsetAsync(a.tile_state, 0, (size_t)a.n_tiles * 16, st); cudaMemsetAsync(a.ticket, 0, 4, st);
     fold_prepare_kernel<<<(unsigned)a.n_tiles, FP_THREADS, 0, st>>>(a); LRB_COUNT_LAUNCH();
+}
+
+// Class order for the class folds (update_gtf.c:501-528 folds each class's rows as a list of its own).  A candidate never sees another
+// sub-stream's entries (fold_event), so grouping the rows of a locus by class, each group in row order, hands every sub-stream the same
+// sequence, and its replay walks only its own range.  The loci are cut on all rows in row order (fold_prepare_kernel's rule), not
+// on the permuted list: the cuts, and so every locus and its path, stay what they are.
+//   class_order_kernel    per tile of rows: locus heads (look-back, max), then one look-back (sum) of the head count and the class
+//                         counts (class 3 is what the others leave); per row its locus and its rank among the earlier rows of its
+//                         class, per locus the class counts before its head (cbase)
+//   class_scatter_kernel  per row: its candidate index (the locus's class ranges follow from two neighbours in cbase)
+__global__ void __launch_bounds__(FP_THREADS) class_order_kernel(MergeArgs a, const uint8_t *__restrict__ row_kls, uint2 *loc_rank)
+{
+    __shared__ uint32_t s_scan[33];
+    __shared__ uint32_t s_tile; __shared__ uint64_t s_excl[2];
+    if (threadIdx.x == 0) s_tile = atomicAdd(a.ticket, 1u);
+    __syncthreads();
+    const int tile = (int)s_tile, lane = lane_id(), w = warp_id();
+    const int64_t n = a.n_cand;
+    const int64_t c0 = ((int64_t)tile * FP_THREADS + threadIdx.x) * FP_ITEMS;
+    const uint32_t head = tile_locus_heads(a.tile_state, tile, c0, n, a.single_locus, a.head, [&](int64_t r, uint64_t &ks, uint64_t &ke) {
+        const uint32_t g = a.rows.ex_beg[r]; const int ni = (int)a.rows.ex_n[r];
+        const uint64_t tk = (uint64_t)(uint32_t)(a.rows.tid[r] + 1) << 32;
+        ke = tk | (uint32_t)a.ex.ee[g + ni - 1];
+        ks = tk | (uint32_t)a.ex.es[g];
+    });
+    uint32_t k[FP_ITEMS], hk0 = __popc(head), k12 = 0;                         // 16-bit counters in pairs: a tile has 1024 rows
+#pragma unroll
+    for (int i = 0; i < FP_ITEMS; ++i) {
+        k[i] = c0 + i < n ? row_kls[c0 + i] : 3u;
+        hk0 += k[i] == 0 ? 1u << 16 : 0u; k12 += k[i] == 1 ? 1u : k[i] == 2 ? 1u << 16 : 0u;
+    }
+    uint32_t t_hk0, t_k12;
+    const uint32_t e_hk0 = block_excl_sum(hk0, s_scan, &t_hk0), e_k12 = block_excl_sum(k12, s_scan, &t_k12);
+    if (w == 0) {
+        const uint64_t x = lookback_exclusive(a.tile_state + a.n_tiles, tile, pack_pair(t_hk0 & 0xFFFFu, t_hk0 >> 16), OpAdd());
+        const uint64_t y = lookback_exclusive(a.tile_state + 2 * a.n_tiles, tile, pack_pair(t_k12 & 0xFFFFu, t_k12 >> 16), OpAdd());
+        if (lane == 0) { s_excl[0] = x; s_excl[1] = y; }
+    }
+    __syncthreads();
+    uint32_t loc = pair_hi(s_excl[0]) + (e_hk0 & 0xFFFFu);                    // loci that start before this thread's first row
+    uint32_t r0 = pair_lo(s_excl[0]) + (e_hk0 >> 16), r1 = pair_hi(s_excl[1]) + (e_k12 & 0xFFFFu), r2 = pair_lo(s_excl[1]) + (e_k12 >> 16);
+    uint32_t r3 = (uint32_t)c0 - r0 - r1 - r2;                                 // rows of each class before it
+#pragma unroll
+    for (int i = 0; i < FP_ITEMS; ++i) {
+        if (c0 + i >= n) break;
+        if ((head >> i) & 1u) { a.locus_start[loc] = (uint32_t)(c0 + i); a.cbase[loc] = make_uint4(r0, r1, r2, r3); ++loc; }
+        const uint32_t rank = k[i] == 0 ? r0++ : k[i] == 1 ? r1++ : k[i] == 2 ? r2++ : r3++;
+        loc_rank[c0 + i] = make_uint2(loc - 1, rank);
+    }
+    if (tile == a.n_tiles - 1 && threadIdx.x == 0) {
+        const uint32_t n_loci = pair_hi(s_excl[0]) + (t_hk0 & 0xFFFFu);
+        const uint32_t q0 = pair_lo(s_excl[0]) + (t_hk0 >> 16), q1 = pair_hi(s_excl[1]) + (t_k12 & 0xFFFFu), q2 = pair_lo(s_excl[1]) + (t_k12 >> 16);
+        a.totals[0] = n_loci;
+        a.cbase[n_loci] = make_uint4(q0, q1, q2, (uint32_t)n - q0 - q1 - q2);
+    }
+}
+__global__ void __launch_bounds__(256) class_scatter_kernel(MergeArgs a, const uint8_t *__restrict__ row_kls, const uint2 *__restrict__ loc_rank,
+                                                            uint32_t *perm, uint8_t *cand_kls)
+{
+    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= a.n_cand) return;
+    const int k = row_kls[r]; const uint2 lr = loc_rank[r];
+    const uint4 b0 = a.cbase[lr.x];
+    int64_t cs, ce; class_range(a, lr.x, a.locus_start[lr.x], k, cs, ce);
+    const int64_t c = cs + lr.y - (k == 0 ? b0.x : k == 1 ? b0.y : k == 2 ? b0.z : b0.w);
+    perm[c] = (uint32_t)r; cand_kls[c] = (uint8_t)k;
+}
+void launch_class_order(MergeArgs a, const uint8_t *row_kls, uint32_t *perm, uint8_t *cand_kls, cudaStream_t st)
+{
+    if (a.n_cand <= 0) return;
+    a.n_tiles = (int)((a.n_cand + FP_THREADS * FP_ITEMS - 1) / (FP_THREADS * FP_ITEMS));
+    uint2 *loc_rank = reinterpret_cast<uint2 *>(a.tlist);                      // tlist: n_cand * 8 bytes, not needed before the fold
+    cudaMemsetAsync(a.tile_state, 0, (size_t)a.n_tiles * 24, st); cudaMemsetAsync(a.ticket, 0, 4, st);
+    class_order_kernel<<<(unsigned)a.n_tiles, FP_THREADS, 0, st>>>(a, row_kls, loc_rank); LRB_COUNT_LAUNCH();
+    class_scatter_kernel<<<(unsigned)((a.n_cand + 255) / 256), 256, 0, st>>>(a, row_kls, loc_rank, perm, cand_kls); LRB_COUNT_LAUNCH();
 }
 
 // check_iden (gtf.c:54-92) between candidate t and fold entry E (first start / last end may have been extended)
@@ -933,7 +1033,7 @@ template <int SLOTS, int CACHE>
 struct FbSlots {
     uint64_t j0[SLOTS], sig[SLOTS];
     int fs[SLOTS], le[SLOTS], end[SLOTS], start[SLOTS], tid[SLOTS], cov[SLOTS];
-    uint32_t gbeg[SLOTS], cand[SLOTS], meta[SLOTS], rep[SLOTS];       // meta: n << 8 | kls << 2 | mono bit 1 | rev bit 0
+    uint32_t gbeg[SLOTS], cand[SLOTS], meta[SLOTS], rep[SLOTS];       // meta: n << 8 | mono bit 1 | rev bit 0
     uint32_t cache[CACHE];                          // partial-match relation of two classes: valid 31 | result 30 | relA 29:15 | relB 14:0
     uint32_t pad[8];                                // group stride = 8 banks mod 32: the four 8-lane groups of a warp read disjoint banks
 };
@@ -946,11 +1046,17 @@ __global__ void __launch_bounds__(256) fold_big_mark_kernel(MergeArgs a)
     for (int64_t loc = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / 32; loc < n_loci; loc += (int64_t)gridDim.x * blockDim.x / 32) {
         int64_t ls, le; locus_range(a, n_loci, loc, ls, le);
         if (le - ls <= FF_MAX && a.hard[ls] == LP_FLAT) continue;
-        // the later passes walk this list, not all loci; an entry is (locus, sub-stream): the four class folds of the summary run over the
-        // same rows but never see each other's entries, so each gets its own replay (and its own, four times shorter, survivor list)
+        // the later passes walk this list, not all loci; an entry is (locus, sub-stream): the four class folds of the summary run over
+        // their own ranges of the locus (class order) and never see each other's entries, so each gets its own replay, and a sub-stream
+        // without rows in the locus gets none (nor class rows: zero classes)
         if (lane < (a.kls ? 4 : 1)) {
-            const uint32_t i = atomicAdd(&a.fb_cnt[0], 1u);
-            if (i < (uint32_t)a.n_cand) a.fb_list[i] = ((uint32_t)loc << 2) | (uint32_t)lane; else a.hard[ls] = LP_MERGE_OVER;    // (cannot happen for loci beyond the masks)
+            int64_t cs = ls, ce = le;
+            if (a.kls) class_range(a, loc, ls, lane, cs, ce);
+            if (ce == cs) ((uint8_t *)&a.locus_cnt[loc])[lane] = 0;
+            else {
+                const uint32_t i = atomicAdd(&a.fb_cnt[0], 1u);
+                if (i < (uint32_t)a.n_cand) a.fb_list[i] = ((uint32_t)loc << 2) | (uint32_t)lane; else a.hard[ls] = LP_MERGE_OVER;    // (cannot happen for loci beyond the masks)
+            }
         }
         for (int64_t c = ls + lane; c < le; c += 32) { a.desc[c] = DESC_BIG; a.lstart[c] = (uint32_t)ls; }
     }
@@ -1016,13 +1122,13 @@ __global__ void __launch_bounds__(256) fold_class_rows_kernel(MergeArgs a, uint3
         if (lane == 0) bi = atomicAdd(next_entry, 1u);               // entries differ by orders of magnitude in size: claimed one at a time
         bi = __shfl_sync(FULL, bi, 0);
         if ((int64_t)bi >= n_big) return;
-        const int64_t loc = a.fb_list[bi] >> 2; const uint32_t my = a.fb_list[bi] & 3u;
-        int64_t ls, le; locus_range(a, n_loci, loc, ls, le);
+        const int64_t loc = a.fb_list[bi] >> 2; const int my = (int)(a.fb_list[bi] & 3u);
+        int64_t ls, le, cs, ce; replay_range(a, n_loci, loc, my, ls, le, cs, ce);
         if (for_merge_fold(a.hard[ls])) continue;
         int K = 0;
-        for (int64_t c0 = ls; c0 < le; c0 += 32) {
+        for (int64_t c0 = cs; c0 < ce; c0 += 32) {
             const int64_t c = c0 + lane;
-            const bool headc = c < le && cd.n[c] > 1 && a.rep[c] == (uint32_t)c && (!a.kls || a.kls[c] == my);
+            const bool headc = c < ce && cd.n[c] > 1 && a.rep[c] == (uint32_t)c;
             const unsigned b = __ballot_sync(FULL, headc);
             if (headc) {
                 const int o = K + __popc(b & ((1u << lane) - 1u));
@@ -1036,8 +1142,7 @@ __global__ void __launch_bounds__(256) fold_class_rows_kernel(MergeArgs a, uint3
         if (lane == 0) ((uint8_t *)&a.locus_cnt[loc])[my] = K <= FB_MAXCLS ? (uint8_t)K : CLASSES_UNTABULATED;
         if (K > FB_MAXCLS) continue;
         __syncwarp();
-        for (int64_t c = ls + lane; c < le; c += 32) {
-            if (a.kls && a.kls[c] != my) continue;
+        for (int64_t c = cs + lane; c < ce; c += 32) {
             if (cd.n[c] < 2) a.cord[c] = (uint8_t)FB_SINGLE;
             else if (a.rep[c] != (uint32_t)c) a.cord[c] = a.cord[a.rep[c]];
         }
@@ -1108,7 +1213,44 @@ LRB_DEVINL void fold_index_append(FbIndex &ix, int lane, int slot, uint32_t ord,
     if (lane == (slot >> 5)) { ix.lo_tid = min(ix.lo_tid, tid); ix.lo_end = min(ix.lo_end, end); }
 }
 
-// tier 0: loci beyond the masks or left over by the flat kernels (LP_TIER0); overflow -> LP_TIER1.  tier 1: overflow -> LP_MERGE_OVER.
+// Tier 0's replay when its slots ran out, kept for tier 1 to go on from: the slots, each lane's class index (slot numbers and chunk
+// bounds mean the same with tier 1's slots), the candidate that found the slots full (tier 1 decides it again: a candidate to be
+// appended changed nothing) and the count of indexed decisions so far.  The relation cache is not kept: it only remembers relations
+// tier 1 can work out again.  One per entry of tier 1's list, at the entry's index.
+static constexpr int FB_SLOTS0 = 128;
+struct FbSaved {
+    uint64_t j0[FB_SLOTS0], sig[FB_SLOTS0];
+    int fs[FB_SLOTS0], le[FB_SLOTS0], end[FB_SLOTS0], start[FB_SLOTS0], tid[FB_SLOTS0], cov[FB_SLOTS0];
+    uint32_t gbeg[FB_SLOTS0], cand[FB_SLOTS0], meta[FB_SLOTS0], rep[FB_SLOTS0];
+    FbIndex ix[32];
+    int64_t next; uint32_t n_indexed;
+};
+// a tier-1 entry holds more than FB_SLOTS0 candidates of its own (a range no other entry shares)
+size_t fold_resume_bytes(int64_t n_cand) { return (size_t)(n_cand / (FB_SLOTS0 + 1) + 1) * sizeof(FbSaved); }
+template <int SLOTS, int CACHE>
+LRB_DEVINL void fb_save(FbSaved &d, const FbSlots<SLOTS, CACHE> &S, const FbIndex &ix, int lane, int64_t next, uint32_t n_indexed)
+{
+    static_assert(SLOTS == FB_SLOTS0, "tier 0 saves");
+    for (int k = lane; k < FB_SLOTS0; k += 32) {
+        d.j0[k] = S.j0[k]; d.sig[k] = S.sig[k]; d.fs[k] = S.fs[k]; d.le[k] = S.le[k]; d.end[k] = S.end[k]; d.start[k] = S.start[k];
+        d.tid[k] = S.tid[k]; d.cov[k] = S.cov[k]; d.gbeg[k] = S.gbeg[k]; d.cand[k] = S.cand[k]; d.meta[k] = S.meta[k]; d.rep[k] = S.rep[k];
+    }
+    d.ix[lane] = ix;
+    if (lane == 0) { d.next = next; d.n_indexed = n_indexed; }
+}
+template <int SLOTS, int CACHE>
+LRB_DEVINL void fb_load(FbSlots<SLOTS, CACHE> &S, FbIndex &ix, const FbSaved &d, int lane)
+{
+    static_assert(SLOTS >= FB_SLOTS0, "tier 1 resumes");
+    for (int k = lane; k < FB_SLOTS0; k += 32) {
+        S.j0[k] = d.j0[k]; S.sig[k] = d.sig[k]; S.fs[k] = d.fs[k]; S.le[k] = d.le[k]; S.end[k] = d.end[k]; S.start[k] = d.start[k];
+        S.tid[k] = d.tid[k]; S.cov[k] = d.cov[k]; S.gbeg[k] = d.gbeg[k]; S.cand[k] = d.cand[k]; S.meta[k] = d.meta[k]; S.rep[k] = d.rep[k];
+    }
+    ix = d.ix[lane];
+}
+
+// tier 0: loci beyond the masks or left over by the flat kernels (LP_TIER0); overflow -> LP_TIER1, which goes on from where tier 0
+// stopped.  tier 1: overflow -> LP_MERGE_OVER.
 // Tier 0 runs 6 blocks per SM (its slots take 222 KB of shared memory): at most 80 registers.
 template <int G, int SLOTS, int CACHE, int TIER>
 __global__ void __launch_bounds__(FB_THREADS, TIER == 0 ? 6 : 1) fold_big_kernel(MergeArgs a, uint32_t *next_locus)
@@ -1130,7 +1272,7 @@ __global__ void __launch_bounds__(FB_THREADS, TIER == 0 ? 6 : 1) fold_big_kernel
         li = __shfl_sync(gm, li, 0, G);
         if (li >= n_list) return;
         const int64_t loc = (int64_t)(list[li] >> 2); const int my = (int)(list[li] & 3u);      // (locus, sub-stream)
-        int64_t ls, le; locus_range(a, n_loci, loc, ls, le);
+        int64_t ls, le, cs, ce; replay_range(a, n_loci, loc, my, ls, le, cs, ce);
         const int hd = a.hard[ls];
         if (TIER == 0 ? for_merge_fold(hd) : hd != LP_TIER1) continue;
         if (le - ls >= FB_MAXREL) { if (lane == 0) a.hard[ls] = LP_MERGE_OVER; continue; }
@@ -1140,26 +1282,27 @@ __global__ void __launch_bounds__(FB_THREADS, TIER == 0 ? 6 : 1) fold_big_kernel
         // last end), untabulated classes and finite end_dis keep the back-scan, the only exact path for them
         const bool indexed = use_rows && a.up.end_dis == INT_MAX;
         FbIndex ix; uint32_t n_indexed = 0;
-        __syncwarp(gm);
         int cnt = 0; bool overflow = false;
-        for (int64_t c0 = ls; c0 < le && !overflow; c0 += G) {
+        int64_t from = cs, next = 0;                                 // next: the candidate that found the slots full
+        if constexpr (TIER == 1) {
+            const FbSaved &d = reinterpret_cast<const FbSaved *>(a.fb_state)[li];
+            fb_load(S, ix, d, lane); cnt = FB_SLOTS0; from = d.next; n_indexed = d.n_indexed;
+        }
+        __syncwarp(gm);
+        for (int64_t c0 = from; c0 < ce && !overflow; c0 += G) {
             // 32 candidates, one per lane
-            const int64_t cl = c0 + lane; const bool have = cl < le;
-            const int l_kls = (have && a.kls) ? a.kls[cl] : 0;
-            const bool mine = have && (!a.kls || l_kls == my);       // rows of the other sub-streams are skipped below: their fields are not loaded
-            if (!__any_sync(gm, mine)) continue;
-            const int l_tid = mine ? cd.tid[cl] : 0, l_start = mine ? cd.start[cl] : 0, l_end = mine ? cd.end[cl] : 0, l_rv = mine ? cd.rev[cl] : 0;
-            const int l_n = mine ? cd.n[cl] : 0, l_fs = mine ? cd.fs[cl] : 0, l_le = mine ? cd.le[cl] : 0; const uint32_t l_gbeg = mine ? cd.gbeg[cl] : 0;
-            const uint64_t l_j0 = mine ? cd.j0[cl] : 0, l_sig = mine ? cd.sig[cl] : 0;
-            const uint32_t l_rep = mine ? a.rep[cl] : 0;
-            const uint32_t l_ord = (mine && use_rows) ? a.cord[cl] : FB_SINGLE;
+            const int64_t cl = c0 + lane; const bool have = cl < ce;
+            const int l_tid = have ? cd.tid[cl] : 0, l_start = have ? cd.start[cl] : 0, l_end = have ? cd.end[cl] : 0, l_rv = have ? cd.rev[cl] : 0;
+            const int l_n = have ? cd.n[cl] : 0, l_fs = have ? cd.fs[cl] : 0, l_le = have ? cd.le[cl] : 0; const uint32_t l_gbeg = have ? cd.gbeg[cl] : 0;
+            const uint64_t l_j0 = have ? cd.j0[cl] : 0, l_sig = have ? cd.sig[cl] : 0;
+            const uint32_t l_rep = have ? a.rep[cl] : 0;
+            const uint32_t l_ord = (have && use_rows) ? a.cord[cl] : FB_SINGLE;
             const uint64_t l_row0 = l_ord != FB_SINGLE ? a.crow[2 * (size_t)l_rep] : 0, l_row1 = l_ord != FB_SINGLE ? a.crow[2 * (size_t)l_rep + 1] : 0;
             int l_alive = 0;
-            const int nb = (int)min((int64_t)G, le - c0);
+            const int nb = (int)min((int64_t)G, ce - c0);
             for (int q = 0; q < nb; ++q) {
-                if (a.kls && __shfl_sync(gm, l_kls, q, G) != my) continue;       // another sub-stream's row: its own replay takes it
                 const int t_tid = __shfl_sync(gm, l_tid, q, G), t_start = __shfl_sync(gm, l_start, q, G), t_end = __shfl_sync(gm, l_end, q, G), t_rv = __shfl_sync(gm, l_rv, q, G);
-                const int t_kls = __shfl_sync(gm, l_kls, q, G), t_n = __shfl_sync(gm, l_n, q, G), t_fs = __shfl_sync(gm, l_fs, q, G), t_le = __shfl_sync(gm, l_le, q, G);
+                const int t_n = __shfl_sync(gm, l_n, q, G), t_fs = __shfl_sync(gm, l_fs, q, G), t_le = __shfl_sync(gm, l_le, q, G);
                 const uint32_t t_gbeg = __shfl_sync(gm, l_gbeg, q, G), t_rep = __shfl_sync(gm, l_rep, q, G);
                 const uint64_t t_j0 = __shfl_sync(gm, l_j0, q, G), t_sig = __shfl_sync(gm, l_sig, q, G);
                 const uint64_t t_row0 = __shfl_sync(gm, l_row0, q, G), t_row1 = __shfl_sync(gm, l_row1, q, G);
@@ -1177,7 +1320,7 @@ __global__ void __launch_bounds__(FB_THREADS, TIER == 0 ? 6 : 1) fold_big_kernel
                         const int e_n = (int)(mt >> 8);
                         // the static relation of two multi-exon classes: the class rows, else the identity of the representatives or the
                         // partial match (the shorter chain's first junction must be a junction of the longer, then the cached relation)
-                        ev = fold_event(a, !a.kls || (int)((mt >> 2) & 3u) == t_kls, t_tid > S.tid[k] || t_start > S.end[k], (t_rv & 1) == (int)(mt & 1u),
+                        ev = fold_event(a, true, t_tid > S.tid[k] || t_start > S.end[k], (t_rv & 1) == (int)(mt & 1u),
                                         t_n, t_fs, t_le, e_n, S.fs[k], S.le[k], [&] {
                             if (use_rows) {
                                 const uint32_t e_ord = S.cand[k] >> 16;
@@ -1208,11 +1351,11 @@ __global__ void __launch_bounds__(FB_THREADS, TIER == 0 ? 6 : 1) fold_big_kernel
                 __syncwarp(gm);
                 if (result == 0 && absorbed_elsewhere(a, c0 + q, lane == 0)) result = 1;
                 if (result == 0) {
-                    if (cnt == SLOTS) { overflow = true; break; }
+                    if (cnt == SLOTS) { overflow = true; next = c0 + q; n_indexed -= indexed && t_ord != FB_SINGLE; break; }
                     if (lane == 0) {
                         S.j0[cnt] = t_j0; S.sig[cnt] = t_sig; S.fs[cnt] = t_fs; S.le[cnt] = t_le; S.end[cnt] = t_end; S.start[cnt] = t_start;
                         S.tid[cnt] = t_tid; S.cov[cnt] = 1; S.gbeg[cnt] = t_gbeg; S.cand[cnt] = (uint32_t)(c0 + q - ls) | (t_ord << 16); S.rep[cnt] = t_rep;
-                        S.meta[cnt] = ((uint32_t)t_n << 8) | ((uint32_t)t_kls << 2) | (uint32_t)(t_rv & 3);
+                        S.meta[cnt] = ((uint32_t)t_n << 8) | (uint32_t)(t_rv & 3);
                     }
                     fold_index_append(ix, lane, cnt, t_ord, t_tid, t_end);
                     ++cnt;
@@ -1220,10 +1363,17 @@ __global__ void __launch_bounds__(FB_THREADS, TIER == 0 ? 6 : 1) fold_big_kernel
                 }
                 __syncwarp(gm);
             }
-            if (!overflow && have && (!a.kls || l_kls == my)) a.alive[cl] = (uint8_t)l_alive;
+            if (have && (!overflow || cl < next)) a.alive[cl] = (uint8_t)l_alive;
         }
-        if (overflow) {                                              // the next tier / merge_fold_kernel redoes the locus from scratch
-            if (lane == 0) { a.hard[ls] = TIER == 0 ? LP_TIER1 : LP_MERGE_OVER; if (TIER == 0) a.fb_list[a.n_cand + atomicAdd(&a.fb_cnt[2], 1u)] = list[li]; }
+        if (overflow) {                                              // tier 1 goes on from here; merge_fold_kernel redoes the locus from scratch
+            if constexpr (TIER == 0) {
+                uint32_t i = 0;
+                if (lane == 0) i = atomicAdd(&a.fb_cnt[2], 1u);
+                i = __shfl_sync(gm, i, 0, G);
+                fb_save(reinterpret_cast<FbSaved *>(a.fb_state)[i], S, ix, lane, next, n_indexed);
+                if (lane == 0) { a.hard[ls] = LP_TIER1; a.fb_list[a.n_cand + i] = list[li]; }
+            } else if (lane == 0) a.hard[ls] = LP_MERGE_OVER;
+            __syncwarp(gm);
             continue;
         }
         if (a.n_indexed && lane == 0 && n_indexed) atomicAdd(a.n_indexed, n_indexed);
@@ -1464,8 +1614,8 @@ void launch_merge_fold(const MergeArgs &a, cudaStream_t st)
         // loci beyond the masks and the ones the flat kernels gave up on: classes through one table, then warp per locus with the survivors
         // in shared memory; what outgrows the slots there (LP_MERGE_OVER) is replayed from global memory
         int64_t bl2 = (a.n_cand / (FF_MAX + 1) + 1 + 3) / 4 + 8; if (bl2 > 148 * 8) bl2 = 148 * 8;
-        using S0 = FbSlots<128, 256>; using S1 = FbSlots<416, 1024>;
-        auto k0 = fold_big_kernel<32, 128, 256, 0>; auto k1 = fold_big_kernel<32, 416, 1024, 1>;
+        using S0 = FbSlots<FB_SLOTS0, 256>; using S1 = FbSlots<416, 1024>;
+        auto k0 = fold_big_kernel<32, FB_SLOTS0, 256, 0>; auto k1 = fold_big_kernel<32, 416, 1024, 1>;
         const size_t smem0 = sizeof(S0) * (FB_THREADS / 32), smem1 = sizeof(S1) * (FB_THREADS / 32);
         static bool attr = false;
         if (!attr) { cudaFuncSetAttribute(k0, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem0); cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1); attr = true; }
