@@ -260,6 +260,17 @@ int lrb_sj_upload(lrb_ctx *ctx, const lrb_sj *sj);        /* sj==NULL or n==0: n
 
 /* Record batch -> device (async on the ctx stream; pinned source recommended). */
 int lrb_batch_upload(lrb_ctx *ctx, const lrb_batch *batch);
+/* Record batch -> device WITHOUT its CIGAR pool, for a batch whose pool does not fit the device (4 B per op; an ONT read carries
+ * hundreds of ops).  The fixed-width columns are copied as lrb_batch_upload copies them; the context's device copy of an earlier
+ * pool is freed.  The later lrb_filter_run, lrb_exon_run and lrb_pipeline_run stream the pool from batch->cigar through two
+ * device staging buffers, in chunks of whole walk tiles of at most chunk_ops ops (the copy of the next chunk runs under the walk
+ * of the current one); every result is the one lrb_batch_upload gives.  A tile whose own ops exceed chunk_ops (a tile is 256
+ * records when the batch averages <= 48 ops per record, 32 otherwise) is staged alone, in staging grown for it.  chunk_ops == 0:
+ * the library sizes the chunks from the free device memory (cudaMemGetInfo).
+ * Contract: batch->cigar stays valid and unchanged until the next lrb_batch_upload / lrb_batch_attach or lrb_ctx_destroy.  Pinned
+ * memory (lrb_host_alloc) lets the copies overlap the walk; pageable memory gives the same results, serialised.  lrb_bam2sj needs
+ * the batch passed to it (b != NULL) after an attach.  LRB_E_ARG if chunk_ops < 0. */
+int lrb_batch_attach(lrb_ctx *ctx, const lrb_batch *batch, int64_t chunk_ops);
 int lrb_chains_upload(lrb_ctx *ctx, const lrb_chains *chains);   /* -m g input */
 
 /* Device-resident stages (no host<->device copies of per-read data). */
@@ -326,6 +337,10 @@ int lrb_elapsed_ms(lrb_ctx *ctx, int slot_from, int slot_to, float *ms);   /* sy
 /* Diagnostics of the last lrb_update_run: split pieces that were absorbed by an entry on ANOTHER chromosome (the reference's
  * back-scan of a piece never stops, update_gtf.c:148; settled in rounds on the device) and folds replayed as one locus. */
 int lrb_update_diag(const lrb_ctx *ctx, int64_t *pieces_across_chromosomes, int64_t *one_locus_replays);
+/* Diagnostics of the last CIGAR walk (lrb_filter_run / lrb_exon_run / lrb_pipeline_run; the repeat of a walk whose exon pool
+ * was regrown counts alone): chunks of an attached batch's pool walked, and the most ops one chunk staged on the device.
+ * Both 0 for a batch uploaded with its pool. */
+int lrb_cigar_stream_diag(const lrb_ctx *ctx, int64_t *chunks, int64_t *max_staged_ops);
 /* Fold census, a test hook: which path of the merge fold (update-gtf's updated_T and class folds, unique-gtf) folded each locus.
  * Counted only when LRB_TEST_FOLD_CENSUS is set to a non-zero number at lrb_ctx_create; each fold then reads its locus table back
  * and synchronises its stream.  Cumulative over the context's life; the repeated folds that settle split pieces absorbed on another

@@ -24,7 +24,7 @@ ENTRY_POINTS = [
     "lrb_mark", "lrb_elapsed_ms", "lrb_host_alloc", "lrb_host_free", "lrb_update_fetch_table", "lrb_filter_fetch_keep",
     "lrb_comm_id", "lrb_comm_init", "lrb_comm_destroy", "lrb_comm_rank", "lrb_tables_broadcast", "lrb_update_gather", "lrb_gather_fetch",
     "lrb_gather_timing", "lrb_shard_cuts_weighted", "lrb_update_diag", "lrb_bam2sj", "lrb_sort3", "lrb_update_gather_reads",
-    "lrb_gather_fetch_reads", "lrb_fold_census",
+    "lrb_gather_fetch_reads", "lrb_fold_census", "lrb_batch_attach", "lrb_cigar_stream_diag",
 ]
 
 # lrb_fold_census counters per stream, in the order of the LRB_FC_* enum
@@ -60,6 +60,7 @@ def load_library():
     L.lrb_rm_upload.argtypes = [vp, P(cabi.Anno)]
     L.lrb_sj_upload.argtypes = [vp, P(cabi.Sj)]
     L.lrb_batch_upload.argtypes = [vp, P(cabi.Batch)]
+    L.lrb_batch_attach.argtypes = [vp, P(cabi.Batch), C.c_int64]
     L.lrb_chains_upload.argtypes = [vp, P(cabi.Chains)]
     L.lrb_filter_run.argtypes = [vp, P(cabi.FilterParams)]
     L.lrb_exon_run.argtypes = [vp, P(cabi.ExonParams), C.c_int]
@@ -99,6 +100,7 @@ def load_library():
     L.lrb_gather_fetch_reads.argtypes = [vp, P(cabi.UpdateResult), P(cabi.FilterResult)]
     L.lrb_update_diag.argtypes = [vp, P(C.c_int64), P(C.c_int64)]
     L.lrb_fold_census.argtypes = [vp, P(C.c_int64), C.c_int]
+    L.lrb_cigar_stream_diag.argtypes = [vp, P(C.c_int64), P(C.c_int64)]
     L.lrb_bam2sj.argtypes = [vp, P(cabi.Batch), cabi.u8p, P(cabi.SjParams), P(cabi.Sj)]
     L.lrb_sort3.argtypes = [vp, cabi.u32p, cabi.u32p, cabi.u32p, C.c_int64, P(cabi.u32p)]
     _lib = L
@@ -154,6 +156,12 @@ class Context:
     def upload(self, batch_soa: dict):
         b, k = cabi.make_batch(batch_soa); self._keep["batch"] = (b, k)
         self._ck(self.L.lrb_batch_upload(self.h, C.byref(b)))
+
+    def attach(self, batch_soa: dict, chunk_ops: int = 0):
+        """The batch without its CIGAR pool on the device: the walk streams batch_soa["cigar"] from host memory in chunks of at most
+        chunk_ops ops (0: the library chooses).  The arrays stay referenced here until the next upload / attach or close()."""
+        b, k = cabi.make_batch(batch_soa); self._keep["batch"] = (b, k)
+        self._ck(self.L.lrb_batch_attach(self.h, C.byref(b), int(chunk_ops)))
 
     def upload_struct(self, b):
         self._ck(self.L.lrb_batch_upload(self.h, C.byref(b)))
@@ -279,6 +287,11 @@ class Context:
     def update_diag(self):
         a = C.c_int64(); b = C.c_int64(); self._ck(self.L.lrb_update_diag(self.h, C.byref(a), C.byref(b)))
         return dict(pieces_across_chromosomes=int(a.value), one_locus_replays=int(b.value))
+
+    def cigar_stream_diag(self) -> dict:
+        """Of the last CIGAR walk: chunks of an attached pool walked, and the most ops one chunk staged on the device (0, 0: uploaded pool)."""
+        a = C.c_int64(); b = C.c_int64(); self._ck(self.L.lrb_cigar_stream_diag(self.h, C.byref(a), C.byref(b)))
+        return dict(chunks=int(a.value), max_staged_ops=int(b.value))
 
     def fold_census(self) -> dict:
         """Loci per merge-fold path since the context was created, {"main": {name: n}, "side": {name: n}} (names: FOLD_CENSUS_NAMES).

@@ -36,9 +36,54 @@ int setup_exons(lrb_ctx *c, int64_t cap)
     return LRB_OK;
 }
 
+// tiles of the CIGAR walk: short CIGARs (Iso-Seq like) are walked thread per read on staged tiles of 256 reads, long CIGARs
+// (ONT like) by the streaming kernel on warp tiles
+bool scan_stream_mode(int64_t n, int64_t n_cigar) { return n > 0 && (double)n_cigar / (double)n > 48.0; }
+int scan_tile_reads(bool stream_mode) { return stream_mode ? stream_reads_per_tile() : scan_reads_per_tile(); }
+
+// the CIGAR walk of one scan attempt (look-back state zeroed by the caller): one launch over the resident pool, or the chunks of an
+// attached pool.  A chunk's launch takes its tiles from its first one on, so its first tile looks back at the last tile of the
+// chunk before, complete by then (same stream): rows and exons are placed as by one launch, with no host round trip in between.
+int walk_cigars(lrb_ctx *c, ScanArgs a, int n_tiles, bool stream_mode, size_t smem)
+{
+    c->n_chunks_walked = 0; c->max_staged_ops = 0;
+    if (!c->attached) {
+        a.ops = c->b.cigar; a.op_base = 0; a.tile_base = 0;
+        CK(cudaMemsetAsync(a.ticket, 0, 4, c->st));
+        launch_cigar_scan(a, n_tiles, stream_mode, smem, c->st);
+        return LRB_OK;
+    }
+    // + 4 words: the last bulk copy of the streaming kernel rounds its length up to 16 bytes
+    for (Buf &s : c->stage) NEED(s, (size_t)(c->stage_ops + 4) * 4);
+    const size_t nk = c->chunks.size();
+    auto copy_chunk = [&](size_t k) -> int {         // chunk k -> staging buffer k & 1, once the walk of chunk k - 2 is done with it
+        const OpChunk &ch = c->chunks[k]; const int s = (int)(k & 1);
+        CK(cudaStreamWaitEvent(c->st_copy, c->ev_walked[s], 0));
+        if (ch.op_end > ch.op_base)
+            CK(cudaMemcpyAsync(c->stage[s].p, c->h_cigar + ch.op_base, (size_t)(ch.op_end - ch.op_base) * 4, cudaMemcpyHostToDevice, c->st_copy));
+        CK(cudaEventRecord(c->ev_copied[s], c->st_copy));
+        return LRB_OK;
+    };
+    int rc;
+    if (nk && (rc = copy_chunk(0))) return rc;
+    for (size_t k = 0; k < nk; ++k) {
+        if (k + 1 < nk && (rc = copy_chunk(k + 1))) return rc;
+        const OpChunk &ch = c->chunks[k]; const int s = (int)(k & 1);
+        CK(cudaStreamWaitEvent(c->st, c->ev_copied[s], 0));
+        a.ops = c->stage[s].as<uint32_t>(); a.op_base = ch.op_base; a.tile_base = ch.tile0;
+        CK(cudaMemsetAsync(a.ticket, 0, 4, c->st));
+        launch_cigar_scan(a, ch.tile1 - ch.tile0, stream_mode, smem, c->st);
+        CK(cudaEventRecord(c->ev_walked[s], c->st));
+        c->max_staged_ops = std::max<int64_t>(c->max_staged_ops, (int64_t)(ch.op_end - ch.op_base));
+    }
+    c->n_chunks_walked = (int64_t)nk;
+    return LRB_OK;
+}
+
 // the scan stage in one of its three modes; on return the counts are known on the host.  Mode 2 (fused pipeline) writes the rows at
 // their record index and runs the selection, the keep list and the kept rows (rows2) behind the walk: its counts are n_pass, ex.n and
-// n_keep, read back in the same round trip.  If the exon pool was too small the walk is repeated once with its exact size.
+// n_keep, read back in the same round trip.  If the exon pool was too small the walk is repeated once with its exact size (all chunks
+// of an attached pool again).
 int run_scan(lrb_ctx *c, int mode, const lrb_filter_params *fp, const lrb_exon_params *ep, const uint8_t *sel_mask)
 {
     const int64_t n = c->b.n;
@@ -48,15 +93,18 @@ int run_scan(lrb_ctx *c, int mode, const lrb_filter_params *fp, const lrb_exon_p
     if (mode != 1) { NEED(c->f_pass, (size_t)n + 1); NEED(c->f_score, (size_t)n * 4 + 4); NEED(c->f_intron, (size_t)n * 4 + 4); }
     if (n == 0) { c->rows.n = 0; c->ex.n = 0; if (mode != 0 && (rc = setup_exons(c, 16)) != LRB_OK) return rc; return LRB_OK; }
     const double avg = (double)c->b.n_cigar / (double)n;
-    // short CIGARs (Iso-Seq like): thread per read on staged tiles of 256 reads; long CIGARs (ONT like): the streaming kernel
-    const bool stream_mode = avg > 48.0;
-    const int R = stream_mode ? stream_reads_per_tile() : 256;
+    const bool stream_mode = scan_stream_mode(n, c->b.n_cigar);
+    const int R = scan_tile_reads(stream_mode);
     int stage_words = (int)(R * avg * 1.3) + 256; stage_words = (stage_words + 255) & ~255; stage_words = std::max(2048, std::min(12288, stage_words));
     if (stream_mode) stage_words = 0;
     const int n_tiles = (int)((n + R - 1) / R);
     if (mode != 0) {
         int64_t bound = c->b.n_cigar + n + 16, est = c->b.n_cigar / 2 + n + 4096;
-        if ((rc = setup_exons(c, std::min(bound, std::max(est, c->ex.cap)))) != LRB_OK) return rc;
+        rc = setup_exons(c, std::min(bound, std::max(est, c->ex.cap)));
+        // the estimate is 4.5 B per op, more than the pool: an attached batch that cannot hold it walks once to count its exons
+        // (the walk writes none when they do not fit), then again with the exact size
+        if (rc == LRB_E_NOMEM && c->attached) rc = setup_exons(c, n + 4096);
+        if (rc != LRB_OK) return rc;
     }
     for (int attempt = 0;; ++attempt) {
         ScanArgs a{};
@@ -65,10 +113,10 @@ int run_scan(lrb_ctx *c, int mode, const lrb_filter_params *fp, const lrb_exon_p
         a.rows = c->rows; a.ex = c->ex; a.tile_state = c->tile_state.as<uint64_t>(); a.ticket = d_ticket(c); a.totals = d_totals(c);
         a.reads_per_tile = R; a.stage_words = stage_words; a.rows_by_record = mode == 2 ? 1 : 0;
         CK(cudaMemsetAsync(c->tile_state.p, 0, (size_t)n_tiles * 8, c->st));
-        CK(cudaMemsetAsync(c->scalars.p, 0, 8 * 8, c->st)); CK(cudaMemsetAsync(d_ticket(c), 0, 4, c->st));
+        CK(cudaMemsetAsync(c->scalars.p, 0, 8 * 8, c->st));
         size_t smem = (size_t)stage_words * 4;
         tick(c, EV_SCAN0);
-        launch_cigar_scan(a, n_tiles, stream_mode, smem, c->st);
+        if ((rc = walk_cigars(c, a, n_tiles, stream_mode, smem)) != LRB_OK) return rc;
         tick(c, EV_SCAN1);
         CK(cudaGetLastError());
         if (mode == 2) {                             // run selection on the record stream -> compaction + row gather
@@ -216,6 +264,8 @@ int lrb_ctx_create(int device, lrb_ctx **out)
     cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming); cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming);
     if (cudaStreamCreateWithFlags(&c->st3, cudaStreamNonBlocking) != cudaSuccess) { cudaStreamDestroy(c->st2); cudaStreamDestroy(c->st); delete c; return LRB_E_CUDA; }
     cudaEventCreateWithFlags(&c->ev_fork3, cudaEventDisableTiming); cudaEventCreateWithFlags(&c->ev_join3, cudaEventDisableTiming);
+    if (cudaStreamCreateWithFlags(&c->st_copy, cudaStreamNonBlocking) != cudaSuccess) { cudaStreamDestroy(c->st3); cudaStreamDestroy(c->st2); cudaStreamDestroy(c->st); delete c; return LRB_E_CUDA; }
+    for (int i = 0; i < 2; ++i) { cudaEventCreateWithFlags(&c->ev_copied[i], cudaEventDisableTiming); cudaEventCreateWithFlags(&c->ev_walked[i], cudaEventDisableTiming); }
     { const char *e = getenv("LRB_TEST_SMALL_NOVEL_CAP"); if (e) c->test_small_novel_cap = atoi(e) != 0; }      // test hook: novel_T sized too small on the first attempt
     { const char *e = getenv("LRB_FORCE_SINGLE_FOLD"); if (e) c->force_single_fold = atoi(e) != 0; }    // test hook: updated_T always folded by the one-locus replay
     { const char *e = getenv("LRB_TEST_FOLD_CENSUS"); if (e) c->fold_census = atoi(e) != 0; }       // test hook: loci tallied by fold path (lrb_fold_census)
@@ -234,12 +284,14 @@ void lrb_ctx_destroy(lrb_ctx *c)
 {
     if (!c) return;
     cudaSetDevice(c->device);
-    cudaStreamSynchronize(c->st); cudaStreamSynchronize(c->st2); cudaStreamSynchronize(c->st3);
+    cudaStreamSynchronize(c->st); cudaStreamSynchronize(c->st2); cudaStreamSynchronize(c->st3); cudaStreamSynchronize(c->st_copy);
     lrbk::multi_release(c);
     for (cudaEvent_t e : c->ev) cudaEventDestroy(e);
     for (int i = 0; i < 8; ++i) cudaEventDestroy(c->marks[i]);
     cudaEventDestroy(c->ev_fork); cudaEventDestroy(c->ev_join);
     cudaEventDestroy(c->ev_fork3); cudaEventDestroy(c->ev_join3); cudaStreamDestroy(c->st3);
+    for (int i = 0; i < 2; ++i) { cudaEventDestroy(c->ev_copied[i]); cudaEventDestroy(c->ev_walked[i]); }
+    cudaStreamDestroy(c->st_copy);
     cudaStreamDestroy(c->st2); cudaStreamDestroy(c->st);
     delete c;                                       // frees the device and pinned buffers
 }
@@ -334,23 +386,58 @@ int lrb_sj_upload(lrb_ctx *c, const lrb_sj *s)
 }
 
 // --------------------------------------------------------------------------------------------------- batch
-int lrb_batch_upload(lrb_ctx *c, const lrb_batch *b)
+// the fixed-width columns of b -> HBM, and the CIGAR pool with them unless it stays in host memory (attach: chunk_ops >= 0)
+static int load_batch(lrb_ctx *c, const lrb_batch *b, int64_t chunk_ops)
 {
     if (!c || !b || b->n < 0) return LRB_E_ARG;
     CK(cudaSetDevice(c->device));
+    const bool attach = chunk_ops >= 0;
     const size_t n = (size_t)b->n;
     const size_t nc = n ? b->cigar_off[n] : 0;
     if (b->n >= (1ll << 31) - 1) return fail(c, LRB_E_ARG, "batch too large: at most 2^31-2 records per batch");
     if (n && b->cigar_off[0] != 0) return fail(c, LRB_E_ARG, "cigar_off[0] must be 0");
     if (nc >= (1ull << 40)) return fail(c, LRB_E_ARG, "batch too large: at most 2^40 CIGAR ops per batch");
+    c->have_batch = false; c->attached = false; c->h_cigar = nullptr; c->chunks.clear();
+    if (attach) c->batch_cols.cigar.release();      // the pool's device column is returned before anything else is sized
+    else { c->stage[0].release(); c->stage[1].release(); }
     static const uint64_t no_cigar = 0;             // cigar_off of an empty batch
     BatchCols<const void *> src;
     src.tid = b->tid; src.pos = b->pos; src.l_qseq = b->l_qseq; src.nm = b->nm; src.flag = b->flag; src.xs = b->xs; src.qhash = b->qname_hash;
     src.cigar_off = n ? b->cigar_off : &no_cigar; src.cigar = b->cigar;
-    if (int rc = copy(c, c->batch_cols, src, Extent{(int64_t)n, (int64_t)nc}, cudaMemcpyHostToDevice)) return rc;
+    if (int rc = copy(c, c->batch_cols, src, Extent{(int64_t)n, attach ? 0 : (int64_t)nc}, cudaMemcpyHostToDevice)) return rc;
     c->b = view(c->batch_cols, DBatch{b->n, (int64_t)nc});
+    if (attach) {
+        c->batch_cols.cigar.release(); c->b.cigar = nullptr;      // (copy() sized it for an empty pool)
+        if (chunk_ops == 0) {                       // two staging buffers of at most 1/64 of the free memory each, 4 MB .. 256 MB
+            size_t fr = 0, tot = 0;
+            CK(cudaMemGetInfo(&fr, &tot));
+            chunk_ops = std::max<int64_t>(1 << 20, std::min<int64_t>(1 << 26, (int64_t)(fr / 64 / 4)));
+        }
+        // chunks of whole tiles, staged from op_base = (the first tile's first op) rounded down to a multiple of 4; a chunk takes
+        // tiles while its staged ops stay within chunk_ops, and at least one
+        const bool sm = scan_stream_mode((int64_t)n, (int64_t)nc);
+        const int64_t R = scan_tile_reads(sm), n_tiles = ((int64_t)n + R - 1) / R;
+        auto tile_end = [&](int64_t t) { return b->cigar_off[std::min<int64_t>((int64_t)n, (t + 1) * R)]; };
+        c->stage_ops = 0;
+        for (int64_t t = 0; t < n_tiles;) {
+            OpChunk ch; ch.tile0 = (int)t; ch.op_base = b->cigar_off[t * R] & ~3ull;
+            do ++t; while (t < n_tiles && tile_end(t) - ch.op_base <= (uint64_t)chunk_ops);
+            ch.tile1 = (int)t; ch.op_end = tile_end(t - 1);
+            c->chunks.push_back(ch);
+            c->stage_ops = std::max<int64_t>(c->stage_ops, (int64_t)(ch.op_end - ch.op_base));
+        }
+        c->h_cigar = b->cigar; c->attached = true;
+    }
     c->have_batch = true; c->have_filter = c->have_exons = c->have_update = c->have_unique = false;
     return LRB_OK;
+}
+
+int lrb_batch_upload(lrb_ctx *c, const lrb_batch *b) { return load_batch(c, b, -1); }
+
+int lrb_batch_attach(lrb_ctx *c, const lrb_batch *b, int64_t chunk_ops)
+{
+    if (chunk_ops < 0) return LRB_E_ARG;
+    return load_batch(c, b, chunk_ops);
 }
 
 // rows straight from exon chains (-m g input): start/end/ex_beg/ex_n derived on device
@@ -1100,6 +1187,13 @@ int lrb_update_diag(const lrb_ctx *c, int64_t *pieces, int64_t *replays)
     if (!c) return LRB_E_ARG;
     if (pieces) *pieces = c->n_xlocus_pieces;
     if (replays) *replays = c->n_xlocus_replays;
+    return LRB_OK;
+}
+int lrb_cigar_stream_diag(const lrb_ctx *c, int64_t *chunks, int64_t *max_staged_ops)
+{
+    if (!c) return LRB_E_ARG;
+    if (chunks) *chunks = c->n_chunks_walked;
+    if (max_staged_ops) *max_staged_ops = c->max_staged_ops;
     return LRB_OK;
 }
 int lrb_fold_census(const lrb_ctx *c, int64_t *out, int n)

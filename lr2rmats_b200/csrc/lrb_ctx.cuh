@@ -6,6 +6,7 @@
 #include <cstring>
 #include <string>
 #include <type_traits>
+#include <vector>
 #include "lrb_common.cuh"
 #include "lrb_kernels.cuh"
 #include "lrb_summary.cuh"
@@ -176,6 +177,10 @@ enum {
 
 struct MultiState;                                  // lrb_multi.cu
 
+struct OpChunk {                                    // one chunk of an attached CIGAR pool: tiles [tile0, tile1), ops [op_base, op_end)
+    int tile0, tile1; uint64_t op_base, op_end;
+};
+
 }  // namespace lrbk
 
 struct lrb_ctx {
@@ -194,6 +199,12 @@ struct lrb_ctx {
     // batch
     DBatch b; lrbk::BatchCols<Buf> batch_cols;
     bool have_batch = false;
+    // an attached batch (lrb_batch_attach): b.cigar is NULL, the walk streams the caller's host pool through two staging buffers,
+    // chunk k + 1 copied on st_copy while chunk k is walked on st.  The chunks are whole tiles of the walk, planned at attach.
+    const uint32_t *h_cigar = nullptr; bool attached = false;
+    std::vector<lrbk::OpChunk> chunks; int64_t stage_ops = 0;       // the plan; the most ops one chunk stages
+    Buf stage[2]; cudaStream_t st_copy = nullptr; cudaEvent_t ev_copied[2] = {}, ev_walked[2] = {};
+    int64_t n_chunks_walked = 0, max_staged_ops = 0;                // lrb_cigar_stream_diag: of the last walk
     // filter
     Buf f_pass, f_score, f_intron, f_keep_row_mask, f_keep_rec_mask, f_keep_idx, f_keep_rows;
     int64_t n_pass = 0, n_keep = 0; bool have_filter = false;

@@ -63,14 +63,20 @@ struct ScanArgs {
     const uint8_t *sel_mask;                        // mode 1: records to walk (NULL = all)
     uint8_t *pass; int32_t *score, *intron_n;       // filter outputs (record level)
     DRows rows; DExons ex;
-    uint64_t *tile_state; uint32_t *ticket;         // look-back state (zeroed per launch)
+    uint64_t *tile_state; uint32_t *ticket;         // look-back state (zeroed per walk), tile ticket (zeroed per launch)
     uint64_t *totals;                               // [0] rows, [1] exons
     int reads_per_tile, stage_words;
     int rows_by_record;                             // 1: a passing record's row is written at its record index (no row compaction)
+    // the ops of the launch's tiles: op k of the batch (cigar_off[r] <= k < cigar_off[r + 1] for a record r of these tiles) is
+    // ops[k - op_base].  The whole pool (ops = b.cigar, op_base = 0), or one chunk of it staged from host memory (op_base a
+    // multiple of 4, so that the 16-byte alignment of the pool holds in the staging buffer).
+    const uint32_t *ops; uint64_t op_base;
+    int tile_base;                                  // a launch walks tiles [tile_base, tile_base + its grid's tiles)
 };
 
 void launch_cigar_scan(const ScanArgs &a, int n_tiles, bool stream_mode, size_t smem_bytes, cudaStream_t st);
 int stream_reads_per_tile();                        // tile size of the long-CIGAR streaming kernel
+int scan_reads_per_tile();                          // tile size of the short-CIGAR kernel
 void launch_select_runs(const DBatch &b, const uint32_t *row_read, int64_t n_rows, const int32_t *score, const int32_t *intron_n,
                         lrb_filter_params fp, uint8_t *keep_row_mask, uint8_t *keep_rec_mask, cudaStream_t st);
 // ordered compaction of the set positions of a byte mask: out[k] = index of k-th nonzero (optionally mapped through `map`)

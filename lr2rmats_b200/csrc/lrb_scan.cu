@@ -27,6 +27,9 @@ enum { OP_M = 0, OP_I, OP_D, OP_N, OP_S, OP_H, OP_P, OP_EQ, OP_X, OP_B };
 
 LRB_DEVINL bool op_ref(unsigned op) { return (0x18Du >> op) & 1u; }   // M D N = X consume reference (bits 0,2,3,7,8)
 
+// op `off` of the batch, from wherever the launch's ops are (see ScanArgs::ops)
+LRB_DEVINL const uint32_t *op_ptr(const ScanArgs &a, uint64_t off) { return a.ops + (off - a.op_base); }
+
 struct WalkStats { int n_exon, intron_n, del_len, ref_len, first_start, last_end; };
 
 // ---- sequential walk (one thread).  EMIT writes exons to es/ee.
@@ -158,7 +161,7 @@ __global__ void __launch_bounds__(SCAN_THREADS) cigar_scan_kernel(ScanArgs a)
     __shared__ uint64_t s_excl;
 
     const int tid = threadIdx.x, R = a.reads_per_tile;
-    if (tid == 0) s_tile = atomicAdd(a.ticket, 1u);
+    if (tid == 0) s_tile = a.tile_base + atomicAdd(a.ticket, 1u);
     __syncthreads();
     const int tile = (int)s_tile;
     const int64_t r0 = (int64_t)tile * R, r1 = min(a.b.n, r0 + R);
@@ -169,7 +172,7 @@ __global__ void __launch_bounds__(SCAN_THREADS) cigar_scan_kernel(ScanArgs a)
     const bool do_filter = a.mode != 1, do_exon = a.mode != 0;
     if (staged) {
         // coalesced stage: scalar head up to 16-byte alignment, then 128-bit streaming loads
-        const uint32_t *src = a.b.cigar + w_lo;
+        const uint32_t *src = op_ptr(a, w_lo);
         uint32_t head = (uint32_t)((4 - (w_lo & 3)) & 3); if (head > nw) head = (uint32_t)nw;
         if ((uint32_t)tid < head) s_words[tid] = ldg_stream_u32(src + tid);
         uint32_t nv = ((uint32_t)nw - head) >> 2;
@@ -188,7 +191,7 @@ __global__ void __launch_bounds__(SCAN_THREADS) cigar_scan_kernel(ScanArgs a)
     // ---- walk 1: statistics, exon count, filter predicate
     auto read_ptr = [&](int64_t r) -> const uint32_t * {
         const uint64_t off = a.b.cigar_off[r];
-        return staged ? (s_words + (off - w_lo)) : (a.b.cigar + off);
+        return staged ? (s_words + (off - w_lo)) : op_ptr(a, off);
     };
     bool parked = false, park_ovf = false; int park_last_start = 0;      // exons parked in the staged words by walk 1
     if (tid < nr) {
@@ -253,7 +256,7 @@ __global__ void __launch_bounds__(SCAN_THREADS) cigar_scan_kernel(ScanArgs a)
             for (int k = 0; k < last; ++k) { es[k] = (int)c[2 * k]; ee[k] = (int)c[2 * k + 1]; }
             es[last] = park_last_start; ee[last] = s_end[tid];
         } else {
-            if (parked) c = a.b.cigar + a.b.cigar_off[r];     // the staged copy is partly overwritten: walk the pool
+            if (parked) c = op_ptr(a, a.b.cigar_off[r]);      // the staged copy is partly overwritten: walk the pool
             WalkStats w; walk_seq<true>(c, n_c, a.b.pos[r], a.ep, es, ee, w);
         }
     }
@@ -325,6 +328,7 @@ __global__ void __launch_bounds__(ST_THREADS) cigar_stream_kernel(ScanArgs a, in
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     tile = __shfl_sync(FULL, tile, 0);
     if (tile >= n_tiles) return;                     // (the grid is rounded up to whole CTAs)
+    tile += a.tile_base;
     const int64_t r0 = (int64_t)tile * ST_R, r1 = min(a.b.n, r0 + ST_R);
     const int nr = (int)(r1 - r0);
     const uint64_t w_lo = a.b.cigar_off[r0], w_hi = a.b.cigar_off[r1];
@@ -336,7 +340,7 @@ __global__ void __launch_bounds__(ST_THREADS) cigar_stream_kernel(ScanArgs a, in
     const int my_pos = mine ? a.b.pos[rr] : 0;
     // the record fields the filter predicate needs and the read's first / last op: loaded now, used after the stream
     const uint32_t my_flag = mine ? a.b.flag[rr] : 4u;
-    const uint32_t c0 = (mine && my_end > my_beg) ? a.b.cigar[w_lo + (uint64_t)my_beg] : 0u, c1 = (mine && my_end > my_beg) ? a.b.cigar[w_lo + (uint64_t)my_end - 1] : 0u;
+    const uint32_t c0 = (mine && my_end > my_beg) ? *op_ptr(a, w_lo + (uint64_t)my_beg) : 0u, c1 = (mine && my_end > my_beg) ? *op_ptr(a, w_lo + (uint64_t)my_end - 1) : 0u;
     S.off[lane] = my_beg; if (lane == 31) S.off[32] = my_end;
     int my_ref = 0, my_del = 0, my_int = 0; uint32_t my_ncut = 0, my_sbeg = 0;
     bool ovf = huge;
@@ -349,7 +353,7 @@ __global__ void __launch_bounds__(ST_THREADS) cigar_stream_kernel(ScanArgs a, in
         const int lead = (int)(w_lo - g_abs);                        // pad words in front of the tile (0..3)
         const int n_words = lead + nw;
         const int n_chunks = (n_words + ST_ROUND - 1) / ST_ROUND;
-        const uint32_t *src = a.b.cigar + g_abs;
+        const uint32_t *src = op_ptr(a, g_abs);                      // op_base is a multiple of 4: still 16-byte aligned
         auto issue = [&](int c) {
             const int s = c % ST_STAGES;
             int words = n_words - c * ST_ROUND; words = words > ST_ROUND ? ST_ROUND : ((words + 3) & ~3);
@@ -471,7 +475,7 @@ __global__ void __launch_bounds__(ST_THREADS) cigar_stream_kernel(ScanArgs a, in
     } else {
         for (int li = 0; li < nr; ++li) {                        // staging overflow: one warp walk per read
             const int64_t q = r0 + li;
-            const uint32_t *cg = a.b.cigar + a.b.cigar_off[q]; const int nc = (int)(a.b.cigar_off[q + 1] - a.b.cigar_off[q]);
+            const uint32_t *cg = op_ptr(a, a.b.cigar_off[q]); const int nc = (int)(a.b.cigar_off[q + 1] - a.b.cigar_off[q]);
             WalkStats t; walk_warp<false>(cg, nc, a.b.pos[q], a.ep, nullptr, nullptr, t);
             if (lane == li) ws = t;
         }
@@ -535,13 +539,14 @@ __global__ void __launch_bounds__(ST_THREADS) cigar_stream_kernel(ScanArgs a, in
             const uint32_t cnt = __shfl_sync(FULL, my_ex, li), lo = __shfl_sync(FULL, ex_excl, li);
             if (!cnt) continue;
             const int64_t q = r0 + li;
-            const uint32_t *cg = a.b.cigar + a.b.cigar_off[q]; const int nc = (int)(a.b.cigar_off[q + 1] - a.b.cigar_off[q]);
+            const uint32_t *cg = op_ptr(a, a.b.cigar_off[q]); const int nc = (int)(a.b.cigar_off[q + 1] - a.b.cigar_off[q]);
             WalkStats t; walk_warp<true>(cg, nc, a.b.pos[q], a.ep, a.ex.es + ex_base + lo, a.ex.ee + ex_base + lo, t);
         }
     }
 }
 
 int stream_reads_per_tile() { return ST_R; }
+int scan_reads_per_tile() { return SCAN_THREADS; }
 
 void launch_cigar_scan(const ScanArgs &a, int n_tiles, bool stream_mode, size_t smem_bytes, cudaStream_t st)
 {

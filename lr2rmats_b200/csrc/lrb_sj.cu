@@ -107,6 +107,7 @@ extern "C" int lrb_bam2sj(lrb_ctx *c, const lrb_batch *b, const uint8_t *is_uniq
     int rc;
     if (b && (rc = lrb_batch_upload(c, b))) return rc;
     if (!c->have_batch) return fail(c, LRB_E_ARG, "lrb_bam2sj: no batch uploaded");
+    if (c->attached) return fail(c, LRB_E_ARG, "lrb_bam2sj: the batch is attached (its CIGARs are in host memory): pass it to lrb_bam2sj");
     CK(cudaSetDevice(c->device));
     const int64_t l0 = total_launches();
     const int64_t n = c->b.n; const size_t nn = (size_t)std::max<int64_t>(n, 1);

@@ -31,39 +31,73 @@ int set_tables(void *s, const lrb_anno *a, const lrb_anno *rm, const lrb_sj *sj)
     if ((rc = lrb_rm_upload(c, rm))) return rc;
     return lrb_sj_upload(c, sj);
 }
-int do_filter(void *s, const lrb_batch *b, const lrb_filter_params *p, lrb_filter_result *o) { return lrb_filter(((CudaEngine *)s)->get(), b, p, o); }
-int do_bam2gtf(void *s, const lrb_batch *b, const lrb_exon_params *p, lrb_exon_result *o) { return lrb_bam2gtf(((CudaEngine *)s)->get(), b, p, o); }
+// A batch goes to the device with its CIGAR pool (lrb_batch_upload).  When that, or a later stage of the same engine call, runs out
+// of device memory, the call runs once more with the batch attached (lrb_batch_attach: the pool streams from host memory through
+// the walk).  Every engine call is a pure function of its inputs, so the second run gives what the first would have.
+// LRB_TEST_CHUNK_OPS=n (test hook): every call takes the attached path from the start, in chunks of n ops.
+int64_t test_chunk_ops() { static const int64_t n = getenv("LRB_TEST_CHUNK_OPS") ? atoll(getenv("LRB_TEST_CHUNK_OPS")) : 0; return n; }
+template <class F> int with_pool_fallback(F &&call)
+{
+    if (test_chunk_ops() > 0) return call(test_chunk_ops());
+    const int rc = call(-1);
+    return rc == LRB_E_NOMEM ? call(0) : rc;
+}
+// chunk_ops < 0: upload the batch, pool included; otherwise attach it with chunks of chunk_ops ops (0: the library's choice)
+int load(lrb_ctx *c, const lrb_batch *b, int64_t chunk_ops) { return chunk_ops < 0 ? lrb_batch_upload(c, b) : lrb_batch_attach(c, b, chunk_ops); }
+
+int do_filter(void *s, const lrb_batch *b, const lrb_filter_params *p, lrb_filter_result *o)
+{
+    lrb_ctx *c = ((CudaEngine *)s)->get();
+    return with_pool_fallback([&](int64_t k) { int rc;
+        if ((rc = load(c, b, k)) || (rc = lrb_filter_run(c, p))) return rc;
+        return lrb_filter_fetch(c, o); });
+}
+int do_bam2gtf(void *s, const lrb_batch *b, const lrb_exon_params *p, lrb_exon_result *o)
+{
+    lrb_ctx *c = ((CudaEngine *)s)->get();
+    return with_pool_fallback([&](int64_t k) { int rc;
+        if ((rc = load(c, b, k)) || (rc = lrb_exon_run(c, p, 0))) return rc;
+        return lrb_exon_fetch(c, o); });
+}
 int do_sort3(void *s, const uint32_t *a, const uint32_t *b, const uint32_t *c, int64_t n, const uint32_t **perm) { return lrb_sort3(((CudaEngine *)s)->get(), a, b, c, n, perm); }
 int do_bam2sj(void *s, const lrb_batch *b, const uint8_t *u, const lrb_sj_params *p, lrb_sj *o) { return lrb_bam2sj(((CudaEngine *)s)->get(), b, u, p, o); }
 // LRB_SORT_INPUT=1: update-gtf takes a BAM that is NOT coordinate sorted (filter's output as it is) and sorts the rows on the
 // device -- the `samtools sort` hop of the pipeline (Snakefile:90) without the extra BAM round trip
 bool sort_input() { static const bool on = getenv("LRB_SORT_INPUT") && atoi(getenv("LRB_SORT_INPUT")) != 0; return on; }
 
+// the rows of an update / unique run: the batch's exon chains (b), or the given chains (-m g)
+int load_rows(lrb_ctx *c, const lrb_batch *b, const lrb_chains *ch, const lrb_exon_params *ep, int64_t chunk_ops)
+{
+    int rc;
+    if (!b) return lrb_chains_upload(c, ch);
+    if ((rc = load(c, b, chunk_ops))) return rc;
+    return lrb_exon_run(c, ep, 0);
+}
 int do_update(void *s, const lrb_batch *b, const lrb_chains *ch, const lrb_exon_params *ep, const lrb_update_params *up, lrb_update_result *o)
 {
-    lrb_ctx *c = ((CudaEngine *)s)->get(); int rc;
-    if (!b) { if ((rc = lrb_chains_upload(c, ch))) return rc; }
-    if (!sort_input()) return lrb_update_gtf(c, b, ep, up, o);
-    if (b) { if ((rc = lrb_batch_upload(c, b))) return rc; if ((rc = lrb_exon_run(c, ep, 0))) return rc; }
-    if ((rc = lrb_rows_sort(c))) return rc;
-    if ((rc = lrb_update_run(c, up))) return rc;
-    return lrb_update_fetch(c, o);
+    lrb_ctx *c = ((CudaEngine *)s)->get();
+    return with_pool_fallback([&](int64_t k) { int rc;
+        if ((rc = load_rows(c, b, ch, ep, k))) return rc;
+        if (sort_input() && (rc = lrb_rows_sort(c))) return rc;
+        if ((rc = lrb_update_run(c, up))) return rc;
+        return lrb_update_fetch(c, o); });
 }
 int do_update_table(void *s, const lrb_batch *b, const lrb_chains *ch, const lrb_exon_params *ep, const lrb_update_params *up,
                     lrb_trans_table *tab, lrb_bed_list *bed, int32_t *summary)
 {
-    lrb_ctx *c = ((CudaEngine *)s)->get(); int rc;
-    if (b) { if ((rc = lrb_batch_upload(c, b))) return rc; if ((rc = lrb_exon_run(c, ep, 0))) return rc; }
-    else if ((rc = lrb_chains_upload(c, ch))) return rc;
-    if (sort_input() && (rc = lrb_rows_sort(c))) return rc;
-    if ((rc = lrb_update_run(c, up))) return rc;
-    return lrb_update_fetch_table(c, tab, bed, summary);
+    lrb_ctx *c = ((CudaEngine *)s)->get();
+    return with_pool_fallback([&](int64_t k) { int rc;
+        if ((rc = load_rows(c, b, ch, ep, k))) return rc;
+        if (sort_input() && (rc = lrb_rows_sort(c))) return rc;
+        if ((rc = lrb_update_run(c, up))) return rc;
+        return lrb_update_fetch_table(c, tab, bed, summary); });
 }
 int do_unique(void *s, const lrb_batch *b, const lrb_chains *ch, const lrb_exon_params *ep, const lrb_update_params *up, lrb_unique_result *o)
 {
     lrb_ctx *c = ((CudaEngine *)s)->get();
-    if (!b) { int rc = lrb_chains_upload(c, ch); if (rc) return rc; }
-    return lrb_unique_gtf(c, b, ep, up, o);
+    return with_pool_fallback([&](int64_t k) { int rc;
+        if ((rc = load_rows(c, b, ch, ep, k)) || (rc = lrb_unique_run(c, up))) return rc;
+        return lrb_unique_fetch(c, o); });
 }
 const char *err(void *s) { return lrb_last_error(((CudaEngine *)s)->get()); }
 }  // namespace
