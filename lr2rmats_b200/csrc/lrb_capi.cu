@@ -80,18 +80,31 @@ int walk_cigars(lrb_ctx *c, ScanArgs a, int n_tiles, bool stream_mode, size_t sm
     return LRB_OK;
 }
 
-// the scan stage in one of its three modes; on return the counts are known on the host.  Mode 2 (fused pipeline) writes the rows at
-// their record index and runs the selection, the keep list and the kept rows (rows2) behind the walk: its counts are n_pass, ex.n and
-// n_keep, read back in the same round trip.  If the exon pool was too small the walk is repeated once with its exact size (all chunks
-// of an attached pool again).
+// the scan stage in one of its three modes: 0 filter, 1 exon chains (of the records in sel_mask, or of all), 2 both in one fused pass.
+// On return the counts are known on the host.  A walk that computes the filter is followed by the qname-run selection on the record
+// stream and the ordered compaction of the kept records: into the keep list (mode 0), or into the keep list and the kept rows, rows2
+// (mode 2, whose walk writes the rows at their record index).  Mode 0 writes no rows.  Rows, exons and kept records come back in one
+// round trip.  If the exon pool was too small the walk is repeated once with its exact size (all chunks of an attached pool again).
 int run_scan(lrb_ctx *c, int mode, const lrb_filter_params *fp, const lrb_exon_params *ep, const uint8_t *sel_mask)
 {
     const int64_t n = c->b.n;
+    const bool do_filter = mode != 1, do_exon = mode != 0;
     int rc;
     if ((rc = ensure_tiles(c, n)) != LRB_OK) return rc;
-    if ((rc = setup_rows(c, c->rows, c->rows_cols, n)) != LRB_OK) return rc;
-    if (mode != 1) { NEED(c->f_pass, (size_t)n + 1); NEED(c->f_score, (size_t)n * 4 + 4); NEED(c->f_intron, (size_t)n * 4 + 4); }
-    if (n == 0) { c->rows.n = 0; c->ex.n = 0; if (mode != 0 && (rc = setup_exons(c, 16)) != LRB_OK) return rc; return LRB_OK; }
+    if (do_exon && (rc = setup_rows(c, c->rows, c->rows_cols, n)) != LRB_OK) return rc;
+    if (do_filter) {
+        NEED(c->f_pass, (size_t)n + 1); NEED(c->f_score, (size_t)n * 4 + 4); NEED(c->f_intron, (size_t)n * 4 + 4);
+        NEED(c->f_keep_rec_mask, (size_t)n + 1); NEED(c->f_keep_idx, (size_t)n * 4 + 4);
+    }
+    if (mode == 2 && (rc = setup_rows(c, c->rows2, c->rows2_cols, n)) != LRB_OK) return rc;
+    // the counts of a walk, t = (rows, exons, kept records); the fused pass's rows are indexed by record
+    auto take = [&](const uint64_t *t) {
+        c->ex.n = (int64_t)t[1];
+        if (do_filter) c->n_keep = (int64_t)t[2];
+        if (do_exon) c->rows.n = mode == 2 ? n : (int64_t)t[0];
+        if (mode == 2) c->rows2.n = c->n_keep;
+    };
+    if (n == 0) { const uint64_t none[3] = {0, 0, 0}; take(none); return do_exon ? setup_exons(c, 16) : LRB_OK; }
     const double avg = (double)c->b.n_cigar / (double)n;
     const bool stream_mode = scan_stream_mode(n, c->b.n_cigar);
     const int R = scan_tile_reads(stream_mode);
@@ -119,39 +132,45 @@ int run_scan(lrb_ctx *c, int mode, const lrb_filter_params *fp, const lrb_exon_p
         if ((rc = walk_cigars(c, a, n_tiles, stream_mode, smem)) != LRB_OK) return rc;
         tick(c, EV_SCAN1);
         CK(cudaGetLastError());
-        if (mode == 2) {                             // run selection on the record stream -> compaction + row gather
-            CK(cudaMemsetAsync(c->f_keep_rec_mask.p, 0, (size_t)n, c->st));
-            launch_select_records(c->b, c->f_pass.as<uint8_t>(), c->f_score.as<int32_t>(), c->f_intron.as<int32_t>(), *fp, c->f_keep_rec_mask.as<uint8_t>(), c->st);
-            launch_compact_gather(c->f_keep_rec_mask.as<uint8_t>(), n, c->rows, c->rows2, c->f_keep_idx.as<uint32_t>(), c->tile_state.as<uint64_t>(),
-                                  d_ticket(c), d_totals(c) + 2, c->st);
+        if (do_filter) {                             // run selection on the record stream -> compaction (+ row gather)
+            uint8_t *keep = c->f_keep_rec_mask.as<uint8_t>();
+            CK(cudaMemsetAsync(keep, 0, (size_t)n, c->st));
+            launch_select_records(c->b, c->f_pass.as<uint8_t>(), c->f_score.as<int32_t>(), c->f_intron.as<int32_t>(), *fp, keep, c->st);
+            if (mode == 2)
+                launch_compact_gather(keep, n, c->rows, c->rows2, c->f_keep_idx.as<uint32_t>(), c->tile_state.as<uint64_t>(), d_ticket(c), d_totals(c) + 2, c->st);
+            else launch_compact_mask(keep, n, c->f_keep_idx.as<uint32_t>(), c->tile_state.as<uint64_t>(), d_ticket(c), d_totals(c) + 2, c->st);
             CK(cudaGetLastError());
         }
-        uint64_t t[3];
-        if ((rc = read_totals(c, t, mode == 2 ? 3 : 2)) != LRB_OK) return rc;
-        if (mode == 2) { c->n_pass = (int64_t)t[0]; c->n_keep = (int64_t)t[2]; }
-        else c->rows.n = (int64_t)t[0];
-        c->ex.n = (int64_t)t[1];
+        uint64_t t[3] = {0, 0, 0};
+        if ((rc = read_totals(c, t, do_filter ? 3 : 2)) != LRB_OK) return rc;
+        take(t);
         if (c->timing) cudaEventElapsedTime(&c->ms[LRB_T_K_SCAN], c->ev[EV_SCAN0], c->ev[EV_SCAN1]);
-        if (mode == 0 || c->ex.n <= c->ex.cap) return LRB_OK;
+        if (!do_exon || c->ex.n <= c->ex.cap) return LRB_OK;
         if (attempt == 1) return fail(c, LRB_E_NOMEM, "exon pool still too small after regrow");
         if ((rc = setup_exons(c, c->ex.n + 16)) != LRB_OK) return rc;          // exact size known now: walk again
     }
 }
 
-int run_select(lrb_ctx *c, const lrb_filter_params *fp)
+// The stages that walk the CIGARs, run_scan in their mode: checks, timing, launch count, and what is current afterwards -- the filter
+// result (modes 0, 2), the rows and exon chains (modes 1, 2).
+int scan_stage(lrb_ctx *c, const char *who, int mode, const lrb_filter_params *fp, const lrb_exon_params *ep, bool use_keep_list)
 {
-    const int64_t n = c->b.n, np = c->rows.n;
-    NEED(c->f_keep_row_mask, (size_t)std::max<int64_t>(np, 1)); NEED(c->f_keep_rec_mask, (size_t)std::max<int64_t>(n, 1));
-    NEED(c->f_keep_idx, (size_t)std::max<int64_t>(np, 1) * 4); NEED(c->f_keep_rows, (size_t)std::max<int64_t>(np, 1) * 4);
-    CK(cudaMemsetAsync(c->f_keep_row_mask.p, 0, (size_t)std::max<int64_t>(np, 1), c->st));
-    CK(cudaMemsetAsync(c->f_keep_rec_mask.p, 0, (size_t)std::max<int64_t>(n, 1), c->st));
-    launch_select_runs(c->b, c->rows.read_idx, np, c->f_score.as<int32_t>(), c->f_intron.as<int32_t>(), *fp,
-                       c->f_keep_row_mask.as<uint8_t>(), c->f_keep_rec_mask.as<uint8_t>(), c->st);
-    launch_compact_mask(c->f_keep_row_mask.as<uint8_t>(), np, c->rows.read_idx, c->f_keep_idx.as<uint32_t>(), c->f_keep_rows.as<uint32_t>(),
-                        c->tile_state.as<uint64_t>(), d_ticket(c), d_totals(c), c->st);
-    CK(cudaGetLastError());
-    uint64_t t; int rc = read_totals(c, &t, 1); if (rc) return rc;
-    c->n_pass = np; c->n_keep = (int64_t)t;
+    if (!c || (mode != 1 && !fp) || (mode != 0 && !ep)) return LRB_E_ARG;
+    if (!c->have_batch) return fail(c, LRB_E_ARG, std::string(who) + ": no batch uploaded");
+    if (use_keep_list && !c->have_filter) return fail(c, LRB_E_ARG, std::string(who) + ": keep list requested but lrb_filter_run has not run");
+    CK(cudaSetDevice(c->device));
+    const int64_t l0 = total_launches(); tick(c, EV_BEGIN);
+    if (int rc = run_scan(c, mode, fp, ep, use_keep_list ? c->f_keep_rec_mask.as<uint8_t>() : nullptr)) return rc;
+    tick(c, EV_END);
+    if (mode != 1) c->have_filter = true;
+    if (mode == 0) c->have_exons = false;
+    else { c->cur = mode == 2 ? &c->rows2 : &c->rows; c->rows_compact = mode == 1; c->have_exons = true; c->have_update = c->have_unique = false; }
+    c->launches_last = total_launches() - l0;
+    if (c->timing) {
+        CK(cudaStreamSynchronize(c->st));
+        cudaEventElapsedTime(&c->ms[mode == 1 ? LRB_T_EXON : LRB_T_FILTER], c->ev[EV_BEGIN], c->ev[EV_END]);
+        if (mode == 2) c->ms[LRB_T_EXON] = 0;
+    }
     return LRB_OK;
 }
 
@@ -475,55 +494,9 @@ int lrb_chains_upload(lrb_ctx *c, const lrb_chains *ch)
 }
 
 // -------------------------------------------------------------------------------------------------- stages
-int lrb_filter_run(lrb_ctx *c, const lrb_filter_params *p)
-{
-    if (!c || !p) return LRB_E_ARG;
-    if (!c->have_batch) return fail(c, LRB_E_ARG, "lrb_filter_run: no batch uploaded");
-    CK(cudaSetDevice(c->device));
-    int64_t l0 = total_launches(); tick(c, EV_BEGIN);
-    int rc = run_scan(c, 0, p, nullptr, nullptr); if (rc) return rc;
-    if ((rc = run_select(c, p))) return rc;
-    tick(c, EV_END);
-    c->have_filter = true; c->have_exons = false; c->launches_last = total_launches() - l0;
-    if (c->timing) { CK(cudaStreamSynchronize(c->st)); cudaEventElapsedTime(&c->ms[LRB_T_FILTER], c->ev[EV_BEGIN], c->ev[EV_END]); }
-    return LRB_OK;
-}
-
-int lrb_exon_run(lrb_ctx *c, const lrb_exon_params *p, int use_keep_list)
-{
-    if (!c || !p) return LRB_E_ARG;
-    if (!c->have_batch) return fail(c, LRB_E_ARG, "lrb_exon_run: no batch uploaded");
-    if (use_keep_list && !c->have_filter) return fail(c, LRB_E_ARG, "lrb_exon_run: keep list requested but lrb_filter_run has not run");
-    CK(cudaSetDevice(c->device));
-    int64_t l0 = total_launches(); tick(c, EV_BEGIN);
-    int rc = run_scan(c, 1, nullptr, p, use_keep_list ? c->f_keep_rec_mask.as<uint8_t>() : nullptr); if (rc) return rc;
-    tick(c, EV_END);
-    c->cur = &c->rows; c->rows_compact = true; c->have_exons = true; c->have_update = c->have_unique = false;
-    c->launches_last = total_launches() - l0;
-    if (c->timing) { CK(cudaStreamSynchronize(c->st)); cudaEventElapsedTime(&c->ms[LRB_T_EXON], c->ev[EV_BEGIN], c->ev[EV_END]); }
-    return LRB_OK;
-}
-
-int lrb_pipeline_run(lrb_ctx *c, const lrb_filter_params *fp, const lrb_exon_params *ep)
-{
-    if (!c || !fp || !ep) return LRB_E_ARG;
-    if (!c->have_batch) return fail(c, LRB_E_ARG, "lrb_pipeline_run: no batch uploaded");
-    CK(cudaSetDevice(c->device));
-    int64_t l0 = total_launches(); tick(c, EV_BEGIN);
-    const int64_t n = c->b.n;
-    int rc;
-    NEED(c->f_keep_rec_mask, (size_t)std::max<int64_t>(n, 1)); NEED(c->f_keep_idx, (size_t)std::max<int64_t>(n, 1) * 4);
-    if ((rc = setup_rows(c, c->rows2, c->rows2_cols, n))) return rc;
-    c->rows.n = 0; c->ex.n = 0; c->n_pass = c->n_keep = 0;
-    if ((rc = n ? run_scan(c, 2, fp, ep, nullptr) : setup_exons(c, 16))) return rc;
-    c->rows.n = n;                                              // record-indexed: only the passing records' rows are valid
-    c->rows2.n = c->n_keep;
-    tick(c, EV_END);
-    c->cur = &c->rows2; c->rows_compact = false; c->have_filter = true; c->have_exons = true; c->have_update = c->have_unique = false;
-    c->launches_last = total_launches() - l0;
-    if (c->timing) { CK(cudaStreamSynchronize(c->st)); cudaEventElapsedTime(&c->ms[LRB_T_FILTER], c->ev[EV_BEGIN], c->ev[EV_END]); c->ms[LRB_T_EXON] = 0; }
-    return LRB_OK;
-}
+int lrb_filter_run(lrb_ctx *c, const lrb_filter_params *p) { return scan_stage(c, "lrb_filter_run", 0, p, nullptr, false); }
+int lrb_exon_run(lrb_ctx *c, const lrb_exon_params *p, int use_keep_list) { return scan_stage(c, "lrb_exon_run", 1, nullptr, p, use_keep_list != 0); }
+int lrb_pipeline_run(lrb_ctx *c, const lrb_filter_params *fp, const lrb_exon_params *ep) { return scan_stage(c, "lrb_pipeline_run", 2, fp, ep, false); }
 
 // the error flags of the update / unique input checks (d_err) as a status
 static int err_status(lrb_ctx *c, uint32_t e)
@@ -838,7 +811,7 @@ int lrb_unique_run(lrb_ctx *c, const lrb_update_params *up)
     c->n_shared = 0;
     if (n) {
         invert_mask_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->st>>>(c->mg.alive.as<uint8_t>(), c->mg.head.as<uint8_t>(), n);
-        launch_compact_mask(c->mg.head.as<uint8_t>(), n, nullptr, c->q_shared.as<uint32_t>(), nullptr, c->tile_state.as<uint64_t>(), d_ticket(c), d_totals(c), c->st);
+        launch_compact_mask(c->mg.head.as<uint8_t>(), n, c->q_shared.as<uint32_t>(), c->tile_state.as<uint64_t>(), d_ticket(c), d_totals(c), c->st);
         CK(cudaGetLastError());
         uint64_t t; if ((rc = read_totals(c, &t, 1))) return rc;
         c->n_shared = (int64_t)t;

@@ -206,8 +206,8 @@ struct lrb_ctx {
     Buf stage[2]; cudaStream_t st_copy = nullptr; cudaEvent_t ev_copied[2] = {}, ev_walked[2] = {};
     int64_t n_chunks_walked = 0, max_staged_ops = 0;                // lrb_cigar_stream_diag: of the last walk
     // filter
-    Buf f_pass, f_score, f_intron, f_keep_row_mask, f_keep_rec_mask, f_keep_idx, f_keep_rows;
-    int64_t n_pass = 0, n_keep = 0; bool have_filter = false;
+    Buf f_pass, f_score, f_intron, f_keep_rec_mask, f_keep_idx;
+    int64_t n_keep = 0; bool have_filter = false;
     // rows + exons
     DRows rows, rows2, rows3; DRows *cur = nullptr; DExons ex;      // rows3: the coordinate-sorted copy made by lrb_rows_sort
     lrbk::RowsCols<Buf> rows_cols, rows2_cols, rows3_cols; Buf r_nonmono;

@@ -59,7 +59,7 @@ struct ScanArgs {
     DBatch b;
     lrb_filter_params fp; lrb_exon_params ep;
     DRmIndex rm;
-    int mode;                                       // 0 filter only, 1 exon only, 2 fused
+    int mode;                                       // 0 filter only (writes no rows), 1 exon only, 2 fused
     const uint8_t *sel_mask;                        // mode 1: records to walk (NULL = all)
     uint8_t *pass; int32_t *score, *intron_n;       // filter outputs (record level)
     DRows rows; DExons ex;
@@ -77,11 +77,8 @@ struct ScanArgs {
 void launch_cigar_scan(const ScanArgs &a, int n_tiles, bool stream_mode, size_t smem_bytes, cudaStream_t st);
 int stream_reads_per_tile();                        // tile size of the long-CIGAR streaming kernel
 int scan_reads_per_tile();                          // tile size of the short-CIGAR kernel
-void launch_select_runs(const DBatch &b, const uint32_t *row_read, int64_t n_rows, const int32_t *score, const int32_t *intron_n,
-                        lrb_filter_params fp, uint8_t *keep_row_mask, uint8_t *keep_rec_mask, cudaStream_t st);
-// ordered compaction of the set positions of a byte mask: out[k] = index of k-th nonzero (optionally mapped through `map`)
-void launch_compact_mask(const uint8_t *mask, int64_t n, const uint32_t *map, uint32_t *out, uint32_t *out2_unmapped,
-                         uint64_t *tile_state, uint32_t *ticket, uint64_t *total, cudaStream_t st);
+// ordered compaction of the set positions of a byte mask: out[k] = index of k-th nonzero
+void launch_compact_mask(const uint8_t *mask, int64_t n, uint32_t *out, uint64_t *tile_state, uint32_t *ticket, uint64_t *total, cudaStream_t st);
 void launch_select_records(const DBatch &b, const uint8_t *pass, const int32_t *score, const int32_t *intron_n, lrb_filter_params fp,
                            uint8_t *keep_rec_mask, cudaStream_t st);
 void launch_compact_gather(const uint8_t *mask, int64_t n, const DRows &src_by_record, DRows &dst, uint32_t *keep_idx,

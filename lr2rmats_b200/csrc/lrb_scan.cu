@@ -227,21 +227,21 @@ __global__ void __launch_bounds__(SCAN_THREADS) cigar_scan_kernel(ScanArgs a)
     const uint32_t row_base = pair_hi(s_excl), ex_base = pair_lo(s_excl);
     if (r1 == a.b.n && tid == 0) { a.totals[0] = (uint64_t)row_base + rows_total; a.totals[1] = (uint64_t)ex_base + ex_total; }
 
+    if (!do_exon) return;
+
     // ---- row records
     if (tid < nr && my_row) {
         int64_t r = r0 + tid; uint32_t row = a.rows_by_record ? (uint32_t)r : row_base + row_excl;
         if ((int64_t)row < a.rows.cap) {
+            int8_t xs = a.b.xs[r];
             a.rows.read_idx[row] = (uint32_t)r;
-            if (do_exon) {
-                int8_t xs = a.b.xs[r];
-                a.rows.tid[row] = a.b.tid[r];
-                a.rows.is_rev[row] = xs == 0 ? ((a.b.flag[r] & 16) != 0) : (xs == '+' ? 0 : 1);    // bam2gtf.c:35-37
-                a.rows.start[row] = s_start[tid]; a.rows.end[row] = s_end[tid];
-                a.rows.ex_beg[row] = ex_base + ex_excl; a.rows.ex_n[row] = my_ex;
-            }
+            a.rows.tid[row] = a.b.tid[r];
+            a.rows.is_rev[row] = xs == 0 ? ((a.b.flag[r] & 16) != 0) : (xs == '+' ? 0 : 1);    // bam2gtf.c:35-37
+            a.rows.start[row] = s_start[tid]; a.rows.end[row] = s_end[tid];
+            a.rows.ex_beg[row] = ex_base + ex_excl; a.rows.ex_n[row] = my_ex;
         }
     }
-    if (!do_exon || ex_total == 0) return;
+    if (ex_total == 0) return;
 
     // ---- walk 2: each read's parked exons move straight to the pools (no staging buffer: 6 resident CTAs per SM cover
     // the look-back waits)
@@ -510,20 +510,19 @@ __global__ void __launch_bounds__(ST_THREADS) cigar_stream_kernel(ScanArgs a, in
         row_base = pair_hi(e); ex_base = pair_lo(e);
         if (r1 == a.b.n && lane == 0) { a.totals[0] = (uint64_t)row_base + rows_total; a.totals[1] = (uint64_t)ex_base + ex_total; }
     }
+    if (!do_exon) return;
     if (my_row) {
         const uint32_t row = a.rows_by_record ? (uint32_t)rr : row_base + row_excl;
         if ((int64_t)row < a.rows.cap) {
+            const int8_t xs = a.b.xs[rr];
             a.rows.read_idx[row] = (uint32_t)rr;
-            if (do_exon) {
-                const int8_t xs = a.b.xs[rr];
-                a.rows.tid[row] = a.b.tid[rr];
-                a.rows.is_rev[row] = xs == 0 ? ((a.b.flag[rr] & 16) != 0) : (xs == '+' ? 0 : 1);    // bam2gtf.c:35-37
-                a.rows.start[row] = ws.first_start; a.rows.end[row] = ws.last_end;
-                a.rows.ex_beg[row] = ex_base + ex_excl; a.rows.ex_n[row] = my_ex;
-            }
+            a.rows.tid[row] = a.b.tid[rr];
+            a.rows.is_rev[row] = xs == 0 ? ((a.b.flag[rr] & 16) != 0) : (xs == '+' ? 0 : 1);    // bam2gtf.c:35-37
+            a.rows.start[row] = ws.first_start; a.rows.end[row] = ws.last_end;
+            a.rows.ex_beg[row] = ex_base + ex_excl; a.rows.ex_n[row] = my_ex;
         }
     }
-    if (!do_exon || ex_total == 0) return;
+    if (ex_total == 0) return;
     if ((int64_t)ex_base + ex_total > a.ex.cap) return;          // host re-runs with a larger pool
     if (!ovf) {
         if (my_ex) {
@@ -560,42 +559,9 @@ void launch_cigar_scan(const ScanArgs &a, int n_tiles, bool stream_mode, size_t 
 }
 
 // ---------------------------------------------------------------------------------------- qname-run selection
-// Rows are the passing records in input order, so a run of equal qname hashes over adjacent rows is exactly the run the
-// reference's state machine sees (bam_filter.c:133-153; SURVEY Q3).  The head row of each run replays the machine.
-__global__ void select_runs_kernel(const uint64_t *__restrict__ qhash, const uint32_t *__restrict__ row_read, int64_t n_rows,
-                                   const int32_t *__restrict__ score, const int32_t *__restrict__ intron_n,
-                                   lrb_filter_params fp, uint8_t *keep_row_mask, uint8_t *keep_rec_mask)
-{
-    int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= n_rows) return;
-    uint32_t r = row_read[k];
-    uint64_t h = qhash[r];
-    if (k > 0 && qhash[row_read[k - 1]] == h) return;          // not a run head
-    int b_score = score[r], s_score = 0, b_intron = intron_n[r]; int64_t best = k;
-    for (int64_t j = k + 1; j < n_rows; ++j) {
-        uint32_t rj = row_read[j];
-        if (qhash[rj] != h) break;
-        int sc = score[rj];
-        if (sc > b_score) { best = j; s_score = b_score; b_score = sc; b_intron = intron_n[rj]; }
-        else if (sc > s_score) s_score = sc;
-    }
-    if ((float)s_score < __fmul_rn(fp.sec_rat, (float)b_score) && b_intron >= fp.min_intron_n) {
-        keep_row_mask[best] = 1;
-        keep_rec_mask[row_read[best]] = 1;
-    }
-}
-
-void launch_select_runs(const DBatch &b, const uint32_t *row_read, int64_t n_rows, const int32_t *score, const int32_t *intron_n,
-                        lrb_filter_params fp, uint8_t *keep_row_mask, uint8_t *keep_rec_mask, cudaStream_t st)
-{
-    if (n_rows <= 0) return;
-    int th = 256; int64_t bl = (n_rows + th - 1) / th;
-    select_runs_kernel<<<(unsigned)bl, th, 0, st>>>(b.qhash, row_read, n_rows, score, intron_n, fp, keep_row_mask, keep_rec_mask);
-    LRB_COUNT_LAUNCH();
-}
-
-// The same state machine on the record stream itself (fused filter + exon pass): the passing subsequence is walked through
-// the pass mask, so no compacted row list -- and no host round trip for its size -- is needed in front of the selection.
+// The reference's state machine (bam_filter.c:133-153; SURVEY Q3) sees the passing records in input order, so a run is a stretch
+// of equal qname hashes over the passing subsequence, walked here through the pass mask: no compacted row list -- and no host
+// round trip for its size -- is needed in front of the selection.  The head record of each run replays the machine.
 __global__ void select_records_kernel(const uint64_t *__restrict__ qhash, const uint8_t *__restrict__ pass, int64_t n,
                                       const int32_t *__restrict__ score, const int32_t *__restrict__ intron_n, lrb_filter_params fp, uint8_t *keep_rec_mask)
 {
@@ -669,8 +635,8 @@ void launch_compact_gather(const uint8_t *mask, int64_t n, const DRows &src, DRo
 
 // -------------------------------------------------------------------------------------------- mask compaction
 static constexpr int CM_THREADS = 256, CM_ITEMS = 8;
-__global__ void __launch_bounds__(CM_THREADS) compact_mask_kernel(const uint8_t *__restrict__ mask, int64_t n, const uint32_t *__restrict__ map,
-                                                                  uint32_t *out, uint32_t *out2, uint64_t *tile_state, uint32_t *ticket, uint64_t *total)
+__global__ void __launch_bounds__(CM_THREADS) compact_mask_kernel(const uint8_t *__restrict__ mask, int64_t n, uint32_t *out,
+                                                                  uint64_t *tile_state, uint32_t *ticket, uint64_t *total)
 {
     __shared__ uint32_t s_scan[33];
     __shared__ uint32_t s_tile; __shared__ uint64_t s_excl;
@@ -687,17 +653,16 @@ __global__ void __launch_bounds__(CM_THREADS) compact_mask_kernel(const uint8_t 
     uint32_t o = (uint32_t)s_excl + excl;
 #pragma unroll
     for (int i = 0; i < CM_ITEMS; ++i)
-        if (m[i]) { uint32_t idx = (uint32_t)(base + i); out[o] = map ? map[idx] : idx; if (out2) out2[o] = idx; ++o; }
+        if (m[i]) out[o++] = (uint32_t)(base + i);
     if ((int64_t)(tile + 1) * CM_THREADS * CM_ITEMS >= n && threadIdx.x == 0) *total = s_excl + tot;
 }
 
-void launch_compact_mask(const uint8_t *mask, int64_t n, const uint32_t *map, uint32_t *out, uint32_t *out2,
-                         uint64_t *tile_state, uint32_t *ticket, uint64_t *total, cudaStream_t st)
+void launch_compact_mask(const uint8_t *mask, int64_t n, uint32_t *out, uint64_t *tile_state, uint32_t *ticket, uint64_t *total, cudaStream_t st)
 {
     if (n <= 0) { cudaMemsetAsync(total, 0, 8, st); return; }
     int64_t per = (int64_t)CM_THREADS * CM_ITEMS, bl = (n + per - 1) / per;
     cudaMemsetAsync(tile_state, 0, (size_t)bl * 8, st); cudaMemsetAsync(ticket, 0, 4, st);
-    compact_mask_kernel<<<(unsigned)bl, CM_THREADS, 0, st>>>(mask, n, map, out, out2, tile_state, ticket, total);
+    compact_mask_kernel<<<(unsigned)bl, CM_THREADS, 0, st>>>(mask, n, out, tile_state, ticket, total);
     LRB_COUNT_LAUNCH();
 }
 

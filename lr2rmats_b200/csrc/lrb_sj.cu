@@ -138,7 +138,7 @@ extern "C" int lrb_bam2sj(lrb_ctx *c, const lrb_batch *b, const uint8_t *is_uniq
         const uint32_t *perm;
         if ((rc = sort3_device(c, a.j_tid, a.j_don, a.j_acc, nj, &perm))) return rc;
         sj_heads_kernel<<<(unsigned)((nj + 255) / 256), 256, 0, c->st>>>(a.j_tid, a.j_don, a.j_acc, perm, c->j_head.as<uint8_t>(), nj);
-        launch_compact_mask(c->j_head.as<uint8_t>(), nj, nullptr, c->j_hpos.as<uint32_t>(), nullptr, c->tile_state.as<uint64_t>(), d_ticket(c), d_totals(c), c->st);
+        launch_compact_mask(c->j_head.as<uint8_t>(), nj, c->j_hpos.as<uint32_t>(), c->tile_state.as<uint64_t>(), d_ticket(c), d_totals(c), c->st);
         CK(cudaGetLastError());
         uint64_t t; if ((rc = read_totals(c, &t, 1))) return rc;
         nd = (int64_t)t;
